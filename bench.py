@@ -2,7 +2,7 @@
 """bench.py -- depth maps/s of the generator forward on N B200s, with in-run parity, the NLSPN roofline and the reference beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3|c2|c5|c4] [--batch GLOBAL] [--precision bf16|fp32]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; the default, c3, is the one `metric` is quoted on):
   c3  RDFC-GAN RDFGenerator (ResNet-18 x2, W-AdaIN, NLSPN TGASS 18 it.) inference, GLOBAL batch 256 @228x304, batch-sharded over
@@ -26,10 +26,15 @@ a barrier + synchronize and the max over ranks is taken.  Rank 0 prints ONE JSON
              achieved = 116 B x pixels per launch / launch time, against MEASURED_PEAKS.json hbm_gbs.
   cpu_baseline / --impl reference: the UNMODIFIED reference Python (baseline/_ref/rdf_generator, DCN served by
              torchvision.ops.deform_conv2d as BASELINE.json prescribes) on all host cores, on a bounded sample.
+
+--dump-outputs DIR writes what the last timed step computed on rank 0 as DIR/<name>.npy: the five maps, float32 (beyond DUMP_BYTES,
+a fixed seeded sample of the images), and for c4 also the step's losses, float64.  Inputs and weights are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 import argparse
 import json
 import os
+import random
 import statistics
 import subprocess
 import sys
@@ -103,6 +108,25 @@ class ClockSampler(threading.Thread):
         reasons = sorted({n for r in self.rows for n, v in zip(names, r[2:6]) if v.lower().startswith("active")})
         return dict(sm_mhz=int(statistics.median(sm)) if sm else None, sm_max_mhz=max(mx) if mx else None, reasons=reasons,
                     samples=len(sm))
+
+
+DUMP_BYTES = 48 << 20                    # --dump-outputs: at most this much array data
+
+
+def sample_outputs(outputs):
+    """name -> [B, ...] device tensor  =>  name -> float32 host array.  Above DUMP_BYTES in all, every map keeps the same sample
+    of images, drawn with a fixed seed from B alone (so it is the same in every run with the same batch)."""
+    B = next(iter(outputs.values())).shape[0]
+    keep = min(B, DUMP_BYTES // sum(t[0].numel() * 4 for t in outputs.values()))
+    idx = list(range(B)) if keep == B else sorted(random.Random(0).sample(range(B), keep))
+    return {k: t[idx].detach().float().cpu().numpy() for k, t in outputs.items()}
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def gen_kwargs(cfg):
@@ -239,7 +263,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (--impl b200 only; with several GPUs, rank 0's "
+                         "shard of the batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.config == "c4":
@@ -325,6 +356,7 @@ def main():
     clocks = sampler.summary()
     t_ms = maxreduce(sum(a.elapsed_time(b) for a, b in evs))
     value = args.batch * args.steps / (t_ms / 1e3)
+    dumped = sample_outputs(dict(zip(KEYS, plan.outputs))) if args.dump_outputs and rank == 0 else None
 
     # ---------------- e2e: public API, pinned host inputs, all five maps back to the host, H2D + D2H inside the timed region
     rgb_h, stem_h, depth_h = rgb.pin_memory(), stem.pin_memory(), depth.pin_memory()
@@ -500,6 +532,8 @@ def main():
             "e2e": {"value": e2e, "unit": "maps/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
             "gpu_launches": n_launch * args.steps, "parity": parity, "value_fp32": value_fp32, "value_fp32_tc": value_fp32_tc, "ref_gpu": ref_gpu,
             "roofline": roofline, "roofline_dense": roofline_dense, "cpu_baseline": cpu}))
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 

@@ -105,6 +105,7 @@ def main(args, rank, world, local):
             "e2e": {"value": val, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
         return
 
+    import numpy as np
     import torch
     import torch.distributed as dist
     from _synth import synth_state_dict
@@ -176,6 +177,11 @@ def main(args, rank, world, local):
     ar_ms = maxreduce(sum(x.elapsed_time(y) for x, y in ar_events)) / args.steps
     value = per_gpu * world * args.steps / (t_ms / 1e3)
     assert all(v == v and abs(v) < 1e6 for v in stats.values()), stats          # finite losses
+    dumped = None
+    if args.dump_outputs and rank == 0:         # the last timed step's generator maps and the loss dict it returned
+        dumped = bench.sample_outputs(dict(zip(bench.KEYS, (model.fake_B_rgb_branch, model.conf_map_rgb_branch, model.fake_B_depth_branch,
+                                                            model.conf_map_depth_branch, model.final_depth))))
+        dumped.update({k: np.float64(v) for k, v in stats.items()})
 
     # e2e: host batch -> set_input (H2D) -> step -> loss dict on the host, wall clock
     barrier()
@@ -190,7 +196,8 @@ def main(args, rank, world, local):
     pk = bench.peaks()
     tflops = 3 * GFLOP_FWD * 1e9 * per_gpu * args.steps / (t_ms / 1e3) / 1e12
     cpu = None
-    if rank == 0 and world == 1 and not args.no_cpu_baseline:
+    import ref_loader
+    if rank == 0 and world == 1 and not args.no_cpu_baseline and ref_loader.available():     # the step has no oracle restatement
         v, cores, ts = reference_step_cpu(1, 2)
         cpu = {"value": v, "unit": "images/s", "cores": cores, "kind": "reference",
                "sample": f"1 image per step x 2 timed steps, fp32, the reference's own modules on torch CPU; {sum(ts):.1f} s timed"}
@@ -209,5 +216,7 @@ def main(args, rank, world, local):
                          "frac": tflops / pk["bf16_sustained"], "traffic": None, "peak_source": pk["src"] + " (sustained cuBLAS bf16)",
                          "note": "3 x 221.4 GFLOP per image (forward, data gradient, filter gradient) over the whole step time"},
             "cpu_baseline": cpu}))
+    if dumped is not None:
+        bench.write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
