@@ -320,7 +320,8 @@ int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, float *workspa
 /* ------------------------------------------------------------------ ESANet guidance glue ---------------------- */
 /* The non-GEMM layers of RDF-GAN's global_guidance_module (F/lib/models/segmentator/esa_net/esa_net_one_modality.py:145-172,
  * decoder.py:137-191, model_utils.py:34-49,99-134; F = /root/reference/RDF-GAN); its GEMM-shaped layers go through
- * rdfc_conv_forward.  All views bf16 NHWC. */
+ * rdfc_conv_forward.  Views are NHWC, bf16 or fp32, C % 8 == 0, 16-byte aligned, pixel stride a multiple of 8 (bf16) or 4 (fp32)
+ * elements; the views of one call share a dtype (else RDFC_ERR_INVALID).  The up-sampling's fp32 NCHW result takes either input dtype. */
 
 /* encoder.conv1 + folded bn1 + ReLU: k x k (<= 7) conv, any stride, from fp32 NCHW x (B, Cin <= 4, Hi, Wi); weight (Cout, Cin, k, k) fp32 */
 int rdfc_first_conv_forward(const float *x_nchw, int B, int Cin, int Hi, int Wi, const float *weight, int k, int stride, int pad,
@@ -336,7 +337,7 @@ int rdfc_adaptive_avgpool_forward(const rdfc_view *x, const rdfc_view *out, int 
 /* F.interpolate(mode='nearest') of a (hs, ws) map to (H, W), written into `out` (a channel slice of a concat buffer) */
 int rdfc_upsample_nearest_forward(const rdfc_view *x, const rdfc_view *out, int B, int hs, int ws, int H, int W, void *stream);
 /* Upsample('learned-3x3-zeropad'): nearest resize (Hi, Wi) -> (Ho, Wo), depth-wise 3x3 conv (weight (C, 1, 3, 3), bias (C)) with zero
- * padding, + skip (or NULL); result to `out` (bf16 NHWC) or, when out_nchw != NULL, to fp32 NCHW (B, C, Ho, Wo) */
+ * padding, + skip (or NULL); result to `out` (NHWC, x's dtype) or, when out_nchw != NULL, to fp32 NCHW (B, C, Ho, Wo) */
 int rdfc_upsample_dw_forward(const rdfc_view *x, const float *weight, const float *bias, const rdfc_view *skip, const rdfc_view *out,
                              float *out_nchw, int B, int Hi, int Wi, int Ho, int Wo, void *stream);
 

@@ -16,18 +16,15 @@ import ctypes
 import torch
 
 from . import _cabi as C
+from .engine import pack_weight
 
 
 def pack_filter(w_oihw):
-    """(Cout, Cin, kh, kw) -> the UMMA filter layout [tap][Cin/8][CoutP][8] bf16 (engine._pack's layout)."""
-    Cout, Cin, kh, kw = w_oihw.shape
+    """(Cout, Cin, kh, kw) -> the UMMA filter layout [tap][Cin/8][CoutP][8] bf16 (engine.pack_weight's layout)."""
+    Cin = w_oihw.shape[1]
     if Cin % 32:
         raise RuntimeError(f"tensor-core conv needs Cin % 32 == 0, got {Cin}")
-    g = w_oihw.detach().float().permute(0, 2, 3, 1).reshape(Cout, kh * kw, Cin)
-    CoutP = (Cout + 15) // 16 * 16
-    if CoutP != Cout:
-        g = torch.cat([g, g.new_zeros(CoutP - Cout, kh * kw, Cin)], 0)
-    return g.reshape(CoutP, kh * kw, Cin // 8, 8).permute(1, 2, 0, 3).contiguous().to(torch.bfloat16)
+    return pack_weight(w_oihw.detach().float(), umma=True)
 
 
 def _run(x, packed, Cout, stride, transposed, out_hw):

@@ -1,5 +1,7 @@
 // Glue kernels of the ESANet guidance network (RDF-GAN's global_guidance_module,
-// F/lib/models/segmentator/esa_net/esa_net_one_modality.py:11-194, F = /root/reference/RDF-GAN), bf16 NHWC.
+// F/lib/models/segmentator/esa_net/esa_net_one_modality.py:11-194, F = /root/reference/RDF-GAN) over NHWC activations, bf16 (the
+// throughput mode) or fp32 (the parity modes).  Every kernel is a template over the activation type T; the bf16 instantiations
+// keep the arithmetic and store order they had before fp32 existed, so the bf16 network's outputs are unchanged.
 //
 // The GEMM-shaped layers of ESANet (ResNet BasicBlocks, 1x1 skip / context convs, decoder 3x3 and factorised 3x1 / 1x3 convs,
 // conv_out) run on conv_umma_kernel; what is left are HBM-bound layers with a handful of input channels or no contraction at
@@ -10,10 +12,45 @@
 namespace rdfc {
 namespace {
 
-// ---- encoder.conv1 + bn1 + ReLU: k x k (k <= 7) stride-s conv from fp32 NCHW (Cin <= 4) to bf16 NHWC (Cout = 64) ----------
+// eight consecutive channels of an NHWC pixel: one 16-byte access in bf16, two in fp32
+template <typename T>
+__device__ __forceinline__ void load8(const T *p, float (&v)[8]);
+template <>
+__device__ __forceinline__ void load8<__nv_bfloat16>(const __nv_bfloat16 *p, float (&v)[8]) {
+    const uint4 a = __ldg(reinterpret_cast<const uint4 *>(p));
+    const __nv_bfloat162 *h = reinterpret_cast<const __nv_bfloat162 *>(&a);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) { const float2 f = __bfloat1622float2(h[q]); v[2 * q] = f.x; v[2 * q + 1] = f.y; }
+}
+template <>
+__device__ __forceinline__ void load8<float>(const float *p, float (&v)[8]) {
+    const float4 a = __ldg(reinterpret_cast<const float4 *>(p)), b = __ldg(reinterpret_cast<const float4 *>(p) + 1);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void store8(__nv_bfloat16 *p, const float (&v)[8]) {
+    uint32_t o[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) { const __nv_bfloat162 h = __floats2bfloat162_rn(v[2 * q], v[2 * q + 1]); o[q] = *reinterpret_cast<const uint32_t *>(&h); }
+    *reinterpret_cast<uint4 *>(p) = make_uint4(o[0], o[1], o[2], o[3]);
+}
+__device__ __forceinline__ void store8(float *p, const float (&v)[8]) {
+    reinterpret_cast<float4 *>(p)[0] = make_float4(v[0], v[1], v[2], v[3]);
+    reinterpret_cast<float4 *>(p)[1] = make_float4(v[4], v[5], v[6], v[7]);
+}
+// copy of eight channels without conversion
+__device__ __forceinline__ void copy8(__nv_bfloat16 *d, const __nv_bfloat16 *s) {
+    *reinterpret_cast<uint4 *>(d) = __ldg(reinterpret_cast<const uint4 *>(s));
+}
+__device__ __forceinline__ void copy8(float *d, const float *s) {
+    reinterpret_cast<float4 *>(d)[0] = __ldg(reinterpret_cast<const float4 *>(s));
+    reinterpret_cast<float4 *>(d)[1] = __ldg(reinterpret_cast<const float4 *>(s) + 1);
+}
+
+// ---- encoder.conv1 + bn1 + ReLU: k x k (k <= 7) stride-s conv from fp32 NCHW (Cin <= 4) to T NHWC (Cout = 64) -------------
 // block = 64 threads (one per output channel) x 4 pixels; the filter bank sits in shared memory as [tap][ci][cout].
+template <typename T>
 __global__ void __launch_bounds__(256) first_conv_kernel(const float *__restrict__ x, const float *__restrict__ w, const float *__restrict__ scale,
-                                                         const float *__restrict__ shift, __nv_bfloat16 *__restrict__ out, int out_stride, int B,
+                                                         const float *__restrict__ shift, T *__restrict__ out, int out_stride, int B,
                                                          int Cin, int Hi, int Wi, int Ho, int Wo, int k, int s, int pad, int Cout, int relu) {
     extern __shared__ float sw[];                       // [k*k*Cin][Cout]
     const int ntaps = k * k * Cin;
@@ -34,13 +71,14 @@ __global__ void __launch_bounds__(256) first_conv_kernel(const float *__restrict
             for (int kx = 0; kx < k; ++kx) {
                 const int ix = ox * s - pad + kx;
                 if (ix < 0 || ix >= Wi) continue;
+#pragma unroll 1                                    // unrolled (Cin <= 4), ptxas spills 16 bytes
                 for (int ci = 0; ci < Cin; ++ci)
                     acc = fmaf(__ldg(x + (((long long)b * Cin + ci) * Hi + iy) * Wi + ix), sw[((ky * k + kx) * Cin + ci) * Cout + co], acc);
             }
         }
         float y = fmaf(acc, scale[co], shift[co]);
         if (relu) y = fmaxf(y, 0.f);
-        out[p * out_stride + co] = __float2bfloat16_rn(y);
+        stf(out + p * out_stride + co, y);
     }
 }
 
@@ -50,8 +88,9 @@ __global__ void __launch_bounds__(256) first_conv_kernel(const float *__restrict
 // the lane reads the 13 patch values its four pixels touch once (three 16-byte loads + one) and per kx eight filter values (two 16-byte,
 // warp-broadcast loads): 224 FMAs per 18 shared-memory loads instead of 1 per 2 in the kernel above (7.1 ms -> 0.3 ms at B = 32, 228 x 304).
 constexpr int FC_TY = 8, FC_TX = 16, FC_PR = 2 * FC_TY + 5, FC_PC = 40;
+template <typename T>
 __global__ void __launch_bounds__(256) first_conv7s2_kernel(const float *__restrict__ x, const float *__restrict__ w, const float *__restrict__ scale,
-                                                            const float *__restrict__ shift, __nv_bfloat16 *__restrict__ out, int out_stride, int B,
+                                                            const float *__restrict__ shift, T *__restrict__ out, int out_stride, int B,
                                                             int Cin, int Hi, int Wi, int Ho, int Wo, int relu) {
     extern __shared__ __align__(16) float fsm[];
     float *sw = fsm;                                    // [49 * Cin][64]
@@ -109,22 +148,21 @@ __global__ void __launch_bounds__(256) first_conv7s2_kernel(const float *__restr
             for (int p = 0; p < 4; ++p) {
                 const int ox = ox0 + 4 * pg + p;
                 if (ox >= Wo) continue;
-                uint32_t o[4];
+                float y[8];
 #pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    float y0 = fmaf(acc[p][2 * c], sc[2 * c], sh[2 * c]), y1 = fmaf(acc[p][2 * c + 1], sc[2 * c + 1], sh[2 * c + 1]);
-                    if (relu) { y0 = fmaxf(y0, 0.f); y1 = fmaxf(y1, 0.f); }
-                    const __nv_bfloat162 h = __floats2bfloat162_rn(y0, y1);
-                    o[c] = *reinterpret_cast<const uint32_t *>(&h);
+                for (int c = 0; c < 8; ++c) {
+                    y[c] = fmaf(acc[p][c], sc[c], sh[c]);
+                    if (relu) y[c] = fmaxf(y[c], 0.f);
                 }
-                *reinterpret_cast<uint4 *>(out + (((long long)b * Ho + oy) * Wo + ox) * out_stride + cg * 8) = make_uint4(o[0], o[1], o[2], o[3]);
+                store8(out + (((long long)b * Ho + oy) * Wo + ox) * out_stride + cg * 8, y);
             }
         }
     }
 }
 
-// ---- max pooling 3x3 / stride 2 / pad 1 over bf16 NHWC, 8 channels per thread -------------------------------------------
-__global__ void __launch_bounds__(256) maxpool_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, __nv_bfloat16 *__restrict__ out,
+// ---- max pooling 3x3 / stride 2 / pad 1 over NHWC, 8 channels per thread ------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(256) maxpool_kernel(const T *__restrict__ x, int x_stride, T *__restrict__ out,
                                                       int out_stride, int B, int C, int Hi, int Wi, int Ho, int Wo) {
     const int cgs = C >> 3;
     const long long total = (long long)B * Ho * Wo * cgs;
@@ -141,23 +179,13 @@ __global__ void __launch_bounds__(256) maxpool_kernel(const __nv_bfloat16 *__res
             for (int kx = 0; kx < 3; ++kx) {
                 const int ix = 2 * ox - 1 + kx;
                 if (ix < 0 || ix >= Wi) continue;
-                const uint4 v = __ldg(reinterpret_cast<const uint4 *>(x + (((long long)b * Hi + iy) * Wi + ix) * x_stride + cg * 8));
-                const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
+                float v[8];
+                load8(x + (((long long)b * Hi + iy) * Wi + ix) * x_stride + cg * 8, v);
 #pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162 *>(&wv[q]));
-                    m[2 * q] = fmaxf(m[2 * q], f.x);
-                    m[2 * q + 1] = fmaxf(m[2 * q + 1], f.y);
-                }
+                for (int q = 0; q < 8; ++q) m[q] = fmaxf(m[q], v[q]);
             }
         }
-        uint32_t o[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const __nv_bfloat162 h = __floats2bfloat162_rn(m[2 * q], m[2 * q + 1]);
-            o[q] = *reinterpret_cast<const uint32_t *>(&h);
-        }
-        *reinterpret_cast<uint4 *>(out + p * out_stride + cg * 8) = make_uint4(o[0], o[1], o[2], o[3]);
+        store8(out + p * out_stride + cg * 8, m);
     }
 }
 
@@ -184,7 +212,8 @@ __global__ void __launch_bounds__(256) se_weights_kernel(const float *__restrict
 }
 
 // ---- adaptive average pooling to bins x bins (torch's window rule: [floor(i*H/n), ceil((i+1)*H/n))) ------------------------
-__global__ void __launch_bounds__(256) adaptive_avgpool_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, __nv_bfloat16 *__restrict__ out,
+template <typename T>
+__global__ void __launch_bounds__(256) adaptive_avgpool_kernel(const T *__restrict__ x, int x_stride, T *__restrict__ out,
                                                                int out_stride, int B, int C, int H, int W, int bins) {
     const long long total = (long long)B * bins * bins * C;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -194,13 +223,14 @@ __global__ void __launch_bounds__(256) adaptive_avgpool_kernel(const __nv_bfloat
         const int y0 = (by * H) / bins, y1 = ((by + 1) * H + bins - 1) / bins, x0 = (bx * W) / bins, x1 = ((bx + 1) * W + bins - 1) / bins;
         float s = 0.f;
         for (int y = y0; y < y1; ++y)
-            for (int xx = x0; xx < x1; ++xx) s += __bfloat162float(x[(((long long)b * H + y) * W + xx) * x_stride + c]);
-        out[p * out_stride + c] = __float2bfloat16_rn(s / (float)((y1 - y0) * (x1 - x0)));
+            for (int xx = x0; xx < x1; ++xx) s += ldf(x + (((long long)b * H + y) * W + xx) * x_stride + c);
+        stf(out + p * out_stride + c, s / (float)((y1 - y0) * (x1 - x0)));
     }
 }
 
 // ---- nearest up-sampling of a (hs x ws) map into a channel slice of a (H x W) NHWC buffer (torch 'nearest': floor(dst*in/out)) --
-__global__ void __launch_bounds__(256) upsample_nearest_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, __nv_bfloat16 *__restrict__ out,
+template <typename T>
+__global__ void __launch_bounds__(256) upsample_nearest_kernel(const T *__restrict__ x, int x_stride, T *__restrict__ out,
                                                                int out_stride, int B, int C, int hs, int ws, int H, int W) {
     const int cgs = C >> 3;
     const long long total = (long long)B * H * W * cgs;
@@ -209,16 +239,15 @@ __global__ void __launch_bounds__(256) upsample_nearest_kernel(const __nv_bfloat
         const long long p = i / cgs;
         const int ox = (int)(p % W), oy = (int)((p / W) % H), b = (int)(p / ((long long)W * H));
         const int sy = min((int)floorf(oy * ((float)hs / H)), hs - 1), sx = min((int)floorf(ox * ((float)ws / W)), ws - 1);
-        *reinterpret_cast<uint4 *>(out + p * out_stride + cg * 8) =
-            __ldg(reinterpret_cast<const uint4 *>(x + (((long long)b * hs + sy) * ws + sx) * x_stride + cg * 8));
+        copy8(out + p * out_stride + cg * 8, x + (((long long)b * hs + sy) * ws + sx) * x_stride + cg * 8);
     }
 }
 
 // ---- the decoder's learned up-sampling (Upsample, decoder.py:137-191, mode 'learned-3x3-zeropad'): nearest resize to (Ho, Wo),
-// depth-wise 3x3 conv with zero padding + bias, optional skip add.  Output: bf16 NHWC, or fp32 NCHW planes (the network's result).
-template <bool kNCHW>
-__global__ void __launch_bounds__(256) upsample_dw_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, const float *__restrict__ w,
-                                                          const float *__restrict__ bias, const __nv_bfloat16 *__restrict__ skip, int skip_stride,
+// depth-wise 3x3 conv with zero padding + bias, optional skip add.  Output: T NHWC, or fp32 NCHW planes (the network's result).
+template <typename T, bool kNCHW>
+__global__ void __launch_bounds__(256) upsample_dw_kernel(const T *__restrict__ x, int x_stride, const float *__restrict__ w,
+                                                          const float *__restrict__ bias, const T *__restrict__ skip, int skip_stride,
                                                           void *__restrict__ out, int out_stride, int B, int C, int Hi, int Wi, int Ho, int Wo) {
     const long long total = (long long)B * Ho * Wo * C;
     const float fy = (float)Hi / Ho, fx = (float)Wi / Wo;
@@ -241,13 +270,13 @@ __global__ void __launch_bounds__(256) upsample_dw_kernel(const __nv_bfloat16 *_
                 const int ux = ox - 1 + kx;
                 if (ux < 0 || ux >= Wo) continue;
                 const int sx = min((int)floorf(ux * fx), Wi - 1);
-                acc = fmaf(w[c * 9 + ky * 3 + kx], __bfloat162float(x[(((long long)b * Hi + sy) * Wi + sx) * x_stride + c]), acc);
+                acc = fmaf(w[c * 9 + ky * 3 + kx], ldf(x + (((long long)b * Hi + sy) * Wi + sx) * x_stride + c), acc);
             }
         }
         const long long p = ((long long)b * Ho + oy) * Wo + ox;
-        if (skip) acc += __bfloat162float(skip[p * skip_stride + c]);
+        if (skip) acc += ldf(skip + p * skip_stride + c);
         if (kNCHW) reinterpret_cast<float *>(out)[(((long long)b * C + c) * Ho + oy) * Wo + ox] = acc;
-        else reinterpret_cast<__nv_bfloat16 *>(out)[p * out_stride + c] = __float2bfloat16_rn(acc);
+        else stf(reinterpret_cast<T *>(out) + p * out_stride + c, acc);
     }
 }
 
@@ -255,9 +284,12 @@ __global__ void __launch_bounds__(256) upsample_dw_kernel(const __nv_bfloat16 *_
 // (1) fp32 NCHW result (the network's last up-sampling, 40 planes at full resolution): with x fastest across the lanes the plain kernel reads
 // 2 bytes out of a different pixel per lane and tap.  Here a CTA owns 64 output pixels of one row x all channels: the (<= 3) source rows are
 // staged in shared memory with coalesced channel-fastest reads, the outputs leave as 256-byte runs per plane (1.36 ms -> ~0.1 ms at B = 32).
+// The staged rows are fp32 whatever T is, so the tile's shared memory (3 x 70 x (C | 1) floats, 34 KB at C = 40) is the same for a
+// bf16 and an fp32 input; an fp32 input takes two 16-byte reads per eight channels instead of one.
 constexpr int UP_TX = 64, UP_NCOL = 70;
-__global__ void __launch_bounds__(256) upsample_dw_nchw_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, const float *__restrict__ w,
-                                                               const float *__restrict__ bias, const __nv_bfloat16 *__restrict__ skip, int skip_stride,
+template <typename T>
+__global__ void __launch_bounds__(256) upsample_dw_nchw_kernel(const T *__restrict__ x, int x_stride, const float *__restrict__ w,
+                                                               const float *__restrict__ bias, const T *__restrict__ skip, int skip_stride,
                                                                float *__restrict__ out, int C, int Hi, int Wi, int Ho, int Wo) {
     extern __shared__ float usrc[];                     // [3][UP_NCOL][CP]
     const int CP = C | 1;
@@ -278,10 +310,10 @@ __global__ void __launch_bounds__(256) upsample_dw_nchw_kernel(const __nv_bfloat
         const int cg = e % cgs, col = (e / cgs) % ncol, ky = e / (cgs * ncol);
         float *dst = usrc + (ky * UP_NCOL + col) * CP + cg * 8;
         if (vy[ky]) {
-            const uint4 v = *reinterpret_cast<const uint4 *>(x + (((long long)b * Hi + sy[ky]) * Wi + sx_lo + col) * x_stride + cg * 8);
-            const __nv_bfloat162 *h = reinterpret_cast<const __nv_bfloat162 *>(&v);
+            float v[8];
+            load8(x + (((long long)b * Hi + sy[ky]) * Wi + sx_lo + col) * x_stride + cg * 8, v);
 #pragma unroll
-            for (int q = 0; q < 4; ++q) { const float2 f = __bfloat1622float2(h[q]); dst[2 * q] = f.x; dst[2 * q + 1] = f.y; }
+            for (int q = 0; q < 8; ++q) dst[q] = v[q];
         } else {
 #pragma unroll
             for (int q = 0; q < 8; ++q) dst[q] = 0.f;
@@ -307,15 +339,16 @@ __global__ void __launch_bounds__(256) upsample_dw_nchw_kernel(const __nv_bfloat
             for (int kx = 0; kx < 3; ++kx)
                 if (vx[kx]) acc = fmaf(w[c * 9 + ky * 3 + kx], usrc[(ky * UP_NCOL + scol[kx]) * CP + c], acc);
         }
-        if (skip) acc += __bfloat162float(skip[(((long long)b * Ho + oy) * Wo + ox) * skip_stride + c]);
+        if (skip) acc += ldf(skip + (((long long)b * Ho + oy) * Wo + ox) * skip_stride + c);
         out[(((long long)b * C + c) * Ho + oy) * Wo + ox] = acc;
     }
 }
 
-// (2) bf16 NHWC result: eight channels per thread (16-byte loads / stores), the depth-wise filters in shared memory as [tap][channel]
-__global__ void __launch_bounds__(256) upsample_dw_nhwc8_kernel(const __nv_bfloat16 *__restrict__ x, int x_stride, const float *__restrict__ w,
-                                                                const float *__restrict__ bias, const __nv_bfloat16 *__restrict__ skip, int skip_stride,
-                                                                __nv_bfloat16 *__restrict__ out, int out_stride, int B, int C, int Hi, int Wi, int Ho,
+// (2) NHWC result: eight channels per thread (16-byte loads / stores), the depth-wise filters in shared memory as [tap][channel]
+template <typename T>
+__global__ void __launch_bounds__(256) upsample_dw_nhwc8_kernel(const T *__restrict__ x, int x_stride, const float *__restrict__ w,
+                                                                const float *__restrict__ bias, const T *__restrict__ skip, int skip_stride,
+                                                                T *__restrict__ out, int out_stride, int B, int C, int Hi, int Wi, int Ho,
                                                                 int Wo) {
     extern __shared__ float usw[];                      // [9][C] then bias[C]
     for (int e = threadIdx.x; e < 9 * C; e += 256) usw[e] = w[(e % C) * 9 + e / C];
@@ -341,27 +374,20 @@ __global__ void __launch_bounds__(256) upsample_dw_nhwc8_kernel(const __nv_bfloa
                 const int ux = ox - 1 + kx;
                 if (ux < 0 || ux >= Wo) continue;
                 const int sx = min((int)floorf(ux * fx), Wi - 1);
-                const uint4 v = *reinterpret_cast<const uint4 *>(x + (((long long)b * Hi + sy) * Wi + sx) * x_stride + c0);
-                const __nv_bfloat162 *h = reinterpret_cast<const __nv_bfloat162 *>(&v);
+                float v[8];
+                load8(x + (((long long)b * Hi + sy) * Wi + sx) * x_stride + c0, v);
                 const float *wt = usw + (ky * 3 + kx) * C + c0;
 #pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float2 f = __bfloat1622float2(h[q]);
-                    acc[2 * q] = fmaf(wt[2 * q], f.x, acc[2 * q]);
-                    acc[2 * q + 1] = fmaf(wt[2 * q + 1], f.y, acc[2 * q + 1]);
-                }
+                for (int q = 0; q < 8; ++q) acc[q] = fmaf(wt[q], v[q], acc[q]);
             }
         }
         if (skip) {
-            const uint4 v = *reinterpret_cast<const uint4 *>(skip + p * skip_stride + c0);
-            const __nv_bfloat162 *h = reinterpret_cast<const __nv_bfloat162 *>(&v);
+            float v[8];
+            load8(skip + p * skip_stride + c0, v);
 #pragma unroll
-            for (int q = 0; q < 4; ++q) { const float2 f = __bfloat1622float2(h[q]); acc[2 * q] += f.x; acc[2 * q + 1] += f.y; }
+            for (int q = 0; q < 8; ++q) acc[q] += v[q];
         }
-        uint32_t o[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) { const __nv_bfloat162 h2 = __floats2bfloat162_rn(acc[2 * q], acc[2 * q + 1]); o[q] = *reinterpret_cast<const uint32_t *>(&h2); }
-        *reinterpret_cast<uint4 *>(out + p * out_stride + c0) = make_uint4(o[0], o[1], o[2], o[3]);
+        store8(out + p * out_stride + c0, acc);
     }
 }
 
@@ -372,18 +398,25 @@ int grid_for(long long total) { return (int)min((long long)cdiv(total, 256), (lo
 
 using namespace rdfc;
 
-static int bf16_view_ok(const rdfc_view *v, const char *what) {
-    RDFC_REQUIRE(v && v->ptr && v->dtype == RDFC_BF16 && !v->nchw && v->C % 8 == 0 && v->pix_stride % 8 == 0 && ((uintptr_t)v->ptr % 16) == 0,
-                 "%s: 16-byte aligned bf16 NHWC view with C %% 8 == 0 expected", what);
+// NHWC activation view: bf16 or fp32, C % 8 == 0, 16-byte aligned at every pixel (eight channels are one or two 16-byte accesses)
+static int act_view_ok(const rdfc_view *v, const char *what) {
+    RDFC_REQUIRE(v && v->ptr && (v->dtype == RDFC_BF16 || v->dtype == RDFC_F32) && !v->nchw && v->C % 8 == 0 &&
+                     v->pix_stride % (v->dtype == RDFC_BF16 ? 8 : 4) == 0 && ((uintptr_t)v->ptr % 16) == 0,
+                 "%s: 16-byte aligned bf16 or fp32 NHWC view with C %% 8 == 0 expected", what);
     return 0;
 }
 
-extern "C" int rdfc_first_conv_forward(const float *x_nchw, int B, int Cin, int Hi, int Wi, const float *weight, int k, int stride, int pad,
-                                       const float *scale, const float *shift, int relu, const rdfc_view *out, void *stream) {
-    RDFC_REQUIRE(x_nchw && weight && scale && shift && out, "first conv: NULL argument");
-    if (int rc = bf16_view_ok(out, "first conv out")) return rc;
-    RDFC_REQUIRE(B > 0 && Cin >= 1 && Cin <= 4 && k >= 1 && k <= 7 && stride >= 1 && out->C <= 256 && 256 % out->C == 0,
-                 "first conv: Cin <= 4, k <= 7, Cout a divisor of 256");
+// both views valid and of one dtype
+static int act_pair_ok(const rdfc_view *x, const rdfc_view *out, const char *what) {
+    if (int rc = act_view_ok(x, what)) return rc;
+    if (int rc = act_view_ok(out, what)) return rc;
+    RDFC_REQUIRE(x->dtype == out->dtype, "%s: input and output views must share a dtype", what);
+    return 0;
+}
+
+template <typename T>
+static int first_conv_launch(const float *x_nchw, int B, int Cin, int Hi, int Wi, const float *weight, int k, int stride, int pad,
+                             const float *scale, const float *shift, int relu, const rdfc_view *out, cudaStream_t st) {
     const int Ho = (Hi + 2 * pad - k) / stride + 1, Wo = (Wi + 2 * pad - k) / stride + 1;
     if (k == 7 && stride == 2 && pad == 3 && out->C == 64 && knob("RDFC_FIRSTCONV_FAST", 1) != 0) {     // ESANet's stem: the register-tiled kernel
         const size_t fsmem = (size_t)(49 * Cin * 64 + Cin * FC_PR * FC_PC) * sizeof(float);
@@ -391,13 +424,12 @@ extern "C" int rdfc_first_conv_forward(const float *x_nchw, int B, int Cin, int 
         int dev = 0;
         RDFC_CUDA(cudaGetDevice(&dev));
         if (!attr[dev & 63]) {
-            RDFC_CUDA(cudaFuncSetAttribute(first_conv7s2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024));
+            RDFC_CUDA(cudaFuncSetAttribute(first_conv7s2_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024));
             attr[dev & 63] = true;
         }
         const long long ntiles = (long long)B * cdiv(Ho, FC_TY) * cdiv(Wo, FC_TX);
         const int grid = (int)min(ntiles, (long long)sm_count() * 3);
-        first_conv7s2_kernel<<<grid, 256, fsmem, (cudaStream_t)stream>>>(x_nchw, weight, scale, shift, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, Cin,
-                                                                         Hi, Wi, Ho, Wo, relu);
+        first_conv7s2_kernel<T><<<grid, 256, fsmem, st>>>(x_nchw, weight, scale, shift, (T *)out->ptr, out->pix_stride, B, Cin, Hi, Wi, Ho, Wo, relu);
         RDFC_CHECK_LAUNCH("first_conv7s2_kernel");
         return 0;
     }
@@ -406,20 +438,34 @@ extern "C" int rdfc_first_conv_forward(const float *x_nchw, int B, int Cin, int 
     const long long npix = (long long)B * Ho * Wo;
     const int npb = 256 / out->C;
     const int grid = (int)min((long long)cdiv(npix, npb), (long long)sm_count() * 8);
-    first_conv_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(x_nchw, weight, scale, shift, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, Cin, Hi,
-                                                                 Wi, Ho, Wo, k, stride, pad, out->C, relu);
+    first_conv_kernel<T><<<grid, 256, smem, st>>>(x_nchw, weight, scale, shift, (T *)out->ptr, out->pix_stride, B, Cin, Hi, Wi, Ho, Wo, k, stride, pad,
+                                                  out->C, relu);
     RDFC_CHECK_LAUNCH("first_conv_kernel");
     return 0;
 }
 
+extern "C" int rdfc_first_conv_forward(const float *x_nchw, int B, int Cin, int Hi, int Wi, const float *weight, int k, int stride, int pad,
+                                       const float *scale, const float *shift, int relu, const rdfc_view *out, void *stream) {
+    RDFC_REQUIRE(x_nchw && weight && scale && shift && out, "first conv: NULL argument");
+    if (int rc = act_view_ok(out, "first conv out")) return rc;
+    RDFC_REQUIRE(B > 0 && Cin >= 1 && Cin <= 4 && k >= 1 && k <= 7 && stride >= 1 && out->C <= 256 && 256 % out->C == 0,
+                 "first conv: Cin <= 4, k <= 7, Cout a divisor of 256");
+    return out->dtype == RDFC_F32
+               ? first_conv_launch<float>(x_nchw, B, Cin, Hi, Wi, weight, k, stride, pad, scale, shift, relu, out, (cudaStream_t)stream)
+               : first_conv_launch<__nv_bfloat16>(x_nchw, B, Cin, Hi, Wi, weight, k, stride, pad, scale, shift, relu, out, (cudaStream_t)stream);
+}
+
 extern "C" int rdfc_maxpool3x3s2_forward(const rdfc_view *x, const rdfc_view *out, int B, int Hi, int Wi, void *stream) {
-    if (int rc = bf16_view_ok(x, "maxpool x")) return rc;
-    if (int rc = bf16_view_ok(out, "maxpool out")) return rc;
+    if (int rc = act_pair_ok(x, out, "maxpool")) return rc;
     RDFC_REQUIRE(x->C == out->C && B > 0 && Hi > 0 && Wi > 0, "maxpool: channel mismatch / empty");
     const int Ho = (Hi - 1) / 2 + 1, Wo = (Wi - 1) / 2 + 1;
-    maxpool_kernel<<<grid_for((long long)B * Ho * Wo * (x->C / 8)), 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16 *)x->ptr, x->pix_stride,
-                                                                                                   (__nv_bfloat16 *)out->ptr, out->pix_stride, B,
-                                                                                                   x->C, Hi, Wi, Ho, Wo);
+    const int grid = grid_for((long long)B * Ho * Wo * (x->C / 8));
+    if (x->dtype == RDFC_F32)
+        maxpool_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>((const float *)x->ptr, x->pix_stride, (float *)out->ptr, out->pix_stride, B, x->C,
+                                                                      Hi, Wi, Ho, Wo);
+    else
+        maxpool_kernel<__nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16 *)x->ptr, x->pix_stride, (__nv_bfloat16 *)out->ptr,
+                                                                              out->pix_stride, B, x->C, Hi, Wi, Ho, Wo);
     RDFC_CHECK_LAUNCH("maxpool_kernel");
     return 0;
 }
@@ -433,55 +479,73 @@ extern "C" int rdfc_se_weights(const float *mean, const float *w1, const float *
 }
 
 extern "C" int rdfc_adaptive_avgpool_forward(const rdfc_view *x, const rdfc_view *out, int B, int H, int W, int bins, void *stream) {
-    if (int rc = bf16_view_ok(x, "adaptive avgpool x")) return rc;
-    if (int rc = bf16_view_ok(out, "adaptive avgpool out")) return rc;
+    if (int rc = act_pair_ok(x, out, "adaptive avgpool")) return rc;
     RDFC_REQUIRE(x->C == out->C && B > 0 && bins > 0 && H > 0 && W > 0, "adaptive avgpool: bad shape");
-    adaptive_avgpool_kernel<<<grid_for((long long)B * bins * bins * x->C), 256, 0, (cudaStream_t)stream>>>(
-        (const __nv_bfloat16 *)x->ptr, x->pix_stride, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, x->C, H, W, bins);
+    const int grid = grid_for((long long)B * bins * bins * x->C);
+    if (x->dtype == RDFC_F32)
+        adaptive_avgpool_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>((const float *)x->ptr, x->pix_stride, (float *)out->ptr, out->pix_stride,
+                                                                               B, x->C, H, W, bins);
+    else
+        adaptive_avgpool_kernel<__nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            (const __nv_bfloat16 *)x->ptr, x->pix_stride, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, x->C, H, W, bins);
     RDFC_CHECK_LAUNCH("adaptive_avgpool_kernel");
     return 0;
 }
 
 extern "C" int rdfc_upsample_nearest_forward(const rdfc_view *x, const rdfc_view *out, int B, int hs, int ws, int H, int W, void *stream) {
-    if (int rc = bf16_view_ok(x, "upsample x")) return rc;
-    if (int rc = bf16_view_ok(out, "upsample out")) return rc;
+    if (int rc = act_pair_ok(x, out, "upsample nearest")) return rc;
     RDFC_REQUIRE(x->C == out->C && B > 0 && hs > 0 && ws > 0 && H > 0 && W > 0, "upsample nearest: bad shape");
-    upsample_nearest_kernel<<<grid_for((long long)B * H * W * (x->C / 8)), 256, 0, (cudaStream_t)stream>>>(
-        (const __nv_bfloat16 *)x->ptr, x->pix_stride, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, x->C, hs, ws, H, W);
+    const int grid = grid_for((long long)B * H * W * (x->C / 8));
+    if (x->dtype == RDFC_F32)
+        upsample_nearest_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>((const float *)x->ptr, x->pix_stride, (float *)out->ptr, out->pix_stride,
+                                                                               B, x->C, hs, ws, H, W);
+    else
+        upsample_nearest_kernel<__nv_bfloat16><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            (const __nv_bfloat16 *)x->ptr, x->pix_stride, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, x->C, hs, ws, H, W);
     RDFC_CHECK_LAUNCH("upsample_nearest_kernel");
+    return 0;
+}
+
+template <typename T>
+static int upsample_dw_launch(const rdfc_view *x, const float *weight, const float *bias, const T *sk, int sk_stride, const rdfc_view *out,
+                              float *out_nchw, int B, int Hi, int Wi, int Ho, int Wo, cudaStream_t st) {
+    const T *xp = (const T *)x->ptr;
+    const long long total = (long long)B * Ho * Wo * x->C;
+    const bool fast = knob("RDFC_UPSAMPLE_FAST", 1) != 0;
+    if (out_nchw && fast && Hi <= Ho && Wi <= Wo && (size_t)3 * UP_NCOL * (x->C | 1) * 4 <= 48 * 1024 && B <= 65535 && Ho <= 65535) {
+        upsample_dw_nchw_kernel<T><<<dim3(cdiv(Wo, UP_TX), Ho, B), 256, (size_t)3 * UP_NCOL * (x->C | 1) * 4, st>>>(
+            xp, x->pix_stride, weight, bias, sk, sk_stride, out_nchw, x->C, Hi, Wi, Ho, Wo);
+    } else if (out_nchw) {
+        upsample_dw_kernel<T, true><<<grid_for(total), 256, 0, st>>>(xp, x->pix_stride, weight, bias, sk, sk_stride, out_nchw, 0, B, x->C, Hi, Wi, Ho, Wo);
+    } else if (fast && (size_t)10 * x->C * 4 <= 48 * 1024) {
+        upsample_dw_nhwc8_kernel<T><<<grid_for(total / 8), 256, (size_t)10 * x->C * 4, st>>>(xp, x->pix_stride, weight, bias, sk, sk_stride,
+                                                                                             (T *)out->ptr, out->pix_stride, B, x->C, Hi, Wi, Ho, Wo);
+    } else {
+        upsample_dw_kernel<T, false><<<grid_for(total), 256, 0, st>>>(xp, x->pix_stride, weight, bias, sk, sk_stride, out->ptr, out->pix_stride, B, x->C,
+                                                                      Hi, Wi, Ho, Wo);
+    }
+    RDFC_CHECK_LAUNCH("upsample_dw_kernel");
     return 0;
 }
 
 extern "C" int rdfc_upsample_dw_forward(const rdfc_view *x, const float *weight, const float *bias, const rdfc_view *skip, const rdfc_view *out,
                                         float *out_nchw, int B, int Hi, int Wi, int Ho, int Wo, void *stream) {
-    if (int rc = bf16_view_ok(x, "upsample dw x")) return rc;
+    if (int rc = act_view_ok(x, "upsample dw x")) return rc;
     RDFC_REQUIRE(weight && bias && B > 0 && Hi > 0 && Wi > 0 && Ho > 0 && Wo > 0, "upsample dw: bad argument");
-    RDFC_REQUIRE((out && out->ptr) != (out_nchw != nullptr), "upsample dw: exactly one of out (bf16 NHWC) / out_nchw (fp32 NCHW)");
-    const __nv_bfloat16 *sk = nullptr;
+    RDFC_REQUIRE((out && out->ptr) != (out_nchw != nullptr), "upsample dw: exactly one of out (NHWC) / out_nchw (fp32 NCHW)");
+    if (!out_nchw) {
+        if (int rc = act_pair_ok(x, out, "upsample dw")) return rc;
+        RDFC_REQUIRE(out->C == x->C, "upsample dw: output channel mismatch");
+    }
+    const void *sk = nullptr;
     int sk_stride = 0;
     if (skip && skip->ptr) {
-        if (int rc = bf16_view_ok(skip, "upsample dw skip")) return rc;
+        if (int rc = act_pair_ok(x, skip, "upsample dw skip")) return rc;
         RDFC_REQUIRE(skip->C == x->C, "upsample dw: skip channel mismatch");
-        sk = (const __nv_bfloat16 *)skip->ptr; sk_stride = skip->pix_stride;
+        sk = skip->ptr; sk_stride = skip->pix_stride;
     }
-    const long long total = (long long)B * Ho * Wo * x->C;
-    const bool fast = knob("RDFC_UPSAMPLE_FAST", 1) != 0;
-    if (out_nchw && fast && Hi <= Ho && Wi <= Wo && (size_t)3 * UP_NCOL * (x->C | 1) * 4 <= 48 * 1024 && B <= 65535 && Ho <= 65535) {
-        upsample_dw_nchw_kernel<<<dim3(cdiv(Wo, UP_TX), Ho, B), 256, (size_t)3 * UP_NCOL * (x->C | 1) * 4, (cudaStream_t)stream>>>(
-            (const __nv_bfloat16 *)x->ptr, x->pix_stride, weight, bias, sk, sk_stride, out_nchw, x->C, Hi, Wi, Ho, Wo);
-    } else if (out_nchw) {
-        upsample_dw_kernel<true><<<grid_for(total), 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16 *)x->ptr, x->pix_stride, weight, bias, sk,
-                                                                                    sk_stride, out_nchw, 0, B, x->C, Hi, Wi, Ho, Wo);
-    } else {
-        if (int rc = bf16_view_ok(out, "upsample dw out")) return rc;
-        RDFC_REQUIRE(out->C == x->C, "upsample dw: output channel mismatch");
-        if (fast && (size_t)10 * x->C * 4 <= 48 * 1024 && (!sk || (sk_stride % 8 == 0 && ((uintptr_t)sk % 16) == 0)))
-            upsample_dw_nhwc8_kernel<<<grid_for(total / 8), 256, (size_t)10 * x->C * 4, (cudaStream_t)stream>>>(
-                (const __nv_bfloat16 *)x->ptr, x->pix_stride, weight, bias, sk, sk_stride, (__nv_bfloat16 *)out->ptr, out->pix_stride, B, x->C, Hi, Wi, Ho, Wo);
-        else
-        upsample_dw_kernel<false><<<grid_for(total), 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16 *)x->ptr, x->pix_stride, weight, bias, sk,
-                                                                                     sk_stride, out->ptr, out->pix_stride, B, x->C, Hi, Wi, Ho, Wo);
-    }
-    RDFC_CHECK_LAUNCH("upsample_dw_kernel");
-    return 0;
+    if (x->dtype == RDFC_F32)
+        return upsample_dw_launch<float>(x, weight, bias, (const float *)sk, sk_stride, out, out_nchw, B, Hi, Wi, Ho, Wo, (cudaStream_t)stream);
+    return upsample_dw_launch<__nv_bfloat16>(x, weight, bias, (const __nv_bfloat16 *)sk, sk_stride, out, out_nchw, B, Hi, Wi, Ho, Wo,
+                                             (cudaStream_t)stream);
 }

@@ -27,6 +27,24 @@ def _down(n):
     return (n - 1) // 2 + 1      # conv k3 s2 p1 (and 1x1 s2 p0)
 
 
+def pack_weight(w, umma, x3=False):
+    """(Cout, Cin, kh, kw) fp32 filters -> the layout rdfc_conv_forward reads for the conv path:
+    RDFC_PATH_SIMT_F32    (umma False)     [tap][cin][cout] fp32;
+    RDFC_PATH_UMMA_BF16   (umma, not x3)   [tap][cin/8][CoutP][8] bf16, Cout zero-padded to CoutP = a multiple of 16;
+    RDFC_PATH_UMMA_F32X3  (umma and x3)    the same layout in fp16 over [W_hi ; W_lo ; W_hi] along Cin (3 Cin channels)."""
+    if x3:       # [W_hi ; W_lo ; W_hi] along Cin, fp16 halves (11 + 11 mantissa bits): the kernel pairs them with x_hi, x_hi, x_lo
+        w_hi = w.to(torch.float16).float()
+        w = torch.cat([w_hi, (w - w_hi).to(torch.float16).float(), w_hi], 1)
+    Cout, Cin, kh, kw = w.shape
+    g = w.permute(0, 2, 3, 1).reshape(Cout, kh * kw, Cin)          # [cout][tap][cin]
+    if not umma:
+        return g.permute(1, 2, 0).contiguous()                      # [tap][cin][cout] fp32
+    CoutP = (Cout + 15) // 16 * 16
+    if CoutP != Cout:
+        g = torch.cat([g, g.new_zeros(CoutP - Cout, kh * kw, Cin)], 0)
+    return g.reshape(CoutP, kh * kw, Cin // 8, 8).permute(1, 2, 0, 3).contiguous().to(torch.float16 if x3 else torch.bfloat16)
+
+
 class _Packed:
     """Persistent device storage for one (possibly fused) conv layer's packed filters and epilogue vectors."""
 
@@ -162,19 +180,7 @@ class GeneratorEngine:
                 sh = bias.detach().float() if bias is not None else torch.zeros(w.shape[0], device=w.device)
             scs.append(sc)
             shs.append(sh)
-        w = torch.cat(ws, 0)
-        if x3:       # [W_hi ; W_lo ; W_hi] along Cin, fp16 halves (11 + 11 mantissa bits): the kernel pairs them with x_hi, x_hi, x_lo
-            w_hi = w.to(torch.float16).float()
-            w = torch.cat([w_hi, (w - w_hi).to(torch.float16).float(), w_hi], 1)
-        Cout, Cin, kh, kw = w.shape
-        g = w.permute(0, 2, 3, 1).reshape(Cout, kh * kw, Cin)          # [cout][tap][cin]
-        if umma:
-            CoutP = (Cout + 15) // 16 * 16
-            if CoutP != Cout:
-                g = torch.cat([g, g.new_zeros(CoutP - Cout, kh * kw, Cin)], 0)
-            packed = g.reshape(CoutP, kh * kw, Cin // 8, 8).permute(1, 2, 0, 3).contiguous().to(torch.float16 if x3 else torch.bfloat16)
-        else:
-            packed = g.permute(1, 2, 0).contiguous()                    # [tap][cin][cout] fp32
+        packed = pack_weight(torch.cat(ws, 0), umma, x3)
         p = self._packed.setdefault((precision, name), _Packed())
         p.store(packed, torch.cat(scs).contiguous(), torch.cat(shs).contiguous())
         return p

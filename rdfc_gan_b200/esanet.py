@@ -4,14 +4,19 @@ F/lib/models/backbone/resnet/resnet.py; F = /root/reference/RDF-GAN): the ``glob
 into the 40-channel semantic map RDF-GAN's stems read (rdf_gan_generator.py:235).
 
 Same constructor keywords, same module / parameter names (``state_dict`` loads into and from the reference class with
-strict=True).  Inference runs on this repo's kernels through one plan per input shape (buffers + a flat list of C-ABI calls,
-captured in a CUDA graph), bf16 NHWC activations:
+strict=True).  Inference runs on this repo's kernels through one plan per input shape and precision (buffers + a flat list of
+C-ABI calls, captured in a CUDA graph), NHWC activations:
 
 * every GEMM-shaped layer -- the ResNet BasicBlocks, the 1x1 skip / pyramid-pooling convs, the decoder's 3x3 convs, its
-  factorised 3x1 / 1x3 convs (as 3x3 filters with zero taps) and conv_out -- on ``rdfc_conv_forward`` (tcgen05), BatchNorm
-  folded, bias / ReLU / residual fused in the epilogue;
+  factorised 3x1 / 1x3 convs (as 3x3 filters with zero taps) and conv_out -- on ``rdfc_conv_forward``, BatchNorm folded,
+  bias / ReLU / residual fused in the epilogue;
 * the 7x7 stride-2 stem, max pooling, squeeze-and-excitation, the pyramid pooling module's average pools / nearest up-sampling
   and the decoder's learned x2 up-sampling (+ skip add) on the small kernels of csrc/esanet.cu.
+
+``set_precision`` selects the arithmetic, with the meanings of the generator's modes (engine.GeneratorEngine):
+  'bf16'    (default) bf16 activations, the convs on the tcgen05 tensor cores (RDFC_PATH_UMMA_BF16): the throughput mode;
+  'fp32'    fp32 activations, every conv on the CUDA cores in fp32 (RDFC_PATH_SIMT_F32): the parity mode;
+  'fp32_tc' fp32 activations, the convs on the tensor cores with split fp16 operands (RDFC_PATH_UMMA_F32X3).
 
 Covered configuration = the one the reference's scripts use (F/bash/test_nyuv2_Ts2T.sh:7-16): ResNet-18 / 34 BasicBlock encoder,
 ``weighting_in_encoder='SE-add'``, ``context_module='ppm'``, ``encoder_decoder_fusion='add'``,
@@ -24,8 +29,10 @@ import torch
 import torch.nn as nn
 
 from . import _cabi as C
+from .engine import pack_weight
 
 _BLOCKS = {'resnet18': (2, 2, 2, 2), 'resnet34': (3, 4, 6, 3)}
+_PRECISIONS = ('bf16', 'fp32', 'fp32_tc')
 
 
 def _no_forward(self, *a, **k):
@@ -176,8 +183,18 @@ class ESANetOneModality(nn.Module):
         bins = (1, 2, 4, 8) if context_module == 'ppm-1-2-4-8' else (1, 5)
         self.context_module = PyramidPoolingModule(512, channels_decoder[0], bins)
         self.decoder = Decoder(channels_decoder[0], channels_decoder, nr_decoder_blocks, num_classes)
+        self.precision = 'bf16'
         self._plans = {}
         self._stamp = None
+
+    def set_precision(self, precision):
+        """'bf16' (the default: tensor cores, bf16 activations), 'fp32' (CUDA-core fp32, the parity mode) or 'fp32_tc' (fp32
+        activations, tensor cores with split fp16 operands).  Returns self.  A generator's ``set_precision`` does not reach the
+        guidance module it holds: set both for an fp32 RDF-GAN end to end."""
+        if precision not in _PRECISIONS:
+            raise ValueError(f"precision must be one of {_PRECISIONS}, got {precision!r}")
+        self.precision = precision
+        return self
 
     # ------------------------------------------------------------------------------------------------------------
     def forward(self, image):
@@ -198,12 +215,12 @@ class ESANetOneModality(nn.Module):
             if stamp != self._stamp:                       # weights changed (or first call): plans bake folded / packed copies
                 self._plans.clear()
                 self._stamp = stamp
-            key = (B, H, W, dev)
+            key = (B, H, W, dev, self.precision)
             plan = self._plans.get(key)
             if plan is None:
                 if len(self._plans) >= 4:
                     del self._plans[next(iter(self._plans))]
-                plan = self._plans[key] = _build_plan(self, B, H, W, dev)
+                plan = self._plans[key] = _build_plan(self, B, H, W, dev, self.precision)
                 plan['inp'].copy_(image)
                 _capture(plan)
             plan['inp'].copy_(image)
@@ -217,32 +234,34 @@ def _fold(bn):
     return scale, bn.bias.detach().float() - bn.running_mean.detach().float() * scale
 
 
-def _pack_umma(w):
-    """(O, I, kh, kw) -> 3x3 (zero taps around factorised / 1x1 kernels stay out: 1x1 is packed as 1 tap) UMMA layout, bf16"""
+def _square(w):
+    """(O, I, kh, kw) -> (filters, k): the factorised 3x1 / 1x3 kernels embedded in 3x3 filters with zero taps; 1x1 and 3x3 as they are"""
     O, I, kh, kw = w.shape
-    if (kh, kw) not in ((1, 1), (3, 3)):
-        full = w.new_zeros(O, I, 3, 3)
-        full[:, :, (3 - kh) // 2:(3 - kh) // 2 + kh, (3 - kw) // 2:(3 - kw) // 2 + kw] = w
-        w, kh, kw = full, 3, 3
-    OP = (O + 15) // 16 * 16
-    g = w.permute(0, 2, 3, 1).reshape(O, kh * kw, I)
-    if OP != O:
-        g = torch.cat([g, g.new_zeros(OP - O, kh * kw, I)], 0)
-    return g.reshape(OP, kh * kw, I // 8, 8).permute(1, 2, 0, 3).contiguous().to(torch.bfloat16), kh
+    if (kh, kw) in ((1, 1), (3, 3)):
+        return w, kh
+    full = w.new_zeros(O, I, 3, 3)
+    full[:, :, (3 - kh) // 2:(3 - kh) // 2 + kh, (3 - kw) // 2:(3 - kw) // 2 + kw] = w
+    return full, 3
 
 
-def _build_plan(net, B, H, W, dev):
+def _build_plan(net, B, H, W, dev, precision='bf16'):
     keep, steps = [], []
+    adt = torch.bfloat16 if precision == 'bf16' else torch.float32
+    x3_descs = []            # fp32_tc: descriptors sharing one split-input workspace, sized once every conv is known
 
-    def new(*shape, dtype=torch.bfloat16):
-        t = torch.empty(shape, dtype=dtype, device=dev)
+    def new(*shape, dtype=None):
+        t = torch.empty(shape, dtype=dtype or adt, device=dev)
         keep.append(t)
         return t
 
     def conv(x, conv_mod, bn, out, act, residual=None, hin=None, stride=1):
-        """x / out / residual: (tensor, c0, C) NHWC slices.  Conv2d (+ folded BatchNorm or bias) + activation on the tensor cores."""
-        w = conv_mod.weight.detach().float()
-        packed, k = _pack_umma(w)
+        """x / out / residual: (tensor, c0, C) NHWC slices.  Conv2d (+ folded BatchNorm or bias) + activation on the plan's conv path."""
+        w, k = _square(conv_mod.weight.detach().float())
+        cin = x[2]
+        # fp32_tc: the split-operand tensor-core path where its shape rules allow (all ESANet convs), else CUDA-core fp32
+        x3 = precision == 'fp32_tc' and cin % 32 == 0 and out[2] >= 16
+        umma = precision == 'bf16' or x3
+        packed = pack_weight(w, umma, x3)
         if bn is not None:
             scale, shift = _fold(bn)
             if conv_mod.bias is not None:            # conv bias in front of a BatchNorm (NonBottleneck1D): bn(conv + b) = scale conv + (scale b + shift)
@@ -256,7 +275,10 @@ def _build_plan(net, B, H, W, dev):
         d = C.ConvDesc()
         d.B, d.Hi, d.Wi, d.Ho, d.Wo = B, Hi, Wi, Ho, Wo
         d.kh = d.kw = k
-        d.stride, d.pad, d.transposed, d.act, d.path = stride, (k - 1) // 2, 0, act, C.PATH_UMMA_BF16
+        d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, 0, act
+        d.path = C.PATH_UMMA_F32X3 if x3 else (C.PATH_UMMA_BF16 if umma else C.PATH_SIMT_F32)
+        if x3:
+            x3_descs.append((d, B * Hi * Wi * cin * 4))
         d.inp, d.in2 = C.view(x[0], x[2], x[1]), C.view(None)
         d.out = C.view(out[0], out[2], out[1])
         d.residual = C.view(None) if residual is None else C.view(residual[0], residual[2], residual[1])
@@ -396,6 +418,10 @@ def _build_plan(net, B, H, W, dev):
         else:
             steps.append(lambda s, v_in=v_in, wq=wq, bq=bq, a=src_hw, b=dst_hw: C.check(C.lib.rdfc_upsample_dw_forward(
                 ctypes.byref(v_in), C.ptr(wq), C.ptr(bq), None, None, C.ptr(out), B, a[0], a[1], b[0], b[1], s)))
+    if x3_descs:             # one stream: the convs run one after the other and can share the [hi | lo] copy of their input
+        ws = new(max(n for _, n in x3_descs), dtype=torch.uint8)
+        for d, _ in x3_descs:
+            d.workspace, d.workspace_bytes = ws.data_ptr(), ws.numel()
     return dict(inp=inp, out=out, steps=steps, keep=keep, graph=None)
 
 

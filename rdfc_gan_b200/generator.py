@@ -172,7 +172,11 @@ class RDFGenerator(_GeneratorBase):
 class DCVGANGenerator(_GeneratorBase):
     """RDF-GAN generator (rdf_gan_generator.py:12-361).  ``fuse_depth_in_rgb_decoder='AdaIN'`` selects the W-AdaIN
     layer there (:133), and the keyword is spelled ``use_nlpsn_refine`` (:28).  ``global_guidance_module`` is any
-    nn.Module mapping rgb -> (B, semantic_channels_in, H, W) (ESANet in the reference's scripts); it is called as is."""
+    nn.Module mapping rgb -> (B, semantic_channels_in, H, W) (ESANet in the reference's scripts); it is called as is.
+
+    The guidance module keeps its own precision: ``set_precision`` sets the generator's arithmetic only (this repo's ESANet
+    stays in its default 'bf16').  RDF-GAN in fp32 end to end is
+    ``G.set_precision('fp32'); G.global_guidance_module.set_precision('fp32')``; ``stream`` calls the module as ``forward`` does."""
 
     def __init__(self, global_guidance_module, encoder_rgb='resnet18', encoder_depth='resnet18',
                  pretrained_on_imagenet=True, semantic_channels_in=40, fuse_depth_in_rgb_decoder='AdaIN', bn=True,
