@@ -48,7 +48,8 @@ typedef enum {
     RDFC_ERR_UNSUPPORTED = -3
 } rdfc_status;
 
-typedef enum { RDFC_F32 = 0, RDFC_F64 = 1, RDFC_BF16 = 2 } rdfc_dtype;
+/* RDFC_F16: the fp16 [hi | lo] split tensors of the fp32_tc training entry points only */
+typedef enum { RDFC_F32 = 0, RDFC_F64 = 1, RDFC_BF16 = 2, RDFC_F16 = 3 } rdfc_dtype;
 
 int rdfc_abi_version(void);
 const char *rdfc_last_error(void);
@@ -284,7 +285,8 @@ int rdfc_depth_metric_sums(const float *pred, const float *gt, const unsigned ch
 /* Batch-statistics BatchNorm fused with the activation and the residual add, and the conv filter gradient: what the
  * reference's train() mode leaves to nn.BatchNorm2d / cuDNN inside conv_bn_relu / convt_bn_relu / BasicBlock
  * (encoder_decoder/common.py:29-61, encoder_decoder/encoder_decoder.py:39-59; training step lib/models/rdf_gan.py:135-207).
- * Activations: bf16 NHWC views over npix = B*H*W pixels; statistics and parameter gradients fp32; deterministic reductions. */
+ * Activations: NHWC views over npix = B*H*W pixels -- bf16, or fp32 for the BatchNorm entry points (one dtype per call; fp32 pixel
+ * strides a multiple of 4); statistics and parameter gradients fp32; deterministic reductions. */
 
 /* floats of workspace for rdfc_bn_stats / rdfc_bn_act_backward */
 int rdfc_bn_workspace_floats(long long npix, int C);
@@ -316,6 +318,25 @@ typedef struct {
 } rdfc_wgrad_desc;
 long long rdfc_conv_wgrad_workspace_floats(const rdfc_wgrad_desc *d);
 int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, float *workspace, void *stream);
+/* The training step's fp32_tc mode: fp32 activations and gradients, contractions on the tensor cores with split fp16 operands
+ * (x = x_hi + x_lo; x_hi W_hi + x_hi W_lo + x_lo W_hi accumulated in fp32).  Each tensor is first scaled by a power of two taken
+ * from its own largest magnitude (fp16's exponent range is narrow: gradients near 1e-5 would lose their low half), and the
+ * factors stay on the device.  C % 32 == 0 everywhere; views 16-byte aligned; invalid arguments fail before any launch.
+ *
+ * rdfc_split_scaled: x = fp32 NHWC view (C channels, pixel stride a multiple of 4) -> out = RDFC_F16 view of 2C channels
+ *   [hi | lo] of s * x per pixel (pixel stride a multiple of 8); *factor (device float) = s, the power of two with
+ *   max|x| * s in [1024, 2048), 1 for an all-zero tensor. */
+int rdfc_split_scaled(const rdfc_view *x, long long npix, const rdfc_view *out, float *factor, void *stream);
+/* rdfc_conv_forward on an already split input: d->in = the RDFC_F16 [hi | lo] view (2 Cin channels), d->path =
+ * RDFC_PATH_UMMA_F32X3 (weight = that path's [W_hi ; W_lo ; W_hi] packing, of the filter scaled by its own power of two),
+ * d->out fp32 NHWC, d->scale REQUIRED: the per-Cout factor 1 / (s_x s_w) that undoes the scaling; no residual, no workspace. */
+int rdfc_conv_forward_split(const rdfc_conv_desc *d, void *stream);
+/* Filter gradient of split operands: d->grad_out / d->input = RDFC_F16 [hi | lo] views (2 O / 2 I channels) of s_g * grad_out and
+ * s_x * input; inv_scale = device float 1 / (s_g s_x).  The three products g_hi x_hi, g_hi x_lo, g_lo x_hi run on the tcgen05
+ * filter-gradient kernel into consecutive chunk ranges of the workspace (rdfc_conv_wgrad_split_workspace_floats(d) floats,
+ * 16-byte aligned); one reduction in a fixed order writes grad_weight (O, I, k, k) fp32: bit-reproducible. */
+long long rdfc_conv_wgrad_split_workspace_floats(const rdfc_wgrad_desc *d);
+int rdfc_conv_wgrad_split(const rdfc_wgrad_desc *d, const float *inv_scale, float *grad_weight, float *workspace, void *stream);
 
 /* ------------------------------------------------------------------ ESANet guidance glue ---------------------- */
 /* The non-GEMM layers of RDF-GAN's global_guidance_module (F/lib/models/segmentator/esa_net/esa_net_one_modality.py:145-172,

@@ -9,7 +9,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librdfc_b200.so")
 
-F32, F64, BF16 = 0, 1, 2
+F32, F64, BF16, F16 = 0, 1, 2, 3          # F16: the split [hi | lo] tensors of the fp32_tc training mode
 ACT_NONE, ACT_RELU, ACT_LEAKY02, ACT_TANH, ACT_SIGMOID = range(5)
 PATH_SIMT_F32, PATH_UMMA_BF16, PATH_UMMA_F32X3 = 0, 1, 2
 AFFINITY = {"AS": 0, "ASS": 1, "TC": 2, "TGASS": 3}
@@ -88,6 +88,11 @@ def _load():
     lib.rdfc_conv_wgrad_workspace_floats.argtypes = [ctypes.POINTER(WgradDesc)]
     lib.rdfc_conv_wgrad_workspace_floats.restype = ctypes.c_longlong
     lib.rdfc_conv_wgrad.argtypes = [ctypes.POINTER(WgradDesc), c_void_p, c_void_p, c_void_p]
+    lib.rdfc_split_scaled.argtypes = [VP, ctypes.c_longlong, VP, c_void_p, c_void_p]
+    lib.rdfc_conv_forward_split.argtypes = [ctypes.POINTER(ConvDesc), c_void_p]
+    lib.rdfc_conv_wgrad_split_workspace_floats.argtypes = [ctypes.POINTER(WgradDesc)]
+    lib.rdfc_conv_wgrad_split_workspace_floats.restype = ctypes.c_longlong
+    lib.rdfc_conv_wgrad_split.argtypes = [ctypes.POINTER(WgradDesc), c_void_p, c_void_p, c_void_p, c_void_p]
     lib.rdfc_first_conv_forward.argtypes = [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, VP, c_void_p]
     lib.rdfc_maxpool3x3s2_forward.argtypes = [VP, VP, c_int, c_int, c_int, c_void_p]
     lib.rdfc_se_weights.argtypes = [c_void_p] * 6 + [c_int, c_int, c_int, c_void_p]
@@ -126,7 +131,8 @@ EXPORTS = ["rdfc_abi_version", "rdfc_last_error", "rdfc_launch_count", "rdfc_dcn
            "rdfc_wadain_tile", "rdfc_wadain_conv_forward", "rdfc_dev_set_knob", "rdfc_dev_umma_timers",
            "rdfc_bn_workspace_floats", "rdfc_bn_stats", "rdfc_affine_act_forward", "rdfc_bn_act_backward",
            "rdfc_conv_wgrad_workspace_floats", "rdfc_conv_wgrad", "rdfc_first_conv_forward", "rdfc_maxpool3x3s2_forward", "rdfc_se_weights",
-           "rdfc_adaptive_avgpool_forward", "rdfc_upsample_nearest_forward", "rdfc_upsample_dw_forward"]
+           "rdfc_adaptive_avgpool_forward", "rdfc_upsample_nearest_forward", "rdfc_upsample_dw_forward",
+           "rdfc_split_scaled", "rdfc_conv_forward_split", "rdfc_conv_wgrad_split_workspace_floats", "rdfc_conv_wgrad_split"]
 
 
 KNOB_UNSET = -(1 << 63)

@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "librdfc_b200.so")
-SOURCES = ["api.cu", "dcn.cu", "nlspn.cu", "conv_simt.cu", "conv_umma.cu", "conv.cu", "norm.cu", "metrics.cu", "train.cu", "wgrad_umma.cu", "esanet.cu"]
+SOURCES = ["api.cu", "dcn.cu", "nlspn.cu", "conv_simt.cu", "conv_umma.cu", "conv.cu", "norm.cu", "metrics.cu", "train.cu", "wgrad_umma.cu", "train_split.cu", "esanet.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "-ccbin", "/usr/bin/g++"] + os.environ.get("RDFC_NVCC_FLAGS", "").split()   # e.g. -DRDFC_UMMA_TIMERS

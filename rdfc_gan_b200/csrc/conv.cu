@@ -12,7 +12,7 @@ int conv_umma_read_dbg(long long *host, int n);
 
 using namespace rdfc;
 
-extern "C" int rdfc_conv_forward(const rdfc_conv_desc *d, void *stream) {
+static int check_conv_geometry(const rdfc_conv_desc *d) {
     RDFC_REQUIRE(d != nullptr, "descriptor is NULL");
     RDFC_REQUIRE(d->in.ptr && d->out.ptr && d->weight, "conv: input / output / weight must not be NULL");
     RDFC_REQUIRE(d->B > 0 && d->Hi > 0 && d->Wi > 0 && d->Ho > 0 && d->Wo > 0 && d->in.C > 0 && d->out.C > 0,
@@ -26,6 +26,11 @@ extern "C" int rdfc_conv_forward(const rdfc_conv_desc *d, void *stream) {
     }
     RDFC_REQUIRE(d->in.nchw || d->in.pix_stride >= d->in.C, "conv: input pixel stride smaller than its channel count");
     RDFC_REQUIRE(d->out.nchw || d->out.pix_stride >= d->out.C, "conv: output pixel stride smaller than its channel count");
+    return 0;
+}
+
+extern "C" int rdfc_conv_forward(const rdfc_conv_desc *d, void *stream) {
+    if (int rc = check_conv_geometry(d)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (d->path == RDFC_PATH_UMMA_BF16) return conv_umma_forward(d, st, nullptr, nullptr, nullptr, 0);
     if (d->path == RDFC_PATH_SIMT_F32) return conv_simt_forward(d, st);
@@ -45,6 +50,20 @@ extern "C" int rdfc_conv_forward(const rdfc_conv_desc *d, void *stream) {
         return conv_umma_forward(&e, st, nullptr, nullptr, nullptr, d->in.C);
     }
     return fail(RDFC_ERR_INVALID, "conv: unknown path %d", d->path);
+}
+
+extern "C" int rdfc_conv_forward_split(const rdfc_conv_desc *d, void *stream) {
+    if (int rc = check_conv_geometry(d)) return rc;
+    RDFC_REQUIRE(d->path == RDFC_PATH_UMMA_F32X3, "conv (split input): path must be RDFC_PATH_UMMA_F32X3");
+    RDFC_REQUIRE(d->in.dtype == RDFC_F16 && !d->in.nchw && d->in.C % 64 == 0,
+                 "conv (split input): an fp16 [hi | lo] view with 2 x Cin channels, Cin %% 32 == 0, expected (got %d channels)", d->in.C);
+    RDFC_REQUIRE(d->out.dtype == RDFC_F32 && !d->out.nchw && !d->in2.ptr && !d->residual.ptr,
+                 "conv (split input): fp32 NHWC output, no second source, no residual");
+    RDFC_REQUIRE(d->scale != nullptr, "conv (split input): the per-Cout inverse scale vector is required");
+    rdfc_conv_desc e = *d;
+    e.in.dtype = RDFC_BF16;                 // 16-bit operands: the split path of the kernel reads them as fp16
+    e.path = RDFC_PATH_UMMA_BF16;
+    return conv_umma_forward(&e, (cudaStream_t)stream, nullptr, nullptr, nullptr, d->in.C / 2);
 }
 
 extern "C" int rdfc_heads_forward(const rdfc_heads_desc *h, void *stream) {

@@ -3,8 +3,8 @@
 //
 // Replaces, for conv_bn_relu / convt_bn_relu / torchvision BasicBlock in train() mode (encoder_decoder/common.py:29-61,
 // encoder_decoder/encoder_decoder.py:39-59), what the reference leaves to cuDNN / ATen: nn.BatchNorm2d's batch statistics and
-// its backward, the (Leaky)ReLU backward, and Conv2d / ConvTranspose2d's weight gradient.  Activations are bf16 NHWC views
-// (pointer, channels, pixel stride), statistics and gradients of parameters fp32, all reductions deterministic (fixed
+// its backward, the (Leaky)ReLU backward, and Conv2d / ConvTranspose2d's weight gradient.  Activations are NHWC views (pointer,
+// channels, pixel stride): bf16, or fp32 in the BatchNorm kernels (the fp32_tc training mode); statistics and gradients of parameters fp32, all reductions deterministic (fixed
 // combination order, no atomics).
 #include "common.cuh"
 
@@ -33,15 +33,30 @@ __device__ __forceinline__ void st8(__nv_bfloat16 *p, const float (&v)[8]) {
     *reinterpret_cast<uint4 *>(p) = make_uint4(w[0], w[1], w[2], w[3]);
 }
 
+// the same for fp32 activations (the fp32_tc training mode): two 16-byte loads / stores
+__device__ __forceinline__ void ld8(const float *p, float (&v)[8]) {
+    const float4 a = __ldg(reinterpret_cast<const float4 *>(p)), b = __ldg(reinterpret_cast<const float4 *>(p) + 1);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void st8(float *p, const float (&v)[8]) {
+    reinterpret_cast<float4 *>(p)[0] = make_float4(v[0], v[1], v[2], v[3]);
+    reinterpret_cast<float4 *>(p)[1] = make_float4(v[4], v[5], v[6], v[7]);
+}
+__device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float to_f(float v) { return v; }
+
+// an NHWC view of bf16 (the default training mode) or fp32 (fp32_tc) activations
+template <typename T>
 struct View {
-    const __nv_bfloat16 *ptr;
+    const T *ptr;
     int stride;
 };
 
 // ---- per-channel batch statistics ---------------------------------------------------------------------------------------
 // Pass 1: grid (nblk, ceil(C/64)), block 256 = 8 channel groups x 32 pixel lanes.  A CTA owns pixels [p0, p1) and emits the
 // (mean, M2) of every channel over them (sums shifted by the CTA's first pixel, so nothing cancels).
-__global__ void __launch_bounds__(256) bn_partial_kernel(View x, int C, long long npix, int per_blk, float *__restrict__ partial) {
+template <typename T>
+__global__ void __launch_bounds__(256) bn_partial_kernel(View<T> x, int C, long long npix, int per_blk, float *__restrict__ partial) {
     __shared__ float red[32][8][17];
     const int cg = threadIdx.x & 7, lane = threadIdx.x >> 3;
     const int c0 = blockIdx.y * 64 + cg * 8;
@@ -52,7 +67,7 @@ __global__ void __launch_bounds__(256) bn_partial_kernel(View x, int C, long lon
 #pragma unroll
     for (int q = 0; q < 8; ++q) s[q] = ss[q] = pivot[q] = 0.f;
     if (c0 < C && n > 0) {
-        const __nv_bfloat16 *base = x.ptr + p0 * x.stride + c0;
+        const T *base = x.ptr + p0 * x.stride + c0;
         ld8(base, pivot);
         for (int p = lane; p < n; p += 32) {
             float v[8];
@@ -81,7 +96,7 @@ __global__ void __launch_bounds__(256) bn_partial_kernel(View x, int C, long lon
             }
             float mean = 0.f, m2 = 0.f;
             if (n > 0) {
-                const float pv = __bfloat162float(x.ptr[p0 * x.stride + c]);
+                const float pv = to_f(x.ptr[p0 * x.stride + c]);
                 mean = pv + ts / n;
                 m2 = fmaxf(tss - ts * ts / n, 0.f);
             }
@@ -134,9 +149,9 @@ __global__ void __launch_bounds__(256) bn_final_kernel(const float *__restrict__
 // kHoist (C / 8 a power of two <= 256, i.e. a divisor of the 256-thread block): a thread's channel group is the same in every iteration
 // of the grid-stride loop, so its eight (scale, shift) pairs are read once and the pixel index advances by an add -- the plain form reads
 // 16 per-channel values through the LSU per 2-3 vector loads of data and divides a 64-bit index per iteration.
-template <bool kHoist>
-__global__ void __launch_bounds__(256) affine_act_kernel(View x, const float *__restrict__ scale, const float *__restrict__ shift, View res,
-                                                         float slope, __nv_bfloat16 *__restrict__ out, int out_stride, int C, long long npix) {
+template <typename T, bool kHoist>
+__global__ void __launch_bounds__(256) affine_act_kernel(View<T> x, const float *__restrict__ scale, const float *__restrict__ shift, View<T> res,
+                                                         float slope, T *__restrict__ out, int out_stride, int C, long long npix) {
     const int cgs = C >> 3;
     if (kHoist) {
         const long long tid = (long long)blockIdx.x * 256 + threadIdx.x, T = (long long)gridDim.x * 256;
@@ -180,7 +195,8 @@ __global__ void __launch_bounds__(256) affine_act_kernel(View x, const float *__
 // act' from the sign of the activation's OUTPUT (ReLU / LeakyReLU keep the sign; slope 1 = no activation).
 __device__ __forceinline__ float dact(float out, float slope) { return out > 0.f ? 1.f : slope; }
 
-__global__ void __launch_bounds__(256) bn_bwd_partial_kernel(View dout, View out, View y, const float *__restrict__ mean,
+template <typename T>
+__global__ void __launch_bounds__(256) bn_bwd_partial_kernel(View<T> dout, View<T> out, View<T> y, const float *__restrict__ mean,
                                                              const float *__restrict__ rstd, float slope, int C, long long npix, int per_blk,
                                                              float *__restrict__ partial) {
     __shared__ float red[32][8][17];
@@ -250,11 +266,11 @@ __global__ void __launch_bounds__(256) sum_final_kernel(const float *__restrict_
 }
 
 // dy = gamma * rstd * (dz - sum_dz / N - xhat * sum_dz_xhat / N);  dres = dz.   kHoist: as in affine_act_kernel (same arithmetic order).
-template <bool kHoist>
-__global__ void __launch_bounds__(256) bn_bwd_apply_kernel(View dout, View out, View y, const float *__restrict__ mean,
+template <typename T, bool kHoist>
+__global__ void __launch_bounds__(256) bn_bwd_apply_kernel(View<T> dout, View<T> out, View<T> y, const float *__restrict__ mean,
                                                            const float *__restrict__ rstd, const float *__restrict__ gamma,
                                                            const float *__restrict__ sum_dz, const float *__restrict__ sum_dzx, float slope,
-                                                           __nv_bfloat16 *__restrict__ dy, int dy_stride, __nv_bfloat16 *__restrict__ dres,
+                                                           T *__restrict__ dy, int dy_stride, T *__restrict__ dres,
                                                            int dres_stride, int C, long long npix) {
     const int cgs = C >> 3;
     const float invn = 1.f / (float)npix;
@@ -485,11 +501,14 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float *__restri
 
 using namespace rdfc;
 
-static inline View mk(const rdfc_view *v) { return View{(const __nv_bfloat16 *)v->ptr, v->pix_stride}; }
-static int check_view(const rdfc_view *v, int C, const char *what) {
+template <typename T>
+static inline View<T> mk(const rdfc_view *v) { return View<T>{(const T *)v->ptr, v->pix_stride}; }
+// `dtype`: the dtype every view of the call must have -- bf16 (pixel stride a multiple of 8) or fp32 (a multiple of 4); 16-byte aligned
+static int check_view(const rdfc_view *v, int C, const char *what, int dtype) {
     RDFC_REQUIRE(v && v->ptr, "%s: NULL view", what);
-    RDFC_REQUIRE(v->dtype == RDFC_BF16 && !v->nchw, "%s: bf16 NHWC views only", what);
-    RDFC_REQUIRE(v->C == C && C % 8 == 0 && v->pix_stride % 8 == 0 && ((uintptr_t)v->ptr % 16) == 0,
+    RDFC_REQUIRE((dtype == RDFC_BF16 || dtype == RDFC_F32) && v->dtype == dtype && !v->nchw,
+                 "%s: NHWC views of one dtype (bf16 or fp32) expected", what);
+    RDFC_REQUIRE(v->C == C && C % 8 == 0 && v->pix_stride % (dtype == RDFC_BF16 ? 8 : 4) == 0 && ((uintptr_t)v->ptr % 16) == 0,
                  "%s: %d channels expected, multiples of 8, 16-byte aligned", what, C);
     return 0;
 }
@@ -506,36 +525,74 @@ extern "C" int rdfc_bn_workspace_floats(long long npix, int C) {
     return red_blocks(npix, &per) * C * 2;
 }
 
-extern "C" int rdfc_bn_stats(const rdfc_view *x, long long npix, float *workspace, float *mean, float *var, void *stream) {
-    RDFC_REQUIRE(x && workspace && mean && var && npix > 0, "bn stats: bad argument");
-    if (int rc = check_view(x, x->C, "bn stats")) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
+template <typename T>
+static int bn_stats(const rdfc_view *x, long long npix, float *workspace, float *mean, float *var, cudaStream_t st) {
     int per;
     const int nblk = red_blocks(npix, &per), C = x->C;
-    bn_partial_kernel<<<dim3(nblk, cdiv(C, 64)), 256, 0, st>>>(mk(x), C, npix, per, workspace);
+    bn_partial_kernel<T><<<dim3(nblk, cdiv(C, 64)), 256, 0, st>>>(mk<T>(x), C, npix, per, workspace);
     RDFC_CHECK_LAUNCH("bn_partial_kernel");
     bn_final_kernel<<<cdiv(C, 8), 256, 0, st>>>(workspace, C, npix, per, nblk, mean, var);
     RDFC_CHECK_LAUNCH("bn_final_kernel");
     return 0;
 }
 
+extern "C" int rdfc_bn_stats(const rdfc_view *x, long long npix, float *workspace, float *mean, float *var, void *stream) {
+    RDFC_REQUIRE(x && workspace && mean && var && npix > 0, "bn stats: bad argument");
+    if (int rc = check_view(x, x->C, "bn stats", x->dtype)) return rc;
+    if (x->dtype == RDFC_F32) return bn_stats<float>(x, npix, workspace, mean, var, (cudaStream_t)stream);
+    return bn_stats<__nv_bfloat16>(x, npix, workspace, mean, var, (cudaStream_t)stream);
+}
+
 static float act_slope(int act) { return act == RDFC_ACT_RELU ? 0.f : (act == RDFC_ACT_LEAKY02 ? 0.2f : 1.f); }
+
+template <typename T>
+static int affine_act(const rdfc_view *x, const float *scale, const float *shift, const rdfc_view *residual, int act, const rdfc_view *out,
+                      long long npix, cudaStream_t st) {
+    const int C = x->C;
+    const View<T> r = (residual && residual->ptr) ? mk<T>(residual) : View<T>{nullptr, 0};
+    const int nblk = (int)min((long long)cdiv(npix * (C / 8), 256), (long long)sm_count() * 16);
+    if (256 % (C >> 3) == 0 && knob("RDFC_BN_HOIST", 1) != 0)
+        affine_act_kernel<T, true><<<nblk, 256, 0, st>>>(mk<T>(x), scale, shift, r, act_slope(act), (T *)out->ptr, out->pix_stride, C, npix);
+    else
+        affine_act_kernel<T, false><<<nblk, 256, 0, st>>>(mk<T>(x), scale, shift, r, act_slope(act), (T *)out->ptr, out->pix_stride, C, npix);
+    RDFC_CHECK_LAUNCH("affine_act_kernel");
+    return 0;
+}
 
 extern "C" int rdfc_affine_act_forward(const rdfc_view *x, const float *scale, const float *shift, const rdfc_view *residual, int act,
                                        const rdfc_view *out, long long npix, void *stream) {
     RDFC_REQUIRE(x && scale && shift && out && npix > 0, "affine act: bad argument");
     RDFC_REQUIRE(act == RDFC_ACT_NONE || act == RDFC_ACT_RELU || act == RDFC_ACT_LEAKY02, "affine act: none / ReLU / LeakyReLU(0.2) only");
-    const int C = x->C;
-    if (int rc = check_view(x, C, "affine act x")) return rc;
-    if (int rc = check_view(out, C, "affine act out")) return rc;
-    if (residual && residual->ptr) if (int rc = check_view(residual, C, "affine act residual")) return rc;
-    const View r = (residual && residual->ptr) ? mk(residual) : View{nullptr, 0};
-    const int nblk = (int)min((long long)cdiv(npix * (C / 8), 256), (long long)sm_count() * 16);
+    const int C = x->C, dt = x->dtype;
+    if (int rc = check_view(x, C, "affine act x", dt)) return rc;
+    if (int rc = check_view(out, C, "affine act out", dt)) return rc;
+    if (residual && residual->ptr) if (int rc = check_view(residual, C, "affine act residual", dt)) return rc;
+    if (dt == RDFC_F32) return affine_act<float>(x, scale, shift, residual, act, out, npix, (cudaStream_t)stream);
+    return affine_act<__nv_bfloat16>(x, scale, shift, residual, act, out, npix, (cudaStream_t)stream);
+}
+
+template <typename T>
+static int bn_act_backward(const rdfc_view *dout, const rdfc_view *out, const rdfc_view *y, const float *mean, const float *rstd, const float *gamma,
+                           int act, const rdfc_view *dy, const rdfc_view *dres, float *workspace, float *sum_dz, float *sum_dz_xhat, long long npix,
+                           cudaStream_t st) {
+    const int C = y->C;
+    int per;
+    const int nblk = red_blocks(npix, &per);
+    const float slope = act_slope(act);
+    bn_bwd_partial_kernel<T><<<dim3(nblk, cdiv(C, 64)), 256, 0, st>>>(mk<T>(dout), mk<T>(out), mk<T>(y), mean, rstd, slope, C, npix, per, workspace);
+    RDFC_CHECK_LAUNCH("bn_bwd_partial_kernel");
+    sum_final_kernel<<<cdiv(C, 8), 256, 0, st>>>(workspace, C, nblk, sum_dz, sum_dz_xhat);
+    RDFC_CHECK_LAUNCH("sum_final_kernel");
+    const int ablk = (int)min((long long)cdiv(npix * (C / 8), 256), (long long)sm_count() * 16);
+    T *dr = (dres && dres->ptr) ? (T *)dres->ptr : nullptr;
+    const int dr_stride = dr ? dres->pix_stride : 0;
     if (256 % (C >> 3) == 0 && knob("RDFC_BN_HOIST", 1) != 0)
-        affine_act_kernel<true><<<nblk, 256, 0, (cudaStream_t)stream>>>(mk(x), scale, shift, r, act_slope(act), (__nv_bfloat16 *)out->ptr, out->pix_stride, C, npix);
+        bn_bwd_apply_kernel<T, true><<<ablk, 256, 0, st>>>(mk<T>(dout), mk<T>(out), mk<T>(y), mean, rstd, gamma, sum_dz, sum_dz_xhat, slope, (T *)dy->ptr,
+                                                           dy->pix_stride, dr, dr_stride, C, npix);
     else
-        affine_act_kernel<false><<<nblk, 256, 0, (cudaStream_t)stream>>>(mk(x), scale, shift, r, act_slope(act), (__nv_bfloat16 *)out->ptr, out->pix_stride, C, npix);
-    RDFC_CHECK_LAUNCH("affine_act_kernel");
+        bn_bwd_apply_kernel<T, false><<<ablk, 256, 0, st>>>(mk<T>(dout), mk<T>(out), mk<T>(y), mean, rstd, gamma, sum_dz, sum_dz_xhat, slope, (T *)dy->ptr,
+                                                            dy->pix_stride, dr, dr_stride, C, npix);
+    RDFC_CHECK_LAUNCH("bn_bwd_apply_kernel");
     return 0;
 }
 
@@ -544,31 +601,15 @@ extern "C" int rdfc_bn_act_backward(const rdfc_view *dout, const rdfc_view *out,
                                     float *sum_dz, float *sum_dz_xhat, long long npix, void *stream) {
     RDFC_REQUIRE(dout && out && y && mean && rstd && gamma && dy && workspace && sum_dz && sum_dz_xhat && npix > 0, "bn backward: bad argument");
     RDFC_REQUIRE(act == RDFC_ACT_NONE || act == RDFC_ACT_RELU || act == RDFC_ACT_LEAKY02, "bn backward: none / ReLU / LeakyReLU(0.2) only");
-    const int C = y->C;
-    if (int rc = check_view(dout, C, "bn backward dout")) return rc;
-    if (int rc = check_view(out, C, "bn backward out")) return rc;
-    if (int rc = check_view(y, C, "bn backward y")) return rc;
-    if (int rc = check_view(dy, C, "bn backward dy")) return rc;
-    if (dres && dres->ptr) if (int rc = check_view(dres, C, "bn backward dres")) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    int per;
-    const int nblk = red_blocks(npix, &per);
-    const float slope = act_slope(act);
-    bn_bwd_partial_kernel<<<dim3(nblk, cdiv(C, 64)), 256, 0, st>>>(mk(dout), mk(out), mk(y), mean, rstd, slope, C, npix, per, workspace);
-    RDFC_CHECK_LAUNCH("bn_bwd_partial_kernel");
-    sum_final_kernel<<<cdiv(C, 8), 256, 0, st>>>(workspace, C, nblk, sum_dz, sum_dz_xhat);
-    RDFC_CHECK_LAUNCH("sum_final_kernel");
-    const int ablk = (int)min((long long)cdiv(npix * (C / 8), 256), (long long)sm_count() * 16);
-    if (256 % (C >> 3) == 0 && knob("RDFC_BN_HOIST", 1) != 0)
-        bn_bwd_apply_kernel<true><<<ablk, 256, 0, st>>>(mk(dout), mk(out), mk(y), mean, rstd, gamma, sum_dz, sum_dz_xhat, slope, (__nv_bfloat16 *)dy->ptr,
-                                                        dy->pix_stride, (dres && dres->ptr) ? (__nv_bfloat16 *)dres->ptr : nullptr,
-                                                        (dres && dres->ptr) ? dres->pix_stride : 0, C, npix);
-    else
-        bn_bwd_apply_kernel<false><<<ablk, 256, 0, st>>>(mk(dout), mk(out), mk(y), mean, rstd, gamma, sum_dz, sum_dz_xhat, slope, (__nv_bfloat16 *)dy->ptr,
-                                                         dy->pix_stride, (dres && dres->ptr) ? (__nv_bfloat16 *)dres->ptr : nullptr,
-                                                         (dres && dres->ptr) ? dres->pix_stride : 0, C, npix);
-    RDFC_CHECK_LAUNCH("bn_bwd_apply_kernel");
-    return 0;
+    const int C = y->C, dt = y->dtype;
+    if (int rc = check_view(dout, C, "bn backward dout", dt)) return rc;
+    if (int rc = check_view(out, C, "bn backward out", dt)) return rc;
+    if (int rc = check_view(y, C, "bn backward y", dt)) return rc;
+    if (int rc = check_view(dy, C, "bn backward dy", dt)) return rc;
+    if (dres && dres->ptr) if (int rc = check_view(dres, C, "bn backward dres", dt)) return rc;
+    if (dt == RDFC_F32)
+        return bn_act_backward<float>(dout, out, y, mean, rstd, gamma, act, dy, dres, workspace, sum_dz, sum_dz_xhat, npix, (cudaStream_t)stream);
+    return bn_act_backward<__nv_bfloat16>(dout, out, y, mean, rstd, gamma, act, dy, dres, workspace, sum_dz, sum_dz_xhat, npix, (cudaStream_t)stream);
 }
 
 // geometry shared by the workspace query and the launch
@@ -619,8 +660,8 @@ extern "C" int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, flo
     WgGeom g;
     if (int rc = wgrad_geom(d, &g)) return rc;
     RDFC_REQUIRE(grad_weight && workspace, "wgrad: NULL output / workspace");
-    if (int rc = check_view(&d->grad_out, d->grad_out.C, "wgrad grad_out")) return rc;
-    if (int rc = check_view(&d->input, d->input.C, "wgrad input")) return rc;
+    if (int rc = check_view(&d->grad_out, d->grad_out.C, "wgrad grad_out", RDFC_BF16)) return rc;
+    if (int rc = check_view(&d->input, d->input.C, "wgrad input", RDFC_BF16)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (wgrad_umma_ok(d)) return wgrad_umma(d, grad_weight, workspace, st);
     WgradParams P{};

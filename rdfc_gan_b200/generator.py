@@ -31,6 +31,7 @@ class _GeneratorBase(nn.Module):
             raise NotImplementedError("channel plans other than the reference defaults are not supported "
                                       "(the ResNet layers fix them, encoder_decoder.py:39-46)")
         self.use_nlspn_refine = use_nlspn_refine
+        self._train_precision = 'bf16'          # set_train_precision; a plain attribute, not part of state_dict
         self.bn = bn
         self.rgb_skip_connection_type = rgb_skip_connection_type
         self.depth_skip_connection_type = depth_skip_connection_type
@@ -102,6 +103,21 @@ class _GeneratorBase(nn.Module):
         self.engine(precision)
         return self
 
+    def set_train_precision(self, precision):
+        """Arithmetic of the train-mode forward / backward (batch-statistics BatchNorm, autograd): 'bf16' (bf16 activations on the
+        tcgen05 tensor cores, the default) or 'fp32_tc' (fp32 activations and gradients; every conv's forward, data gradient and
+        filter gradient on the tensor cores with split fp16 operands, each scaled by a power of two from its own largest magnitude;
+        fp32 BatchNorm; the cuDNN stems / heads with TF32 off) -- the reference's fp32 training at tensor-core speed.  Strict
+        CUDA-core fp32 training is not provided.  Leaves ``set_precision`` (the eval-mode engine) alone, and the reverse; not part of
+        ``state_dict``.  Returns self."""
+        if precision == 'fp32':
+            raise ValueError("train precision 'fp32' (CUDA-core training) is not provided: use 'fp32_tc' for fp32 training on the "
+                             "tensor cores, or 'bf16'")
+        if precision not in ('bf16', 'fp32_tc'):
+            raise ValueError(f"train precision must be 'bf16' or 'fp32_tc', got {precision!r}")
+        self._train_precision = precision
+        return self
+
     def _check_inference(self, *tensors):
         for t in tensors:
             if not t.is_cuda:
@@ -116,7 +132,8 @@ class _GeneratorBase(nn.Module):
             from .train_forward import generator_forward_train
             if self.bn is not True or self.fuse_kind not in ('WAdaIN', 'AdaIN', 'IN'):
                 raise NotImplementedError("training-mode forward covers bn=True generators")
-            return generator_forward_train(self, stem_in, depth)
+            dtype = torch.float32 if getattr(self, '_train_precision', 'bf16') == 'fp32_tc' else torch.bfloat16
+            return generator_forward_train(self, stem_in, depth, dtype)
         self._check_inference(stem_in, depth)
         return self.engine().forward(stem_in, depth)
 
@@ -136,7 +153,9 @@ class _GeneratorBase(nn.Module):
 
 
 class RDFGenerator(_GeneratorBase):
-    """rdf_generator.py:31-414"""
+    """rdf_generator.py:31-414.  Eval mode runs the inference engine (``set_precision('bf16' | 'fp32' | 'fp32_tc')``); train mode
+    runs batch-statistics BatchNorm with autograd in bf16 or, after ``set_train_precision('fp32_tc')``, in fp32 on split-operand
+    tensor-core arithmetic."""
 
     def __init__(self, encoder_rgb='resnet18', encoder_depth='resnet18', pretrained_on_imagenet=True,
                  semantic_channels_in=3, fuse_depth_in_rgb_decoder='WAdaIN', bn=True,
@@ -174,6 +193,7 @@ class DCVGANGenerator(_GeneratorBase):
     layer there (:133), and the keyword is spelled ``use_nlpsn_refine`` (:28).  ``global_guidance_module`` is any
     nn.Module mapping rgb -> (B, semantic_channels_in, H, W) (ESANet in the reference's scripts); it is called as is.
 
+    ``set_train_precision('bf16' | 'fp32_tc')`` selects the train-mode arithmetic (see _GeneratorBase.set_train_precision).
     The guidance module keeps its own precision: ``set_precision`` sets the generator's arithmetic only (this repo's ESANet
     stays in its default 'bf16').  RDF-GAN in fp32 end to end is
     ``G.set_precision('fp32'); G.global_guidance_module.set_precision('fp32')``; ``stream`` calls the module as ``forward`` does."""

@@ -1,5 +1,7 @@
 """Training-mode forward of the generator (batch-statistics BatchNorm, autograd), rdf_generator.py:280-414 /
-rdf_gan_generator.py:233-361, composed of the differentiable ops of train_ops.py over bf16 NHWC tensors.
+rdf_gan_generator.py:233-361, composed of the differentiable ops of train_ops.py over NHWC tensors: bf16 (the default training
+mode) or fp32 (the ``fp32_tc`` mode: split-operand tensor-core arithmetic in the ops, and the PyTorch convs that stay on cuDNN --
+stems, ``*_dec0`` heads -- run in true fp32, with TF32 off in their forward and backward).
 
 The convolutions with >= 32 input channels -- every encoder / decoder / ``*_dec1`` layer and the per-pixel EqualLinear of
 W-AdaIN, > 99 % of the FLOPs -- run forward, data gradient and filter gradient on this repo's kernels; BatchNorm (+ residual +
@@ -7,6 +9,8 @@ activation) runs on the fused batch-statistics kernels; the NLSPN runs its fused
 stems (3 / 1 input channels), the ``*_dec0`` heads (<= 8 output channels), the InstanceNorm + modulation of the fusion layers
 and the output fusion are differentiable PyTorch expressions on the same tensors.
 """
+import contextlib
+
 import torch
 import torch.nn.functional as F
 
@@ -19,6 +23,46 @@ BF = torch.bfloat16
 
 def _nhwc(x_nchw):
     return x_nchw.permute(0, 2, 3, 1).contiguous()
+
+
+@contextlib.contextmanager
+def _no_tf32():
+    """cuDNN convs in true fp32 (torch lets them use TF32 by default, ~1e-3 relative); the caller's setting comes back after."""
+    prev = torch.backends.cudnn.allow_tf32
+    torch.backends.cudnn.allow_tf32 = False
+    try:
+        yield
+    finally:
+        torch.backends.cudnn.allow_tf32 = prev
+
+
+class _ConvFP32(torch.autograd.Function):
+    """F.conv2d(x, w, b, padding) (stride 1) with TF32 off in the forward AND the backward: autograd would run the backward
+    under whatever TF32 setting is current when it gets there."""
+    @staticmethod
+    def forward(ctx, x, w, b, padding):
+        with _no_tf32():
+            y = F.conv2d(x, w, b, padding=padding)
+        ctx.save_for_backward(x, w)
+        ctx.cfg = (padding, None if b is None else tuple(b.shape))
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, w = ctx.saved_tensors
+        padding, bshape = ctx.cfg
+        mask = [ctx.needs_input_grad[0], ctx.needs_input_grad[1], bshape is not None and ctx.needs_input_grad[2]]
+        with _no_tf32():
+            gx, gw, gb = torch.ops.aten.convolution_backward(gy, x, w, list(bshape) if bshape else None, [1, 1], [padding, padding], [1, 1],
+                                                             False, [0, 0], 1, mask)
+        return gx, gw, gb, None
+
+
+def _conv(x, w, b, padding, dt):
+    """the stems' and heads' cuDNN conv: as is in bf16 mode, true fp32 in fp32_tc mode"""
+    if dt == torch.float32:
+        return _ConvFP32.apply(x, w, b, padding)
+    return F.conv2d(x, w, b, padding=padding)
 
 
 def _conv_bn_act(x, seq, k=3, stride=1, transposed=False, act=C.ACT_LEAKY02, residual=None):
@@ -37,11 +81,12 @@ def _basic_block(x, blk):
 
 
 def _small_conv(x_nhwc, conv, act=None):
-    """A conv too thin for the tensor-core kernel (<= 8 output channels): torch, on the NHWC tensor viewed as channels-last NCHW.
-    -> fp32 NCHW"""
+    """A conv too thin for the tensor-core kernel (<= 8 output channels): torch, on the NHWC tensor viewed as channels-last NCHW,
+    in the activations' dtype.  -> fp32 NCHW"""
+    dt = x_nhwc.dtype
     x = x_nhwc.permute(0, 3, 1, 2)                      # channels-last view; channels-last filters keep cuDNN from converting layouts
-    w = conv.weight.to(BF).contiguous(memory_format=torch.channels_last)
-    y = F.conv2d(x, w, None if conv.bias is None else conv.bias.to(BF), stride=1, padding=1).float()
+    w = conv.weight.to(dt).contiguous(memory_format=torch.channels_last)
+    y = _conv(x, w, None if conv.bias is None else conv.bias.to(dt), 1, dt).float()
     if act == 'tanh':
         y = torch.tanh(y)
     elif act == 'sigmoid':
@@ -58,7 +103,8 @@ def _instance_norm(x, eps=1e-5, unbiased=False):
 
 
 def _fuse(layer, xr, xd):
-    """fuse_layer{n}(rgb feature, depth feature), model_utils.py:53-129, NHWC in / out"""
+    """fuse_layer{n}(rgb feature, depth feature), model_utils.py:53-129, NHWC in / out (the inputs' dtype)"""
+    dt = xr.dtype
     if isinstance(layer, AdaptiveInstanceNorm):
         lin = layer.style.linear
         Cx = xr.shape[3]
@@ -73,17 +119,17 @@ def _fuse(layer, xr, xd):
             out = gw * gamma * out + bw * beta
         else:
             out = gamma * out + beta
-        return out.to(BF)
+        return out.to(dt)
     if isinstance(layer, AdaIN):
         xf, cm, cv = _instance_norm(xr, unbiased=True)
         sf, sm, sv = _instance_norm(xd, unbiased=True)
-        return ((xf - cm) / torch.sqrt(cv + 1e-5) * torch.sqrt(sv + 1e-5) + sm).to(BF)
+        return ((xf - cm) / torch.sqrt(cv + 1e-5) * torch.sqrt(sv + 1e-5) + sm).to(dt)
     if isinstance(layer, IN):
         both = torch.cat([xr, xd], 3)
         bf, mean, var = _instance_norm(both)
-        normed = ((bf - mean) * torch.rsqrt(var + 1e-5)).to(BF)
+        normed = ((bf - mean) * torch.rsqrt(var + 1e-5)).to(dt)
         dc = layer.down_channel
-        return (conv2d_nhwc(normed, dc.weight, 1, 1).float() + dc.bias.float()).to(BF)
+        return (conv2d_nhwc(normed, dc.weight, 1, 1).float() + dc.bias.float()).to(dt)
     raise NotImplementedError(type(layer))
 
 
@@ -92,14 +138,17 @@ def _crop_cat(fd, fe):
     return torch.cat([fd[:, :fe.shape[1], :fe.shape[2]], fe], 3)
 
 
-def generator_forward_train(g, stem_in, depth):
-    """g: RDFGenerator / DCVGANGenerator (train mode).  stem_in (B, Cs, H, W), depth (B, 1, H, W) fp32 CUDA.
+def generator_forward_train(g, stem_in, depth, dtype=BF):
+    """g: RDFGenerator / DCVGANGenerator (train mode).  stem_in (B, Cs, H, W), depth (B, 1, H, W) fp32 CUDA.  dtype: the activations'
+    dtype, torch.bfloat16 (default) or torch.float32 (the fp32_tc training mode).
     -> (depth_map_1, confidence_map_1, depth_map_2, confidence_map_2, pred_depth), fp32 NCHW, attached to the autograd graph."""
     C.require_cuda(stem_in, depth)
+    if dtype not in (torch.bfloat16, torch.float32):
+        raise ValueError(f"training activations are bf16 or fp32, not {dtype}")
     L = C.ACT_LEAKY02
     # ---- stems (rdf_generator.py:286-292): 3 / 1 input channels, bias, LeakyReLU -- torch
     def stem(x, seq):                                   # fp32 conv (cuDNN's NCHW fp32 kernels), cast BEFORE the layout change (half the bytes)
-        return _nhwc(F.leaky_relu(F.conv2d(x, seq[0].weight, seq[0].bias, padding=1), 0.2).to(BF))
+        return _nhwc(F.leaky_relu(_conv(x, seq[0].weight, seq[0].bias, 1, dtype), 0.2).to(dtype))
     fe1 = {'r': stem(stem_in, g.rgb_branch_en1),
            'd': torch.cat([stem(stem_in, g.depth_branch_en1_rgb), stem(depth, g.depth_branch_en1_depth)], 3)}
     # ---- encoders
