@@ -313,8 +313,8 @@ typedef struct {
     int Hg, Wg;             /* grid of grad_out */
     int Hi, Wi;             /* grid of input */
     int k, stride, pad;     /* k in {1, 3}, stride in {1, 2}, pad = (k - 1) / 2 */
-    rdfc_view grad_out;     /* bf16 NHWC, O channels */
-    rdfc_view input;        /* bf16 NHWC, I channels */
+    rdfc_view grad_out;     /* bf16 NHWC, O channels, O % 8 == 0 */
+    rdfc_view input;        /* bf16 NHWC, I channels, I % 8 == 0 */
 } rdfc_wgrad_desc;
 long long rdfc_conv_wgrad_workspace_floats(const rdfc_wgrad_desc *d);
 int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, float *workspace, void *stream);

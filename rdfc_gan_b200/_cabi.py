@@ -13,7 +13,7 @@ F32, F64, BF16, F16 = 0, 1, 2, 3          # F16: the split [hi | lo] tensors of 
 ACT_NONE, ACT_RELU, ACT_LEAKY02, ACT_TANH, ACT_SIGMOID = range(5)
 PATH_SIMT_F32, PATH_UMMA_BF16, PATH_UMMA_F32X3 = 0, 1, 2
 AFFINITY = {"AS": 0, "ASS": 1, "TC": 2, "TGASS": 3}
-_DT = {torch.float32: F32, torch.float64: F64, torch.bfloat16: BF16}
+_DT = {torch.float32: F32, torch.float64: F64, torch.bfloat16: BF16, torch.float16: F16}
 
 c_int, c_void_p, c_float = ctypes.c_int, ctypes.c_void_p, ctypes.c_float
 

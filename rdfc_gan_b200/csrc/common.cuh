@@ -50,6 +50,18 @@ __device__ __forceinline__ float ldf(const __nv_bfloat16 *p) { return __bfloat16
 __device__ __forceinline__ void stf(float *p, float v) { *p = v; }
 __device__ __forceinline__ void stf(__nv_bfloat16 *p, float v) { *p = __float2bfloat16_rn(v); }
 
+// Split-precision operands are fp16 halves x = hi + lo, and fp16 has a narrow exponent range: a tensor is scaled by the power of two s
+// with amax * s in [1024, 2048) before it is split, so that lo keeps 11 significant bits down to ~3e-5 of the largest element.
+// 1 for an all-zero (or non-finite) tensor.
+__device__ __forceinline__ float pow2_scale(float amax) {
+    if (!(amax > 0.f) || !(amax < 3.0e38f)) return 1.f;
+    int ex;
+    frexpf(amax, &ex);                       // amax = f * 2^ex, f in [0.5, 1)
+    ex = 11 - ex;
+    ex = ex > 100 ? 100 : (ex < -100 ? -100 : ex);
+    return exp2f((float)ex);
+}
+
 __device__ __forceinline__ float apply_act(float v, int act) {
     switch (act) {
         case RDFC_ACT_RELU: return fmaxf(v, 0.f);

@@ -6,8 +6,6 @@
 // NCHW tensor.  Reference layers: encoder_decoder/common.py:29-61, rdf_generator.py:60-102.
 #include <type_traits>
 
-#include <cuda_fp16.h>
-
 #include "common.cuh"
 
 namespace rdfc {
@@ -349,41 +347,6 @@ int conv_simt_forward(const rdfc_conv_desc *d, cudaStream_t st) {
     if (it == RDFC_BF16 && ot == RDFC_BF16) return launch<__nv_bfloat16, __nv_bfloat16>(g, st);
     if (it == RDFC_BF16 && ot == RDFC_F32) return launch<__nv_bfloat16, float>(g, st);
     return fail(RDFC_ERR_UNSUPPORTED, "conv (SIMT): unsupported dtype pair (%d,%d)", it, ot);
-}
-
-// fp32 NHWC view -> dense fp16 [pixel][hi(C) | lo(C)]: hi = fp16(x), lo = fp16(x - hi).  8 channels per thread.
-__global__ void __launch_bounds__(256) split_f32_kernel(const float *__restrict__ x, int C, int stride, __half *__restrict__ out,
-                                                        long long npix) {
-    const int cgs = C >> 3;
-    const long long total = npix * cgs;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const long long p = i / cgs;
-        const int c0 = (int)(i - p * cgs) * 8;
-        const float4 a = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0)), b = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0) + 1);
-        const float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-        uint32_t hi[4], lo[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const __half2 h = __floats2half2_rn(v[2 * q], v[2 * q + 1]);
-            const float2 hf = __half22float2(h);
-            const __half2 l = __floats2half2_rn(v[2 * q] - hf.x, v[2 * q + 1] - hf.y);
-            hi[q] = *reinterpret_cast<const uint32_t *>(&h);
-            lo[q] = *reinterpret_cast<const uint32_t *>(&l);
-        }
-        __half *o = out + p * (2 * C) + c0;
-        *reinterpret_cast<uint4 *>(o) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-        *reinterpret_cast<uint4 *>(o + C) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-    }
-}
-
-int split_f32_forward(const rdfc_view *x, void *out_bf16, long long npix, cudaStream_t st) {
-    RDFC_REQUIRE(x && x->ptr && out_bf16 && x->dtype == RDFC_F32 && !x->nchw && x->C % 8 == 0 && x->pix_stride % 4 == 0 &&
-                     ((uintptr_t)x->ptr % 16) == 0,
-                 "split: 16-byte aligned fp32 NHWC view with C % 8 == 0 expected");
-    const int nblk = (int)min((long long)cdiv(npix * (x->C / 8), 256), (long long)sm_count() * 16);
-    split_f32_kernel<<<nblk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, (__half *)out_bf16, npix);
-    RDFC_CHECK_LAUNCH("split_f32_kernel");
-    return 0;
 }
 
 }  // namespace rdfc

@@ -322,15 +322,6 @@ __global__ void __launch_bounds__(NT) dcn_amax_kernel(AmaxArgs a, unsigned *am) 
     for (int sft = 16; sft > 0; sft >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, sft));
     if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(am + seg, __float_as_uint(m));
 }
-// power of two s with amax * s in [1024, 2048); 1 for an all-zero (or non-finite) tensor
-__device__ __forceinline__ float pow2_scale(float amax) {
-    if (!(amax > 0.f) || !(amax < 3.0e38f)) return 1.f;
-    int ex;
-    frexpf(amax, &ex);                       // amax = f * 2^ex, f in [0.5, 1)
-    ex = 11 - ex;
-    ex = ex > 100 ? 100 : (ex < -100 ? -100 : ex);
-    return exp2f((float)ex);
-}
 __device__ __forceinline__ float scale_cols(const unsigned *am) { return pow2_scale(__uint_as_float(am[0]) * (am[1] ? __uint_as_float(am[1]) : 1.f)); }
 __device__ __forceinline__ float scale_w(const unsigned *am) { return pow2_scale(__uint_as_float(am[2])); }
 __device__ __forceinline__ float scale_g(const unsigned *am) { return pow2_scale(__uint_as_float(am[3])); }

@@ -1,5 +1,5 @@
 // Training-step kernels (SURVEY 8f rank 1): batch-statistics BatchNorm forward / backward fused with the activation and the
-// residual add, and the convolution filter gradient.
+// residual add, and the entry points of the convolution filter gradient (its tcgen05 kernel is in wgrad_umma.cu).
 //
 // Replaces, for conv_bn_relu / convt_bn_relu / torchvision BasicBlock in train() mode (encoder_decoder/common.py:29-61,
 // encoder_decoder/encoder_decoder.py:39-59), what the reference leaves to cuDNN / ATen: nn.BatchNorm2d's batch statistics and
@@ -323,179 +323,6 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(View<T> dout, View<T>
     }
 }
 
-// ---------------------------------------------------------------------------------------------------------------------------
-// Filter gradient.   dW[o][i][ky][kx] = sum over (b, py, px) of  G[b, py, px, o] * I[b, s*py - pad + ky, s*px - pad + kx, i]
-// G = gradient w.r.t. the conv output (grid Hg x Wg, O channels), I = the conv input (grid Hi x Wi, I channels); the transposed
-// convolution's filter gradient is the same sum with the roles of its input and its output gradient exchanged (host side).
-// A GEMM with K = pixels: per CTA a 64 (o) x 64 (i) block of every tap over a chunk of G rows ("split K"), partial results to a
-// workspace, reduced in chunk order by wgrad_reduce_kernel.  Both operands sit pixel-major in shared memory ([pixel][channel],
-// rows padded to 144 bytes against bank conflicts), i.e. "transposed" for the tensor-core fragments: ldmatrix.trans delivers
-// them.  Warp-level mma.sync (m16n8k16, bf16 -> fp32): this first version does not use tcgen05 (DESIGN.md, open items).
-constexpr int WG_OB = 64, WG_IB = 64, WG_ROWP = 72;      // block sizes; smem row pitch in elements (64 channels + 8 pad)
-constexpr int WG_TW = 32;                                  // G pixels per tile row (two K = 16 steps)
-
-__device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t (&r)[4]) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void cp16(uint32_t dst, const void *src, bool ok) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(ok ? 16u : 0u) : "memory");
-}
-
-struct WgradParams {
-    const __nv_bfloat16 *G, *I;
-    int g_stride, i_stride, O, Ich;
-    int B, Hg, Wg, Hi, Wi, k, s, pad;
-    int rows_per_cta;            // G rows (over all images) per CTA
-    int TR;                      // G rows per tile
-    int ksplit;                  // warps that share one (tap, half) by taking K steps round-robin (k = 1 layers)
-    float *partial;              // [chunk][tap][64][64]
-    int nchunk_cta;              // CTAs along the pixel dimension
-};
-
-// warp w: tap = w / (2 * ksplit), half = (w / ksplit) & 1, ks = w % ksplit.  Accumulators: 64 (o) x 32 (i) = 4 x 4 mma tiles.
-__global__ void __launch_bounds__(576) wgrad_kernel(WgradParams P) {
-    extern __shared__ __align__(16) unsigned char wsm[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int ntap = P.k * P.k, nwarps = blockDim.x >> 5;
-    const int tap = warp / (2 * P.ksplit), half = (warp / P.ksplit) & 1, ks = warp % P.ksplit;
-    const int ky = tap / P.k, kx = tap - ky * P.k;
-    const int o0 = blockIdx.y * WG_OB, i0 = blockIdx.z * WG_IB;
-    // tile geometry: TR rows x WG_TW columns of G; the I patch that its taps touch
-    const int TR = P.TR, IR = P.s * (TR - 1) + P.k, IC = P.s * (WG_TW - 1) + P.k;
-    const int g_tile = TR * WG_TW * WG_ROWP * 2, i_tile = IR * IC * WG_ROWP * 2;       // bytes per buffer
-    const uint32_t sG = (uint32_t)__cvta_generic_to_shared(wsm), sI = sG + 2u * (uint32_t)g_tile;
-    const long long total_rows = (long long)P.B * P.Hg;
-    const long long row0 = (long long)blockIdx.x * P.rows_per_cta;
-    const long long row1 = row0 + P.rows_per_cta < total_rows ? row0 + P.rows_per_cta : total_rows;
-    const int xtiles = (P.Wg + WG_TW - 1) / WG_TW;
-
-    float acc[4][4][4];
-#pragma unroll
-    for (int a = 0; a < 4; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) acc[a][b][c] = 0.f;
-
-    // tiles of this CTA: (row group, x tile); a row group never crosses an image
-    // enumerate lazily: state (row, xt)
-    auto issue_tile = [&](long long row, int xt, int buf) {
-        const int b = (int)(row / P.Hg), gy0 = (int)(row - (long long)b * P.Hg), gx0 = xt * WG_TW;
-        long long nr = row1 - row;
-        if (nr > P.Hg - gy0) nr = P.Hg - gy0;
-        if (nr > TR) nr = TR;
-        // G tile: TR x WG_TW pixels x 64 channels (8 chunks of 16 bytes per pixel)
-        for (int e = threadIdx.x; e < TR * WG_TW * 8; e += blockDim.x) {
-            const int ch = e & 7, px = (e >> 3) % WG_TW, r = (e >> 3) / WG_TW;
-            const int gy = gy0 + r, gx = gx0 + px, c = o0 + ch * 8;
-            const bool ok = r < nr && gx < P.Wg && c < P.O;
-            const __nv_bfloat16 *src = ok ? P.G + (((long long)b * P.Hg + gy) * P.Wg + gx) * P.g_stride + c : P.G;
-            cp16(sG + (uint32_t)buf * g_tile + (uint32_t)((r * WG_TW + px) * WG_ROWP + ch * 8) * 2u, src, ok);
-        }
-        const int iy0 = P.s * gy0 - P.pad, ix0 = P.s * gx0 - P.pad;
-        for (int e = threadIdx.x; e < IR * IC * 8; e += blockDim.x) {
-            const int ch = e & 7, px = (e >> 3) % IC, r = (e >> 3) / IC;
-            const int iy = iy0 + r, ix = ix0 + px, c = i0 + ch * 8;
-            const bool ok = iy >= 0 && iy < P.Hi && ix >= 0 && ix < P.Wi && c < P.Ich && r < P.s * ((int)nr - 1) + P.k;
-            const __nv_bfloat16 *src = ok ? P.I + (((long long)b * P.Hi + iy) * P.Wi + ix) * P.i_stride + c : P.I;
-            cp16(sI + (uint32_t)buf * i_tile + (uint32_t)((r * IC + px) * WG_ROWP + ch * 8) * 2u, src, ok);
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        return (int)nr;
-    };
-
-    long long row = row0;
-    int xt = 0, buf = 0;
-    int nr_cur = 0;
-    if (row < row1) nr_cur = issue_tile(row, 0, 0);
-    // lane-constant parts of the ldmatrix row addresses
-    const int lrow = lane & 7, lmat = lane >> 3;
-    while (row < row1) {
-        // next tile
-        long long nrow = row;
-        int nxt = xt + 1;
-        if (nxt == xtiles) { nxt = 0; nrow = row + nr_cur; }
-        int nr_next = 0;
-        if (nrow < row1) nr_next = issue_tile(nrow, nxt, buf ^ 1);
-        else asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        __syncthreads();
-        if (tap < ntap) {
-            const uint32_t gb = sG + (uint32_t)buf * g_tile, ib = sI + (uint32_t)buf * i_tile;
-            const int nsteps = TR * (WG_TW / 16);
-            for (int st = ks; st < nsteps; st += P.ksplit) {
-                const int r = st / (WG_TW / 16), x16 = (st - r * (WG_TW / 16)) * 16;
-                // A fragments (o x pixels): matrices (k0, m0), (k0, m0 + 8), (k0 + 8, m0), (k0 + 8, m0 + 8) of S[k = pixel][m = o]
-                uint32_t afr[4][4];
-#pragma unroll
-                for (int mb = 0; mb < 4; ++mb) {
-                    const int kk = x16 + lrow + 8 * (lmat >> 1), mm = mb * 16 + 8 * (lmat & 1);
-                    ldsm_x4_t(gb + (uint32_t)((r * WG_TW + kk) * WG_ROWP + mm) * 2u, afr[mb]);
-                }
-                // B fragments (pixels x i): matrices (k0, n0), (k0 + 8, n0), (k0, n0 + 8), (k0 + 8, n0 + 8) of S'[k = pixel][n = i];
-                // the pixel of K index kk under this tap is (s * r + ky, s * (x16 + kk) + kx) of the I patch
-                uint32_t bfr[2][4];
-#pragma unroll
-                for (int nb = 0; nb < 2; ++nb) {
-                    const int kk = lrow + 8 * (lmat & 1), nn = half * 32 + nb * 16 + 8 * (lmat >> 1);
-                    const int pr = P.s * r + ky, pc = P.s * (x16 + kk) + kx;
-                    ldsm_x4_t(ib + (uint32_t)((pr * IC + pc) * WG_ROWP + nn) * 2u, bfr[nb]);
-                }
-#pragma unroll
-                for (int mb = 0; mb < 4; ++mb)
-#pragma unroll
-                    for (int nb = 0; nb < 2; ++nb) {
-                        mma16816(acc[mb][2 * nb], afr[mb], bfr[nb][0], bfr[nb][1]);
-                        mma16816(acc[mb][2 * nb + 1], afr[mb], bfr[nb][2], bfr[nb][3]);
-                    }
-            }
-        }
-        __syncthreads();
-        row = nrow; xt = nxt; buf ^= 1; nr_cur = nr_next;
-    }
-    // partial results: chunk id = (CTA along pixels) * ksplit + ks
-    if (tap < ntap) {
-        const int g = lane >> 2, t = lane & 3;
-        const long long chunk = (long long)blockIdx.x * P.ksplit + ks;
-        const long long nchunks = (long long)P.nchunk_cta * P.ksplit;
-        const int nob = gridDim.y, nib = gridDim.z;
-        float *base = P.partial + ((((long long)(blockIdx.y * nib + blockIdx.z) * nchunks + chunk) * ntap + tap) * WG_OB) * WG_IB;
-        (void)nob;
-#pragma unroll
-        for (int mb = 0; mb < 4; ++mb)
-#pragma unroll
-            for (int nb = 0; nb < 4; ++nb) {
-                const int m = mb * 16 + g, n = half * 32 + nb * 8 + 2 * t;
-                *reinterpret_cast<float2 *>(base + m * WG_IB + n) = make_float2(acc[mb][nb][0], acc[mb][nb][1]);
-                *reinterpret_cast<float2 *>(base + (m + 8) * WG_IB + n) = make_float2(acc[mb][nb][2], acc[mb][nb][3]);
-            }
-    }
-    (void)nwarps;
-}
-
-// dW[o][i][tap] (torch layout (O, I, kh, kw)) = sum over chunks, in chunk order
-__global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float *__restrict__ partial, float *__restrict__ dw, int O, int Ich, int ntap,
-                                                           int nchunks, int nib) {
-    const long long total = (long long)O * Ich * ntap;
-    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
-        // consecutive threads walk i fastest inside a 64 x 64 block for coalesced partial reads
-        const int i = (int)(e % Ich);
-        const int tap = (int)((e / Ich) % ntap);
-        const int o = (int)(e / ((long long)Ich * ntap));
-        const int ob = o / WG_OB, ib = i / WG_IB;
-        const float *src = partial + (((long long)(ob * nib + ib) * nchunks * ntap + tap) * WG_OB + (o % WG_OB)) * WG_IB + (i % WG_IB);
-        const long long cstride = (long long)ntap * WG_OB * WG_IB;
-        float s = 0.f;
-        for (int c = 0; c < nchunks; ++c) s += __ldg(src + (long long)c * cstride);
-        dw[((long long)o * Ich + i) * ntap + tap] = s;
-    }
-}
-
 }  // namespace
 }  // namespace rdfc
 
@@ -612,76 +439,30 @@ extern "C" int rdfc_bn_act_backward(const rdfc_view *dout, const rdfc_view *out,
     return bn_act_backward<__nv_bfloat16>(dout, out, y, mean, rstd, gamma, act, dy, dres, workspace, sum_dz, sum_dz_xhat, npix, (cudaStream_t)stream);
 }
 
-// geometry shared by the workspace query and the launch
-struct WgGeom { int nob, nib, nchunk_cta, rows_per_cta, TR, ksplit, nwarps; size_t smem; long long ws_floats; };
-static int wgrad_geom(const rdfc_wgrad_desc *d, WgGeom *g) {
+// argument checks shared by the workspace query and the launch
+static int check_wgrad(const rdfc_wgrad_desc *d) {
     RDFC_REQUIRE(d && (d->k == 1 || d->k == 3) && (d->stride == 1 || d->stride == 2) && d->pad == (d->k - 1) / 2,
                  "wgrad: 3x3 / 1x1 kernels, stride 1 / 2, padding (k-1)/2");
     RDFC_REQUIRE(d->B > 0 && d->Hg > 0 && d->Wg > 0 && d->Hi > 0 && d->Wi > 0, "wgrad: empty dimension");
     RDFC_REQUIRE(d->Hg == (d->Hi + 2 * d->pad - d->k) / d->stride + 1 && d->Wg == (d->Wi + 2 * d->pad - d->k) / d->stride + 1,
                  "wgrad: gradient grid (%d,%d) does not match the input grid (%d,%d)", d->Hg, d->Wg, d->Hi, d->Wi);
-    const int O = d->grad_out.C, I = d->input.C;
-    RDFC_REQUIRE(O % 8 == 0 && I % 8 == 0, "wgrad: channel counts must be multiples of 8");
-    g->nob = cdiv(O, WG_OB); g->nib = cdiv(I, WG_IB);
-    g->ksplit = d->k == 1 ? 8 : 1;
-    g->nwarps = d->k * d->k * 2 * g->ksplit;             // 18 (3x3) or 16 (1x1)
-    g->TR = d->stride == 1 ? 4 : 2;
-    const int IR = d->stride * (g->TR - 1) + d->k, IC = d->stride * (WG_TW - 1) + d->k;
-    g->smem = 2 * ((size_t)g->TR * WG_TW + (size_t)IR * IC) * WG_ROWP * 2;
-    RDFC_REQUIRE(g->smem <= 220 * 1024, "wgrad: tile does not fit shared memory");
-    const long long rows = (long long)d->B * d->Hg;
-    long long want = (long long)sm_count() * 2 / ((long long)g->nob * g->nib);     // ~2 CTAs' worth of work per SM in total
-    if (want < 1) want = 1;
-    long long rpc = (rows + want - 1) / want;
-    if (rpc < g->TR) rpc = g->TR;
-    g->rows_per_cta = (int)rpc;
-    g->nchunk_cta = (int)((rows + rpc - 1) / rpc);
-    g->ws_floats = (long long)g->nob * g->nib * g->nchunk_cta * g->ksplit * d->k * d->k * WG_OB * WG_IB;
+    RDFC_REQUIRE(d->grad_out.C % 8 == 0 && d->input.C % 8 == 0, "wgrad: channel counts must be multiples of 8");
     return 0;
 }
 
 namespace rdfc {
-bool wgrad_umma_ok(const rdfc_wgrad_desc *d);                       // wgrad_umma.cu: 3x3 filter gradients on tcgen05
-long long wgrad_umma_workspace_floats(const rdfc_wgrad_desc *d);
+long long wgrad_umma_workspace_floats(const rdfc_wgrad_desc *d);    // wgrad_umma.cu: the filter gradient on tcgen05
 int wgrad_umma(const rdfc_wgrad_desc *d, float *grad_weight, float *workspace, cudaStream_t st);
 }  // namespace rdfc
 
 extern "C" long long rdfc_conv_wgrad_workspace_floats(const rdfc_wgrad_desc *d) {
-    WgGeom g;
-    if (wgrad_geom(d, &g) != 0) return -1;
-    if (wgrad_umma_ok(d)) {                                         // either path may serve the call (knob): size for both
-        const long long u = wgrad_umma_workspace_floats(d);
-        return u > g.ws_floats ? u : g.ws_floats;
-    }
-    return wgrad_geom(d, &g) == 0 ? g.ws_floats : -1;
+    return check_wgrad(d) == 0 ? wgrad_umma_workspace_floats(d) : -1;
 }
 
 extern "C" int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, float *workspace, void *stream) {
-    WgGeom g;
-    if (int rc = wgrad_geom(d, &g)) return rc;
+    if (int rc = check_wgrad(d)) return rc;
     RDFC_REQUIRE(grad_weight && workspace, "wgrad: NULL output / workspace");
     if (int rc = check_view(&d->grad_out, d->grad_out.C, "wgrad grad_out", RDFC_BF16)) return rc;
     if (int rc = check_view(&d->input, d->input.C, "wgrad input", RDFC_BF16)) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (wgrad_umma_ok(d)) return wgrad_umma(d, grad_weight, workspace, st);
-    WgradParams P{};
-    P.G = (const __nv_bfloat16 *)d->grad_out.ptr; P.I = (const __nv_bfloat16 *)d->input.ptr;
-    P.g_stride = d->grad_out.pix_stride; P.i_stride = d->input.pix_stride; P.O = d->grad_out.C; P.Ich = d->input.C;
-    P.B = d->B; P.Hg = d->Hg; P.Wg = d->Wg; P.Hi = d->Hi; P.Wi = d->Wi; P.k = d->k; P.s = d->stride; P.pad = d->pad;
-    P.rows_per_cta = g.rows_per_cta; P.TR = g.TR; P.ksplit = g.ksplit; P.partial = workspace; P.nchunk_cta = g.nchunk_cta;
-    static bool attr[64] = {};
-    int dev = 0;
-    RDFC_CUDA(cudaGetDevice(&dev));
-    if (!attr[dev & 63]) {
-        RDFC_CUDA(cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-        attr[dev & 63] = true;
-    }
-    wgrad_kernel<<<dim3(g.nchunk_cta, g.nob, g.nib), g.nwarps * 32, g.smem, st>>>(P);
-    RDFC_CHECK_LAUNCH("wgrad_kernel");
-    const int ntap = d->k * d->k;
-    const long long total = (long long)P.O * P.Ich * ntap;
-    const int nblk = (int)min((long long)cdiv(total, 256), (long long)sm_count() * 8);
-    wgrad_reduce_kernel<<<nblk, 256, 0, st>>>(workspace, grad_weight, P.O, P.Ich, ntap, g.nchunk_cta * g.ksplit, g.nib);
-    RDFC_CHECK_LAUNCH("wgrad_reduce_kernel");
-    return 0;
+    return wgrad_umma(d, grad_weight, workspace, (cudaStream_t)stream);
 }

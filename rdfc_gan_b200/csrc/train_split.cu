@@ -5,18 +5,18 @@
 //   rdfc_conv_wgrad_split   the filter gradient of wgrad_umma.cu on fp16 halves, run for the three products g_hi.x_hi, g_hi.x_lo,
 //                           g_lo.x_hi into consecutive chunk ranges of one workspace, then ONE reduction in a fixed order that also
 //                           applies 1 / (s_g s_x)  (bit-reproducible)
-// (the conv forward / data gradient on an already split input is rdfc_conv_forward_split, conv.cu.)
+// (the conv forward / data gradient on an already split input is rdfc_conv_forward_split, conv.cu.)  The split kernel also serves,
+// unscaled, the fp32 inputs of the inference path's RDFC_PATH_UMMA_F32X3 convs and fp32 heads (split_f32_forward).
 //
 // Why the scaling: fp16 keeps 11 significant bits down to 6.1e-5 only, and the training step's gradients start near 1e-5 (the
 // reference's image_loss_weight = mask / mask.sum()).  Scaled so that the largest magnitude lies in [1024, 2048), the low half keeps
-// 11 bits down to ~3e-5 of the largest element -- the scheme of the DCN path (dcn.cu, pow2_scale).  The factor never leaves the
+// 11 bits down to ~3e-5 of the largest element -- the scheme of the DCN path (common.cuh, pow2_scale).  The factor never leaves the
 // device: no host synchronisation per conv.
 #include <cuda_fp16.h>
 
 #include "common.cuh"
 
 namespace rdfc {
-bool wgrad_umma_ok(const rdfc_wgrad_desc *d);
 long long wgrad_umma_workspace_floats(const rdfc_wgrad_desc *d);
 int wgrad_umma_partials(const rdfc_wgrad_desc *d, float *workspace, int fp16, cudaStream_t st, int *nchunk);
 
@@ -37,27 +37,23 @@ __global__ void __launch_bounds__(256) split_amax_kernel(const float *__restrict
     if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(am, __float_as_uint(m));
 }
 
-// power of two s with amax * s in [1024, 2048); 1 for an all-zero (or non-finite) tensor (dcn.cu's pow2_scale)
-__device__ __forceinline__ float pow2_scale(float amax) {
-    if (!(amax > 0.f) || !(amax < 3.0e38f)) return 1.f;
-    int ex;
-    frexpf(amax, &ex);
-    ex = 11 - ex;
-    ex = ex > 100 ? 100 : (ex < -100 ? -100 : ex);
-    return exp2f((float)ex);
-}
-
 // fp32 NHWC view -> fp16 [pixel][hi(C) | lo(C)] of s * x, hi = fp16(s x), lo = fp16(s x - hi).  8 channels per thread.
-__global__ void __launch_bounds__(256) split_scaled_kernel(const float *__restrict__ x, int C, int stride, __half *__restrict__ out, int out_stride,
-                                                           long long npix, const unsigned *__restrict__ am) {
-    const float s = pow2_scale(__uint_as_float(__ldg(am)));
+// kScaled: s = pow2_scale(max |x|), read from `am`; otherwise s = 1 -- no load of `am`, no multiply (the inference path's split).
+template <bool kScaled>
+__global__ void __launch_bounds__(256) split_kernel(const float *__restrict__ x, int C, int stride, __half *__restrict__ out, int out_stride,
+                                                    long long npix, const unsigned *__restrict__ am) {
+    float s = 1.f;
+    if (kScaled) s = pow2_scale(__uint_as_float(__ldg(am)));
     const int cgs = C >> 3;
     const long long total = npix * cgs;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long p = i / cgs;
         const int c0 = (int)(i - p * cgs) * 8;
         const float4 a = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0)), b = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0) + 1);
-        const float v[8] = {a.x * s, a.y * s, a.z * s, a.w * s, b.x * s, b.y * s, b.z * s, b.w * s};
+        float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        if (kScaled)
+#pragma unroll
+            for (int q = 0; q < 8; ++q) v[q] *= s;
         uint32_t hi[4], lo[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
@@ -104,6 +100,24 @@ static int check_split_view(const rdfc_view *v, const char *what) {
     return 0;
 }
 
+template <bool kScaled>
+static int split_launch(const rdfc_view *x, __half *out, int out_stride, long long npix, const unsigned *am, cudaStream_t st) {
+    const int nblk = (int)min((long long)cdiv(npix * (x->C / 8), 256), (long long)sm_count() * 16);
+    split_kernel<kScaled><<<nblk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, out, out_stride, npix, am);
+    RDFC_CHECK_LAUNCH("split_kernel");
+    return 0;
+}
+
+namespace rdfc {
+// the unscaled split into a dense [hi | lo] workspace: the fp32 input of the RDFC_PATH_UMMA_F32X3 conv and of the fp32 heads (conv.cu)
+int split_f32_forward(const rdfc_view *x, void *out, long long npix, cudaStream_t st) {
+    RDFC_REQUIRE(x && x->ptr && out && x->dtype == RDFC_F32 && !x->nchw && x->C % 8 == 0 && x->pix_stride % 4 == 0 &&
+                     ((uintptr_t)x->ptr % 16) == 0,
+                 "split: 16-byte aligned fp32 NHWC view with C % 8 == 0 expected");
+    return split_launch<false>(x, (__half *)out, 2 * x->C, npix, nullptr, st);
+}
+}  // namespace rdfc
+
 extern "C" int rdfc_split_scaled(const rdfc_view *x, long long npix, const rdfc_view *out, float *factor, void *stream) {
     RDFC_REQUIRE(x && out && factor && npix > 0, "split: bad argument");
     RDFC_REQUIRE(x->ptr && x->dtype == RDFC_F32 && !x->nchw, "split: the source must be an fp32 NHWC view");
@@ -117,10 +131,7 @@ extern "C" int rdfc_split_scaled(const rdfc_view *x, long long npix, const rdfc_
     const int ablk = (int)min((long long)cdiv(npix * (x->C / 4), 256 * 8), (long long)sm_count() * 4);
     split_amax_kernel<<<ablk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, npix, (unsigned *)factor);
     RDFC_CHECK_LAUNCH("split_amax_kernel");
-    const int nblk = (int)min((long long)cdiv(npix * (x->C / 8), 256), (long long)sm_count() * 16);
-    split_scaled_kernel<<<nblk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, (__half *)out->ptr, out->pix_stride, npix,
-                                              (const unsigned *)factor);
-    RDFC_CHECK_LAUNCH("split_scaled_kernel");
+    if (int rc = split_launch<true>(x, (__half *)out->ptr, out->pix_stride, npix, (const unsigned *)factor, st)) return rc;
     split_factor_kernel<<<1, 1, 0, st>>>(factor);
     RDFC_CHECK_LAUNCH("split_factor_kernel");
     return 0;
@@ -163,7 +174,6 @@ extern "C" int rdfc_conv_wgrad_split(const rdfc_wgrad_desc *d, const float *inv_
                  "wgrad (split): the workspace must be 16-byte aligned");
     rdfc_wgrad_desc parts[3];
     for (int t = 0; t < 3; ++t) parts[t] = split_part(d, t);
-    RDFC_REQUIRE(wgrad_umma_ok(&parts[0]), "wgrad (split): the tcgen05 filter-gradient kernel is unavailable (driver entry point or knob)");
     cudaStream_t st = (cudaStream_t)stream;
     const int O = parts[0].grad_out.C, I = parts[0].input.C, ntap = d->k * d->k;
     const long long blk = (long long)ntap * O * I;

@@ -232,12 +232,6 @@ TmapEncodeFn tmap_encoder() {
 
 }  // namespace
 
-// the tcgen05 path takes every 3x3 / 1x1 filter gradient whose channel counts are multiples of 16 (RDFC_WGRAD_UMMA = 0 keeps the mma.sync kernel)
-bool wgrad_umma_ok(const rdfc_wgrad_desc *d) {
-    return (d->k == 3 || d->k == 1) && d->pad == (d->k - 1) / 2 && (d->stride == 1 || d->stride == 2) && d->grad_out.C % 16 == 0 && d->grad_out.C >= 16 && d->input.C % 8 == 0 &&
-           d->input.pix_stride % 8 == 0 && d->grad_out.pix_stride % 8 == 0 && knob("RDFC_WGRAD_UMMA", 1) != 0 && tmap_encoder() != nullptr;
-}
-
 struct WuGeom { WuParams P; int nchunk; size_t smem; long long ws_floats; };
 
 static int wgrad_umma_geom(const rdfc_wgrad_desc *d, WuGeom *g) {
@@ -250,7 +244,7 @@ static int wgrad_umma_geom(const rdfc_wgrad_desc *d, WuGeom *g) {
     P.TR = (P.s == 1 || d->k == 1) ? (P.TW == 32 ? 4 : 8) : (P.TW == 32 ? 2 : 4);
     if (P.TR > P.Hg) P.TR = P.Hg;
     P.nob = cdiv(P.O, 96);
-    P.NB = cdiv(cdiv(P.O, P.nob), 16) * 16;
+    P.NB = cdiv(cdiv(P.O, P.nob), 16) * 16;          // the MMA's N; channels past O (O % 16 == 8) are TMA zero fill, masked in the epilogue
     P.nib = cdiv(P.Ich, 64);
     P.ncol = (uint32_t)P.NB;
     P.g_boxes = P.NB > 64 ? 2 : 1;
@@ -314,6 +308,7 @@ int wgrad_umma_partials(const rdfc_wgrad_desc *d, float *workspace, int fp16, cu
     P.partial = workspace;
     P.fp16 = fp16;
     RDFC_REQUIRE(((uintptr_t)d->grad_out.ptr % 16) == 0 && ((uintptr_t)d->input.ptr % 16) == 0, "wgrad (tcgen05): 16-byte aligned tensors");
+    RDFC_REQUIRE(tmap_encoder() != nullptr, "wgrad (tcgen05): the CUDA driver does not provide cuTensorMapEncodeTiled");
     {
         const cuuint64_t gdim[4] = {(cuuint64_t)P.O, (cuuint64_t)d->Wg, (cuuint64_t)d->Hg, (cuuint64_t)d->B};
         const cuuint64_t ps = (cuuint64_t)d->grad_out.pix_stride * 2;

@@ -4,8 +4,8 @@ What the reference gets from autograd + cuDNN inside ``conv_bn_relu`` / ``convt_
 train() mode (encoder_decoder/common.py:29-61, encoder_decoder/encoder_decoder.py:39-59) becomes two autograd Functions over
 bf16 NHWC tensors:
 
-* ``conv2d_nhwc``   forward = ``rdfc_conv_forward`` (tcgen05 implicit GEMM); data gradient = the same kernel with a transformed
-                    filter (flipped / transposed-conv form, conv_grad.py); filter gradient = ``rdfc_conv_wgrad``.
+* ``conv2d_nhwc``   forward = ``rdfc_conv_forward`` (tcgen05 implicit GEMM); data gradient = the same kernel in one of the conv
+                    forms, with a transformed filter (_Conv2dNHWC.backward); filter gradient = ``rdfc_conv_wgrad``.
 * ``bn_act``        BatchNorm2d with BATCH statistics (+ running-stat update) fused with the residual add and the
                     (Leaky)ReLU: ``rdfc_bn_stats`` + ``rdfc_affine_act_forward``; backward = ``rdfc_bn_act_backward``.
 
@@ -24,28 +24,7 @@ import ctypes
 import torch
 
 from . import _cabi as C
-from .conv_grad import pack_filter
 from .engine import pack_weight
-
-
-def _conv_umma(x, w_oihw, k, stride, transposed, out_hw):
-    """x (B,H,W,Cin) bf16 contiguous; w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) bf16, no bias / activation."""
-    B, H, W, Cin = x.shape
-    O = w_oihw.shape[0]
-    if Cin % 32 or O % 8 or w_oihw.shape[1] != Cin:
-        raise RuntimeError(f"tensor-core conv needs Cin % 32 == 0 and Cout % 8 == 0, got {Cin} -> {O}")
-    out = torch.empty((B, out_hw[0], out_hw[1], O), dtype=torch.bfloat16, device=x.device)
-    packed = pack_filter(w_oihw)
-    d = C.ConvDesc()
-    d.B, d.Hi, d.Wi, d.Ho, d.Wo = B, H, W, out_hw[0], out_hw[1]
-    d.kh = d.kw = k
-    d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, int(transposed), C.ACT_NONE
-    d.path = C.PATH_UMMA_BF16
-    d.inp, d.in2, d.out, d.residual = C.view(x), C.view(None), C.view(out), C.view(None)
-    d.weight, d.scale, d.shift = packed.data_ptr(), None, None
-    with torch.cuda.device(x.device):
-        C.check(C.lib.rdfc_conv_forward(ctypes.byref(d), C.stream_ptr(x.device)))
-    return out
 
 
 def _dense(t):
@@ -54,24 +33,86 @@ def _dense(t):
     return t if C.nhwc_viewable(t) else t.contiguous()
 
 
-def _wgrad(grad_out, inp, k, stride):
-    """sum_p grad_out[p, o] * inp[stride * p - pad + tap, i] -> (O, I, k, k) fp32."""
+def _pow2_factor(t):
+    """The power of two s with max|t| * s in [1024, 2048) (1 for an all-zero or non-finite tensor), as rdfc_split_scaled chooses
+    it, computed on the device: a 1-element fp32 tensor."""
+    amax = t.detach().abs().amax().float().reshape(1)
+    _, e = torch.frexp(amax)
+    s = torch.exp2((11 - e).clamp(-100, 100).float())
+    return torch.where((amax > 0) & torch.isfinite(amax), s, torch.ones_like(s))
+
+
+def _split(t):
+    """fp32 NHWC tensor (or channel slice) -> (fp16 (B, H, W, 2C) = [hi | lo] of s * t, s as a 1-element device tensor)."""
+    B, H, W, Cc = t.shape
+    xs = torch.empty((B, H, W, 2 * Cc), dtype=torch.float16, device=t.device)
+    s = torch.empty(1, dtype=torch.float32, device=t.device)
+    vx, vo = C.view(t), C.view(xs)
+    with torch.cuda.device(t.device):
+        C.check(C.lib.rdfc_split_scaled(ctypes.byref(vx), B * H * W, ctypes.byref(vo), C.ptr(s), C.stream_ptr(t.device)))
+    return xs, s
+
+
+def _operand(t):
+    """An activation as the contractions read it: (t, None) for bf16; for fp32 (the fp32_tc mode) its split and factor, _split(t)."""
+    return _split(t) if t.dtype == torch.float32 else (t, None)
+
+
+def _conv(x, sx, w_oihw, k, stride, transposed, out_hw):
+    """(x, sx) = _operand(input); w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) = conv(input, w), no bias / activation: bf16 from a bf16
+    input, fp32 from a split one (x_hi W_hi + x_hi W_lo + x_lo W_hi of the scaled operands, the inverse scales in the epilogue)."""
+    B, H, W, Cx = x.shape
+    Cin, O = (Cx if sx is None else Cx // 2), w_oihw.shape[0]
+    if Cin % 32 or O % 8 or w_oihw.shape[1] != Cin:
+        raise RuntimeError(f"tensor-core conv needs Cin % 32 == 0 and Cout % 8 == 0, got {Cin} -> {O}")
+    w = w_oihw.detach().float()
+    d = C.ConvDesc()
+    d.B, d.Hi, d.Wi, d.Ho, d.Wo = B, H, W, out_hw[0], out_hw[1]
+    d.kh = d.kw = k
+    d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, int(transposed), C.ACT_NONE
+    if sx is None:
+        packed, inv = pack_weight(w, umma=True), None
+        d.path, fn, dtype = C.PATH_UMMA_BF16, C.lib.rdfc_conv_forward, torch.bfloat16
+    else:
+        sw = _pow2_factor(w)
+        packed = pack_weight(w * sw, umma=True, x3=True)                   # [W_hi ; W_lo ; W_hi] of the scaled filter
+        inv = (1.0 / (sx * sw)).expand((O + 15) // 16 * 16).contiguous()   # exact: powers of two
+        d.path, fn, dtype = C.PATH_UMMA_F32X3, C.lib.rdfc_conv_forward_split, torch.float32
+    out = torch.empty((B, out_hw[0], out_hw[1], O), dtype=dtype, device=x.device)
+    d.inp, d.in2, d.out, d.residual = C.view(x), C.view(None), C.view(out), C.view(None)
+    d.weight, d.scale, d.shift = packed.data_ptr(), None if inv is None else inv.data_ptr(), None
+    with torch.cuda.device(x.device):
+        C.check(fn(ctypes.byref(d), C.stream_ptr(x.device)))
+    return out
+
+
+def _wgrad(grad_out, inp, k, stride, sg=None, sx=None):
+    """sum_p grad_out[p, o] * inp[stride * p - pad + tap, i] -> (O, I, k, k) fp32.  bf16 operands, or split ones with their factors
+    ((grad_out, sg), (inp, sx) from _split: the three products reduced once, the inverse scales applied there)."""
     B, Hg, Wg, O = grad_out.shape
     _, Hi, Wi, I = inp.shape
+    if sx is not None:
+        O, I = O // 2, I // 2
     d = C.WgradDesc()
     d.B, d.Hg, d.Wg, d.Hi, d.Wi, d.k, d.stride, d.pad = B, Hg, Wg, Hi, Wi, k, stride, (k - 1) // 2
     d.grad_out, d.input = C.view(grad_out), C.view(inp)
-    n = C.lib.rdfc_conv_wgrad_workspace_floats(ctypes.byref(d))
+    n = (C.lib.rdfc_conv_wgrad_workspace_floats if sx is None else C.lib.rdfc_conv_wgrad_split_workspace_floats)(ctypes.byref(d))
     if n < 0:
         raise RuntimeError(C.lib.rdfc_last_error().decode("utf-8", "replace"))
     ws = torch.empty(n, dtype=torch.float32, device=inp.device)
     gw = torch.empty((O, I, k, k), dtype=torch.float32, device=inp.device)
     with torch.cuda.device(inp.device):
-        C.check(C.lib.rdfc_conv_wgrad(ctypes.byref(d), C.ptr(gw), C.ptr(ws), C.stream_ptr(inp.device)))
+        if sx is None:
+            C.check(C.lib.rdfc_conv_wgrad(ctypes.byref(d), C.ptr(gw), C.ptr(ws), C.stream_ptr(inp.device)))
+        else:
+            inv = 1.0 / (sg * sx)
+            C.check(C.lib.rdfc_conv_wgrad_split(ctypes.byref(d), C.ptr(inv), C.ptr(gw), C.ptr(ws), C.stream_ptr(inp.device)))
     return gw
 
 
 class _Conv2dNHWC(torch.autograd.Function):
+    """The conv forms and their data-gradient transforms; the arithmetic follows the input's dtype (_operand).  In the fp32_tc mode the
+    split input (as many bytes as the fp32 input) is kept for the filter gradient instead of the input itself."""
     @staticmethod
     def forward(ctx, x, weight, k, stride, transposed):
         C.require_cuda(x, weight)
@@ -84,155 +125,38 @@ class _Conv2dNHWC(torch.autograd.Function):
             p = (k - 1) // 2
             out_hw = ((H + 2 * p - k) // stride + 1, (W + 2 * p - k) // stride + 1)
             w_oihw = weight.detach()
-        ctx.save_for_backward(x, weight)
+        x, sx = _operand(x)
+        ctx.save_for_backward(x, sx, weight)
         ctx.cfg = (k, stride, transposed)
-        return _conv_umma(x, w_oihw, k, stride, transposed, out_hw)
+        return _conv(x, sx, w_oihw, k, stride, transposed, out_hw)
 
     @staticmethod
     def backward(ctx, gy):
-        x, weight = ctx.saved_tensors
+        x, sx, weight = ctx.saved_tensors
         k, stride, transposed = ctx.cfg
-        gy = _dense(gy)
-        B, H, W, Cin = x.shape
+        g, sg = _operand(_dense(gy))
+        B, H, W = x.shape[:3]
         w = weight.detach()
         gx = gw = None
         if ctx.needs_input_grad[0]:
             if transposed:                  # dgrad of the transposed conv = the stride-2 conv with the SAME filter (O = Cin, I = Cout)
-                gx = _conv_umma(gy, w, 3, 2, False, (H, W))
+                gx = _conv(g, sg, w, 3, 2, False, (H, W))
             elif k == 3 and stride == 1:    # flipped filter, (Cout, Cin) swapped
-                gx = _conv_umma(gy, w.flip(2, 3).permute(1, 0, 2, 3), 3, 1, False, (H, W))
+                gx = _conv(g, sg, w.flip(2, 3).permute(1, 0, 2, 3), 3, 1, False, (H, W))
             elif k == 3:                    # stride 2: the transposed conv with the same filter, cropped to the input size
-                gx = _conv_umma(gy, w.permute(1, 0, 2, 3), 3, 2, True, (H, W))
+                gx = _conv(g, sg, w.permute(1, 0, 2, 3), 3, 2, True, (H, W))
             else:                           # 1x1: W^T per pixel; stride 2 scatters onto the even grid
-                t = _conv_umma(gy, w.permute(1, 0, 2, 3), 1, 1, False, tuple(gy.shape[1:3]))
+                t = _conv(g, sg, w.permute(1, 0, 2, 3), 1, 1, False, tuple(gy.shape[1:3]))
                 if stride == 1:
                     gx = t
                 else:
-                    gx = torch.zeros_like(x)
+                    gx = t.new_zeros((B, H, W, t.shape[3]))
                     gx[:, ::2, ::2] = t
         if ctx.needs_input_grad[1]:
             if transposed:                  # roles exchanged: "gradient" = the layer's input, "input" = d(output), stride-2 form
-                gw = _wgrad(x, gy, 3, 2)                       # (Cin, Cout, 3, 3) = ConvTranspose2d's weight layout
+                gw = _wgrad(x, g, 3, 2, sx, sg)                # (Cin, Cout, 3, 3) = ConvTranspose2d's weight layout
             else:
-                gw = _wgrad(gy, x, k, stride)                  # (Cout, Cin, k, k)
-            gw = gw.to(weight.dtype)
-        return gx, gw, None, None, None
-
-
-# ---- fp32_tc: split operands --------------------------------------------------------------------------------------------
-def _pow2_factor(t):
-    """The power of two s with max|t| * s in [1024, 2048) (1 for an all-zero or non-finite tensor), as rdfc_split_scaled chooses
-    it, computed on the device: a 1-element fp32 tensor."""
-    amax = t.detach().abs().amax().float().reshape(1)
-    _, e = torch.frexp(amax)
-    s = torch.exp2((11 - e).clamp(-100, 100).float())
-    return torch.where((amax > 0) & torch.isfinite(amax), s, torch.ones_like(s))
-
-
-def _f16_view(t):
-    """View of a dense (B, H, W, 2C) fp16 split tensor [hi | lo]."""
-    return C.View(t.data_ptr(), C.F16, t.shape[3], t.shape[3], 0)
-
-
-def _split(t):
-    """fp32 NHWC tensor (or channel slice) -> (fp16 (B, H, W, 2C) = [hi | lo] of s * t, s as a 1-element device tensor)."""
-    B, H, W, Cc = t.shape
-    xs = torch.empty((B, H, W, 2 * Cc), dtype=torch.float16, device=t.device)
-    s = torch.empty(1, dtype=torch.float32, device=t.device)
-    vx, vo = C.view(t), _f16_view(xs)
-    with torch.cuda.device(t.device):
-        C.check(C.lib.rdfc_split_scaled(ctypes.byref(vx), B * H * W, ctypes.byref(vo), C.ptr(s), C.stream_ptr(t.device)))
-    return xs, s
-
-
-def _conv_split(xs, sx, w_oihw, k, stride, transposed, out_hw):
-    """xs, sx = _split(x); w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) fp32 = conv(x, w), no bias / activation."""
-    B, H, W, C2 = xs.shape
-    Cin, O = C2 // 2, w_oihw.shape[0]
-    if Cin % 32 or O % 8 or w_oihw.shape[1] != Cin:
-        raise RuntimeError(f"tensor-core conv needs Cin % 32 == 0 and Cout % 8 == 0, got {Cin} -> {O}")
-    w = w_oihw.detach().float()
-    sw = _pow2_factor(w)
-    packed = pack_weight(w * sw, umma=True, x3=True)                   # [W_hi ; W_lo ; W_hi] of the scaled filter
-    inv = (1.0 / (sx * sw)).expand((O + 15) // 16 * 16).contiguous()   # exact: powers of two
-    out = torch.empty((B, out_hw[0], out_hw[1], O), dtype=torch.float32, device=xs.device)
-    d = C.ConvDesc()
-    d.B, d.Hi, d.Wi, d.Ho, d.Wo = B, H, W, out_hw[0], out_hw[1]
-    d.kh = d.kw = k
-    d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, int(transposed), C.ACT_NONE
-    d.path = C.PATH_UMMA_F32X3
-    d.inp, d.in2, d.out, d.residual = _f16_view(xs), C.view(None), C.view(out), C.view(None)
-    d.weight, d.scale, d.shift = packed.data_ptr(), inv.data_ptr(), None
-    with torch.cuda.device(xs.device):
-        C.check(C.lib.rdfc_conv_forward_split(ctypes.byref(d), C.stream_ptr(xs.device)))
-    return out
-
-
-def _wgrad_split(gs, sg, xs, sx, k, stride):
-    """Filter gradient from split operands (gs, sg = _split(grad_out); xs, sx = _split(input)) -> (O, I, k, k) fp32."""
-    B, Hg, Wg, O2 = gs.shape
-    _, Hi, Wi, I2 = xs.shape
-    d = C.WgradDesc()
-    d.B, d.Hg, d.Wg, d.Hi, d.Wi, d.k, d.stride, d.pad = B, Hg, Wg, Hi, Wi, k, stride, (k - 1) // 2
-    d.grad_out, d.input = _f16_view(gs), _f16_view(xs)
-    n = C.lib.rdfc_conv_wgrad_split_workspace_floats(ctypes.byref(d))
-    if n < 0:
-        raise RuntimeError(C.lib.rdfc_last_error().decode("utf-8", "replace"))
-    ws = torch.empty(n, dtype=torch.float32, device=xs.device)
-    gw = torch.empty((O2 // 2, I2 // 2, k, k), dtype=torch.float32, device=xs.device)
-    inv = 1.0 / (sg * sx)
-    with torch.cuda.device(xs.device):
-        C.check(C.lib.rdfc_conv_wgrad_split(ctypes.byref(d), C.ptr(inv), C.ptr(gw), C.ptr(ws), C.stream_ptr(xs.device)))
-    return gw
-
-
-class _Conv2dNHWCSplit(torch.autograd.Function):
-    """_Conv2dNHWC on fp32 tensors: the same conv forms and data-gradient transforms, split-operand arithmetic.  Keeps the split
-    input (as many bytes as the fp32 input) for the filter gradient instead of the input itself."""
-    @staticmethod
-    def forward(ctx, x, weight, k, stride, transposed):
-        C.require_cuda(x, weight)
-        x = _dense(x)
-        B, H, W, _ = x.shape
-        if transposed:
-            out_hw = (2 * H, 2 * W)
-            w_oihw = weight.detach().permute(1, 0, 2, 3)
-        else:
-            p = (k - 1) // 2
-            out_hw = ((H + 2 * p - k) // stride + 1, (W + 2 * p - k) // stride + 1)
-            w_oihw = weight.detach()
-        xs, sx = _split(x)
-        ctx.save_for_backward(xs, sx, weight)
-        ctx.cfg = (k, stride, transposed)
-        return _conv_split(xs, sx, w_oihw, k, stride, transposed, out_hw)
-
-    @staticmethod
-    def backward(ctx, gy):
-        xs, sx, weight = ctx.saved_tensors
-        k, stride, transposed = ctx.cfg
-        gs, sg = _split(_dense(gy))
-        B, H, W, C2 = xs.shape
-        w = weight.detach()
-        gx = gw = None
-        if ctx.needs_input_grad[0]:
-            if transposed:
-                gx = _conv_split(gs, sg, w, 3, 2, False, (H, W))
-            elif k == 3 and stride == 1:
-                gx = _conv_split(gs, sg, w.flip(2, 3).permute(1, 0, 2, 3), 3, 1, False, (H, W))
-            elif k == 3:
-                gx = _conv_split(gs, sg, w.permute(1, 0, 2, 3), 3, 2, True, (H, W))
-            else:
-                t = _conv_split(gs, sg, w.permute(1, 0, 2, 3), 1, 1, False, tuple(gy.shape[1:3]))
-                if stride == 1:
-                    gx = t
-                else:
-                    gx = torch.zeros((B, H, W, C2 // 2), dtype=torch.float32, device=t.device)
-                    gx[:, ::2, ::2] = t
-        if ctx.needs_input_grad[1]:
-            if transposed:
-                gw = _wgrad_split(xs, sx, gs, sg, 3, 2)
-            else:
-                gw = _wgrad_split(gs, sg, xs, sx, k, stride)
+                gw = _wgrad(g, x, k, stride, sg, sx)           # (Cout, Cin, k, k)
             gw = gw.to(weight.dtype)
         return gx, gw, None, None, None
 
@@ -240,8 +164,6 @@ class _Conv2dNHWCSplit(torch.autograd.Function):
 def conv2d_nhwc(x, weight, k=3, stride=1, transposed=False):
     """NHWC convolution (3x3 / 1x1, stride 1 / 2, padding (k-1)/2) or ConvTranspose2d(k3, s2, p1, op1) without bias.
     bf16 ``x``: bf16 operands and result; fp32 ``x``: the fp32_tc split-operand arithmetic, fp32 result."""
-    if x.dtype == torch.float32:
-        return _Conv2dNHWCSplit.apply(x, weight, k, stride, transposed)
     return _Conv2dNHWC.apply(x, weight, k, stride, transposed)
 
 

@@ -1,10 +1,9 @@
-"""Development aid: filter-gradient kernels on the training step's layer shapes (B = 16 per GPU, 228x304): the tcgen05 kernel
-(csrc/wgrad_umma.cu) against the mma.sync kernel (RDFC_WGRAD_UMMA = 0) and cuDNN's wgrad (torch.nn.grad.conv2d_weight, bf16)."""
+"""Development aid: the filter gradient on the training step's layer shapes (B = 16 per GPU, 228x304): the tcgen05 kernel
+(csrc/wgrad_umma.cu) against cuDNN's wgrad (torch.nn.grad.conv2d_weight, bf16)."""
 import os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from rdfc_gan_b200 import _cabi as C
 from rdfc_gan_b200.train_ops import _wgrad
 
 B = int(os.environ.get("B", 16))
@@ -35,23 +34,21 @@ def timeit(fn, reps=10):
     torch.cuda.synchronize()
     return sorted(a.elapsed_time(b) for a, b in ev)[reps // 2]
 
-tot = {"umma": 0.0, "mma.sync": 0.0}
+tot = {"umma": 0.0, "cuDNN": 0.0}
 for O, I, (Hg, Wg), (Hi, Wi), s, cnt, name in LAYERS[:int(os.environ.get("NLAYERS", len(LAYERS)))]:
     g = torch.Generator(device="cuda").manual_seed(1)
     gy = torch.randn(B, Hg, Wg, O, device="cuda", generator=g).to(torch.bfloat16)
     x = torch.randn(B, Hi, Wi, I, device="cuda", generator=g).to(torch.bfloat16)
     flops = 2.0 * O * I * 9 * B * Hg * Wg
-    res = {}
-    for tag, v in (("umma", 1), ("mma.sync", 0)):
-        C.set_knob("RDFC_WGRAD_UMMA", v)
-        res[tag] = (timeit(lambda: _wgrad(gy, x, 3, s)), _wgrad(gy, x, 3, s))
-        tot[tag] += cnt * res[tag][0]
-    C.set_knob("RDFC_WGRAD_UMMA", None)
-    rel = float((res["umma"][1] - res["mma.sync"][1]).norm() / res["mma.sync"][1].norm())
-    line = f"{name:42s} umma {res['umma'][0]*1e3:7.1f} us ({flops/res['umma'][0]/1e9:6.0f} TF/s) | mma.sync {res['mma.sync'][0]*1e3:7.1f} us ({flops/res['mma.sync'][0]/1e9:5.0f} TF/s) | rel diff {rel:.1e}"
+    t = timeit(lambda: _wgrad(gy, x, 3, s))
+    tot["umma"] += cnt * t
+    line = f"{name:42s} umma {t*1e3:7.1f} us ({flops/t/1e9:6.0f} TF/s)"
     if os.environ.get("CUDNN", "1") == "1":
         xn, gn = x.permute(0, 3, 1, 2), gy.permute(0, 3, 1, 2)        # channels-last views
-        t = timeit(lambda: torch.nn.grad.conv2d_weight(xn, (O, I, 3, 3), gn, stride=s, padding=1))
-        line += f" | cuDNN bf16 {t*1e3:7.1f} us"
+        tc = timeit(lambda: torch.nn.grad.conv2d_weight(xn, (O, I, 3, 3), gn, stride=s, padding=1))
+        tot["cuDNN"] += cnt * tc
+        ref = torch.nn.grad.conv2d_weight(xn, (O, I, 3, 3), gn, stride=s, padding=1).float()
+        rel = float((_wgrad(gy, x, 3, s) - ref).norm() / ref.norm())
+        line += f" | cuDNN bf16 {tc*1e3:7.1f} us | rel diff {rel:.1e}"
     print(line, flush=True)
-print(f"per training step (counts weighted): umma {tot['umma']:.2f} ms, mma.sync {tot['mma.sync']:.2f} ms")
+print(f"per training step (counts weighted): umma {tot['umma']:.2f} ms, cuDNN {tot['cuDNN']:.2f} ms")

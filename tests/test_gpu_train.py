@@ -21,7 +21,9 @@ def _rel(a, b):
     # B, Cin, Cout, H, W, k, stride
     (2, 64, 64, 36, 52, 3, 1), (3, 64, 128, 37, 50, 3, 2), (2, 128, 32, 19, 45, 3, 1), (1, 192, 384, 29, 38, 1, 1),
     (2, 64, 128, 40, 41, 1, 2), (2, 96, 160, 17, 23, 3, 1), (1, 512, 512, 15, 19, 3, 1), (4, 64, 64, 228, 304, 3, 1),
-    (2, 192, 64, 29, 38, 3, 2), (1, 128, 256, 58, 77, 3, 2), (2, 256, 80, 9, 100, 3, 1)])
+    (2, 192, 64, 29, 38, 3, 2), (1, 128, 256, 58, 77, 3, 2), (2, 256, 80, 9, 100, 3, 1),
+    # Cout % 16 == 8: the kernel's N is rounded up to 16, the channels past Cout are zero fill and masked
+    (2, 64, 24, 36, 52, 3, 1), (2, 64, 40, 29, 38, 3, 2), (1, 128, 8, 15, 19, 1, 1), (2, 96, 24, 20, 28, 1, 2)])
 def test_filter_gradient_against_torch(case):
     from rdfc_gan_b200.train_ops import _wgrad
     B, Cin, Cout, H, W, k, s = case
@@ -36,23 +38,17 @@ def test_filter_gradient_against_torch(case):
     assert _rel(got, want) <= 2e-5, _rel(got, want)          # fp32 accumulation of exact bf16 products
     again = _wgrad(gy, x, k, s)
     assert torch.equal(got, again), "the split-K reduction must be deterministic"
-    if True:
-        # filter gradients run on tcgen05 (csrc/wgrad_umma.cu); every tile width of that kernel and the mma.sync kernel
-        # (RDFC_WGRAD_UMMA = 0) must give the same sums
-        from rdfc_gan_b200 import _cabi as C
-        try:
-            for knobs in ({"RDFC_WGRAD_TW": 16}, {"RDFC_WGRAD_TW": 32}, {"RDFC_WGRAD_UMMA": 0}):
-                for name, v in knobs.items():
-                    C.set_knob(name, v)
-                n0 = C.launch_count()
-                other = _wgrad(gy, x, k, s)
-                assert C.launch_count() - n0 == 2
-                assert _rel(other, want) <= 2e-5, (knobs, _rel(other, want))
-                for name in knobs:
-                    C.set_knob(name, None)
-        finally:
-            for name in ("RDFC_WGRAD_TW", "RDFC_WGRAD_UMMA"):
-                C.set_knob(name, None)
+    # every tile width of the tcgen05 kernel (csrc/wgrad_umma.cu) must give the same sums, in two launches (partials, reduction)
+    from rdfc_gan_b200 import _cabi as C
+    try:
+        for tw in (16, 32):
+            C.set_knob("RDFC_WGRAD_TW", tw)
+            n0 = C.launch_count()
+            other = _wgrad(gy, x, k, s)
+            assert C.launch_count() - n0 == 2
+            assert _rel(other, want) <= 2e-5, (tw, _rel(other, want))
+    finally:
+        C.set_knob("RDFC_WGRAD_TW", None)
 
 
 @pytest.mark.parametrize("case", [(2, 64, 64, 20, 28, 3, 1, False), (2, 64, 128, 21, 27, 3, 2, False), (2, 128, 64, 10, 13, 3, 2, True),
@@ -77,6 +73,58 @@ def test_conv_function_gradients(case):
     yr.backward(gy.float().permute(0, 3, 1, 2).double())
     assert _rel(x.grad.float().permute(0, 3, 1, 2), xr.grad) <= 6e-3
     assert _rel(w.grad, wr.grad) <= 1e-4
+
+
+@pytest.mark.parametrize("case", [(2, 64, 64, 36, 52, 1), (2, 64, 128, 37, 50, 2), (1, 128, 256, 30, 44, 2), (2, 256, 256, 19, 26, 1)])
+def test_conv_input_grad_on_the_forward_kernel(case):
+    """conv2d_nhwc's data gradient of the generator's 3x3 convs (stride-1 / transposed convs on the tensor-core kernel), with a filter
+    that needs no gradient, against torch.nn.grad.conv2d_input on the same bf16-rounded operands."""
+    from rdfc_gan_b200.train_ops import conv2d_nhwc
+    B, Cin, Cout, H, W, stride = case
+    gen = torch.Generator().manual_seed(sum(case))
+    w = (torch.randn(Cout, Cin, 3, 3, generator=gen) / math.sqrt(Cout * 9)).bfloat16().float()
+    Ho, Wo = (H + 2 - 3) // stride + 1, (W + 2 - 3) // stride + 1
+    go = torch.randn(B, Cout, Ho, Wo, generator=gen).bfloat16().float()
+    ref = torch.nn.grad.conv2d_input((B, Cin, H, W), w.double(), go.double(), stride=stride, padding=1).float()
+    x = torch.zeros(B, H, W, Cin, dtype=BF, device="cuda", requires_grad=True)
+    wd = w.cuda()
+    conv2d_nhwc(x, wd, 3, stride).backward(go.permute(0, 2, 3, 1).bfloat16().contiguous().cuda())
+    assert wd.grad is None
+    got = x.grad.float().permute(0, 3, 1, 2).cpu()
+    assert tuple(got.shape) == (B, Cin, H, W)
+    err = (got - ref).abs().max().item()
+    assert err <= 1.5e-2 * max(1.0, ref.abs().max().item()), (case, err)        # one bf16 rounding of the output
+
+
+def test_conv_transpose_input_grad_on_the_forward_kernel():
+    from rdfc_gan_b200.train_ops import conv2d_nhwc
+    B, Cin, Cout, H, W = 2, 192, 64, 19, 26
+    gen = torch.Generator().manual_seed(4)
+    w = (torch.randn(Cin, Cout, 3, 3, generator=gen) / math.sqrt(Cout * 9)).bfloat16().float()
+    xr = torch.zeros(B, Cin, H, W, dtype=torch.double, requires_grad=True)
+    yr = F.conv_transpose2d(xr, w.double(), None, stride=2, padding=1, output_padding=1)
+    go = torch.randn(yr.shape, generator=gen).bfloat16().float()
+    (ref,) = torch.autograd.grad(yr, xr, go.double())
+    x = torch.zeros(B, H, W, Cin, dtype=BF, device="cuda", requires_grad=True)
+    wd = w.cuda()
+    conv2d_nhwc(x, wd, 3, 2, True).backward(go.permute(0, 2, 3, 1).bfloat16().contiguous().cuda())
+    assert wd.grad is None
+    got = x.grad.float().permute(0, 3, 1, 2).cpu()
+    assert tuple(got.shape) == (B, Cin, H, W)
+    assert (got - ref.float()).abs().max().item() <= 1.5e-2 * max(1.0, ref.abs().max().item())
+
+
+@pytest.mark.parametrize("dtype", [BF, torch.float32])
+def test_conv_function_rejects_cin_off_the_tensor_core_rule(dtype):
+    """conv2d_nhwc needs Cin % 32 == 0 (bf16 and fp32_tc alike): Cin = 24 raises a RuntimeError naming the rule before any launch."""
+    from rdfc_gan_b200 import _cabi as C
+    from rdfc_gan_b200.train_ops import conv2d_nhwc
+    x = torch.randn(1, 8, 8, 24, device="cuda").to(dtype)
+    w = torch.randn(16, 24, 3, 3, device="cuda")
+    n0 = C.launch_count()
+    with pytest.raises(RuntimeError, match="% 32|multiple of 32"):
+        conv2d_nhwc(x, w)
+    assert C.launch_count() == n0
 
 
 @pytest.mark.parametrize("case", [(2, 19, 27, 64, 1, True), (3, 12, 10, 128, 2, False), (1, 30, 44, 32, 0, True), (2, 114, 152, 64, 2, True)])

@@ -24,17 +24,14 @@ def test_plan_lanes_and_sync_marks():
     assert p.sync == {1: ['fork'], 5: ['join', 'fork'], 8: ['join']}
 
 
-def test_conv_grad_filter_packing_matches_the_engine_layout():
-    """conv_grad.pack_filter must produce engine._pack's UMMA layout [tap][Cin/8][CoutP][8] (bf16), padded to 16 output rows;
-    host-side only (no kernel launch)."""
-    import pytest
+def test_umma_filter_packing_layout():
+    """engine.pack_weight(umma=True), the filter layout of the tensor-core conv (train_ops.conv2d_nhwc packs with it too):
+    [tap][Cin/8][CoutP][8] (bf16), padded to 16 output rows; host-side only (no kernel launch)."""
     import torch
-    from rdfc_gan_b200.conv_grad import pack_filter
+    from rdfc_gan_b200.engine import pack_weight
     w = torch.randn(40, 64, 3, 3)
-    p = pack_filter(w)
+    p = pack_weight(w, umma=True)
     assert p.dtype == torch.bfloat16 and tuple(p.shape) == (9, 8, 48, 8)
     for tap, chunk, co, e in ((0, 0, 0, 0), (4, 3, 17, 5), (8, 7, 39, 7)):
         assert p[tap, chunk, co, e] == w[co, chunk * 8 + e, tap // 3, tap % 3].bfloat16()
     assert (p[:, :, 40:, :] == 0).all()
-    with pytest.raises(RuntimeError):
-        pack_filter(torch.randn(16, 24, 3, 3))          # Cin % 32 != 0: not a tensor-core layer
