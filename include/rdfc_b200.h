@@ -79,6 +79,20 @@ int rdfc_dcn_backward(const void *input, const void *weight, const void *offset,
                       const void *grad_output, void *grad_input, void *grad_offset, void *grad_mask,
                       void *grad_weight, void *grad_bias, const rdfc_dcn_shape *s, int dtype, void *stream);
 
+/* Flags of the *_ex backward entry points.  RDFC_DETERMINISTIC: the scatters that rdfc_dcn_backward,
+ * rdfc_nlspn_affinity_backward and rdfc_nlspn_propagate_backward do with floating-point atomics (so that their last bits depend
+ * on the execution order) accumulate instead in 64-bit fixed point, scaled by a power of two taken on the device from a bound on
+ * the largest possible sum; the results are then bit-identical from run to run on the same GPU and build.  A NaN or Inf input
+ * still gives non-finite results.  flags == 0 calls the entry point without _ex; other bits are refused before any launch.
+ * The deterministic paths allocate their workspace stream-ordered (cudaMallocAsync) and free it before returning.  Bindings that
+ * follow torch.use_deterministic_algorithms pass RDFC_DETERMINISTIC when torch.are_deterministic_algorithms_enabled(). */
+#define RDFC_DETERMINISTIC 1
+
+/* rdfc_dcn_backward's arguments plus flags */
+int rdfc_dcn_backward_ex(const void *input, const void *weight, const void *offset, const void *mask,
+                         const void *grad_output, void *grad_input, void *grad_offset, void *grad_mask,
+                         void *grad_weight, void *grad_bias, const rdfc_dcn_shape *s, int dtype, void *stream, int flags);
+
 /* ------------------------------------------------------------------ NLSPN ------------------------------------- */
 typedef enum { RDFC_AFF_AS = 0, RDFC_AFF_ASS = 1, RDFC_AFF_TC = 2, RDFC_AFF_TGASS = 3 } rdfc_affinity;
 
@@ -124,7 +138,8 @@ int rdfc_nlspn_propagate_forward_packed(const float *feat_init, const void *pack
  * grad_conv (B,24,H,W) = dL/d conv_offset_aff(guidance) (the caller back-propagates the 8 -> 24 channel conv itself),
  * grad_confidence (B,1,H,W, overwritten; required when conf_prop) through the 1x1 DCN gathers of nlspn_model.py:96-119 (their
  * offsets are detached in the reference), grad_aff_scale (1 float, overwritten; NULL to skip) for TGASS's learnable scale
- * (nlspn_model.py:86-87).  offset = the forward's output.  fp32 atomics in the confidence scatter and the scale reduction. */
+ * (nlspn_model.py:86-87).  offset = the forward's output.  fp32 atomics in the confidence scatter and the scale reduction
+ * (rdfc_nlspn_affinity_backward_ex with RDFC_DETERMINISTIC has none). */
 int rdfc_nlspn_affinity_backward(const float *guidance, const float *confidence, const float *conv_w, const float *conv_b,
                                  const float *aff_scale, int affinity, int conf_prop, const float *offset,
                                  const float *grad_offset, const float *grad_aff, float *grad_conv, float *grad_confidence,
@@ -136,11 +151,23 @@ int rdfc_nlspn_affinity_backward(const float *guidance, const float *confidence,
  * preserve_input as in the forward; inter = the forward's `inter` buffer (required when prop_time > 1).
  * Writes grad_feat_init (B,1,H,W), grad_offset (B,18,H,W), grad_aff (B,9,H,W) (overwritten, not accumulated).
  * scratch: (prop_time + 1) * B*H*W floats.  The input-gradient scatter uses fp32 atomics (as the reference's col2im does), so
- * the last bits depend on the execution order. */
+ * the last bits depend on the execution order (rdfc_nlspn_propagate_backward_ex with RDFC_DETERMINISTIC: they do not). */
 int rdfc_nlspn_propagate_backward(const float *grad_out, const float *grad_inter, const float *feat_init,
                                   const float *inter, const float *offset, const float *aff, const float *feat_fix,
                                   int preserve_input, float *grad_feat_init, float *grad_offset, float *grad_aff,
                                   float *scratch, int B, int H, int W, int prop_time, void *stream);
+
+/* The two NLSPN backwards with a trailing flags argument (RDFC_DETERMINISTIC, see rdfc_dcn_backward_ex).  Deterministic, the
+ * propagation backward runs two kernels per iteration instead of one (the fixed-point scatter, then its conversion fused with the
+ * per-iteration finalisation) and the affinity backward four instead of one. */
+int rdfc_nlspn_affinity_backward_ex(const float *guidance, const float *confidence, const float *conv_w, const float *conv_b,
+                                    const float *aff_scale, int affinity, int conf_prop, const float *offset,
+                                    const float *grad_offset, const float *grad_aff, float *grad_conv, float *grad_confidence,
+                                    float *grad_aff_scale, int B, int H, int W, void *stream, int flags);
+int rdfc_nlspn_propagate_backward_ex(const float *grad_out, const float *grad_inter, const float *feat_init,
+                                     const float *inter, const float *offset, const float *aff, const float *feat_fix,
+                                     int preserve_input, float *grad_feat_init, float *grad_offset, float *grad_aff,
+                                     float *scratch, int B, int H, int W, int prop_time, void *stream, int flags);
 
 /* pred = softmax([c1,c2]) . [d1, clamp(d2)] ; d2_clamped receives clamp(d2,-1,1) (may alias d2). n = B*H*W. */
 int rdfc_fuse_depth_forward(const float *d1, const float *c1, const float *d2, const float *c2, float *d2_clamped,

@@ -13,6 +13,7 @@ F32, F64, BF16, F16 = 0, 1, 2, 3          # F16: the split [hi | lo] tensors of 
 ACT_NONE, ACT_RELU, ACT_LEAKY02, ACT_TANH, ACT_SIGMOID = range(5)
 PATH_SIMT_F32, PATH_UMMA_BF16, PATH_UMMA_F32X3 = 0, 1, 2
 AFFINITY = {"AS": 0, "ASS": 1, "TC": 2, "TGASS": 3}
+DETERMINISTIC = 1                         # flags of the *_ex backward entry points
 _DT = {torch.float32: F32, torch.float64: F64, torch.bfloat16: BF16, torch.float16: F16}
 
 c_int, c_void_p, c_float = ctypes.c_int, ctypes.c_void_p, ctypes.c_float
@@ -103,6 +104,8 @@ def _load():
     lib.rdfc_depth_metric_sums.argtypes = [c_void_p] * 3 + [ctypes.c_float] * 3 + [c_void_p] * 2 + [c_int, ctypes.c_longlong, c_void_p]
     lib.rdfc_nlspn_affinity_backward.argtypes = [c_void_p] * 5 + [c_int] * 2 + [c_void_p] * 6 + [c_int] * 3 + [c_void_p]
     lib.rdfc_nlspn_propagate_backward.argtypes = [c_void_p] * 7 + [c_int] + [c_void_p] * 4 + [c_int] * 4 + [c_void_p]
+    for name in ("rdfc_dcn_backward", "rdfc_nlspn_affinity_backward", "rdfc_nlspn_propagate_backward"):
+        getattr(lib, name + "_ex").argtypes = getattr(lib, name).argtypes + [c_int]
     lib.rdfc_conv_forward.argtypes = [ctypes.POINTER(ConvDesc), c_void_p]
     lib.rdfc_heads_forward.argtypes = [ctypes.POINTER(HeadsDesc), c_void_p]
     lib.rdfc_stem_forward.argtypes = [ctypes.POINTER(StemDesc), c_void_p]
@@ -132,7 +135,8 @@ EXPORTS = ["rdfc_abi_version", "rdfc_last_error", "rdfc_launch_count", "rdfc_dcn
            "rdfc_bn_workspace_floats", "rdfc_bn_stats", "rdfc_affine_act_forward", "rdfc_bn_act_backward",
            "rdfc_conv_wgrad_workspace_floats", "rdfc_conv_wgrad", "rdfc_first_conv_forward", "rdfc_maxpool3x3s2_forward", "rdfc_se_weights",
            "rdfc_adaptive_avgpool_forward", "rdfc_upsample_nearest_forward", "rdfc_upsample_dw_forward",
-           "rdfc_split_scaled", "rdfc_conv_forward_split", "rdfc_conv_wgrad_split_workspace_floats", "rdfc_conv_wgrad_split"]
+           "rdfc_split_scaled", "rdfc_conv_forward_split", "rdfc_conv_wgrad_split_workspace_floats", "rdfc_conv_wgrad_split",
+           "rdfc_dcn_backward_ex", "rdfc_nlspn_affinity_backward_ex", "rdfc_nlspn_propagate_backward_ex"]
 
 
 KNOB_UNSET = -(1 << 63)
@@ -142,6 +146,15 @@ def set_knob(name, value=None):
     """Development knobs (the RDFC_* environment variables, cached by the library on first use): override one at run time;
     value None restores the default."""
     check(lib.rdfc_dev_set_knob(name.encode(), KNOB_UNSET if value is None else int(value)))
+
+
+def backward_call(name, *args):
+    """Call the backward entry point `name`; under torch.use_deterministic_algorithms (read at call time, warn_only included) its
+    _ex variant with DETERMINISTIC, whose scatters accumulate in 64-bit fixed point and are bit-reproducible."""
+    if torch.are_deterministic_algorithms_enabled():
+        check(getattr(lib, name + "_ex")(*args, DETERMINISTIC))
+    else:
+        check(getattr(lib, name)(*args))
 
 
 def check(rc):

@@ -8,6 +8,7 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "fixed_point.cuh"
 
 namespace rdfc {
 int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads_desc *heads, const rdfc_stem_desc *stem,
@@ -126,12 +127,17 @@ __global__ void __launch_bounds__(NT) dcn_fwd_kernel(const T *__restrict__ input
 // One thread per (b, gd, k, pixel): loops the channels of the deformable group, forms
 // gcol = sum_co W[co,ci,k] * gout[b,co,pix]  (modulated_deform_conv_cuda.cu:217-222), then
 // grad_mask / grad_offset (col2im_coord, cuh:257-328) and the grad_input scatter (col2im, cuh:197-254).
-template <typename T, bool kMask>
+// kDet (RDFC_DETERMINISTIC): the scatter goes to gacc in fixed point, bounded per destination by K * P contributions of at most
+// am[0] = max |grad_output| x am[1] = max over (ci, tap) of sum_o |W| x am[2] = max |mask|.
+template <typename T, bool kMask, bool kDet>
 __global__ void __launch_bounds__(NT) dcn_bwd_data_kernel(const T *__restrict__ input, const T *__restrict__ weight,
                                                            const T *__restrict__ offset, const T *__restrict__ mask,
                                                            const T *__restrict__ gout, T *__restrict__ gin,
-                                                           T *__restrict__ goff, T *__restrict__ gmask, Geo g) {
+                                                           T *__restrict__ goff, T *__restrict__ gmask, Geo g,
+                                                           long long *__restrict__ gacc, const unsigned long long *__restrict__ am) {
     const int K = g.kh * g.kw, P = g.Ho * g.Wo;
+    const Fx<T> fx(kDet ? (double)K * P : 1.0, am, kDet ? (kMask ? 3 : 2) : 0);
+    const bool scatter = kDet ? gacc != nullptr : gin != nullptr;
     const int cpg = g.Cin / g.group, opg = g.Cout / g.group, cpdg = g.Cin / g.dg;
     const long long total = (long long)g.B * g.dg * K * P;
     for (long long idx = (long long)blockIdx.x * NT + threadIdx.x; idx < total; idx += (long long)gridDim.x * NT) {
@@ -161,8 +167,8 @@ __global__ void __launch_bounds__(NT) dcn_bwd_data_kernel(const T *__restrict__ 
             s_mask += gcol * val;
             s_y += gcol * m * gy;
             s_x += gcol * m * gx;
-            if (gin && valid) {
-                T *gim = gin + ((size_t)b * g.Cin + ci) * g.H * g.W;
+            if (scatter && valid) {
+                const size_t plane = ((size_t)b * g.Cin + ci) * g.H * g.W;
                 const T top = gcol * m;
 #pragma unroll
                 for (int a = 0; a < 2; ++a)
@@ -171,7 +177,8 @@ __global__ void __launch_bounds__(NT) dcn_bwd_data_kernel(const T *__restrict__ 
                         const int yy = yl + a, xx = xl + c2;
                         if (yy >= 0 && yy <= g.H - 1 && xx >= 0 && xx <= g.W - 1) {
                             const T wgt = (a ? ly : (T)1 - ly) * (c2 ? lx : (T)1 - lx);
-                            atomicAdd(gim + (size_t)yy * g.W + xx, wgt * top);
+                            if (kDet) fx_add(gacc + plane + (size_t)yy * g.W + xx, fx.to_fixed(wgt * top));
+                            else atomicAdd(gin + plane + (size_t)yy * g.W + xx, wgt * top);
                         }
                     }
             }
@@ -183,6 +190,21 @@ __global__ void __launch_bounds__(NT) dcn_bwd_data_kernel(const T *__restrict__ 
         }
         if (kMask && gmask) gmask[((size_t)(b * g.dg + gd) * K + k) * P + pix] = s_mask;
     }
+}
+
+// am[0] = max over (ci, tap) of sum_o |W[o, ci, tap]| (the bound of one column gradient per unit grad_output)
+template <typename T>
+__global__ void __launch_bounds__(NT) dcn_wsum_max_kernel(const T *__restrict__ weight, Geo g, unsigned long long *__restrict__ am) {
+    const int K = g.kh * g.kw, cpg = g.Cin / g.group, opg = g.Cout / g.group;
+    unsigned long long m = 0;
+    for (int e = blockIdx.x * NT + threadIdx.x; e < g.Cin * K; e += gridDim.x * NT) {
+        const int ci = e / K, k = e % K, grp = ci / cpg, cil = ci % cpg;
+        T s = (T)0;
+        for (int o = 0; o < opg; ++o) s += fabs(ld(weight + ((size_t)(grp * opg + o) * cpg + cil) * K + k));
+        const unsigned long long bits = fx_bits((double)s);
+        m = bits > m ? bits : m;
+    }
+    fx_warp_max(m, am);
 }
 
 // ---------------------------------------------------------------- backward: filters ---------------------------
@@ -540,11 +562,14 @@ __global__ void __launch_bounds__(NT) dcn_pack_t_x3_kernel(const float *__restri
 // of 64 channels of one tap is read with the lanes along the channels, goes through a shared-memory tile, and is consumed with one lane per
 // PIXEL (coalesced image reads and atomics), the position / bilinear weights computed once per (pixel, tap, deformable group); the per-pixel
 // sums over the channels of a deformable group are combined through shared memory in a fixed order.
+// kDet (RDFC_DETERMINISTIC): grad_input goes to gacc in fixed point, bounded per destination by K * P contributions of at most
+// am[0] = max |gcols| x am[1] = max |mask|.
 constexpr int MAXDG = 16;
-template <bool kMask>
+template <bool kMask, bool kDet>
 __global__ void __launch_bounds__(NT) dcn_col2im_coord_kernel(const float *__restrict__ input, const float *__restrict__ offset, const float *__restrict__ mask,
                                                               const float *__restrict__ gcols, float *__restrict__ gin, float *__restrict__ goff,
-                                                              float *__restrict__ gmask, Geo g) {
+                                                              float *__restrict__ gmask, Geo g, long long *__restrict__ gacc,
+                                                              const unsigned long long *__restrict__ am) {
     __shared__ float tile[64][33];
     __shared__ float part[NT / 32][3][32];
     __shared__ float acc[MAXDG][3][32];
@@ -555,6 +580,8 @@ __global__ void __launch_bounds__(NT) dcn_col2im_coord_kernel(const float *__res
     const long long HW = (long long)g.H * g.W;
     const float *img = input + (long long)b * g.Cin * HW;
     float *gimg = gin ? gin + (long long)b * g.Cin * HW : nullptr;
+    long long *gacc_img = kDet && gacc ? gacc + (long long)b * g.Cin * HW : nullptr;
+    const Fx<float> fx(kDet ? (double)K * P : 1.0, am, kDet ? (kMask ? 2 : 1) : 0);
     for (int tap = 0; tap < K; ++tap) {
         const int ky = tap / g.kw, kx = tap - ky * g.kw;
         for (int i = threadIdx.x; i < g.dg * 96; i += NT) (&acc[0][0][0])[i] = 0.f;
@@ -593,7 +620,14 @@ __global__ void __launch_bounds__(NT) dcn_col2im_coord_kernel(const float *__res
                             sm += gcol * val;
                             sy += gcol * mk * (hx * (v3 - v1) + lx * (v4 - v2));
                             sx += gcol * mk * (hy * (v2 - v1) + ly * (v4 - v3));
-                            if (gimg) {
+                            if (kDet && gacc_img) {
+                                const float top = gcol * mk;
+                                long long *ga = gacc_img + pl;
+                                if (f1) fx_add(ga + i1, fx.to_fixed(hy * hx * top));
+                                if (f2) fx_add(ga + i2, fx.to_fixed(hy * lx * top));
+                                if (f3) fx_add(ga + i3, fx.to_fixed(ly * hx * top));
+                                if (f4) fx_add(ga + i4, fx.to_fixed(ly * lx * top));
+                            } else if (!kDet && gimg) {
                                 const float top = gcol * mk;
                                 float *gi = gimg + pl;
                                 if (f1) atomicAdd(gi + i1, hy * hx * top);
@@ -644,12 +678,15 @@ bool bwd_tc_ok(const Geo &g) {
     return Kg % 32 == 0 && Cg % 8 == 0 && cpd % 8 == 0 && Cog % 32 == 0 && g.dg <= MAXDG && knob("RDFC_DCN_TC", 1) != 0;
 }
 
+// det: grad_input through dcn_col2im_coord_kernel<kMask, true> and a conversion (stream-ordered workspace: the maxima, the int64 image)
 int bwd_tc(const float *input, const float *weight, const float *offset, const float *mask, const float *gout, float *gin, float *goff, float *gmask,
-           float *gw, float *gb, const Geo &g, cudaStream_t st) {
+           float *gw, float *gb, const Geo &g, cudaStream_t st, bool det) {
     const int K = g.kh * g.kw, P = g.Ho * g.Wo, Cg = g.Cin / g.group, Kg = Cg * K, Cog = g.Cout / g.group, KgP = (Kg + 15) / 16 * 16;
     const long long npix = (long long)g.B * P;
     __half *gs = nullptr, *cols = nullptr, *packed = nullptr;
     float *gcols = nullptr, *ws = nullptr;
+    unsigned long long *fx = nullptr;                                   // det: [am: 2][acc: B * Cin * H * W]
+    const long long nin = (long long)g.B * g.Cin * g.H * g.W;
     Aux aux{};
     const bool need_data = gin || goff || gmask;
     int rc = aux_alloc(&aux, KgP, st);
@@ -657,7 +694,12 @@ int bwd_tc(const float *input, const float *weight, const float *offset, const f
         rc = amax_launch(aux, input, (long long)g.B * g.Cin * g.H * g.W, mask, mask ? (long long)g.B * g.dg * K * P : 0, weight, (long long)g.Cout * Kg, gout,
                          npix * g.Cout, st);
     if (rc) return rc;
-    if (gin) RDFC_CUDA(cudaMemsetAsync(gin, 0, sizeof(float) * (size_t)g.B * g.Cin * g.H * g.W, st));
+    if (gin && det) {
+        RDFC_CUDA(cudaMallocAsync((void **)&fx, 8 * (2 + (size_t)nin), st));
+        RDFC_CUDA(cudaMemsetAsync(fx, 0, 8 * (2 + (size_t)nin), st));
+    } else if (gin) {
+        RDFC_CUDA(cudaMemsetAsync(gin, 0, sizeof(float) * (size_t)g.B * g.Cin * g.H * g.W, st));
+    }
     RDFC_CUDA(cudaMallocAsync((void **)&gs, (size_t)npix * g.group * 2 * Cog * sizeof(__half), st));
     dcn_gout_split_kernel<<<dim3(cdiv(P, 32), cdiv(g.Cout, 32), g.B), NT, 0, st>>>(gout, gs, g.Cout, Cog, P, aux.am);
     count_launch();
@@ -675,10 +717,20 @@ int bwd_tc(const float *input, const float *weight, const float *offset, const f
             d.weight = packed; d.scale = aux.vec; d.shift = nullptr;
             rc = conv_umma_forward(&d, st, nullptr, nullptr, nullptr, Cog);
         }
-        if (rc == 0) {
+        if (rc == 0 && fx) {
+            rc = fx_amax(gcols, npix * g.group * Kg, fx, st);
+            if (rc == 0 && mask) rc = fx_amax(mask, (long long)g.B * g.dg * K * P, fx + 1, st);
+            if (rc == 0) {
+                const dim3 grid(cdiv(P, 32), g.B);
+                if (mask) dcn_col2im_coord_kernel<true, true><<<grid, NT, 0, st>>>(input, offset, mask, gcols, nullptr, goff, gmask, g, (long long *)(fx + 2), fx);
+                else dcn_col2im_coord_kernel<false, true><<<grid, NT, 0, st>>>(input, offset, nullptr, gcols, nullptr, goff, nullptr, g, (long long *)(fx + 2), fx);
+                count_launch();
+                rc = fx_convert((const long long *)(fx + 2), gin, nin, (double)K * P, fx, mask ? 2 : 1, st);
+            }
+        } else if (rc == 0) {
             const dim3 grid(cdiv(P, 32), g.B);
-            if (mask) dcn_col2im_coord_kernel<true><<<grid, NT, 0, st>>>(input, offset, mask, gcols, gin, goff, gmask, g);
-            else dcn_col2im_coord_kernel<false><<<grid, NT, 0, st>>>(input, offset, nullptr, gcols, gin, goff, nullptr, g);
+            if (mask) dcn_col2im_coord_kernel<true, false><<<grid, NT, 0, st>>>(input, offset, mask, gcols, gin, goff, gmask, g, nullptr, nullptr);
+            else dcn_col2im_coord_kernel<false, false><<<grid, NT, 0, st>>>(input, offset, nullptr, gcols, gin, goff, nullptr, g, nullptr, nullptr);
             count_launch();
         }
     }
@@ -721,26 +773,60 @@ int bwd_tc(const float *input, const float *weight, const float *offset, const f
     if (packed) cudaFreeAsync(packed, st);
     if (cols) cudaFreeAsync(cols, st);
     if (ws) cudaFreeAsync(ws, st);
+    if (fx) cudaFreeAsync(fx, st);
     cudaFreeAsync(aux.am, st);
+    return rc;
+}
+
+// det: grad_input through dcn_bwd_data_kernel<T, kMask, true> and a conversion (stream-ordered workspace: the maxima, the int64 image)
+template <typename T>
+int bwd_data_det(const T *input, const T *weight, const T *offset, const T *mask, const T *gout, T *gin, T *goff, T *gmask,
+                 const Geo &g, cudaStream_t st) {
+    const int K = g.kh * g.kw, P = g.Ho * g.Wo;
+    const long long nin = (long long)g.B * g.Cin * g.H * g.W, total = (long long)g.B * g.dg * K * P;
+    unsigned long long *fx = nullptr;                                   // [am: 3][acc: nin]
+    RDFC_CUDA(cudaMallocAsync((void **)&fx, 8 * (3 + (size_t)nin), st));
+    long long *acc = (long long *)(fx + 3);
+    int rc = 0;
+    if (cudaMemsetAsync(fx, 0, 8 * (3 + (size_t)nin), st) != cudaSuccess) rc = fail(RDFC_ERR_CUDA, "rdfc_dcn_backward_ex: memset failed");
+    if (rc == 0) rc = fx_amax(gout, (long long)g.B * g.Cout * P, fx, st);
+    if (rc == 0) {
+        dcn_wsum_max_kernel<T><<<cdiv((long long)g.Cin * K, NT), NT, 0, st>>>(weight, g, fx + 1);
+        count_launch();
+    }
+    if (rc == 0 && mask) rc = fx_amax(mask, (long long)g.B * g.dg * K * P, fx + 2, st);
+    if (rc == 0) {
+        const int blocks = (int)min((long long)cdiv(total, NT), (long long)sm_count() * 16);
+        if (mask) dcn_bwd_data_kernel<T, true, true><<<blocks, NT, 0, st>>>(input, weight, offset, mask, gout, nullptr, goff, gmask, g, acc, fx);
+        else dcn_bwd_data_kernel<T, false, true><<<blocks, NT, 0, st>>>(input, weight, offset, nullptr, gout, nullptr, goff, nullptr, g, acc, fx);
+        count_launch();
+        rc = fx_convert(acc, gin, nin, (double)K * P, fx, mask ? 3 : 2, st);
+    }
+    if (rc == 0 && cudaGetLastError() != cudaSuccess) rc = fail(RDFC_ERR_CUDA, "rdfc_dcn_backward_ex: kernel launch failed");
+    cudaFreeAsync(fx, st);
     return rc;
 }
 
 template <typename T>
 int bwd(const void *input, const void *weight, const void *offset, const void *mask, const void *gout, void *gin,
-        void *goff, void *gmask, void *gw, void *gb, const Geo &g, cudaStream_t st) {
+        void *goff, void *gmask, void *gw, void *gb, const Geo &g, cudaStream_t st, bool det) {
     const int K = g.kh * g.kw, P = g.Ho * g.Wo;
-    if (gin) RDFC_CUDA(cudaMemsetAsync(gin, 0, sizeof(T) * (size_t)g.B * g.Cin * g.H * g.W, st));
-    if (gin || goff || gmask) {
+    if (gin && det) {
+        if (int rc = bwd_data_det<T>((const T *)input, (const T *)weight, (const T *)offset, (const T *)mask, (const T *)gout, (T *)gin,
+                                     (T *)goff, (T *)gmask, g, st))
+            return rc;
+    } else if (gin || goff || gmask) {
+        if (gin) RDFC_CUDA(cudaMemsetAsync(gin, 0, sizeof(T) * (size_t)g.B * g.Cin * g.H * g.W, st));
         const long long total = (long long)g.B * g.dg * K * P;
         const int blocks = (int)min((long long)cdiv(total, NT), (long long)sm_count() * 16);
         if (mask)
-            dcn_bwd_data_kernel<T, true><<<blocks, NT, 0, st>>>((const T *)input, (const T *)weight,
-                                                                (const T *)offset, (const T *)mask, (const T *)gout,
-                                                                (T *)gin, (T *)goff, (T *)gmask, g);
+            dcn_bwd_data_kernel<T, true, false><<<blocks, NT, 0, st>>>((const T *)input, (const T *)weight,
+                                                                       (const T *)offset, (const T *)mask, (const T *)gout,
+                                                                       (T *)gin, (T *)goff, (T *)gmask, g, nullptr, nullptr);
         else
-            dcn_bwd_data_kernel<T, false><<<blocks, NT, 0, st>>>((const T *)input, (const T *)weight,
-                                                                 (const T *)offset, nullptr, (const T *)gout,
-                                                                 (T *)gin, (T *)goff, nullptr, g);
+            dcn_bwd_data_kernel<T, false, false><<<blocks, NT, 0, st>>>((const T *)input, (const T *)weight,
+                                                                        (const T *)offset, nullptr, (const T *)gout,
+                                                                        (T *)gin, (T *)goff, nullptr, g, nullptr, nullptr);
         RDFC_CHECK_LAUNCH("dcn_bwd_data_kernel");
     }
     if (gw) {
@@ -790,10 +876,9 @@ extern "C" int rdfc_dcn_forward(const void *input, const void *weight, const voi
                 dtype);
 }
 
-extern "C" int rdfc_dcn_backward(const void *input, const void *weight, const void *offset, const void *mask,
-                                 const void *grad_output, void *grad_input, void *grad_offset, void *grad_mask,
-                                 void *grad_weight, void *grad_bias, const rdfc_dcn_shape *s, int dtype,
-                                 void *stream) {
+static int dcn_backward(const void *input, const void *weight, const void *offset, const void *mask, const void *grad_output,
+                        void *grad_input, void *grad_offset, void *grad_mask, void *grad_weight, void *grad_bias,
+                        const rdfc_dcn_shape *s, int dtype, void *stream, bool det) {
     Geo g;
     if (int rc = check_shape(s, g)) return rc;
     RDFC_REQUIRE(input && weight && offset && grad_output, "input / weight / offset / grad_output must not be NULL");
@@ -802,12 +887,29 @@ extern "C" int rdfc_dcn_backward(const void *input, const void *weight, const vo
     // GEMM-sized layers: both contractions of the backward on tcgen05 at fp32 fidelity; thin layers / fp64: the CUDA-core kernels
     if (dtype == RDFC_F32 && bwd_tc_ok(g))
         return bwd_tc((const float *)input, (const float *)weight, (const float *)offset, (const float *)mask, (const float *)grad_output,
-                      (float *)grad_input, (float *)grad_offset, (float *)grad_mask, (float *)grad_weight, (float *)grad_bias, g, st);
+                      (float *)grad_input, (float *)grad_offset, (float *)grad_mask, (float *)grad_weight, (float *)grad_bias, g, st, det);
     if (dtype == RDFC_F32)
         return bwd<float>(input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask, grad_weight,
-                          grad_bias, g, st);
+                          grad_bias, g, st, det);
     if (dtype == RDFC_F64)
         return bwd<double>(input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask, grad_weight,
-                           grad_bias, g, st);
+                           grad_bias, g, st, det);
     return fail(RDFC_ERR_UNSUPPORTED, "rdfc_dcn_backward: dtype %d not supported", dtype);
+}
+
+extern "C" int rdfc_dcn_backward(const void *input, const void *weight, const void *offset, const void *mask,
+                                 const void *grad_output, void *grad_input, void *grad_offset, void *grad_mask,
+                                 void *grad_weight, void *grad_bias, const rdfc_dcn_shape *s, int dtype,
+                                 void *stream) {
+    return dcn_backward(input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask, grad_weight, grad_bias, s, dtype,
+                        stream, false);
+}
+
+extern "C" int rdfc_dcn_backward_ex(const void *input, const void *weight, const void *offset, const void *mask,
+                                    const void *grad_output, void *grad_input, void *grad_offset, void *grad_mask,
+                                    void *grad_weight, void *grad_bias, const rdfc_dcn_shape *s, int dtype,
+                                    void *stream, int flags) {
+    RDFC_REQUIRE((flags & ~RDFC_DETERMINISTIC) == 0, "rdfc_dcn_backward_ex: unknown flags 0x%x", flags);
+    return dcn_backward(input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask, grad_weight, grad_bias, s, dtype,
+                        stream, (flags & RDFC_DETERMINISTIC) != 0);
 }

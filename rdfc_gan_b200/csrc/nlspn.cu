@@ -12,6 +12,7 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "fixed_point.cuh"
 
 namespace rdfc {
 namespace {
@@ -641,12 +642,16 @@ extern "C" int rdfc_nlspn_propagate_forward_packed(const float *feat_init, const
 // offsets detached there) and accumulates dL/d aff_scale_const (TGASS).  The raw affinity channels are recomputed (8 of the 24
 // conv outputs); the offsets are read back from the forward's output.  The conv's own backward (8 <-> 24 channels, 0.24 GFLOP per
 // image) is left to the caller.
+// kDet (RDFC_DETERMINISTIC): no atomics.  The confidence scatter's per-tap values go to g_tap (B,8,H,W) with their maximum in
+// am[0], for nlspn_conf_scatter_det_kernel; the per-CTA sums of dL/d aff_scale go to g_scale[CTA index], for nlspn_sum_kernel.
+template <bool kDet>
 __global__ void __launch_bounds__(TX *TY) nlspn_affinity_bwd_kernel(const float *__restrict__ guidance, const float *__restrict__ confidence,
                                                                     const float *__restrict__ conv_w, const float *__restrict__ conv_b,
                                                                     const float *__restrict__ aff_scale, int affinity, int conf_prop,
                                                                     const float *__restrict__ offset, const float *__restrict__ g_offset,
                                                                     const float *__restrict__ g_aff, float *__restrict__ g_conv,
-                                                                    float *__restrict__ g_conf, float *__restrict__ g_scale, int H, int W) {
+                                                                    float *__restrict__ g_conf, float *__restrict__ g_scale, int H, int W,
+                                                                    float *__restrict__ g_tap, unsigned long long *__restrict__ am) {
     __shared__ __align__(16) float s_w[72 * 8];      // the 8 affinity channels: [(ci*9 + tap)][8]
     __shared__ float s_b[8];
     __shared__ float s_g[8][TY + 2][TX + 2];
@@ -666,6 +671,7 @@ __global__ void __launch_bounds__(TX *TY) nlspn_affinity_bwd_kernel(const float 
     const int x = x0 + threadIdx.x, y = y0 + threadIdx.y;
     const bool live = x < W && y < H;
     float gs = 0.f;                                  // this pixel's contribution to dL/d aff_scale_const
+    unsigned long long tap_max = 0;                  // kDet: max |per-tap confidence gradient|
     if (live) {
         float r[8];
 #pragma unroll
@@ -720,7 +726,12 @@ __global__ void __launch_bounds__(TX *TY) nlspn_affinity_bwd_kernel(const float 
                 gu = ga[j] / abs_sum - (clamped ? 0.f : dot / (abs_sum * abs_sum) * sgn);
             }
             const float gv = gu * c[j];
-            if (conf_prop) {                              // dL/d confidence: transposed bilinear gather at (y + dy, x + dx)
+            if (conf_prop && kDet) {
+                const float gcj = gu * v[j];
+                g_tap[((long long)b * 8 + j) * P + pix] = gcj;
+                const unsigned long long bits = fx_bits(gcj);
+                tap_max = bits > tap_max ? bits : tap_max;
+            } else if (conf_prop) {                       // dL/d confidence: transposed bilinear gather at (y + dy, x + dx)
                 const float gcj = gu * v[j], sy = (float)y + dy[j], sx = (float)x + dx[j];
                 if (gcj != 0.f && sy > -1.f && sx > -1.f && sy < (float)H && sx < (float)W) {
                     const float fy = floorf(sy), fx = floorf(sx);
@@ -748,6 +759,7 @@ __global__ void __launch_bounds__(TX *TY) nlspn_affinity_bwd_kernel(const float 
             gc[(long long)(2 * j + 1) * P] = __ldg(gop + (long long)(2 * k + 1) * P);
         }
     }
+    if (kDet && conf_prop) fx_warp_max(tap_max, am);
     if (g_scale) {                                    // block reduction, one atomic per CTA
         for (int o = 16; o > 0; o >>= 1) gs += __shfl_down_sync(0xffffffffu, gs, o);
         if ((tid & 31) == 0) s_red[tid >> 5] = gs;
@@ -755,9 +767,58 @@ __global__ void __launch_bounds__(TX *TY) nlspn_affinity_bwd_kernel(const float 
         if (tid == 0) {
             float tot = 0.f;
             for (int w = 0; w < TX * TY / 32; ++w) tot += s_red[w];
-            if (tot != 0.f) atomicAdd(g_scale, tot);
+            if (kDet) g_scale[((long long)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] = tot;
+            else if (tot != 0.f) atomicAdd(g_scale, tot);
         }
     }
+}
+
+// kDet confidence scatter: g_tap (B,8,H,W) -> acc (B,H,W) in fixed point.  Destination bound: the 8 taps of every pixel of the
+// image, each at most max |g_tap| (the four bilinear weights sum to 1).  grid (ceil(P / 256), B).
+__global__ void __launch_bounds__(256) nlspn_conf_scatter_det_kernel(const float *__restrict__ g_tap, const float *__restrict__ offset,
+                                                                     long long *__restrict__ acc, const unsigned long long *__restrict__ am,
+                                                                     int H, int W) {
+    const long long P = (long long)H * W;
+    const int b = blockIdx.y;
+    const long long pix = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (pix >= P) return;
+    const Fx<float> fx(8.0 * (double)P, am, 1);
+    const int y = (int)(pix / W), x = (int)(pix - (long long)y * W);
+    const float *offp = offset + (long long)b * 18 * P + pix;
+    long long *gim = acc + (long long)b * P;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const int k = j < 4 ? j : j + 1;
+        const float gcj = __ldg(g_tap + ((long long)b * 8 + j) * P + pix);
+        const float sy = (float)y + __ldg(offp + (long long)(2 * k) * P), sx = (float)x + __ldg(offp + (long long)(2 * k + 1) * P);
+        if (gcj != 0.f && sy > -1.f && sx > -1.f && sy < (float)H && sx < (float)W) {
+            const float fy = floorf(sy), fxl = floorf(sx);
+            const int yl = (int)fy, xl = (int)fxl;
+            const float ly = sy - fy, lx = sx - fxl;
+#pragma unroll
+            for (int aa = 0; aa < 2; ++aa)
+#pragma unroll
+                for (int cc = 0; cc < 2; ++cc) {
+                    const int yy = yl + aa, xx = xl + cc;
+                    if (yy >= 0 && yy <= H - 1 && xx >= 0 && xx <= W - 1)
+                        fx_add(gim + (long long)yy * W + xx, fx.to_fixed((aa ? ly : 1.f - ly) * (cc ? lx : 1.f - lx) * gcj));
+                }
+        }
+    }
+}
+
+// out[0] = sum of part[0..n) in a fixed order (one CTA: strided per-thread sums, then a fixed tree)
+__global__ void __launch_bounds__(256) nlspn_sum_kernel(const float *__restrict__ part, int n, float *__restrict__ out) {
+    __shared__ float red[256];
+    float s = 0.f;
+    for (int i = threadIdx.x; i < n; i += 256) s += part[i];
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int h = 128; h > 0; h >>= 1) {
+        if (threadIdx.x < h) red[threadIdx.x] += red[threadIdx.x + h];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) out[0] = red[0];
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -876,6 +937,89 @@ __global__ void nlspn_bwd_final_kernel(const float *__restrict__ g0, const float
         out[i] = (fix && __ldg(fix + i) > 0.f) ? 0.f : g0[i];
 }
 
+// Deterministic propagation backward (RDFC_DETERMINISTIC), per iteration t = T..1:
+//   nlspn_bwd_det_scatter_kernel   acc += fixed(A^T g_t) with 2^k from the bound P * max_p sum_k |aff_k[p]| * max |g_t|
+//                                  (no tap crosses an image boundary, the four bilinear weights of a tap sum to 1)
+//   nlspn_bwd_det_finalize_kernel  g_{t-1} = float(acc), then for t-1 >= 1 the finalisation of nlspn_bwd_scatter_kernel
+//                                  ((1 - mask_fix), + grad_inter), acc = 0 for the next iteration, max |g_{t-1}|
+// am[0] = max_p sum_k |aff_k[p]|, am[t] = max |g_t| after its finalisation.
+__global__ void __launch_bounds__(256) nlspn_bwd_det_scatter_kernel(const float *__restrict__ g, const float *__restrict__ offset,
+                                                                    const float *__restrict__ aff, long long *__restrict__ acc,
+                                                                    const unsigned long long *__restrict__ am_aff,
+                                                                    const unsigned long long *__restrict__ am_g, int H, int W) {
+    const long long P = (long long)H * W;
+    const int b = blockIdx.y;
+    const long long pix = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (pix >= P) return;
+    const float gv = g[(long long)b * P + pix];
+    if (gv == 0.f) return;
+    const unsigned long long am[2] = {*am_aff, *am_g};
+    const Fx<float> fx((double)P, am, 2);
+    const int y = (int)(pix / W), x = (int)(pix - (long long)y * W);
+    const float *offp = offset + (long long)b * 18 * P + pix;
+    const float *affp = aff + (long long)b * 9 * P + pix;
+    long long *gim = acc + (long long)b * P;
+#pragma unroll
+    for (int k = 0; k < 9; ++k) {
+        const float sy = (float)(y - 1 + k / 3) + __ldg(offp + (long long)(2 * k) * P);
+        const float sx = (float)(x - 1 + k % 3) + __ldg(offp + (long long)(2 * k + 1) * P);
+        const BwdPos q = bwd_pos(sy, sx, H, W);
+        if (!q.valid) continue;
+        const float top = gv * __ldg(affp + (long long)k * P);
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                const int yy = q.yl + a, xx = q.xl + c;
+                if (yy >= 0 && yy <= H - 1 && xx >= 0 && xx <= W - 1)
+                    fx_add(gim + (long long)yy * W + xx, fx.to_fixed((a ? q.ly : 1.f - q.ly) * (c ? q.lx : 1.f - q.lx) * top));
+            }
+    }
+}
+
+// acc == NULL: g already holds the raw values (t = T).  src_aff, src_g: the two maxima of the scatter that filled acc.  fix / ginter as in
+// nlspn_bwd_scatter_kernel's finalisation (NULL: not applied).  am_out: max |result| (NULL: not needed).  aff != NULL: also
+// am_aff = max_p sum_k |aff_k[p]|.  Grid-stride over the B*P pixels (whole warps, for the maxima).
+__global__ void __launch_bounds__(256) nlspn_bwd_det_finalize_kernel(long long *__restrict__ acc, const unsigned long long *__restrict__ src_aff,
+                                                                     const unsigned long long *__restrict__ src_g,
+                                                                     float *__restrict__ g, const float *__restrict__ fix,
+                                                                     const float *__restrict__ ginter, unsigned long long *__restrict__ am_out,
+                                                                     const float *__restrict__ aff, unsigned long long *__restrict__ am_aff,
+                                                                     long long P, long long BP) {
+    unsigned long long m = 0, ma = 0;
+    float dn1 = 1.f, dn2 = 1.f;
+    bool ok = true;
+    if (acc) {
+        const unsigned long long src[2] = {*src_aff, *src_g};
+        const Fx<float> fx((double)P, src, 2);
+        dn1 = fx.dn1; dn2 = fx.dn2; ok = fx.ok;
+    }
+    for (long long o = (long long)blockIdx.x * 256 + threadIdx.x; o < BP; o += (long long)gridDim.x * 256) {
+        float gv;
+        if (acc) {
+            gv = ok ? __ll2float_rn(acc[o]) * dn1 * dn2 : __int_as_float(0x7fffffff);
+            acc[o] = 0;
+        } else {
+            gv = g[o];
+        }
+        if (fix && __ldg(fix + o) > 0.f) gv = 0.f;
+        if (ginter) gv += __ldg(ginter + o);
+        g[o] = gv;
+        const unsigned long long bits = fx_bits(gv);
+        m = bits > m ? bits : m;
+        if (aff) {
+            const long long b = o / P, pix = o - b * P;
+            float sa = 0.f;
+#pragma unroll
+            for (int k = 0; k < 9; ++k) sa += fabsf(__ldg(aff + (b * 9 + k) * P + pix));
+            const unsigned long long ab = fx_bits(sa);
+            ma = ab > ma ? ab : ma;
+        }
+    }
+    if (am_out) fx_warp_max(m, am_out);
+    if (aff) fx_warp_max(ma, am_aff);
+}
+
 extern "C" int rdfc_nlspn_affinity_backward(const float *guidance, const float *confidence, const float *conv_w, const float *conv_b,
                                             const float *aff_scale, int affinity, int conf_prop, const float *offset,
                                             const float *grad_offset, const float *grad_aff, float *grad_conv, float *grad_confidence,
@@ -888,10 +1032,65 @@ extern "C" int rdfc_nlspn_affinity_backward(const float *guidance, const float *
     if (conf_prop) RDFC_CUDA(cudaMemsetAsync(grad_confidence, 0, sizeof(float) * (size_t)B * H * W, st));
     if (grad_aff_scale) RDFC_CUDA(cudaMemsetAsync(grad_aff_scale, 0, sizeof(float), st));
     dim3 grid(cdiv(W, TX), cdiv(H, TY), B), block(TX, TY);
-    nlspn_affinity_bwd_kernel<<<grid, block, 0, st>>>(guidance, confidence, conv_w, conv_b, aff_scale, affinity, conf_prop, offset,
-                                                      grad_offset, grad_aff, grad_conv, grad_confidence, grad_aff_scale, H, W);
+    nlspn_affinity_bwd_kernel<false><<<grid, block, 0, st>>>(guidance, confidence, conv_w, conv_b, aff_scale, affinity, conf_prop, offset,
+                                                             grad_offset, grad_aff, grad_conv, grad_confidence, grad_aff_scale, H, W,
+                                                             nullptr, nullptr);
     RDFC_CHECK_LAUNCH("nlspn_affinity_bwd_kernel");
     return 0;
+}
+
+// RDFC_DETERMINISTIC: the confidence scatter in fixed point (per-tap values, their maximum, then the scatter and the conversion),
+// dL/d aff_scale as per-CTA partials summed in a fixed order.  Workspace: stream-ordered, freed before returning.
+static int affinity_backward_det(const float *guidance, const float *confidence, const float *conv_w, const float *conv_b,
+                                 const float *aff_scale, int affinity, int conf_prop, const float *offset, const float *grad_offset,
+                                 const float *grad_aff, float *grad_conv, float *grad_confidence, float *grad_aff_scale, int B, int H,
+                                 int W, cudaStream_t st) {
+    const long long P = (long long)H * W, BP = (long long)B * P;
+    dim3 grid(cdiv(W, TX), cdiv(H, TY), B), block(TX, TY);
+    const long long nctas = (long long)grid.x * grid.y * grid.z;
+    // [am: 1 u64][acc: B*P i64][g_tap: 8*B*P f32][partials: nctas f32]
+    const size_t acc_off = 8, tap_off = acc_off + 8 * (size_t)(conf_prop ? BP : 0), part_off = tap_off + 4 * (size_t)(conf_prop ? 8 * BP : 0);
+    char *ws = nullptr;
+    RDFC_CUDA(cudaMallocAsync((void **)&ws, part_off + 4 * (size_t)nctas, st));
+    unsigned long long *am = (unsigned long long *)ws;
+    long long *acc = (long long *)(ws + acc_off);
+    float *g_tap = (float *)(ws + tap_off), *part = (float *)(ws + part_off);
+    int rc = 0;
+    if (cudaMemsetAsync(ws, 0, tap_off, st) != cudaSuccess) rc = fail(RDFC_ERR_CUDA, "rdfc_nlspn_affinity_backward_ex: memset failed");
+    if (rc == 0) {
+        nlspn_affinity_bwd_kernel<true><<<grid, block, 0, st>>>(guidance, confidence, conv_w, conv_b, aff_scale, affinity, conf_prop, offset,
+                                                                grad_offset, grad_aff, grad_conv, nullptr, grad_aff_scale ? part : nullptr,
+                                                                H, W, g_tap, am);
+        count_launch();
+    }
+    if (rc == 0 && conf_prop) {
+        nlspn_conf_scatter_det_kernel<<<dim3((unsigned)cdiv(P, 256), (unsigned)B), 256, 0, st>>>(g_tap, offset, acc, am, H, W);
+        count_launch();
+        rc = fx_convert<float>(acc, grad_confidence, BP, 8.0 * (double)P, am, 1, st);
+    }
+    if (rc == 0 && grad_aff_scale) {
+        nlspn_sum_kernel<<<1, 256, 0, st>>>(part, (int)nctas, grad_aff_scale);
+        count_launch();
+    }
+    if (rc == 0 && cudaGetLastError() != cudaSuccess) rc = fail(RDFC_ERR_CUDA, "rdfc_nlspn_affinity_backward_ex: kernel launch failed");
+    cudaFreeAsync(ws, st);
+    return rc;
+}
+
+extern "C" int rdfc_nlspn_affinity_backward_ex(const float *guidance, const float *confidence, const float *conv_w, const float *conv_b,
+                                               const float *aff_scale, int affinity, int conf_prop, const float *offset,
+                                               const float *grad_offset, const float *grad_aff, float *grad_conv, float *grad_confidence,
+                                               float *grad_aff_scale, int B, int H, int W, void *stream, int flags) {
+    RDFC_REQUIRE((flags & ~RDFC_DETERMINISTIC) == 0, "rdfc_nlspn_affinity_backward_ex: unknown flags 0x%x", flags);
+    if (!(flags & RDFC_DETERMINISTIC))
+        return rdfc_nlspn_affinity_backward(guidance, confidence, conv_w, conv_b, aff_scale, affinity, conf_prop, offset, grad_offset,
+                                            grad_aff, grad_conv, grad_confidence, grad_aff_scale, B, H, W, stream);
+    RDFC_REQUIRE(guidance && conv_w && conv_b && aff_scale && offset && grad_offset && grad_aff && grad_conv, "NULL pointer argument");
+    RDFC_REQUIRE(!conf_prop || (confidence && grad_confidence), "conf_prop requires confidence and grad_confidence");
+    RDFC_REQUIRE(B > 0 && H > 0 && W > 0 && B <= 65535, "bad shape (%d,%d,%d)", B, H, W);
+    RDFC_REQUIRE(affinity >= RDFC_AFF_AS && affinity <= RDFC_AFF_TGASS, "unknown affinity mode %d", affinity);
+    return affinity_backward_det(guidance, confidence, conv_w, conv_b, aff_scale, affinity, conf_prop, offset, grad_offset, grad_aff,
+                                 grad_conv, grad_confidence, grad_aff_scale, B, H, W, (cudaStream_t)stream);
 }
 
 extern "C" int rdfc_nlspn_propagate_backward(const float *grad_out, const float *grad_inter, const float *feat_init,
@@ -933,6 +1132,66 @@ extern "C" int rdfc_nlspn_propagate_backward(const float *grad_out, const float 
         nlspn_bwd_coord_kernel<false><<<grid, 256, 0, st>>>(feat_init, inter, fix, G, offset, aff, grad_offset, grad_aff, B, H, W, T);
     RDFC_CHECK_LAUNCH("nlspn_bwd_coord_kernel");
     return 0;
+}
+
+// RDFC_DETERMINISTIC: phase 1 as fixed-point scatters into one int64 plane, converted and finalised per iteration; phase 2 and the
+// final kernel as in rdfc_nlspn_propagate_backward.  Workspace: stream-ordered, freed before returning.
+static int propagate_backward_det(const float *grad_out, const float *grad_inter, const float *feat_init, const float *inter,
+                                  const float *offset, const float *aff, const float *fix, float *grad_feat_init, float *grad_offset,
+                                  float *grad_aff, float *G, int B, int H, int W, int T, cudaStream_t st) {
+    const long long P = (long long)H * W, BP = (long long)B * P;
+    // [am: T + 1 u64][acc: B*P i64]
+    char *ws = nullptr;
+    RDFC_CUDA(cudaMallocAsync((void **)&ws, 8 * ((size_t)T + 1 + (size_t)BP), st));
+    unsigned long long *am = (unsigned long long *)ws;
+    long long *acc = (long long *)(ws + 8 * ((size_t)T + 1));
+    int rc = 0;
+    if (cudaMemsetAsync(ws, 0, 8 * ((size_t)T + 1 + (size_t)BP), st) != cudaSuccess ||
+        cudaMemcpyAsync(G + (long long)T * BP, grad_out, sizeof(float) * BP, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+        rc = fail(RDFC_ERR_CUDA, "rdfc_nlspn_propagate_backward_ex: memset / copy failed");
+    const int nblk = fx_blocks(BP);
+    const dim3 grid((unsigned)cdiv(P, 256), (unsigned)B);
+    if (rc == 0) {          // g_T: the last iteration's output is not blended, only list_feat's gradient is added; + max sum |aff|
+        nlspn_bwd_det_finalize_kernel<<<nblk, 256, 0, st>>>(nullptr, nullptr, nullptr, G + (long long)T * BP, nullptr,
+                                                            grad_inter ? grad_inter + (long long)(T - 1) * BP : nullptr, am + T, aff, am, P, BP);
+        count_launch();
+    }
+    for (int t = T; t >= 1 && rc == 0; --t) {
+        nlspn_bwd_det_scatter_kernel<<<grid, 256, 0, st>>>(G + (long long)t * BP, offset, aff, acc, am, am + t, H, W);
+        const bool fin = t - 1 >= 1;
+        nlspn_bwd_det_finalize_kernel<<<nblk, 256, 0, st>>>(acc, am, am + t, G + (long long)(t - 1) * BP, fin ? fix : nullptr,
+                                                            (fin && grad_inter) ? grad_inter + (long long)(t - 2) * BP : nullptr,
+                                                            fin ? am + t - 1 : nullptr, nullptr, nullptr, P, BP);
+        count_launch(2);
+    }
+    if (rc == 0) {
+        nlspn_bwd_final_kernel<<<nblk, 256, 0, st>>>(G, fix, grad_feat_init, BP);
+        if (fix)
+            nlspn_bwd_coord_kernel<true><<<grid, 256, 0, st>>>(feat_init, inter, fix, G, offset, aff, grad_offset, grad_aff, B, H, W, T);
+        else
+            nlspn_bwd_coord_kernel<false><<<grid, 256, 0, st>>>(feat_init, inter, fix, G, offset, aff, grad_offset, grad_aff, B, H, W, T);
+        count_launch(2);
+    }
+    if (rc == 0 && cudaGetLastError() != cudaSuccess) rc = fail(RDFC_ERR_CUDA, "rdfc_nlspn_propagate_backward_ex: kernel launch failed");
+    cudaFreeAsync(ws, st);
+    return rc;
+}
+
+extern "C" int rdfc_nlspn_propagate_backward_ex(const float *grad_out, const float *grad_inter, const float *feat_init,
+                                                const float *inter, const float *offset, const float *aff, const float *feat_fix,
+                                                int preserve_input, float *grad_feat_init, float *grad_offset, float *grad_aff,
+                                                float *scratch, int B, int H, int W, int prop_time, void *stream, int flags) {
+    RDFC_REQUIRE((flags & ~RDFC_DETERMINISTIC) == 0, "rdfc_nlspn_propagate_backward_ex: unknown flags 0x%x", flags);
+    // T == 0 copies and zero-fills: nothing to scatter
+    if (!(flags & RDFC_DETERMINISTIC) || prop_time == 0)
+        return rdfc_nlspn_propagate_backward(grad_out, grad_inter, feat_init, inter, offset, aff, feat_fix, preserve_input, grad_feat_init,
+                                             grad_offset, grad_aff, scratch, B, H, W, prop_time, stream);
+    RDFC_REQUIRE(grad_out && feat_init && offset && aff && grad_feat_init && grad_offset && grad_aff && scratch, "NULL pointer argument");
+    RDFC_REQUIRE(!preserve_input || feat_fix, "preserve_input requires feat_fix (nlspn_model.py:157-158)");
+    RDFC_REQUIRE(B > 0 && H > 0 && W > 0 && prop_time > 0 && B <= 65535, "bad shape (%d,%d,%d) x %d", B, H, W, prop_time);
+    RDFC_REQUIRE(prop_time <= 1 || inter, "the backward needs the forward's intermediate results (inter)");
+    return propagate_backward_det(grad_out, grad_inter, feat_init, inter, offset, aff, preserve_input ? feat_fix : nullptr, grad_feat_init,
+                                  grad_offset, grad_aff, scratch, B, H, W, prop_time, (cudaStream_t)stream);
 }
 
 extern "C" int rdfc_fuse_depth_forward(const float *d1, const float *c1, const float *d2, const float *c2,

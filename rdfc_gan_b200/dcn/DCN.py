@@ -2,7 +2,8 @@
 
 Same six names, same positional signatures, same return conventions (fresh contiguous NCHW tensors; backward returns
 a list), same RuntimeError conditions -- but the work is done by librdfc_b200.so through its C ABI
-(include/rdfc_b200.h: rdfc_dcn_forward / rdfc_dcn_backward).  ``install()`` registers this module as
+(include/rdfc_b200.h: rdfc_dcn_forward / rdfc_dcn_backward; under torch.use_deterministic_algorithms the backward calls
+rdfc_dcn_backward_ex with RDFC_DETERMINISTIC, whose grad_input scatter is bit-reproducible).  ``install()`` registers this module as
 ``sys.modules['DCN']`` so the reference's unmodified ``modulated_deform_conv_func.py`` / ``nlspn_model.py`` import it.
 """
 import sys
@@ -81,9 +82,9 @@ def _backward(input, weight, bias, offset, mask, grad_output, *geo):
     grad_weight = torch.empty_like(weight)
     grad_bias = torch.empty_like(bias)
     with torch.cuda.device(input.device):
-        C.check(C.lib.rdfc_dcn_backward(C.ptr(input), C.ptr(weight), C.ptr(offset), C.ptr(mask), C.ptr(grad_output),
-                                        C.ptr(grad_input), C.ptr(grad_offset), C.ptr(grad_mask), C.ptr(grad_weight),
-                                        C.ptr(grad_bias), s, C.dtype_code(input), C.stream_ptr(input.device)))
+        C.backward_call("rdfc_dcn_backward", C.ptr(input), C.ptr(weight), C.ptr(offset), C.ptr(mask), C.ptr(grad_output),
+                        C.ptr(grad_input), C.ptr(grad_offset), C.ptr(grad_mask), C.ptr(grad_weight),
+                        C.ptr(grad_bias), s, C.dtype_code(input), C.stream_ptr(input.device))
     return grad_input, grad_offset, grad_mask, grad_weight, grad_bias
 
 

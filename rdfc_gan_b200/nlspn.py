@@ -4,7 +4,9 @@ Same constructor arguments, parameter names / shapes (state_dict compatible: ``a
 ``w_conf``, ``conv_offset_aff.{weight,bias}``), asserts and return tuples.  The forward pass runs two fused sm_100a
 kernels through the C ABI (rdfc_nlspn_affinity_forward, rdfc_nlspn_propagate_forward) instead of the reference's
 26 DCN calls + ~25 ATen kernels; with gradients enabled the same two stages run as two differentiable ops whose
-backwards are fused kernels as well (rdfc_nlspn_affinity_backward, rdfc_nlspn_propagate_backward).  There is no CPU
+backwards are fused kernels as well (rdfc_nlspn_affinity_backward, rdfc_nlspn_propagate_backward).  Under
+torch.use_deterministic_algorithms the backwards call their _ex variants with RDFC_DETERMINISTIC: fixed-point scatters,
+bit-reproducible gradients.  There is no CPU
 path and no re-statement of the reference's per-call composition: configurations the fused kernels do not cover
 (``prop_kernel != 3``, guidance with other than 8 channels, non-fp32 tensors) raise.
 """
@@ -51,10 +53,11 @@ class _PropagateFused(torch.autograd.Function):
         g_feat, g_off, g_aff = torch.empty_like(feat_init), torch.empty_like(offset), torch.empty_like(aff)
         scratch = torch.empty((prop_time + 1,) + tuple(feat_init.shape), dtype=torch.float32, device=feat_init.device)
         with torch.cuda.device(feat_init.device):
-            C.check(C.lib.rdfc_nlspn_propagate_backward(
+            C.backward_call(
+                "rdfc_nlspn_propagate_backward",
                 C.ptr(grad_out), C.ptr(g_inter), C.ptr(feat_init), C.ptr(inter), C.ptr(offset), C.ptr(aff),
                 C.ptr(fix) if has_fix else None, int(preserve), C.ptr(g_feat), C.ptr(g_off), C.ptr(g_aff), C.ptr(scratch),
-                B, H, W, prop_time, C.stream_ptr(feat_init.device)))
+                B, H, W, prop_time, C.stream_ptr(feat_init.device))
         return g_feat, g_off, g_aff, None, None, None
 
 
@@ -88,10 +91,11 @@ class _AffinityFused(torch.autograd.Function):
         g_conf = torch.empty((B, 1, H, W), dtype=torch.float32, device=guidance.device) if has_conf else None
         g_scale = torch.empty((1,), dtype=torch.float32, device=guidance.device) if affinity == 'TGASS' else None
         with torch.cuda.device(guidance.device):
-            C.check(C.lib.rdfc_nlspn_affinity_backward(
+            C.backward_call(
+                "rdfc_nlspn_affinity_backward",
                 C.ptr(guidance), C.ptr(conf) if has_conf else None, C.ptr(weight), C.ptr(bias), C.ptr(scale), C.AFFINITY[affinity],
                 int(conf_prop and has_conf), C.ptr(offset), C.ptr(g_offset.contiguous()), C.ptr(g_aff.contiguous()), C.ptr(g_conv),
-                C.ptr(g_conf), C.ptr(g_scale), B, H, W, C.stream_ptr(guidance.device)))
+                C.ptr(g_conf), C.ptr(g_scale), B, H, W, C.stream_ptr(guidance.device))
         need = ctx.needs_input_grad
         g_guid = torch.nn.grad.conv2d_input(guidance.shape, weight, g_conv, padding=1) if need[0] else None
         g_w = torch.nn.grad.conv2d_weight(guidance, weight.shape, g_conv, padding=1) if need[2] else None
