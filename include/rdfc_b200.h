@@ -365,6 +365,16 @@ int rdfc_conv_forward_split(const rdfc_conv_desc *d, void *stream);
 long long rdfc_conv_wgrad_split_workspace_floats(const rdfc_wgrad_desc *d);
 int rdfc_conv_wgrad_split(const rdfc_wgrad_desc *d, const float *inv_scale, float *grad_weight, float *workspace, void *stream);
 
+/* nn.ReflectionPad2d / nn.ReplicationPad2d of ResnetGenerator (G_B2A) on NHWC views: bf16 or fp32 (one dtype per call), any channel
+ * count, the same channel count in both views, pointers aligned to their elements (16-byte chunks are used where the channel count,
+ * the pixel strides and the pointers allow).  Invalid arguments fail before any launch. */
+typedef enum { RDFC_PAD_REFLECT = 0, RDFC_PAD_REPLICATE = 1 } rdfc_pad_mode;
+/* out (B, H+2p, W+2p, C) = pad(x (B, H, W, C)); symmetric p on all four sides; reflect needs p < H and p < W (torch's rule) */
+int rdfc_pad_nhwc_forward(const rdfc_view *x, int B, int H, int W, int pad, int mode, const rdfc_view *out, void *stream);
+/* grad_in (B, H, W, C) = sum of grad_out over the padded positions that map to each pixel -- OVERWRITTEN, not accumulated.  A gather
+ * in a fixed order (rows, then columns, ascending; fp32 compensated sum, rounded once): bit-reproducible, no atomics. */
+int rdfc_pad_nhwc_backward(const rdfc_view *grad_out, int B, int H, int W, int pad, int mode, const rdfc_view *grad_in, void *stream);
+
 /* ------------------------------------------------------------------ ESANet guidance glue ---------------------- */
 /* The non-GEMM layers of RDF-GAN's global_guidance_module (F/lib/models/segmentator/esa_net/esa_net_one_modality.py:145-172,
  * decoder.py:137-191, model_utils.py:34-49,99-134; F = /root/reference/RDF-GAN); its GEMM-shaped layers go through

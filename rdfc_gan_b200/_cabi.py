@@ -14,6 +14,7 @@ ACT_NONE, ACT_RELU, ACT_LEAKY02, ACT_TANH, ACT_SIGMOID = range(5)
 PATH_SIMT_F32, PATH_UMMA_BF16, PATH_UMMA_F32X3 = 0, 1, 2
 AFFINITY = {"AS": 0, "ASS": 1, "TC": 2, "TGASS": 3}
 DETERMINISTIC = 1                         # flags of the *_ex backward entry points
+PAD_REFLECT, PAD_REPLICATE = 0, 1
 _DT = {torch.float32: F32, torch.float64: F64, torch.bfloat16: BF16, torch.float16: F16}
 
 c_int, c_void_p, c_float = ctypes.c_int, ctypes.c_void_p, ctypes.c_float
@@ -94,6 +95,8 @@ def _load():
     lib.rdfc_conv_wgrad_split_workspace_floats.argtypes = [ctypes.POINTER(WgradDesc)]
     lib.rdfc_conv_wgrad_split_workspace_floats.restype = ctypes.c_longlong
     lib.rdfc_conv_wgrad_split.argtypes = [ctypes.POINTER(WgradDesc), c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.rdfc_pad_nhwc_forward.argtypes = [VP] + [c_int] * 5 + [VP, c_void_p]
+    lib.rdfc_pad_nhwc_backward.argtypes = [VP] + [c_int] * 5 + [VP, c_void_p]
     lib.rdfc_first_conv_forward.argtypes = [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, VP, c_void_p]
     lib.rdfc_maxpool3x3s2_forward.argtypes = [VP, VP, c_int, c_int, c_int, c_void_p]
     lib.rdfc_se_weights.argtypes = [c_void_p] * 6 + [c_int, c_int, c_int, c_void_p]
@@ -136,7 +139,8 @@ EXPORTS = ["rdfc_abi_version", "rdfc_last_error", "rdfc_launch_count", "rdfc_dcn
            "rdfc_conv_wgrad_workspace_floats", "rdfc_conv_wgrad", "rdfc_first_conv_forward", "rdfc_maxpool3x3s2_forward", "rdfc_se_weights",
            "rdfc_adaptive_avgpool_forward", "rdfc_upsample_nearest_forward", "rdfc_upsample_dw_forward",
            "rdfc_split_scaled", "rdfc_conv_forward_split", "rdfc_conv_wgrad_split_workspace_floats", "rdfc_conv_wgrad_split",
-           "rdfc_dcn_backward_ex", "rdfc_nlspn_affinity_backward_ex", "rdfc_nlspn_propagate_backward_ex"]
+           "rdfc_dcn_backward_ex", "rdfc_nlspn_affinity_backward_ex", "rdfc_nlspn_propagate_backward_ex",
+           "rdfc_pad_nhwc_forward", "rdfc_pad_nhwc_backward"]
 
 
 KNOB_UNSET = -(1 << 63)

@@ -2,7 +2,7 @@
 
 What the reference gets from autograd + cuDNN inside ``conv_bn_relu`` / ``convt_bn_relu`` / torchvision ``BasicBlock`` in
 train() mode (encoder_decoder/common.py:29-61, encoder_decoder/encoder_decoder.py:39-59) becomes two autograd Functions over
-bf16 NHWC tensors:
+bf16 NHWC tensors (plus the reflection / replication padding of ResnetGenerator, ``pad_nhwc``):
 
 * ``conv2d_nhwc``   forward = ``rdfc_conv_forward`` (tcgen05 implicit GEMM); data gradient = the same kernel in one of the conv
                     forms, with a transformed filter (_Conv2dNHWC.backward); filter gradient = ``rdfc_conv_wgrad``.
@@ -223,3 +223,46 @@ def bn_act(y, bn, residual=None, act=C.ACT_NONE):
     """act(BatchNorm2d_train(y) + residual) over a bf16 or fp32 NHWC tensor (residual of the same dtype); ``bn`` is the nn.BatchNorm2d holding weight / bias and the
     running statistics (updated in place, as nn.BatchNorm2d.forward does in train mode)."""
     return _BNAct.apply(y, bn.weight, bn.bias, residual, act, bn.eps, bn)
+
+
+_PAD_MODES = {'reflect': C.PAD_REFLECT, 'replicate': C.PAD_REPLICATE}
+
+
+class _PadNHWC(torch.autograd.Function):
+    """Forward = ``rdfc_pad_nhwc_forward`` (a copy); backward = ``rdfc_pad_nhwc_backward``, a gather in a fixed order (no atomics):
+    reproducible under torch.use_deterministic_algorithms, where PyTorch's own CUDA backward of these pads raises."""
+    @staticmethod
+    def forward(ctx, x, pad, mode):
+        C.require_cuda(x)
+        x = _dense(x)
+        B, H, W, Cc = x.shape
+        out = torch.empty((B, H + 2 * pad, W + 2 * pad, Cc), dtype=x.dtype, device=x.device)
+        vx, vo = C.view(x), C.view(out)
+        with torch.cuda.device(x.device):
+            C.check(C.lib.rdfc_pad_nhwc_forward(ctypes.byref(vx), B, H, W, pad, mode, ctypes.byref(vo), C.stream_ptr(x.device)))
+        ctx.cfg = (B, H, W, pad, mode)
+        return out
+
+    @staticmethod
+    def backward(ctx, gy):
+        B, H, W, pad, mode = ctx.cfg
+        g = _dense(gy)
+        gx = torch.empty((B, H, W, g.shape[3]), dtype=g.dtype, device=g.device)
+        vg, vx = C.view(g), C.view(gx)
+        with torch.cuda.device(g.device):
+            C.check(C.lib.rdfc_pad_nhwc_backward(ctypes.byref(vg), B, H, W, pad, mode, ctypes.byref(vx), C.stream_ptr(g.device)))
+        return gx, None, None
+
+
+def pad_nhwc(x, pad, mode):
+    """F.pad(x, (p,) * 4, mode) over a bf16 or fp32 NHWC tensor (B, H, W, C) -> (B, H + 2p, W + 2p, C).  ``pad``: p, or the 4-tuple
+    (left, right, top, bottom) of nn.ReflectionPad2d / nn.ReplicationPad2d.padding, all four equal; ``mode``: 'reflect' or
+    'replicate'.  The forward is a copy (bit for bit F.pad); the backward is a deterministic gather."""
+    if mode not in _PAD_MODES:
+        raise ValueError(f"pad mode must be 'reflect' or 'replicate', got {mode!r}")
+    p = (pad,) * 4 if isinstance(pad, int) else tuple(pad)
+    if len(p) != 4 or len(set(p)) != 1:
+        raise RuntimeError(f"pad_nhwc pads all four sides alike, got padding {pad}")
+    if x.dtype not in (torch.bfloat16, torch.float32):
+        raise RuntimeError(f"pad_nhwc takes bf16 or fp32 tensors, not {x.dtype}")
+    return _PadNHWC.apply(x, int(p[0]), _PAD_MODES[mode])
