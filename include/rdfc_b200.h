@@ -329,6 +329,14 @@ int rdfc_affine_act_forward(const rdfc_view *x, const float *scale, const float 
 int rdfc_bn_act_backward(const rdfc_view *dout, const rdfc_view *out, const rdfc_view *y, const float *mean, const float *rstd,
                          const float *gamma, int act, const rdfc_view *dy, const rdfc_view *dres, float *workspace,
                          float *sum_dz, float *sum_dz_xhat, long long npix, void *stream);
+/* Backward of a FROZEN BatchNorm (running statistics) folded into its conv, out = act(s * y + t + residual):
+ *   dz = dout * act'(out)  (act' from the sign of `out`; written when dz is not NULL),   sum_dz[c] = sum dz (= d beta).
+ * act: none / ReLU / LeakyReLU(0.2); with RDFC_ACT_NONE, `out` is not read (may be NULL) and dz may be NULL: dout is then dz and
+ * only the sum is computed; an activation needs dz.  dout / out / dz: NHWC views of one dtype (bf16 or fp32), C % 8 == 0,
+ * 16-byte aligned; workspace: rdfc_bn_workspace_floats(npix, C) floats.  Per-CTA partials summed in a fixed order (no atomics):
+ * bit-reproducible. */
+int rdfc_bn_frozen_backward(const rdfc_view *dout, const rdfc_view *out, int act, const rdfc_view *dz, float *workspace, float *sum_dz,
+                            long long npix, void *stream);
 
 /* Filter gradient of y = conv2d(input, W (O, I, k, k), stride, padding (k-1)/2):
  *   grad_weight[o][i][ky][kx] = sum_{b,py,px} grad_out[b,py,px,o] * input[b, stride*py - pad + ky, stride*px - pad + kx, i]
@@ -356,7 +364,9 @@ int rdfc_conv_wgrad(const rdfc_wgrad_desc *d, float *grad_weight, float *workspa
 int rdfc_split_scaled(const rdfc_view *x, long long npix, const rdfc_view *out, float *factor, void *stream);
 /* rdfc_conv_forward on an already split input: d->in = the RDFC_F16 [hi | lo] view (2 Cin channels), d->path =
  * RDFC_PATH_UMMA_F32X3 (weight = that path's [W_hi ; W_lo ; W_hi] packing, of the filter scaled by its own power of two),
- * d->out fp32 NHWC, d->scale REQUIRED: the per-Cout factor 1 / (s_x s_w) that undoes the scaling; no residual, no workspace. */
+ * d->out fp32 NHWC, d->scale REQUIRED: the per-Cout factor 1 / (s_x s_w) that undoes the scaling (times a folded BatchNorm's
+ * scale, if any); d->shift, d->act as rdfc_conv_forward; d->residual NULL or an fp32 NHWC view of Cout channels (16-byte aligned,
+ * pixel stride % 8 == 0); no second source, no workspace. */
 int rdfc_conv_forward_split(const rdfc_conv_desc *d, void *stream);
 /* Filter gradient of split operands: d->grad_out / d->input = RDFC_F16 [hi | lo] views (2 O / 2 I channels) of s_g * grad_out and
  * s_x * input; inv_scale = device float 1 / (s_g s_x).  The three products g_hi x_hi, g_hi x_lo, g_lo x_hi run on the tcgen05

@@ -87,6 +87,7 @@ def _load():
     lib.rdfc_affine_act_forward.argtypes = [VP, c_void_p, c_void_p, VP, c_int, VP, ctypes.c_longlong, c_void_p]
     lib.rdfc_bn_act_backward.argtypes = [VP, VP, VP, c_void_p, c_void_p, c_void_p, c_int, VP, VP, c_void_p, c_void_p, c_void_p,
                                          ctypes.c_longlong, c_void_p]
+    lib.rdfc_bn_frozen_backward.argtypes = [VP, VP, c_int, VP, c_void_p, c_void_p, ctypes.c_longlong, c_void_p]
     lib.rdfc_conv_wgrad_workspace_floats.argtypes = [ctypes.POINTER(WgradDesc)]
     lib.rdfc_conv_wgrad_workspace_floats.restype = ctypes.c_longlong
     lib.rdfc_conv_wgrad.argtypes = [ctypes.POINTER(WgradDesc), c_void_p, c_void_p, c_void_p]
@@ -140,7 +141,7 @@ EXPORTS = ["rdfc_abi_version", "rdfc_last_error", "rdfc_launch_count", "rdfc_dcn
            "rdfc_adaptive_avgpool_forward", "rdfc_upsample_nearest_forward", "rdfc_upsample_dw_forward",
            "rdfc_split_scaled", "rdfc_conv_forward_split", "rdfc_conv_wgrad_split_workspace_floats", "rdfc_conv_wgrad_split",
            "rdfc_dcn_backward_ex", "rdfc_nlspn_affinity_backward_ex", "rdfc_nlspn_propagate_backward_ex",
-           "rdfc_pad_nhwc_forward", "rdfc_pad_nhwc_backward"]
+           "rdfc_pad_nhwc_forward", "rdfc_pad_nhwc_backward", "rdfc_bn_frozen_backward"]
 
 
 KNOB_UNSET = -(1 << 63)

@@ -57,8 +57,10 @@ extern "C" int rdfc_conv_forward_split(const rdfc_conv_desc *d, void *stream) {
     RDFC_REQUIRE(d->path == RDFC_PATH_UMMA_F32X3, "conv (split input): path must be RDFC_PATH_UMMA_F32X3");
     RDFC_REQUIRE(d->in.dtype == RDFC_F16 && !d->in.nchw && d->in.C % 64 == 0,
                  "conv (split input): an fp16 [hi | lo] view with 2 x Cin channels, Cin %% 32 == 0, expected (got %d channels)", d->in.C);
-    RDFC_REQUIRE(d->out.dtype == RDFC_F32 && !d->out.nchw && !d->in2.ptr && !d->residual.ptr,
-                 "conv (split input): fp32 NHWC output, no second source, no residual");
+    RDFC_REQUIRE(d->out.dtype == RDFC_F32 && !d->out.nchw && !d->in2.ptr, "conv (split input): fp32 NHWC output, no second source");
+    RDFC_REQUIRE(!d->residual.ptr || (d->residual.dtype == RDFC_F32 && !d->residual.nchw && d->residual.C == d->out.C &&
+                                      d->residual.pix_stride % 8 == 0 && ((uintptr_t)d->residual.ptr % 16) == 0),
+                 "conv (split input): the residual must be an fp32 NHWC view with Cout channels, 16-byte aligned, pixel stride %% 8 == 0");
     RDFC_REQUIRE(d->scale != nullptr, "conv (split input): the per-Cout inverse scale vector is required");
     rdfc_conv_desc e = *d;
     e.in.dtype = RDFC_BF16;                 // 16-bit operands: the split path of the kernel reads them as fp16

@@ -1,5 +1,6 @@
 // Training-step kernels (SURVEY 8f rank 1): batch-statistics BatchNorm forward / backward fused with the activation and the
-// residual add, and the entry points of the convolution filter gradient (its tcgen05 kernel is in wgrad_umma.cu).
+// residual add, the backward of a frozen (running-statistics) BatchNorm folded into its conv, and the entry points of the
+// convolution filter gradient (its tcgen05 kernel is in wgrad_umma.cu).
 //
 // Replaces, for conv_bn_relu / convt_bn_relu / torchvision BasicBlock in train() mode (encoder_decoder/common.py:29-61,
 // encoder_decoder/encoder_decoder.py:39-59), what the reference leaves to cuDNN / ATen: nn.BatchNorm2d's batch statistics and
@@ -323,6 +324,63 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(View<T> dout, View<T>
     }
 }
 
+// ---- frozen BatchNorm backward: dz = dout * act'(out) (written when dz is not NULL), per-CTA partial sums of dz ------------
+template <typename T> __device__ __forceinline__ float rnd(float v);
+template <> __device__ __forceinline__ float rnd<float>(float v) { return v; }
+template <> __device__ __forceinline__ float rnd<__nv_bfloat16>(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+
+// Same grid and CTA layout as bn_bwd_partial_kernel; partial[blk][C] holds one float per channel, summed by sum1_final_kernel.
+template <typename T>
+__global__ void __launch_bounds__(256) bn_frozen_partial_kernel(View<T> dout, View<T> out, float slope, T *__restrict__ dz, int dz_stride,
+                                                                int C, long long npix, int per_blk, float *__restrict__ partial) {
+    __shared__ float red[32][8][9];
+    const int cg = threadIdx.x & 7, lane = threadIdx.x >> 3;
+    const int c0 = blockIdx.y * 64 + cg * 8;
+    const long long p0 = (long long)blockIdx.x * per_blk;
+    const long long p1 = p0 + per_blk < npix ? p0 + per_blk : npix;
+    const int n = (int)(p1 - p0);
+    float s[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) s[q] = 0.f;
+    if (c0 < C && n > 0) {
+#pragma unroll 1                                    // unrolled, the bf16 instantiation spills
+        for (int p = lane; p < n; p += 32) {
+            float g[8];
+            ld8(dout.ptr + (p0 + p) * dout.stride + c0, g);
+            if (out.ptr) {                      // an activation: its derivative from the sign of the output
+                float o[8];
+                ld8(out.ptr + (p0 + p) * out.stride + c0, o);
+#pragma unroll
+                for (int q = 0; q < 8; ++q) g[q] = rnd<T>(g[q] * dact(o[q], slope));
+            }
+            if (dz) st8(dz + (p0 + p) * dz_stride + c0, g);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) s[q] += g[q];      // the sum of dz as stored: d gamma = rstd (<W, G(dz)> - rm sum dz) cancels exactly
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < 8; ++q) red[lane][cg][q] = s[q];
+    __syncthreads();
+    if (threadIdx.x < 64) {
+        const int g2 = threadIdx.x >> 3, q = threadIdx.x & 7, c = blockIdx.y * 64 + g2 * 8 + q;
+        if (c < C) {
+            float ts = 0.f;
+            for (int l = 0; l < 32; ++l) ts += red[l][g2][q];
+            partial[(long long)blockIdx.x * C + c] = ts;
+        }
+    }
+}
+
+// one warp per channel: lane l sums blocks l, l + 32, ... in order (fp64), then a fixed butterfly
+__global__ void __launch_bounds__(256) sum1_final_kernel(const float *__restrict__ partial, int C, int nblk, float *__restrict__ s0) {
+    const int c = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (c >= C) return;
+    double a = 0.0;
+    for (int k = lane; k < nblk; k += 32) a += __ldg(partial + (long long)k * C + c);
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    if (lane == 0) s0[c] = (float)a;
+}
+
 }  // namespace
 }  // namespace rdfc
 
@@ -437,6 +495,37 @@ extern "C" int rdfc_bn_act_backward(const rdfc_view *dout, const rdfc_view *out,
     if (dt == RDFC_F32)
         return bn_act_backward<float>(dout, out, y, mean, rstd, gamma, act, dy, dres, workspace, sum_dz, sum_dz_xhat, npix, (cudaStream_t)stream);
     return bn_act_backward<__nv_bfloat16>(dout, out, y, mean, rstd, gamma, act, dy, dres, workspace, sum_dz, sum_dz_xhat, npix, (cudaStream_t)stream);
+}
+
+template <typename T>
+static int bn_frozen_backward(const rdfc_view *dout, const rdfc_view *out, int act, const rdfc_view *dz, float *workspace, float *sum_dz,
+                              long long npix, cudaStream_t st) {
+    const int C = dout->C;
+    int per;
+    const int nblk = red_blocks(npix, &per);
+    const View<T> o = act == RDFC_ACT_NONE ? View<T>{nullptr, 0} : mk<T>(out);
+    T *d = (dz && dz->ptr) ? (T *)dz->ptr : nullptr;
+    bn_frozen_partial_kernel<T><<<dim3(nblk, cdiv(C, 64)), 256, 0, st>>>(mk<T>(dout), o, act_slope(act), d, d ? dz->pix_stride : 0, C, npix,
+                                                                         per, workspace);
+    RDFC_CHECK_LAUNCH("bn_frozen_partial_kernel");
+    sum1_final_kernel<<<cdiv(C, 8), 256, 0, st>>>(workspace, C, nblk, sum_dz);
+    RDFC_CHECK_LAUNCH("sum1_final_kernel");
+    return 0;
+}
+
+extern "C" int rdfc_bn_frozen_backward(const rdfc_view *dout, const rdfc_view *out, int act, const rdfc_view *dz, float *workspace,
+                                       float *sum_dz, long long npix, void *stream) {
+    RDFC_REQUIRE(dout && workspace && sum_dz && npix > 0, "bn frozen backward: bad argument");
+    RDFC_REQUIRE(act == RDFC_ACT_NONE || act == RDFC_ACT_RELU || act == RDFC_ACT_LEAKY02,
+                 "bn frozen backward: none / ReLU / LeakyReLU(0.2) only");
+    const bool has_dz = dz && dz->ptr;
+    RDFC_REQUIRE(act == RDFC_ACT_NONE || has_dz, "bn frozen backward: an activation needs a dz destination");
+    const int C = dout->C, dt = dout->dtype;
+    if (int rc = check_view(dout, C, "bn frozen backward dout", dt)) return rc;
+    if (act != RDFC_ACT_NONE) if (int rc = check_view(out, C, "bn frozen backward out", dt)) return rc;
+    if (has_dz) if (int rc = check_view(dz, C, "bn frozen backward dz", dt)) return rc;
+    if (dt == RDFC_F32) return bn_frozen_backward<float>(dout, out, act, dz, workspace, sum_dz, npix, (cudaStream_t)stream);
+    return bn_frozen_backward<__nv_bfloat16>(dout, out, act, dz, workspace, sum_dz, npix, (cudaStream_t)stream);
 }
 
 // argument checks shared by the workspace query and the launch

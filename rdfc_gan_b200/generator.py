@@ -128,7 +128,8 @@ class _GeneratorBase(nn.Module):
 
     def _run(self, stem_in, depth):
         if self.training:
-            # train(): batch-statistics BatchNorm (running stats updated) and autograd, whatever the grad mode -- as the reference
+            # train(): autograd, whatever the grad mode, and each BatchNorm by its own flag (train(): batch statistics, running stats
+            # updated; eval(): frozen, running statistics) -- as the reference
             from .train_forward import generator_forward_train
             if self.bn is not True or self.fuse_kind not in ('WAdaIN', 'AdaIN', 'IN'):
                 raise NotImplementedError("training-mode forward covers bn=True generators")

@@ -6,8 +6,11 @@ Sequential of standard modules (state_dict keys ``model.<i>...`` load into / fro
 residual-block convs) and the two ConvTranspose2d(k3, s2, p1, op1) layers -- all with >= 64 input channels, > 97 % of the FLOPs --
 run on the tcgen05 conv kernel through ``train_ops.conv2d_nhwc`` (forward, data gradient, filter gradient), BatchNorm2d in train()
 mode on the fused batch-statistics kernels, the reflection / replication pads on ``train_ops.pad_nhwc`` (a copy forward, a
-fixed-order gather backward: reproducible under torch.use_deterministic_algorithms).  The two 7x7 convolutions (1 or 3 channels on
-one side), LeakyReLU(0.01) / PReLU / Tanh and eval-mode / instance normalisation are differentiable PyTorch ops on the same tensors.
+fixed-order gather backward: reproducible under torch.use_deterministic_algorithms).  Each BatchNorm2d follows its own flag, as in
+PyTorch: in a train()-mode generator, a frozen one (eval() mode, running statistics) after a tensor-core conv is folded into that
+conv (``train_ops.conv_bn_act_frozen``, no activation; its buffers stay untouched), and one after a 7x7 conv runs as the PyTorch
+module.  The two 7x7 convolutions (1 or 3 channels on one side), LeakyReLU(0.01) / PReLU / Tanh and eval-mode / instance
+normalisation are differentiable PyTorch ops on the same tensors.
 
 ``set_train_precision`` picks the activations' dtype: bf16 (default) or fp32 (``'fp32_tc'``: split-operand tensor-core convs, fp32
 BatchNorm, the 7x7 convs in true fp32 with TF32 off).  G_B2A has no separate inference engine, so the setting holds in train() and
@@ -20,7 +23,7 @@ import torch.nn.functional as F
 from . import _cabi as C
 from .generator import _GeneratorBase
 from .train_forward import _ConvFP32
-from .train_ops import bn_act, conv2d_nhwc, pad_nhwc
+from .train_ops import bn_act, bn_frozen, conv2d_nhwc, conv_bn_act_frozen, pad_nhwc
 
 
 def _nchw(t):
@@ -104,20 +107,29 @@ class ResnetGenerator(nn.Module):
         fp32 = dt == torch.float32
         def via_torch(mod, t):
             return mod(t.permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
-        prev = None
-        for m in seq:
+        mods = list(seq)
+        prev, fused = None, None
+        for i, m in enumerate(mods):
             after_pad, prev = isinstance(prev, (nn.ReflectionPad2d, nn.ReplicationPad2d)), m
+            if m is fused:                                               # folded into the conv before it
+                continue
             if isinstance(m, ResnetBlock):
                 x = x + self._walk(m.conv_block, x)
             elif isinstance(m, (nn.ReflectionPad2d, nn.ReplicationPad2d)):
                 x = pad_nhwc(x, m.padding, 'reflect' if isinstance(m, nn.ReflectionPad2d) else 'replicate')
             elif isinstance(m, (nn.Conv2d, nn.ConvTranspose2d)) and self._tc_ok(m, x) and (m.padding != (0, 0) or m.stride == (1, 1)):
-                if isinstance(m, nn.ConvTranspose2d):
-                    y = conv2d_nhwc(x, m.weight, 3, 2, transposed=True)
-                elif m.padding == (0, 0):        # the input was padded explicitly (reflection): zero-pad conv, then drop the border
-                    y = conv2d_nhwc(x, m.weight, 3, 1)[:, 1:-1, 1:-1]
+                nxt = mods[i + 1] if i + 1 < len(mods) else None
+                if self.training and m.bias is None and isinstance(nxt, nn.BatchNorm2d) and bn_frozen(nxt):
+                    fused = nxt                                          # conv + frozen BatchNorm in one launch
+                    conv = lambda t, k, s, tr=False: conv_bn_act_frozen(t, m.weight, nxt, k, s, tr)
                 else:
-                    y = conv2d_nhwc(x, m.weight, 3, m.stride[0])
+                    conv = lambda t, k, s, tr=False: conv2d_nhwc(t, m.weight, k, s, tr)
+                if isinstance(m, nn.ConvTranspose2d):
+                    y = conv(x, 3, 2, True)
+                elif m.padding == (0, 0):        # the input was padded explicitly (reflection): zero-pad conv, then drop the border
+                    y = conv(x, 3, 1)[:, 1:-1, 1:-1]
+                else:
+                    y = conv(x, 3, m.stride[0])
                 x = y if m.bias is None else (y.float() + m.bias).to(dt)
             elif isinstance(m, (nn.Conv2d, nn.ConvTranspose2d)):         # 7x7 / thin convs: fp32 cuDNN (true fp32 in fp32_tc)
                 xin = _nchw(x) if after_pad else x.permute(0, 3, 1, 2)
@@ -131,10 +143,10 @@ class ResnetGenerator(nn.Module):
                 else:
                     y = _ConvFP32.apply(xin, m.weight, m.bias, m.padding[0])
                 x = y.permute(0, 2, 3, 1).to(dt)
-            elif isinstance(m, nn.BatchNorm2d) and self.training and x.shape[3] % 8 == 0:
+            elif isinstance(m, nn.BatchNorm2d) and self.training and not bn_frozen(m) and x.shape[3] % 8 == 0:
                 x = bn_act(x.contiguous(), m, None, C.ACT_NONE)
             elif isinstance(m, (nn.BatchNorm2d, nn.InstanceNorm2d)):
-                x = via_torch(m, x.float()).to(dt)                      # eval-mode or instance normalisation: fp32 PyTorch
+                x = via_torch(m, x.float()).to(dt)                      # eval-mode / frozen or instance normalisation: fp32 PyTorch
             elif isinstance(m, nn.LeakyReLU):                            # not in place: the producer saved its output for backward
                 x = F.leaky_relu(x, m.negative_slope)
             elif isinstance(m, nn.PReLU):                                # fp32 slope parameter: evaluate in fp32

@@ -1,11 +1,14 @@
-"""Training-mode forward of the generator (batch-statistics BatchNorm, autograd), rdf_generator.py:280-414 /
+"""Training-mode forward of the generator (autograd), rdf_generator.py:280-414 /
 rdf_gan_generator.py:233-361, composed of the differentiable ops of train_ops.py over NHWC tensors: bf16 (the default training
 mode) or fp32 (the ``fp32_tc`` mode: split-operand tensor-core arithmetic in the ops, and the PyTorch convs that stay on cuDNN --
 stems, ``*_dec0`` heads -- run in true fp32, with TF32 off in their forward and backward).
 
 The convolutions with >= 32 input channels -- every encoder / decoder / ``*_dec1`` layer and the per-pixel EqualLinear of
-W-AdaIN, > 99 % of the FLOPs -- run forward, data gradient and filter gradient on this repo's kernels; BatchNorm (+ residual +
-activation) runs on the fused batch-statistics kernels; the NLSPN runs its fused forward / backward pair (nlspn.py).  The three
+W-AdaIN, > 99 % of the FLOPs -- run forward, data gradient and filter gradient on this repo's kernels.  Each BatchNorm decides for
+itself, as nn.BatchNorm2d does: one in train() mode (+ residual + activation) runs on the fused batch-statistics kernels and
+updates its running statistics; a frozen one (eval() mode with running statistics, ``bn_frozen``) is folded with its conv,
+residual and activation into one tcgen05 launch (``conv_bn_act_frozen``) and leaves its buffers alone.  The NLSPN runs its fused
+forward / backward pair (nlspn.py).  The three
 stems (3 / 1 input channels), the ``*_dec0`` heads (<= 8 output channels), the InstanceNorm + modulation of the fusion layers
 and the output fusion are differentiable PyTorch expressions on the same tensors.
 """
@@ -16,7 +19,7 @@ import torch.nn.functional as F
 
 from . import _cabi as C
 from .model_utils import IN, AdaIN, AdaptiveInstanceNorm
-from .train_ops import bn_act, conv2d_nhwc
+from .train_ops import bn_act, bn_frozen, conv2d_nhwc, conv_bn_act_frozen
 
 BF = torch.bfloat16
 
@@ -65,19 +68,25 @@ def _conv(x, w, b, padding, dt):
     return F.conv2d(x, w, b, padding=padding)
 
 
+def _conv_bn(x, weight, bn, k, stride, transposed=False, residual=None, act=C.ACT_NONE):
+    """act(bn(conv(x)) + residual): a frozen ``bn`` folded into the conv, else the conv, then the batch-statistics BatchNorm"""
+    if bn_frozen(bn):
+        return conv_bn_act_frozen(x, weight, bn, k, stride, transposed, residual, act)
+    return bn_act(conv2d_nhwc(x, weight, k, stride, transposed), bn, residual, act)
+
+
 def _conv_bn_act(x, seq, k=3, stride=1, transposed=False, act=C.ACT_LEAKY02, residual=None):
     """conv_bn_relu / convt_bn_relu Sequential (common.py:29-61): [0] conv (no bias with BN), [1] BatchNorm2d, LeakyReLU(0.2)."""
-    y = conv2d_nhwc(x, seq[0].weight, k, stride, transposed)
-    return bn_act(y, seq[1], residual, act)
+    return _conv_bn(x, seq[0].weight, seq[1], k, stride, transposed, residual, act)
 
 
 def _basic_block(x, blk):
     """torchvision BasicBlock: relu(bn2(conv2(relu(bn1(conv1(x))))) + identity)"""
     identity = x
     if blk.downsample is not None:
-        identity = bn_act(conv2d_nhwc(x, blk.downsample[0].weight, 1, blk.stride), blk.downsample[1], None, C.ACT_NONE)
-    out = bn_act(conv2d_nhwc(x, blk.conv1.weight, 3, blk.stride), blk.bn1, None, C.ACT_RELU)
-    return bn_act(conv2d_nhwc(out, blk.conv2.weight, 3, 1), blk.bn2, identity, C.ACT_RELU)
+        identity = _conv_bn(x, blk.downsample[0].weight, blk.downsample[1], 1, blk.stride)
+    out = _conv_bn(x, blk.conv1.weight, blk.bn1, 3, blk.stride, act=C.ACT_RELU)
+    return _conv_bn(out, blk.conv2.weight, blk.bn2, 3, 1, residual=identity, act=C.ACT_RELU)
 
 
 def _small_conv(x_nhwc, conv, act=None):
@@ -139,7 +148,7 @@ def _crop_cat(fd, fe):
 
 
 def generator_forward_train(g, stem_in, depth, dtype=BF):
-    """g: RDFGenerator / DCVGANGenerator (train mode).  stem_in (B, Cs, H, W), depth (B, 1, H, W) fp32 CUDA.  dtype: the activations'
+    """g: RDFGenerator / DCVGANGenerator (train mode; BatchNorms in eval() mode inside it use their running statistics).  stem_in (B, Cs, H, W), depth (B, 1, H, W) fp32 CUDA.  dtype: the activations'
     dtype, torch.bfloat16 (default) or torch.float32 (the fp32_tc training mode).
     -> (depth_map_1, confidence_map_1, depth_map_2, confidence_map_2, pred_depth), fp32 NCHW, attached to the autograd graph."""
     C.require_cuda(stem_in, depth)

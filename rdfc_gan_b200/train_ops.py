@@ -1,13 +1,17 @@
 """Differentiable building blocks of the TRAINING step on the sm_100a kernels (SURVEY 8f rank 1).
 
 What the reference gets from autograd + cuDNN inside ``conv_bn_relu`` / ``convt_bn_relu`` / torchvision ``BasicBlock`` in
-train() mode (encoder_decoder/common.py:29-61, encoder_decoder/encoder_decoder.py:39-59) becomes two autograd Functions over
+train() mode (encoder_decoder/common.py:29-61, encoder_decoder/encoder_decoder.py:39-59) becomes autograd Functions over
 bf16 NHWC tensors (plus the reflection / replication padding of ResnetGenerator, ``pad_nhwc``):
 
 * ``conv2d_nhwc``   forward = ``rdfc_conv_forward`` (tcgen05 implicit GEMM); data gradient = the same kernel in one of the conv
                     forms, with a transformed filter (_Conv2dNHWC.backward); filter gradient = ``rdfc_conv_wgrad``.
 * ``bn_act``        BatchNorm2d with BATCH statistics (+ running-stat update) fused with the residual add and the
-                    (Leaky)ReLU: ``rdfc_bn_stats`` + ``rdfc_affine_act_forward``; backward = ``rdfc_bn_act_backward``.
+                    (Leaky)ReLU: ``rdfc_bn_stats`` + ``rdfc_affine_act_forward``; backward = ``rdfc_bn_act_backward``.  For a
+                    BatchNorm in train() mode; nn.BatchNorm2d decides per module (``bn_frozen``).
+* ``conv_bn_act_frozen``  conv + a FROZEN BatchNorm2d (eval() mode: running statistics, no update) + residual + activation in
+                    one tcgen05 launch (the BatchNorm folded into the epilogue's per-channel scale / shift); backward =
+                    ``rdfc_bn_frozen_backward`` + the conv's data / filter gradients, without the pre-BatchNorm tensor.
 
 Both dispatch on the activation dtype.  bf16 is the default training mode.  fp32 tensors select the ``fp32_tc`` mode: the same
 conv forms, every contraction (forward, data gradient, filter gradient) on the tensor cores with split fp16 operands
@@ -22,9 +26,10 @@ the repo's kernels yet).
 import ctypes
 
 import torch
+import torch.nn.functional as F
 
 from . import _cabi as C
-from .engine import pack_weight
+from .engine import GeneratorEngine, pack_weight
 
 
 def _dense(t):
@@ -58,29 +63,37 @@ def _operand(t):
     return _split(t) if t.dtype == torch.float32 else (t, None)
 
 
-def _conv(x, sx, w_oihw, k, stride, transposed, out_hw):
-    """(x, sx) = _operand(input); w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) = conv(input, w), no bias / activation: bf16 from a bf16
-    input, fp32 from a split one (x_hi W_hi + x_hi W_lo + x_lo W_hi of the scaled operands, the inverse scales in the epilogue)."""
+def _conv(x, sx, w_oihw, k, stride, transposed, out_hw, fold=None, residual=None, act=C.ACT_NONE):
+    """(x, sx) = _operand(input); w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) = conv(input, w): bf16 from a bf16 input, fp32 from a
+    split one (x_hi W_hi + x_hi W_lo + x_lo W_hi of the scaled operands, the inverse scales in the epilogue).  Without ``fold``: no
+    bias / activation.  With ``fold`` = (s, t), fp32 (O,) device vectors: act(conv * s + t + residual) in the same launch
+    (``residual``: an NHWC tensor of the output's dtype and shape, or None)."""
     B, H, W, Cx = x.shape
     Cin, O = (Cx if sx is None else Cx // 2), w_oihw.shape[0]
     if Cin % 32 or O % 8 or w_oihw.shape[1] != Cin:
         raise RuntimeError(f"tensor-core conv needs Cin % 32 == 0 and Cout % 8 == 0, got {Cin} -> {O}")
     w = w_oihw.detach().float()
+    CoutP = (O + 15) // 16 * 16
     d = C.ConvDesc()
     d.B, d.Hi, d.Wi, d.Ho, d.Wo = B, H, W, out_hw[0], out_hw[1]
     d.kh = d.kw = k
-    d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, int(transposed), C.ACT_NONE
+    d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, int(transposed), act
     if sx is None:
-        packed, inv = pack_weight(w, umma=True), None
+        packed, scale = pack_weight(w, umma=True), None
         d.path, fn, dtype = C.PATH_UMMA_BF16, C.lib.rdfc_conv_forward, torch.bfloat16
     else:
         sw = _pow2_factor(w)
         packed = pack_weight(w * sw, umma=True, x3=True)                   # [W_hi ; W_lo ; W_hi] of the scaled filter
-        inv = (1.0 / (sx * sw)).expand((O + 15) // 16 * 16).contiguous()   # exact: powers of two
+        scale = (1.0 / (sx * sw)).expand(CoutP).contiguous()               # exact: powers of two
         d.path, fn, dtype = C.PATH_UMMA_F32X3, C.lib.rdfc_conv_forward_split, torch.float32
+    shift = None
+    if fold is not None:
+        s, t = (F.pad(v.float(), (0, CoutP - O)) for v in fold)
+        scale = s if scale is None else scale * s
+        shift = t.contiguous()
     out = torch.empty((B, out_hw[0], out_hw[1], O), dtype=dtype, device=x.device)
-    d.inp, d.in2, d.out, d.residual = C.view(x), C.view(None), C.view(out), C.view(None)
-    d.weight, d.scale, d.shift = packed.data_ptr(), None if inv is None else inv.data_ptr(), None
+    d.inp, d.in2, d.out, d.residual = C.view(x), C.view(None), C.view(out), C.view(residual)
+    d.weight, d.scale, d.shift = packed.data_ptr(), C.ptr(scale), C.ptr(shift)
     with torch.cuda.device(x.device):
         C.check(fn(ctypes.byref(d), C.stream_ptr(x.device)))
     return out
@@ -110,6 +123,15 @@ def _wgrad(grad_out, inp, k, stride, sg=None, sx=None):
     return gw
 
 
+def _conv_form(x, weight, k, stride, transposed):
+    """-> (output (Ho, Wo), the filter as (O, I, k, k)) of conv2d_nhwc's conv forms"""
+    B, H, W, _ = x.shape
+    if transposed:                      # ConvTranspose2d(k3, s2, p1, op1): weight (Cin, Cout, 3, 3), output exactly 2x
+        return (2 * H, 2 * W), weight.detach().permute(1, 0, 2, 3)
+    p = (k - 1) // 2
+    return ((H + 2 * p - k) // stride + 1, (W + 2 * p - k) // stride + 1), weight.detach()
+
+
 class _Conv2dNHWC(torch.autograd.Function):
     """The conv forms and their data-gradient transforms; the arithmetic follows the input's dtype (_operand).  In the fp32_tc mode the
     split input (as many bytes as the fp32 input) is kept for the filter gradient instead of the input itself."""
@@ -117,14 +139,7 @@ class _Conv2dNHWC(torch.autograd.Function):
     def forward(ctx, x, weight, k, stride, transposed):
         C.require_cuda(x, weight)
         x = _dense(x)
-        B, H, W, _ = x.shape
-        if transposed:                      # ConvTranspose2d(k3, s2, p1, op1): weight (Cin, Cout, 3, 3), output exactly 2x
-            out_hw = (2 * H, 2 * W)
-            w_oihw = weight.detach().permute(1, 0, 2, 3)
-        else:
-            p = (k - 1) // 2
-            out_hw = ((H + 2 * p - k) // stride + 1, (W + 2 * p - k) // stride + 1)
-            w_oihw = weight.detach()
+        out_hw, w_oihw = _conv_form(x, weight, k, stride, transposed)
         x, sx = _operand(x)
         ctx.save_for_backward(x, sx, weight)
         ctx.cfg = (k, stride, transposed)
@@ -135,30 +150,37 @@ class _Conv2dNHWC(torch.autograd.Function):
         x, sx, weight = ctx.saved_tensors
         k, stride, transposed = ctx.cfg
         g, sg = _operand(_dense(gy))
-        B, H, W = x.shape[:3]
         w = weight.detach()
         gx = gw = None
         if ctx.needs_input_grad[0]:
-            if transposed:                  # dgrad of the transposed conv = the stride-2 conv with the SAME filter (O = Cin, I = Cout)
-                gx = _conv(g, sg, w, 3, 2, False, (H, W))
-            elif k == 3 and stride == 1:    # flipped filter, (Cout, Cin) swapped
-                gx = _conv(g, sg, w.flip(2, 3).permute(1, 0, 2, 3), 3, 1, False, (H, W))
-            elif k == 3:                    # stride 2: the transposed conv with the same filter, cropped to the input size
-                gx = _conv(g, sg, w.permute(1, 0, 2, 3), 3, 2, True, (H, W))
-            else:                           # 1x1: W^T per pixel; stride 2 scatters onto the even grid
-                t = _conv(g, sg, w.permute(1, 0, 2, 3), 1, 1, False, tuple(gy.shape[1:3]))
-                if stride == 1:
-                    gx = t
-                else:
-                    gx = t.new_zeros((B, H, W, t.shape[3]))
-                    gx[:, ::2, ::2] = t
+            gx = _conv_dgrad(g, sg, w, k, stride, transposed, x.shape[:3])
         if ctx.needs_input_grad[1]:
-            if transposed:                  # roles exchanged: "gradient" = the layer's input, "input" = d(output), stride-2 form
-                gw = _wgrad(x, g, 3, 2, sx, sg)                # (Cin, Cout, 3, 3) = ConvTranspose2d's weight layout
-            else:
-                gw = _wgrad(g, x, k, stride, sg, sx)           # (Cout, Cin, k, k)
-            gw = gw.to(weight.dtype)
+            gw = _conv_wgrad(g, sg, x, sx, k, stride, transposed).to(weight.dtype)
         return gx, gw, None, None, None
+
+
+def _conv_dgrad(g, sg, w, k, stride, transposed, in_bhw):
+    """(g, sg) = _operand(d(output)); w: the layer's weight (as conv2d_nhwc takes it) -> d(input) (B, H, W, Cin) of that conv form."""
+    B, H, W = in_bhw
+    if transposed:                  # dgrad of the transposed conv = the stride-2 conv with the SAME filter (O = Cin, I = Cout)
+        return _conv(g, sg, w, 3, 2, False, (H, W))
+    if k == 3 and stride == 1:      # flipped filter, (Cout, Cin) swapped
+        return _conv(g, sg, w.flip(2, 3).permute(1, 0, 2, 3), 3, 1, False, (H, W))
+    if k == 3:                      # stride 2: the transposed conv with the same filter, cropped to the input size
+        return _conv(g, sg, w.permute(1, 0, 2, 3), 3, 2, True, (H, W))
+    t = _conv(g, sg, w.permute(1, 0, 2, 3), 1, 1, False, tuple(g.shape[1:3]))     # 1x1: W^T per pixel
+    if stride == 1:
+        return t
+    gx = t.new_zeros((B, H, W, t.shape[3]))                                       # stride 2 scatters onto the even grid
+    gx[:, ::2, ::2] = t
+    return gx
+
+
+def _conv_wgrad(g, sg, x, sx, k, stride, transposed):
+    """The unscaled filter gradient in the layer's weight layout, fp32: (Cout, Cin, k, k), or (Cin, Cout, 3, 3) for the transposed conv."""
+    if transposed:                  # roles exchanged: "gradient" = the layer's input, "input" = d(output), stride-2 form
+        return _wgrad(x, g, 3, 2, sx, sg)
+    return _wgrad(g, x, k, stride, sg, sx)
 
 
 def conv2d_nhwc(x, weight, k=3, stride=1, transposed=False):
@@ -221,8 +243,88 @@ class _BNAct(torch.autograd.Function):
 
 def bn_act(y, bn, residual=None, act=C.ACT_NONE):
     """act(BatchNorm2d_train(y) + residual) over a bf16 or fp32 NHWC tensor (residual of the same dtype); ``bn`` is the nn.BatchNorm2d holding weight / bias and the
-    running statistics (updated in place, as nn.BatchNorm2d.forward does in train mode)."""
+    running statistics (updated in place, as nn.BatchNorm2d.forward does in train mode).  Always BATCH statistics, whatever
+    ``bn.training`` says: the generators send a frozen BatchNorm (``bn_frozen``) to ``conv_bn_act_frozen`` instead."""
     return _BNAct.apply(y, bn.weight, bn.bias, residual, act, bn.eps, bn)
+
+
+def bn_frozen(bn):
+    """nn.BatchNorm2d's own rule: a BatchNorm in eval() mode that has running statistics normalises with them and updates nothing,
+    whatever mode its parent is in (the usual way to freeze BatchNorm while fine-tuning at a small batch)."""
+    return not bn.training and bn.running_mean is not None and bn.running_var is not None
+
+
+class _ConvBNActFrozen(torch.autograd.Function):
+    """out = act(s * conv(x, W) + t + residual) with the frozen BatchNorm's s = gamma rsqrt(rv + eps), t = beta - rm s (fp32, on the
+    device) in the conv's epilogue.  Saved: the conv's input operand (bf16 input or fp32_tc split), W, s, rstd, rm and -- with an
+    activation -- the output; not the pre-BatchNorm tensor.  Backward, with dz = dout act'(out) and G = the unscaled filter gradient
+    of dz: d beta = sum dz, d gamma = rstd (<W_c, G_c> - rm_c sum dz_c) (sum_p dz y = <W, G>: y is linear in W), dW = s_c G_c,
+    dx = the conv's data gradient of the filter W s applied to dz, d residual = dz."""
+    @staticmethod
+    def forward(ctx, x, weight, gamma, beta, residual, k, stride, transposed, act, bn):
+        C.require_cuda(x, weight, residual)
+        x = _dense(x)
+        out_hw, w_oihw = _conv_form(x, weight, k, stride, transposed)
+        rm = bn.running_mean.detach().float()
+        rstd = torch.rsqrt(bn.running_var.detach().float() + bn.eps)
+        s, t = GeneratorEngine._bn_fold(bn) if gamma is not None else (rstd, -rm * rstd)
+        res = None
+        if residual is not None:
+            res = _dense(residual)
+            want = (x.shape[0], out_hw[0], out_hw[1], w_oihw.shape[0])
+            if res.dtype != x.dtype or tuple(res.shape) != want:
+                raise RuntimeError(f"conv_bn_act_frozen: residual must be {x.dtype} of shape {want}, got {res.dtype} {tuple(res.shape)}")
+        xo, sx = _operand(x)
+        out = _conv(xo, sx, w_oihw, k, stride, transposed, out_hw, (s, t), res, act)
+        ctx.save_for_backward(xo, sx, weight, out if act != C.ACT_NONE else None, s, rstd, rm)
+        ctx.cfg = (k, stride, transposed, act, None if gamma is None else gamma.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        xo, sx, weight, out, s, rstd, rm = ctx.saved_tensors
+        k, stride, transposed, act, pdt = ctx.cfg
+        need_x, need_w, need_g, need_b, need_r = ctx.needs_input_grad[:5]
+        gout = _dense(gout)
+        B, H, W, Cc = gout.shape
+        npix, dev = B * H * W, gout.device
+        dz = gout if act == C.ACT_NONE else torch.empty(gout.shape, dtype=gout.dtype, device=dev)
+        ws = torch.empty(C.lib.rdfc_bn_workspace_floats(npix, Cc), dtype=torch.float32, device=dev)
+        sum_dz = torch.empty(Cc, device=dev)
+        vg, vo, vz = C.view(gout), C.view(out), C.view(dz)
+        with torch.cuda.device(dev):
+            C.check(C.lib.rdfc_bn_frozen_backward(ctypes.byref(vg), ctypes.byref(vo) if out is not None else None, act,
+                                                  ctypes.byref(vz) if act != C.ACT_NONE else None, C.ptr(ws), C.ptr(sum_dz), npix,
+                                                  C.stream_ptr(dev)))
+        w = weight.detach()
+        bshape = (1, -1, 1, 1) if transposed else (-1, 1, 1, 1)          # the BatchNorm channel: dim 1 of a ConvTranspose2d weight
+        gx = gw = gg = gb = None
+        if need_x or need_w or need_g:
+            g, sg = _operand(dz)
+        if need_w or need_g:
+            G = _conv_wgrad(g, sg, xo, sx, k, stride, transposed)
+            if need_w:
+                gw = (G * s.view(bshape)).to(weight.dtype)
+            if need_g:                      # the filter the forward multiplied: bf16-rounded in the bf16 mode
+                wq = w.float() if sx is not None else w.to(torch.bfloat16).float()
+                gg = (rstd * ((wq * G).sum((0, 2, 3) if transposed else (1, 2, 3)) - rm * sum_dz)).to(pdt)
+        if need_x:
+            gx = _conv_dgrad(g, sg, w.float() * s.view(bshape), k, stride, transposed, xo.shape[:3])
+        if need_b:
+            gb = sum_dz.to(pdt)
+        return gx, gw, gg, gb, (dz if need_r else None), None, None, None, None, None
+
+
+def conv_bn_act_frozen(x, weight, bn, k=3, stride=1, transposed=False, residual=None, act=C.ACT_NONE):
+    """act(BatchNorm2d_eval(conv(x, weight)) + residual): conv2d_nhwc's conv forms and precision (bf16 ``x``: bf16; fp32 ``x``: the
+    fp32_tc split-operand arithmetic) followed by the frozen BatchNorm ``bn`` -- its running statistics, which stay untouched --
+    the residual add and none / ReLU / LeakyReLU(0.2), in one tcgen05 launch.  gamma / beta may train (or not, requires_grad=False);
+    gradients follow the usual autograd rules for x, weight, gamma, beta and the residual."""
+    if not (bn.running_mean is not None and bn.running_var is not None):
+        raise RuntimeError("conv_bn_act_frozen needs a BatchNorm2d with running statistics")
+    if act not in (C.ACT_NONE, C.ACT_RELU, C.ACT_LEAKY02):
+        raise ValueError(f"conv_bn_act_frozen: activation none / ReLU / LeakyReLU(0.2), got {act}")
+    return _ConvBNActFrozen.apply(x, weight, bn.weight, bn.bias, residual, k, stride, transposed, act, bn)
 
 
 _PAD_MODES = {'reflect': C.PAD_REFLECT, 'replicate': C.PAD_REPLICATE}
