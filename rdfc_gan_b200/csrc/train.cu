@@ -317,7 +317,9 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(View<T> dout, View<T>
             const float dz = g[q] * dact(o[q], slope);
             const float rs = __ldg(rstd + c), xh = (v[q] - __ldg(mean + c)) * rs;
             dzv[q] = dz;
-            v[q] = __ldg(gamma + c) * rs * (dz - __ldg(sum_dz + c) * invn - xh * __ldg(sum_dzx + c) * invn);
+            // __fmul_rn: sum_dz / N rounded on its own, as the hoisted form's k1 is -- contracted into dz - sum_dz * invn, one fma
+            // would round once and the two forms would differ in the last bit
+            v[q] = __ldg(gamma + c) * rs * (dz - __fmul_rn(__ldg(sum_dz + c), invn) - xh * __ldg(sum_dzx + c) * invn);
         }
         st8(dy + p * dy_stride + c0, v);
         if (dres) st8(dres + p * dres_stride + c0, dzv);

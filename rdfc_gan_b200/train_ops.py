@@ -63,6 +63,14 @@ def _operand(t):
     return _split(t) if t.dtype == torch.float32 else (t, None)
 
 
+def _pad32(t):
+    """An NHWC tensor with its channels zero-padded to the next multiple of 32; t itself when C % 32 == 0.  The data gradient reads
+    d(output) as the conv kernel's input, and that kernel (and the fp32_tc split) takes Cin % 32 == 0 only, while the forward
+    accepts any Cout % 8 == 0."""
+    n = -t.shape[3] % 32
+    return F.pad(t, (0, n)) if n else t
+
+
 def _conv(x, sx, w_oihw, k, stride, transposed, out_hw, fold=None, residual=None, act=C.ACT_NONE):
     """(x, sx) = _operand(input); w_oihw (O, I, k, k) float -> (B, Ho, Wo, O) = conv(input, w): bf16 from a bf16 input, fp32 from a
     split one (x_hi W_hi + x_hi W_lo + x_lo W_hi of the scaled operands, the inverse scales in the epilogue).  Without ``fold``: no
@@ -149,19 +157,23 @@ class _Conv2dNHWC(torch.autograd.Function):
     def backward(ctx, gy):
         x, sx, weight = ctx.saved_tensors
         k, stride, transposed = ctx.cfg
-        g, sg = _operand(_dense(gy))
+        g, sg = _operand(_pad32(_dense(gy)))
         w = weight.detach()
         gx = gw = None
         if ctx.needs_input_grad[0]:
             gx = _conv_dgrad(g, sg, w, k, stride, transposed, x.shape[:3])
         if ctx.needs_input_grad[1]:
-            gw = _conv_wgrad(g, sg, x, sx, k, stride, transposed).to(weight.dtype)
+            gw = _conv_wgrad(g, sg, x, sx, k, stride, transposed, gy.shape[3]).to(weight.dtype)
         return gx, gw, None, None, None
 
 
 def _conv_dgrad(g, sg, w, k, stride, transposed, in_bhw):
-    """(g, sg) = _operand(d(output)); w: the layer's weight (as conv2d_nhwc takes it) -> d(input) (B, H, W, Cin) of that conv form."""
+    """(g, sg) = _operand(_pad32(d(output))); w: the layer's weight (as conv2d_nhwc takes it) -> d(input) (B, H, W, Cin) of that conv
+    form.  The filter's output channels are zero-padded to g's: the padded channels add exact zeros."""
     B, H, W = in_bhw
+    n = (g.shape[3] if sg is None else g.shape[3] // 2) - w.shape[1 if transposed else 0]
+    if n:
+        w = F.pad(w, (0, 0, 0, 0, 0, n) if transposed else (0, 0, 0, 0, 0, 0, 0, n))
     if transposed:                  # dgrad of the transposed conv = the stride-2 conv with the SAME filter (O = Cin, I = Cout)
         return _conv(g, sg, w, 3, 2, False, (H, W))
     if k == 3 and stride == 1:      # flipped filter, (Cout, Cin) swapped
@@ -176,16 +188,18 @@ def _conv_dgrad(g, sg, w, k, stride, transposed, in_bhw):
     return gx
 
 
-def _conv_wgrad(g, sg, x, sx, k, stride, transposed):
-    """The unscaled filter gradient in the layer's weight layout, fp32: (Cout, Cin, k, k), or (Cin, Cout, 3, 3) for the transposed conv."""
+def _conv_wgrad(g, sg, x, sx, k, stride, transposed, cout):
+    """The unscaled filter gradient in the layer's weight layout, fp32: (Cout, Cin, k, k), or (Cin, Cout, 3, 3) for the transposed conv
+    (the filters of the zero channels _pad32 added to g dropped)."""
     if transposed:                  # roles exchanged: "gradient" = the layer's input, "input" = d(output), stride-2 form
-        return _wgrad(x, g, 3, 2, sx, sg)
-    return _wgrad(g, x, k, stride, sg, sx)
+        return _wgrad(x, g, 3, 2, sx, sg)[:, :cout].contiguous()
+    return _wgrad(g, x, k, stride, sg, sx)[:cout]
 
 
 def conv2d_nhwc(x, weight, k=3, stride=1, transposed=False):
     """NHWC convolution (3x3 / 1x1, stride 1 / 2, padding (k-1)/2) or ConvTranspose2d(k3, s2, p1, op1) without bias.
-    bf16 ``x``: bf16 operands and result; fp32 ``x``: the fp32_tc split-operand arithmetic, fp32 result."""
+    bf16 ``x``: bf16 operands and result; fp32 ``x``: the fp32_tc split-operand arithmetic, fp32 result.  Cin % 32 == 0 and
+    Cout % 8 == 0, in the forward and the backward alike."""
     return _Conv2dNHWC.apply(x, weight, k, stride, transposed)
 
 
@@ -300,9 +314,9 @@ class _ConvBNActFrozen(torch.autograd.Function):
         bshape = (1, -1, 1, 1) if transposed else (-1, 1, 1, 1)          # the BatchNorm channel: dim 1 of a ConvTranspose2d weight
         gx = gw = gg = gb = None
         if need_x or need_w or need_g:
-            g, sg = _operand(dz)
+            g, sg = _operand(_pad32(dz))
         if need_w or need_g:
-            G = _conv_wgrad(g, sg, xo, sx, k, stride, transposed)
+            G = _conv_wgrad(g, sg, xo, sx, k, stride, transposed, Cc)
             if need_w:
                 gw = (G * s.view(bshape)).to(weight.dtype)
             if need_g:                      # the filter the forward multiplied: bf16-rounded in the bf16 mode
@@ -319,7 +333,8 @@ def conv_bn_act_frozen(x, weight, bn, k=3, stride=1, transposed=False, residual=
     """act(BatchNorm2d_eval(conv(x, weight)) + residual): conv2d_nhwc's conv forms and precision (bf16 ``x``: bf16; fp32 ``x``: the
     fp32_tc split-operand arithmetic) followed by the frozen BatchNorm ``bn`` -- its running statistics, which stay untouched --
     the residual add and none / ReLU / LeakyReLU(0.2), in one tcgen05 launch.  gamma / beta may train (or not, requires_grad=False);
-    gradients follow the usual autograd rules for x, weight, gamma, beta and the residual."""
+    gradients follow the usual autograd rules for x, weight, gamma, beta and the residual.  Cin % 32 == 0 and Cout % 8 == 0, in the
+    forward and the backward alike."""
     if not (bn.running_mean is not None and bn.running_var is not None):
         raise RuntimeError("conv_bn_act_frozen needs a BatchNorm2d with running statistics")
     if act not in (C.ACT_NONE, C.ACT_RELU, C.ACT_LEAKY02):

@@ -111,7 +111,9 @@ def test_frozen_rule():
 # ------------------------------------------------------------------------------------------------ per op, GPU
 # B, Cin, Cout, H, W, k, stride, transposed
 FORMS = [(2, 64, 64, 20, 28, 3, 1, False), (2, 64, 128, 21, 27, 3, 2, False), (1, 96, 64, 17, 23, 1, 1, False),
-         (2, 64, 128, 14, 15, 1, 2, False), (2, 128, 64, 10, 13, 3, 2, True)]
+         (2, 64, 128, 14, 15, 1, 2, False), (2, 128, 64, 10, 13, 3, 2, True),
+         # Cout % 32 != 0: dz reaches the data gradient's kernel zero-padded to 32-channel multiples
+         (2, 64, 24, 20, 28, 3, 1, False), (2, 96, 48, 10, 13, 3, 2, True)]
 ACTS = {0: "none", 1: "relu", 2: "leaky02"}
 # Relative L2 against fp64 autograd.  bf16: one bf16 rounding of the output and of dz (measured <= 1.7e-3 output, 2.4e-3 dx,
 # <= 3.5e-4 elsewhere).  fp32_tc: the split-operand contraction (measured <= 3.0e-6 output / dx, <= 2.9e-7 dW / d gamma / d beta).
@@ -204,7 +206,7 @@ def _op_case(form, dtype, act, with_res, gen, sliced=False, big_mean=False, trai
 
 @gpu
 @pytest.mark.parametrize("dtype", [BF, torch.float32], ids=["bf16", "fp32_tc"])
-@pytest.mark.parametrize("form", FORMS, ids=lambda f: f"{f[5]}x{f[5]}s{f[6]}{'T' if f[7] else ''}")
+@pytest.mark.parametrize("form", FORMS, ids=lambda f: f"{f[5]}x{f[5]}s{f[6]}{'T' if f[7] else ''}" + (f"o{f[2]}" if f[2] % 32 else ""))
 def test_conv_bn_act_frozen_against_fp64(form, dtype):
     """Every conv form x every activation x residual on / off: output and the gradients of x, W, gamma, beta and the residual;
     the BatchNorm's running_mean / running_var / num_batches_tracked bit-identical afterwards."""
@@ -243,10 +245,15 @@ def test_conv_bn_act_frozen_special_cases(dtype):
 @pytest.mark.parametrize("dtype", [BF, torch.float32], ids=["bf16", "fp32"])
 def test_frozen_backward_kernel(dtype):
     """rdfc_bn_frozen_backward against torch: dz = dout act'(out) and sum dz over channel-slice views, for every activation; with
-    ACT_NONE and no dz only the sum; three calls bit-identical."""
+    ACT_NONE and no dz only the sum; three calls bit-identical.  Also at the training benchmark's 16 x 228 x 304, where one
+    reduction block sums ~1 900 pixels instead of 64, with 64 and 96 channels (measured sum dz <= 2.1e-7 there)."""
     from rdfc_gan_b200 import _cabi as C
     gen = torch.Generator(device="cuda").manual_seed(1)
-    B, H, W, Cc = 3, 37, 45, 96
+    for B, H, W, Cc in ((3, 37, 45, 96), (16, 228, 304, 64), (16, 228, 304, 96)):
+        _frozen_backward_case(C, B, H, W, Cc, dtype, gen)
+
+
+def _frozen_backward_case(C, B, H, W, Cc, dtype, gen):
     dout = torch.randn(B, H, W, Cc + 32, device="cuda", generator=gen).to(dtype)[..., 32:]
     outb = torch.randn(B, H, W, Cc + 16, device="cuda", generator=gen).to(dtype)[..., :Cc]
     npix = B * H * W
@@ -265,6 +272,7 @@ def test_frozen_backward_kernel(dtype):
             runs.append((None if dz is None else dz.clone(), s.clone()))
         if act:
             assert torch.equal(runs[0][0], dz_want)
+        _dump({"case": f"frozen_backward_{B}x{H}x{W}x{Cc}_{act}_{dtype}", "errs": {"sum_dz": _rel(runs[0][1], sum_want)}})
         assert _rel(runs[0][1], sum_want) <= 1e-6, _rel(runs[0][1], sum_want)
         assert all(torch.equal(r[1], runs[0][1]) and (r[0] is None or torch.equal(r[0], runs[0][0])) for r in runs)
 

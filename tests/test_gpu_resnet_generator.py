@@ -272,11 +272,15 @@ def test_fp32_tc_matches_fp32_composition(monkeypatch):
 @gpu
 def test_fp32_tc_refuses_convs_off_the_tensor_cores():
     """ngf = 48: the stride-2 conv reads 48 channels, which the tensor-core conv does not take -- fp32_tc raises instead of running a
-    cuDNN conv; bf16 keeps its fp32 PyTorch route for such layers."""
+    cuDNN conv; bf16 keeps its fp32 PyTorch route for that layer, and trains (forward and backward) the 96 -> 48 transposed conv,
+    whose 48 output channels the tensor-core conv takes, on the tensor cores."""
     from rdfc_gan_b200.resnet_generator import ResnetGenerator
     G = ResnetGenerator(1, 3, ngf=48, n_blocks=1).cuda().train()
     x = torch.rand(1, 1, 32, 32, device="cuda")
-    assert torch.isfinite(G(x)).all()
+    y = G(x)
+    assert torch.isfinite(y).all()
+    y.square().sum().backward()
+    assert all(p.grad is not None and torch.isfinite(p.grad).all() for p in G.parameters())
     G.set_train_precision('fp32_tc')
     with pytest.raises(RuntimeError, match="input channels % 32 == 0"):
         G(x)

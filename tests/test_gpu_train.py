@@ -9,6 +9,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from _channel_cases import THIN_BN_CASES, THIN_COUT_CASES
+
 pytestmark = pytest.mark.gpu
 BF = torch.bfloat16
 
@@ -23,14 +25,20 @@ def _rel(a, b):
     (2, 64, 128, 40, 41, 1, 2), (2, 96, 160, 17, 23, 3, 1), (1, 512, 512, 15, 19, 3, 1), (4, 64, 64, 228, 304, 3, 1),
     (2, 192, 64, 29, 38, 3, 2), (1, 128, 256, 58, 77, 3, 2), (2, 256, 80, 9, 100, 3, 1),
     # Cout % 16 == 8: the kernel's N is rounded up to 16, the channels past Cout are zero fill and masked
-    (2, 64, 24, 36, 52, 3, 1), (2, 64, 40, 29, 38, 3, 2), (1, 128, 8, 15, 19, 1, 1), (2, 96, 24, 20, 28, 1, 2)])
+    (2, 64, 24, 36, 52, 3, 1), (2, 64, 40, 29, 38, 3, 2), (1, 128, 8, 15, 19, 1, 1), (2, 96, 24, 20, 28, 1, 2),
+    # an input of 8 / 24 / 40 channels: one partial 64-channel block of the input, the channels past it TMA zero fill
+    (2, 24, 64, 20, 28, 3, 2), (2, 40, 96, 17, 23, 3, 2), (2, 8, 64, 15, 19, 3, 2), (1, 40, 128, 15, 19, 3, 1), (2, 24, 32, 20, 28, 1, 1),
+    # the input as channels [0, 96) of a 128-channel tensor: the second 64-channel block is partial, and the 32 channels past it in
+    # memory hold data the kernel must not read
+    (2, 96, 64, 29, 38, 3, 1, 128)])
 def test_filter_gradient_against_torch(case):
     from rdfc_gan_b200.train_ops import _wgrad
-    B, Cin, Cout, H, W, k, s = case
+    B, Cin, Cout, H, W, k, s = case[:7]
+    pitch = case[7] if len(case) > 7 else Cin                   # the input's channel pitch: Cin, or a wider tensor it is a slice of
     g = torch.Generator(device="cuda").manual_seed(sum(case))
     p = (k - 1) // 2
     Ho, Wo = (H + 2 * p - k) // s + 1, (W + 2 * p - k) // s + 1
-    x = torch.randn(B, H, W, Cin, device="cuda", generator=g).to(BF)
+    x = torch.randn(B, H, W, pitch, device="cuda", generator=g).to(BF)[..., :Cin]
     gy = torch.randn(B, Ho, Wo, Cout, device="cuda", generator=g).to(BF)
     got = _wgrad(gy, x, k, s)
     want = torch.nn.grad.conv2d_weight(x.permute(0, 3, 1, 2).double(), (Cout, Cin, k, k), gy.permute(0, 3, 1, 2).double(), stride=s, padding=p)
@@ -52,10 +60,11 @@ def test_filter_gradient_against_torch(case):
 
 
 @pytest.mark.parametrize("case", [(2, 64, 64, 20, 28, 3, 1, False), (2, 64, 128, 21, 27, 3, 2, False), (2, 128, 64, 10, 13, 3, 2, True),
-                                  (1, 192, 384, 9, 12, 1, 1, False), (2, 64, 128, 14, 15, 1, 2, False)])
+                                  (1, 192, 384, 9, 12, 1, 1, False), (2, 64, 128, 14, 15, 1, 2, False)] + THIN_COUT_CASES)
 def test_conv_function_gradients(case):
     """conv2d_nhwc forward, data gradient (forward kernel with transformed filters) and filter gradient against autograd of
-    F.conv2d / F.conv_transpose2d on the same bf16-rounded tensors."""
+    F.conv2d / F.conv_transpose2d on the same bf16-rounded tensors.  Cout % 32 != 0 included: the data gradient reads d(output),
+    zero-padded to 32-channel multiples, as the kernel's input."""
     from rdfc_gan_b200.train_ops import conv2d_nhwc
     B, Cin, Cout, H, W, k, s, tr = case
     g = torch.Generator(device="cuda").manual_seed(sum(case[:7]) + 3)
@@ -127,7 +136,8 @@ def test_conv_function_rejects_cin_off_the_tensor_core_rule(dtype):
     assert C.launch_count() == n0
 
 
-@pytest.mark.parametrize("case", [(2, 19, 27, 64, 1, True), (3, 12, 10, 128, 2, False), (1, 30, 44, 32, 0, True), (2, 114, 152, 64, 2, True)])
+@pytest.mark.parametrize("case", [(2, 19, 27, 64, 1, True), (3, 12, 10, 128, 2, False), (1, 30, 44, 32, 0, True), (2, 114, 152, 64, 2, True)]
+                         + THIN_BN_CASES)
 def test_batchnorm_activation_function(case):
     """bn_act = act(BatchNorm2d_train(y) + residual): outputs, running statistics and the gradients w.r.t. y, gamma, beta and the
     residual against nn.BatchNorm2d + autograd in fp64 on the same bf16-rounded input."""

@@ -13,6 +13,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from _channel_cases import THIN_BN_CASES, THIN_COUT_CASES
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 gpu = pytest.mark.gpu
 
@@ -104,7 +106,7 @@ CONV_CASES = [(2, 64, 64, 36, 52, 3, 1, False), (3, 64, 128, 37, 50, 3, 2, False
               (1, 512, 512, 15, 19, 3, 1, False), (4, 64, 64, 228, 304, 3, 1, False), (2, 192, 64, 29, 38, 3, 2, False),
               (1, 128, 256, 58, 77, 3, 2, False), (2, 256, 96, 9, 100, 3, 1, False),
               (2, 64, 64, 20, 28, 3, 1, False), (2, 64, 128, 21, 27, 3, 2, False), (2, 128, 64, 10, 13, 3, 2, True),
-              (1, 192, 384, 9, 12, 1, 1, False), (2, 64, 128, 14, 15, 1, 2, False), (2, 256, 128, 29, 38, 3, 2, True)]
+              (1, 192, 384, 9, 12, 1, 1, False), (2, 64, 128, 14, 15, 1, 2, False), (2, 256, 128, 29, 38, 3, 2, True)] + THIN_COUT_CASES
 # Relative L2 bounds.  Forward and data gradient: the tensor cores' fp32 accumulation costs ~5e-9 per unit of the contraction length
 # K (measured 4.9e-9 .. 5.2e-9 x K on every case, K = Cin k^2 forward, Cout k^2 data gradient; 2.3e-5 at 512 -> 512 3x3, <= 8.7e-6
 # elsewhere), so the bound is twice that with K = max(Cin, Cout) k^2.  Filter gradient (K = pixels, split-K partials summed in
@@ -162,11 +164,14 @@ def test_conv_fp32_against_fp64(case):
     assert float(x.grad.abs().max()) == 0.0 and float(w.grad.abs().max()) == 0.0
 
 
-BN_BOUND = 4e-7            # relative L2 of every quantity: measured <= 1.8e-7 (running statistics), <= 1.5e-7 (gradients)
+# relative L2 of every quantity: measured <= 1.8e-7 (running statistics), <= 1.5e-7 (gradients).  One case is close to the bound, not
+# at half of it: the running statistics of 320 channels over 126 pixels, measured 2.8e-7
+BN_BOUND = 4e-7
 
 
 @gpu
-@pytest.mark.parametrize("case", [(2, 19, 27, 64, 1, True), (3, 12, 10, 128, 2, False), (1, 30, 44, 32, 0, True), (2, 114, 152, 64, 2, True)])
+@pytest.mark.parametrize("case", [(2, 19, 27, 64, 1, True), (3, 12, 10, 128, 2, False), (1, 30, 44, 32, 0, True), (2, 114, 152, 64, 2, True)]
+                         + THIN_BN_CASES)
 def test_batchnorm_activation_fp32_against_fp64(case):
     """bn_act on fp32 NHWC tensors (and a channel-sliced input) against nn.BatchNorm2d + autograd in fp64 on the same tensors:
     outputs, running statistics, and the gradients w.r.t. y, gamma, beta and the residual."""
