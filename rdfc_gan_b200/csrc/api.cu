@@ -35,6 +35,18 @@ int sm_count() {
     return n;
 }
 
+TmapEncodeFn tmap_encoder() {
+    static const TmapEncodeFn fn = [] {
+        cudaDriverEntryPointQueryResult q;
+        void *p = nullptr;
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                        q == cudaDriverEntryPointSuccess;
+        (void)cudaGetLastError();
+        return ok ? (TmapEncodeFn)p : nullptr;
+    }();
+    return fn;
+}
+
 // Development knobs (RDFC_* environment variables): read ONCE per name, then served from a table, so no launch path calls
 // getenv; rdfc_dev_set_knob overrides a value at run time (tests sweep the NLSPN band halo that way).
 static std::mutex g_knob_mu;

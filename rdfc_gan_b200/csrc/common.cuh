@@ -1,5 +1,6 @@
 // Shared helpers for librdfc_b200.so (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdarg.h>
@@ -39,6 +40,13 @@ static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b)
 
 // number of SMs of the current device (cached)
 int sm_count();
+
+// cuTensorMapEncodeTiled through the runtime's driver entry point query, so that the library links only cudart; nullptr if
+// the driver does not provide it
+typedef CUresult (*TmapEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
+                                 const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+TmapEncodeFn tmap_encoder();
 
 // development knob `name` (an RDFC_* environment variable, read once and cached; rdfc_dev_set_knob overrides it), or dflt
 constexpr long long KNOB_UNSET = (long long)0x8000000000000000ull;

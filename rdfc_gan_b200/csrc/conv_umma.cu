@@ -19,8 +19,8 @@
 //                   plane (input leaves L2 ~1.2x, not 9x).  Stride-2 layers load the four input-parity planes with
 //                   element stride 2; a transposed conv enumerates its four output phases as separate tiles, each a
 //                   1/2/2/4-tap conv over the input grid.
-//                   (warps 0-5 are cp.async producers of a no-swizzle [cin/8][pixel][16 B] layout when RDFC_UMMA_TMA=0,
-//                   and the im2col builders of the fused input stems.)
+//                   (warps 0-5 are the im2col builders of the fused input stems, which stage a no-swizzle
+//                   [cin/8][pixel][16 B] layout.)
 //       warp 7      B loader: one stage = the pre-packed (32-cin, BN) filter blocks of all nine taps of a k-block (3x3 convs
 //                   with N <= 128; one filter row = 3 taps when two such stages do not fit), cp.async.bulk (TMA 1-D) issued
 //                   by all lanes.
@@ -46,14 +46,15 @@ constexpr int KCH = BK / 8;       // 16-byte cin chunks per stage
 constexpr int TH = 16;            // tile rows (= 8-row groups of one M=128 MMA)
 // 16 warps: the register file is split per scheduler (16K registers each), so 4 warps per scheduler leave 128
 // registers per thread; 18 warps (5 on two schedulers) would cap every thread at 96 and spill the epilogue.
-constexpr int NPROD_WARPS = 6, NPROD = NPROD_WARPS * 32;   // A producer threads (warps 0-5)
+constexpr int NPROD_WARPS = 6, NPROD = NPROD_WARPS * 32;   // A producer threads of the stems (warps 0-5)
 constexpr int PIXPASS = NPROD / 4;                         // pixels staged per pass of the producer threads (48)
-constexpr int JMAX = 24;          // pixel slots per producer thread and k-block: a stage holds <= JMAX * PIXPASS pixels
 constexpr int MMA_WARP = 6, BLOAD_WARP = 7, EPI_WARP0 = 8, NEPI_WARPS = 8;
 constexpr int MMA2_WARP = 5;       // second MMA issuer (TMA mode only, where warps 1-5 have no staging work); another scheduler than MMA_WARP
 constexpr int NTHREADS = 16 * 32;
 constexpr int MAX_PLANES = 4, MAX_TAPS = 9;
-constexpr int BAR_BYTES = (3 * 8 + 3 * 16 + 4 + 4) * 8 + 16;   // mbarriers for <= 8 A stages, <= 16 B stages, 2+2 accumulator sets, 4 residual slabs; TMEM slot
+// mbarriers for <= 8 A stages, <= 16 B stages, 2+2 accumulator sets, 4 residual slabs; TMEM slot.  The last 192 bytes are
+// unused: they keep `fixed` in the tile planner, and with it the stage counts every layer was tuned with, as they are.
+constexpr int BAR_BYTES = (2 * 8 + 2 * 16 + 4 + 4) * 8 + 16 + 192;
 constexpr int EPI_SLAB_BYTES = 128 * 64;      // one staged epilogue slab: 128 pixels x 32 bf16 channels
 
 struct Plane {
@@ -87,13 +88,13 @@ struct Params {
     int split_c;                   // C (input channels of the layer) when split, else 0
     int out_f32;
     int dual;                      // two MMA issuer warps (MMA_WARP and MMA2_WARP), each owning a subset of the accumulators
-    int pair;                      // cta_group::2: two CTAs (a cluster) work on two pixel tiles with ONE stream of M = 256 MMAs; each
-                                   // holds its own A stages and HALF of every filter stage (per-SM shared-memory reads per MMA: 4 KB + N*16 B)
     int fast9;                     // nacc == 1, gtaps == 9, TMA operands, one phase: the MMA warp issues a stage as one statement (RDFC_UMMA_FAST9)
     int epi_split;                 // one-accumulator tiles: the two epilogue groups share the accumulator's column steps (RDFC_UMMA_EPISPLIT)
     int kbs;                       // 1x1 convs: 32-channel k-blocks per A stage (plane j = channels 32 j.. of the same pixels, tap j = its filter block)
-    int a_tma, px16, a_plane_bytes, a_tx_bytes;   // a_tx_bytes: bytes the TMA loads of one stage deliver (planes x rows x cols x 64)
-    int _pad_tma;   // px16: 16-byte units per staged pixel (4 with TMA: [pixel][64 B]; 1: [cin/8][pixel][16 B])
+    // a_tma: the A operand arrives through tmap_a (every layer but the stems, whose producers build it);
+    // a_tx_bytes: bytes the TMA loads of one stage deliver (planes x rows x cols x 64)
+    int a_tma, px16, a_plane_bytes, a_tx_bytes;
+    int _pad_tma;   // px16: 16-byte units per staged pixel (4 with TMA: [pixel][64 B]; 1 in the stems: [cin/8][pixel][16 B])
     const __nv_bfloat16 *in;
     int in_stride, B, Hi, Wi;
     int Ht, Wt, tiles_y, tiles_x, n_tiles_n, nphases, ntiles;   // tile space
@@ -105,7 +106,7 @@ struct Params {
     int res_stride;
     const float *scale, *shift;
     int act, nacc, nax, bn, sa, sb, npix, npix_pad, nplanes, tmem_cols, nsets;   // nacc accumulators = nax across x (nacc / nax) down
-    int planar, ncols;             // planar != 0: fp32 output planes, one per output column (fused decode heads)
+    int ncols;                     // fused decode heads: fp32 output planes, one per output column
     int tstep_y, tstep_x, torg;    // tile origin = index * step + torg (shift-add heads: overlapping 16x16 regions, step 14, origin -1)
     float *plane[16];
     long long plane_bstride[16];
@@ -139,22 +140,11 @@ struct Params {
 struct Tile {
     int b, ty0, tx0, n0, z;
 };
-// rank: the CTA's rank in its pair (0 without pairs).  In pair mode `tile` counts pairs of spatial tiles of one (image, phase,
-// Cout tile): the two CTAs take linear positions 2 * pp + rank of the image's tile grid; a position past its end is a dummy
-// tile (all coordinates out of bounds: the TMA zero-fills, the epilogue stores nothing).
-template <bool kPair>
-__device__ __forceinline__ Tile decode_tile(const Params &P, int tile, int rank) {
+__device__ __forceinline__ Tile decode_tile(const Params &P, int tile) {
     Tile t;
     const int nt = tile % P.n_tiles_n; tile /= P.n_tiles_n;      // Cout tile fastest: the A halo stays hot in L2
-    int txi, tyi;
-    if constexpr (kPair) {
-        const int per = (P.tiles_x * P.tiles_y + 1) >> 1;
-        const int l = 2 * (tile % per) + rank; tile /= per;
-        tyi = l / P.tiles_x; txi = l - tyi * P.tiles_x;
-    } else {
-        txi = tile % P.tiles_x; tile /= P.tiles_x;
-        tyi = tile % P.tiles_y; tile /= P.tiles_y;
-    }
+    const int txi = tile % P.tiles_x; tile /= P.tiles_x;
+    const int tyi = tile % P.tiles_y; tile /= P.tiles_y;
     t.z = tile % P.nphases; tile /= P.nphases;
     t.b = tile;
     t.ty0 = tyi * P.tstep_y + P.torg; t.tx0 = txi * P.tstep_x + P.torg; t.n0 = nt * P.bn;
@@ -199,12 +189,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
         }
     }
 }
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void *src, uint32_t src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
@@ -215,13 +199,6 @@ __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence:
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc)
-        : "memory");
 }
 // descriptors passed as (lo, hi) words: advancing an operand is one 32-bit add on the start-address field
 __device__ __forceinline__ void tc_mma2(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
@@ -299,35 +276,6 @@ __device__ __forceinline__ void tc_mma_stage9(uint32_t d_tmem, const uint32_t (&
           "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc0), "r"(b_tap16), "r"(aks), "r"(bks)
         : "memory");
 }
-__device__ __forceinline__ void tc_mma2_pair(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
-                                             uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tsetp.ne.b32 p, %6, 0;\n\t"
-        "mov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}" ::"r"(d_tmem),
-        "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc)
-        : "memory");
-}
-// arrives on the barrier at this shared-memory offset in BOTH CTAs of the pair once all prior MMAs are complete
-__device__ __forceinline__ void tc_commit_pair(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-// arrive on the barrier at the same offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t rank) {
-    uint32_t raddr;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(bar), "r"(rank));
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-__device__ __forceinline__ uint32_t map_to_rank(uint32_t saddr, uint32_t rank) {
-    uint32_t raddr;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(saddr), "r"(rank));
-    return raddr;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
     asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
@@ -336,7 +284,7 @@ __device__ __forceinline__ bool elect_one() {
 // all MMAs of one (k-block, tap): BK/16 k-steps x NACC accumulators, fully unrolled
 // accumulator j = (jy, jx) covers the 16 x 8 pixel block at rows 16 jy, columns 8 jx of the tile: its A view starts
 // jy * 16 plane rows + jx * 8 pixels further (jx_step = 8, jy_step = 16 * plane pitch, in 16-byte units)
-template <int NACC, bool kPair>
+template <int NACC>
 __device__ __forceinline__ void issue_tap(uint32_t d_base, uint32_t bn, uint32_t a_lo, uint32_t a_hi, uint32_t a_kstep,
                                           uint32_t b_lo, uint32_t b_hi, uint32_t b_kstep, uint32_t idesc, uint32_t acc0,
                                           const uint32_t (&jy16)[4], const uint32_t (&jx8)[4]) {
@@ -348,12 +296,8 @@ __device__ __forceinline__ void issue_tap(uint32_t d_base, uint32_t bn, uint32_t
     for (int k2 = 0; k2 < BK / 16; ++k2)
 #pragma unroll
         for (int j = 0; j < NACC; ++j)      // consecutive MMAs target different accumulators
-            if constexpr (kPair)
-                tc_mma2_pair(d_base + (uint32_t)j * bn, a_lo + joff[j] + (uint32_t)k2 * a_kstep, a_hi, b_lo + (uint32_t)k2 * b_kstep, b_hi,
-                             idesc, k2 ? 1u : acc0);
-            else
-                tc_mma2(d_base + (uint32_t)j * bn, a_lo + joff[j] + (uint32_t)k2 * a_kstep, a_hi, b_lo + (uint32_t)k2 * b_kstep, b_hi,
-                        idesc, k2 ? 1u : acc0);
+            tc_mma2(d_base + (uint32_t)j * bn, a_lo + joff[j] + (uint32_t)k2 * a_kstep, a_hi, b_lo + (uint32_t)k2 * b_kstep, b_hi,
+                    idesc, k2 ? 1u : acc0);
 }
 // issue only; the registers are valid after tc_wait_ld(v)
 __device__ __forceinline__ void tc_ld16_issue(uint32_t taddr, uint32_t (&v)[16]) {
@@ -378,12 +322,6 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
           "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
         : "r"(taddr));
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// no-swizzle K-major shared-memory matrix descriptor (cute/arch/mma_sm100_desc.hpp: SmemDescriptor)
-__device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((addr & 0x3FFFF) >> 4) | ((uint64_t)(lbo_bytes >> 4) << 16) | ((uint64_t)(sbo_bytes >> 4) << 32) |
-           (1ull << 46);
 }
 
 // opaque register copy: stops ptxas from re-reading a kernel parameter from the constant bank inside hot loops (with a
@@ -415,14 +353,12 @@ __device__ __forceinline__ void ld_global_v8(const void *p, uint32_t (&o)[8]) {
 #define DBG_T0() const long long _t0 = DBG_ON ? clock64() : 0
 #define DBG_ACC(var) if (DBG_ON) var += clock64() - _t0
 
-// kGeneral = false: the hot variant (bf16 NHWC output, act in {none, ReLU, LeakyReLU}); true adds the planar decode-head
-// outputs and tanh / sigmoid, whose code would otherwise cost the hot epilogue registers.
+// kGeneral = false: the hot variant (bf16 NHWC output, act in {none, ReLU, LeakyReLU}); true adds tanh / sigmoid, partial
+// channel steps, unaligned slices and fp32 output, whose code would otherwise cost the hot epilogue registers.
 // kMode = MODE_WADAIN: W-AdaIN epilogue over [gamma | beta] column tiles.  kMode = MODE_HEADS: the decode heads as ONE
 // 1x1 GEMM to 9 * ncols columns (tap-major) over overlapping 16x16 pixel regions + a shift-add through shared memory.
 enum { MODE_STD = 0, MODE_GENERAL = 1, MODE_WADAIN = 2, MODE_HEADS = 3 };
-// kPair: the cta_group::2 instantiation (its instructions make ptxas require an even cluster size, so the single-CTA
-// kernels are separate instantiations).
-template <int kMode, bool kPair>
+template <int kMode>
 __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_constant__ Params P) {
     constexpr bool kGeneral = kMode == MODE_GENERAL;
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -434,12 +370,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
     const long long t_kernel0 = DBG_ON ? clock64() : 0;
     if (DBG_ON && threadIdx.x == 0) { unsigned long long gt; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt)); P.dbg[blockIdx.x * 16 + 15] = (long long)gt; }
     const int a_stage_bytes = P.a_tma ? P.nplanes * P.a_plane_bytes : KCH * P.npix_pad * 16;
-    const int bn_cta = kPair ? P.bn >> 1 : P.bn;                 // filter rows this CTA stages (half with cta_group::2)
-    const int b_tap_bytes = KCH * bn_cta * 16, b_stage_bytes = P.gtaps * b_tap_bytes;
-    uint32_t rank_u = 0;
-    if constexpr (kPair) asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank_u));
-    const int rank = kPair ? (int)rank_u : 0;
-    const int tile0 = kPair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, tile_step = kPair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+    const int b_tap_bytes = KCH * P.bn * 16, b_stage_bytes = P.gtaps * b_tap_bytes;
+    const int tile0 = blockIdx.x, tile_step = gridDim.x;
     // stages start on a 1 KB boundary (the SWIZZLE_64B pattern the TMA writes repeats every 1 KB; the host adds the slack)
     unsigned char *sA = smem + ((1024u - (smem_u32(smem) & 1023u)) & 1023u);
     unsigned char *sB = sA + (size_t)P.sa * a_stage_bytes;
@@ -451,13 +383,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
     // barrier map: a_full[sa] a_empty[sa] b_full[sb] b_empty[sb] acc_full[2] acc_empty[2]
     const uint32_t bar0 = smem_u32(bars);
     auto BAR = [&](int i) { return bar0 + 8u * (uint32_t)i; };
-    // pair mode adds peer_a_full[sa] peer_b_full[sb] (leader only: the peer CTA forwards its own full signals there)
     const uint32_t kz = opaque_zero();
     const int sa_k = keep(P.sa), sb_k = keep(P.sb);
     const int A_FULL = 0, A_EMPTY = sa_k, B_FULL = 2 * sa_k, B_EMPTY = B_FULL + sb_k, ACC_FULL = B_EMPTY + sb_k,
-              ACC_EMPTY = ACC_FULL + 2, PEER_A = ACC_EMPTY + 2, PEER_B = PEER_A + P.sa;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + PEER_B + P.sb);
-    const int RES_FULL = PEER_B + P.sb + 1;           // [group][buffer]: a residual slab has landed
+              ACC_EMPTY = ACC_FULL + 2;
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + ACC_EMPTY + 2);
+    const int RES_FULL = ACC_EMPTY + 3;               // [group][buffer]: a residual slab has landed
     // per-channel epilogue vectors, padded to CoutP with (1, 0): 16-byte aligned after the barrier block
     float *s_scale = reinterpret_cast<float *>(sE + epi_bytes + BAR_BYTES);
     float *s_shift = s_scale + P.CoutP;
@@ -477,30 +408,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         const int nissue = P.dual ? 2 : 1;           // every issuer commits on the "empty" / "accumulator full" barriers
         for (int i = 0; i < P.sa; ++i) { mbar_init(BAR(A_FULL + i), P.a_tma ? 1 : NPROD); mbar_init(BAR(A_EMPTY + i), nissue); }
         for (int i = 0; i < P.sb; ++i) { mbar_init(BAR(B_FULL + i), 1); mbar_init(BAR(B_EMPTY + i), nissue); }
-        for (int i = 0; i < 2; ++i) { mbar_init(BAR(ACC_FULL + i), nissue); mbar_init(BAR(ACC_EMPTY + i), kPair ? 2 * NEPI_WARPS : NEPI_WARPS); }
-        if constexpr (kPair) {
-            for (int i = 0; i < P.sa; ++i) mbar_init(BAR(PEER_A + i), 1);
-            for (int i = 0; i < P.sb; ++i) mbar_init(BAR(PEER_B + i), 1);
-        }
+        for (int i = 0; i < 2; ++i) { mbar_init(BAR(ACC_FULL + i), nissue); mbar_init(BAR(ACC_EMPTY + i), NEPI_WARPS); }
         for (int i = 0; i < 4; ++i) mbar_init(BAR(RES_FULL + i), 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == MMA_WARP) {
-        if constexpr (kPair) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                         "r"((uint32_t)P.tmem_cols)
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                         "r"((uint32_t)P.tmem_cols)
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                     "r"((uint32_t)P.tmem_cols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
-    if constexpr (kPair) cluster_sync_all();          // both CTAs' barriers exist before any remote arrive / multicast commit
-    else __syncthreads();
+    __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int set_cols = P.nacc * P.bn;
@@ -515,19 +434,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         // The whole warp walks the loop convergently (barrier waits, ring bookkeeping); one elected lane issues.  Per
         // MMA the issue cost is one 32-bit add on a descriptor word; the per-tap descriptor words come from the
         // shared-memory table and are fetched before the wait on the filter stage.
-        // instruction descriptor: bf16 x bf16 -> fp32, N = bn, M = 128 (one CTA) or 256 (cta_group::2: 128 rows per CTA)
+        // instruction descriptor: bf16 x bf16 -> fp32, N = bn, M = 128
 #ifdef RDFC_UMMA_TIMERS
         // RDFC_UMMA_SKIP & 4: issue every MMA with N = 16 (wrong results): is the loop bound by issue or by the tensor pipe?
-        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(((P.dbg_flags & 4) ? 16 : P.bn) >> 3) << 17) | ((kPair ? 16u : 8u) << 24);
+        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(((P.dbg_flags & 4) ? 16 : P.bn) >> 3) << 17) | (8u << 24);
 #else
         // operand format: bf16 (1), or fp16 (0) for the split fp32-faithful mode (11 + 11 mantissa bits per operand)
         const uint32_t fmt = P.split_c ? 0u : 1u;
-        const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(P.bn >> 3) << 17) | ((kPair ? 16u : 8u) << 24);
+        const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(P.bn >> 3) << 17) | (8u << 24);
 #endif
         // one k-step = 16 channels: two chunk planes further in the [cin/8][pixel][16 B] layout, 32 bytes in [pixel][64 B]
-        const uint32_t a_kstep = keep(P.a_tma ? 2u : 2u * (uint32_t)P.npix_pad), b_kstep = keep(2u * (uint32_t)bn_cta);
+        const uint32_t a_kstep = keep(P.a_tma ? 2u : 2u * (uint32_t)P.npix_pad), b_kstep = keep(2u * (uint32_t)P.bn);
         const uint32_t b_hi = (128u >> 4) | (1u << 14);                                     // SBO = 128 B, version bit 46
-        const uint32_t b_lo0 = keep(((smem_u32(sB) & 0x3FFFFu) >> 4) | ((uint32_t)bn_cta << 16));   // LBO = staged rows * 16 B
+        const uint32_t b_lo0 = keep(((smem_u32(sB) & 0x3FFFFu) >> 4) | ((uint32_t)P.bn << 16));    // LBO = staged rows * 16 B
         const uint32_t a_lo0 = keep((smem_u32(sA) & 0x3FFFFu) >> 4);
         const uint32_t a_stage16 = keep((uint32_t)a_stage_bytes >> 4), b_stage16 = keep((uint32_t)b_stage_bytes >> 4);
         const uint32_t b_tap16 = keep((uint32_t)b_tap_bytes >> 4);
@@ -540,8 +459,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         uint32_t jy16[4], jx8[4];                  // accumulator j: 16 * (rows down) and 8 * (blocks across), decoded once
 #pragma unroll
         for (int j = 0; j < 4; ++j) { jy16[j] = keep(16u * (uint32_t)((j + jb) / nax)); jx8[j] = keep(8u * (uint32_t)P.px16 * (uint32_t)((j + jb) % nax)); }
-        // one accumulator, 9-tap stages, TMA operands, single CTA: the stage is one asm statement over register-resident tap words
-        const bool fast9 = !kPair && keep(P.fast9) != 0;
+        // one accumulator, 9-tap stages, TMA operands: the stage is one asm statement over register-resident tap words
+        const bool fast9 = keep(P.fast9) != 0;
         uint32_t tlo9[9], thi9 = 0;
 #pragma unroll
         for (int q = 0; q < 9; ++q) tlo9[q] = 0;
@@ -554,27 +473,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         uint32_t a_par = 0, b_par = 0;
         long long t_acc = 0, t_a = 0, t_b = 0, t_mma = 0, t_commit = 0;
         const long long t_start = DBG_ON ? clock64() : 0;
-        constexpr bool pair = kPair;
-        if (pair && rank != 0) {
-            // peer CTA of a pair: no MMAs to issue.  Forward "my stage is full" to the leader, in consumption order (a TMA / bulk
-            // copy of the peer cannot complete on the leader's mbarrier directly: measured, it never arrives).
-            for (int tile = tile0; tile < P.ntiles; tile += tile_step) {
-                const Tile t = decode_tile<kPair>(P, tile, rank);
-                const int ngroups = P.ntaps[t.z] / gtaps;
-                for (int i = 0; i < nkb; ++i) {
-                    mbar_wait(BAR(A_FULL + s), a_par);
-                    if (lane == 0) mbar_arrive_remote(BAR(PEER_A + s), 0);
-                    for (int gi = 0; gi < ngroups; ++gi) {
-                        mbar_wait(BAR(B_FULL + sb), b_par);
-                        if (lane == 0) mbar_arrive_remote(BAR(PEER_B + sb), 0);
-                        if (++sb == sb_n) { sb = 0; b_par ^= 1u; }
-                    }
-                    if (++s == sa_n) { s = 0; a_par ^= 1u; }
-                }
-            }
-        } else
         for (int tile = tile0; tile < P.ntiles; tile += tile_step, ++it) {
-            const Tile t = decode_tile<kPair>(P, tile, rank);
+            const Tile t = decode_tile(P, tile);
             const int z = t.z, ngroups = P.ntaps[z] / gtaps;
             const uint2 *ztap = s_tap + z * MAX_TAPS;
             const int set = nsets == 2 ? (it & 1) : 0;
@@ -583,11 +483,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
             tc_fence_after();
             const uint32_t d_base = tmem_base + (uint32_t)(set * set_cols) + (uint32_t)jb * bn;
             for (int i = 0; i < nkb; ++i) {
-                { DBG_T0(); mbar_wait(BAR(A_FULL + s), a_par); if (pair) mbar_wait(BAR(PEER_A + s), a_par); DBG_ACC(t_a); }
+                { DBG_T0(); mbar_wait(BAR(A_FULL + s), a_par); DBG_ACC(t_a); }
                 const uint32_t a_stage_lo = a_lo0 + (uint32_t)s * a_stage16;
                 for (int gi = 0; gi < ngroups; ++gi) {
                     const uint32_t b_lo = b_lo0 + (uint32_t)sb * b_stage16;
-                    { DBG_T0(); mbar_wait(BAR(B_FULL + sb), b_par); if (pair) mbar_wait(BAR(PEER_B + sb), b_par); DBG_ACC(t_b); }
+                    { DBG_T0(); mbar_wait(BAR(B_FULL + sb), b_par); DBG_ACC(t_b); }
                     tc_fence_after();
                     if (elect_one()) {
                         const long long _tm0 = DBG_ON ? clock64() : 0;
@@ -605,34 +505,26 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                                 const uint32_t a_lo = td[tg].x + a_stage_lo, a_hi = td[tg].y, bl = b_lo + (uint32_t)(r3 + tg) * b_tap16;
                                 switch (nacc) {
                                     case 1:
-                                        issue_tap<1, kPair>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
+                                        issue_tap<1>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
                                         break;
                                     case 2:
-                                        issue_tap<2, kPair>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
+                                        issue_tap<2>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
                                         break;
                                     case 3:
-                                        issue_tap<3, kPair>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
+                                        issue_tap<3>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
                                         break;
                                     default:
-                                        issue_tap<4, kPair>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
+                                        issue_tap<4>(d_base, bn, a_lo, a_hi, a_kstep, bl, b_hi, b_kstep, idesc, acc0, jy16, jx8);
                                         break;
                                 }
                             }
                         }
                         }
                         const long long _tm1 = DBG_ON ? clock64() : 0;
-                        if constexpr (kPair) {        // the same barriers in both CTAs of the pair
-                            tc_commit_pair(BAR(B_EMPTY + sb));
-                            if (gi == ngroups - 1) {
-                                tc_commit_pair(BAR(A_EMPTY + s));
-                                if (i == nkb - 1) tc_commit_pair(BAR(ACC_FULL + set));
-                            }
-                        } else {
-                            tc_commit(BAR(B_EMPTY + sb));
-                            if (gi == ngroups - 1) {
-                                tc_commit(BAR(A_EMPTY + s));
-                                if (i == nkb - 1) tc_commit(BAR(ACC_FULL + set));
-                            }
+                        tc_commit(BAR(B_EMPTY + sb));
+                        if (gi == ngroups - 1) {
+                            tc_commit(BAR(A_EMPTY + s));
+                            if (i == nkb - 1) tc_commit(BAR(ACC_FULL + set));
                         }
                         if (DBG_ON) { const long long _tm2 = clock64(); t_mma += _tm1 - _tm0; t_commit += _tm2 - _tm1; }
                     }
@@ -662,7 +554,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
             int s = 0;
             uint32_t par = 1;
             for (int tile = tile0; tile < P.ntiles; tile += tile_step) {
-                const Tile t = decode_tile<kPair>(P, tile, rank);
+                const Tile t = decode_tile(P, tile);
                 for (int i = 0; i < nkb; ++i) {
                     mbar_wait(BAR(A_EMPTY + s), par);
                     const uint32_t full = BAR(A_FULL + s);
@@ -686,7 +578,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 }
             }
         }
-    } else if (warp < NPROD_WARPS && P.stem_in0) {
+    } else if (warp < NPROD_WARPS) {
         // ================= A producers, stem mode =================
         // The "input" of the 1x1 GEMM is the im2col matrix of the 3x3 stems, built on the fly: slot (pixel p, chunk ch)
         // of k-block i holds rows k = 32 i + 8 ch .. + 8, row k = (channel k / 9, tap k % 9).  Per tile the producers
@@ -718,7 +610,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         // as long as building a whole tile -- is off the critical path.
         const int patch_stride = nch * plane_sz + 4;               // floats per buffer: cells, the zero cell, padding
         auto fill_patch = [&](int tile, int buf) {
-            const Tile t = decode_tile<kPair>(P, tile, rank);
+            const Tile t = decode_tile(P, tile);
             const float *b0 = P.stem_in0 + (long long)t.b * P.stem_c0 * HW;
             const float *b1 = P.stem_in1 ? P.stem_in1 + (long long)t.b * HW : b0;
             const uint32_t patch_s = smem_u32(patch + buf * patch_stride);
@@ -774,98 +666,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 if (++s == P.sa) { s = 0; par ^= 1u; }
             }
         }
-    } else if (warp < NPROD_WARPS) {
-        // ================= A producers =================
-        // Thread t owns 16-byte chunk (t & 3) of pixel slots (t >> 2) + PIXPASS * j of every stage.  Which plane pixel a slot
-        // is never changes, so its plane-relative input coordinates are decoded once per kernel; per tile they become
-        // a byte offset into the image + a validity bit (outside the image = the conv zero padding); per k-block a
-        // slot costs one add and one cp.async.  Publication of k-block i is deferred until k-block i+LAG is in flight.
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        const int ch = threadIdx.x & 3, p0 = threadIdx.x >> 2;
-        const int nj = (P.npix + PIXPASS - 1) / PIXPASS;
-        uint32_t rel2[JMAX / 2];    // per slot 16 bits: (plane-relative input row + 1) | (column + 1) << 8 ; 0xffff = unused
-#pragma unroll
-        for (int j = 0; j < JMAX; ++j) {
-            const int p = j * PIXPASS + p0;
-            uint32_t v = 0xffffu;
-            if (j < nj && p < P.npix) {
-                int pl = 0;
-                while (pl + 1 < P.nplanes && p >= P.planes[pl + 1].base) ++pl;
-                const Plane &q = P.planes[pl];
-                const int r = (p - q.base) / q.cols, c = (p - q.base) % q.cols;
-                v = (uint32_t)(q.ystep * r + q.yoff + 1) | ((uint32_t)(q.xstep * c + q.xoff + 1) << 8);
-            }
-            if (j & 1) rel2[j >> 1] |= v << 16; else rel2[j >> 1] = v;
-        }
-        const int ystep = keep(P.planes[0].ystep), xstep = keep(P.planes[0].xstep);     // the same for every plane of a layer
-        const int Hi = keep(P.Hi), Wi = keep(P.Wi), in_stride = keep(P.in_stride), nkb = keep(P.nkb), sa_n = keep(P.sa);
-        const uint32_t dst_thread = smem_u32(sA) + (uint32_t)(ch * P.npix_pad + p0) * 16u;
-        // cp.async groups kept in flight before the oldest is published.  Publishing k-block i-lag needs k-block i
-        // issued, i.e. the stage of k-block i-sa drained by the MMAs: lag <= sa - 2 keeps one published stage for the
-        // tensor core to work on meanwhile (lag = sa - 1 serialises MMA and staging).
-        const int lag = P.sa >= 4 ? 2 : (P.sa == 3 ? 1 : 0);
-        int s = 0;                  // ring position, continues across tiles
-        uint32_t par = 1;           // parity to wait for on A_EMPTY[s]
-        long long t_wait_empty = 0, t_issue = 0, t_wait_group = 0;
-        int issued = 0;             // k-blocks committed so far
-        int pub = 0;                // next stage to publish
-        for (int tile = tile0; tile < P.ntiles; tile += tile_step) {
-            const Tile t = decode_tile<kPair>(P, tile, rank);
-            const char *img = reinterpret_cast<const char *>(P.in + (long long)t.b * Hi * Wi * in_stride) + ch * 16;
-            const int y0 = ystep * t.ty0 - 1, x0 = xstep * t.tx0 - 1;
-            uint32_t off[JMAX];
-            uint32_t vmask = 0;
-#pragma unroll
-            for (int j = 0; j < JMAX; ++j) {
-                const uint32_t rj = (rel2[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-                const int iy = y0 + (int)(rj & 0xffu), ix = x0 + (int)(rj >> 8);
-                const bool ok = rj != 0xffffu && (unsigned)iy < (unsigned)Hi && (unsigned)ix < (unsigned)Wi;
-                off[j] = ok ? (uint32_t)((iy * Wi + ix) * in_stride) * 2u : 0u;
-                vmask |= ok ? (1u << j) : 0u;
-            }
-            for (int i = 0; i < nkb; ++i, img += BK * 2) {
-                { DBG_T0(); mbar_wait(BAR(A_EMPTY + s), par); DBG_ACC(t_wait_empty); }
-                const long long _ti = DBG_ON ? clock64() : 0;
-                const uint32_t dst = dst_thread + (uint32_t)s * (uint32_t)a_stage_bytes;
-#pragma unroll
-                for (int j = 0; j < JMAX; ++j)
-                    if (j < nj && ((rel2[j >> 1] >> (16 * (j & 1))) & 0xffffu) != 0xffffu)
-                        cp_async16(dst + (uint32_t)j * (uint32_t)(PIXPASS * 16), img + off[j], (vmask >> j) & 1u ? 16u : 0u);
-                cp_async_commit();
-                if (DBG_ON) t_issue += clock64() - _ti;
-                ++issued;
-                if (issued > lag) {               // publish the oldest k-block in flight
-                    { DBG_T0(); if (lag == 2) cp_async_wait<2>(); else if (lag == 1) cp_async_wait<1>(); else cp_async_wait<0>(); DBG_ACC(t_wait_group); }
-                    fence_proxy_async();
-                    mbar_arrive(BAR(A_FULL + pub));
-                    if (++pub == sa_n) pub = 0;
-                }
-                if (++s == sa_n) { s = 0; par ^= 1u; }
-            }
-        }
-        // drain: publish what is still in flight, oldest first
-        const int left = issued < lag ? issued : lag;
-        if (left == 2) {
-            cp_async_wait<1>();
-            fence_proxy_async();
-            mbar_arrive(BAR(A_FULL + pub));
-            if (++pub == P.sa) pub = 0;
-        }
-        if (left >= 1) {
-            cp_async_wait<0>();
-            fence_proxy_async();
-            mbar_arrive(BAR(A_FULL + pub));
-        }
-        if (DBG_ON && threadIdx.x == 0) {
-            P.dbg[blockIdx.x * 16 + 6] = t_wait_empty; P.dbg[blockIdx.x * 16 + 7] = t_issue; P.dbg[blockIdx.x * 16 + 8] = t_wait_group;
-        }
     } else if (warp == BLOAD_WARP) {
         // ================= B loader (TMA 1-D bulk copies of pre-packed filter blocks) =================
         // The warp walks the ring convergently; lane 0 posts the byte count, then every lane issues its share of the stage's
-        // copies (a 9-tap stage of a filter view that is not contiguous over the k-block is 36 copies of ~1 KB: issued by one
-        // thread they took as long as the MMAs of the stage, which starved the issuer in cta_group::2 mode).
+        // copies.  A 9-tap stage of a filter view that is not contiguous over the k-block is 36 copies of ~1 KB; issued by one
+        // thread they took as long as the MMAs of the stage (measured with CTA pairs).
         {
-            const uint32_t piece = keep((uint32_t)bn_cta * 16u);          // one cin chunk of this CTA's filter rows
+            const uint32_t piece = keep((uint32_t)P.bn * 16u);            // one cin chunk of the tile's filter rows
             const long long chunk_stride = (long long)P.CoutP * 8;
             const uint32_t sB0 = smem_u32(sB);
             const int sb_n = keep(P.sb), nkb = keep(P.nkb), gtaps = keep(P.gtaps), b_contig = keep(P.b_contig);
@@ -873,9 +680,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
             uint32_t par = 1;
             long long t_be = 0;
             for (int tile = tile0; tile < P.ntiles; tile += tile_step) {
-                const Tile t = decode_tile<kPair>(P, tile, rank);
+                const Tile t = decode_tile(P, tile);
                 const int z = t.z, ngroups = P.ntaps[z] / gtaps;
-                const __nv_bfloat16 *w_n0 = P.w + (long long)(t.n0 + rank * bn_cta) * 8;    // pair: rank r stages rows [r * bn / 2, ..)
+                const __nv_bfloat16 *w_n0 = P.w + (long long)t.n0 * 8;
                 for (int i = 0; i < nkb; ++i, w_n0 += P.w_kb_stride)
                     for (int gi = 0; gi < ngroups; ++gi) {
                         const uint32_t dst = sB0 + (uint32_t)sb * (uint32_t)b_stage_bytes;
@@ -912,11 +719,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         const int wq = warp & 3, grp = (warp - EPI_WARP0) >> 2;
         const int r = 4 * wq + (lane >> 3), c = lane & 7;     // MMA row m = 32*wq + lane = 8*r + c
         const int bn = P.bn, Cout = P.Cout, out_stride = P.out_stride, res_stride = P.res_stride;
-        // bit 0 planar, bit 1 vec32, bits 2.. development skip flags: one register for the inner-loop switches
-        const int flags = (P.planar == 1 ? 1 : 0) | (P.vec32 ? 2 : 0) | (P.dbg_flags << 2);
+        // bit 1 vec32, bits 2.. development skip flags: one register for the inner-loop switches
+        const int flags = (P.vec32 ? 2 : 0) | (P.dbg_flags << 2);
         const int act = P.act, nacc = P.nacc, nax = P.nax, nsets = P.nsets;
         const int Ht = P.Ht, Wt = P.Wt, Ho = P.Ho, Wo = P.Wo, oys = P.oys, oxs = P.oxs;
-#define planar (kGeneral && (flags & 1))
 #define vec32 (kMode == MODE_STD || (flags & 2))      // MODE_STD: the host guarantees 32-byte aligned slices and Cout % 16 == 0
 #define skip (flags >> 2)
         const float slope = act == RDFC_ACT_RELU ? 0.f : (act == RDFC_ACT_LEAKY02 ? 0.2f : 1.f);
@@ -936,13 +742,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         const bool leader = wq == 0 && lane == 0;
         const uint32_t row_off = (uint32_t)(32 * wq + lane) * 64u, swz = (uint32_t)(((32 * wq + lane) >> 1) & 3);
         uint32_t ctr = 0;
-        for (int tile = tile0; tile < P.ntiles; tile += tile_step, ++it) {
-            const Tile t = decode_tile<kPair>(P, tile, rank);
-            const int oyo = P.oyo[t.z], oxo = P.oxo[t.z];
-            const int set = nsets == 2 ? (it & 1) : 0;
-            const int use = nsets == 2 ? (it >> 1) : it;
-            const long long _te = DBG_ON ? clock64() : 0;
-            if (tma_epi) {
+        if (tma_epi) {
+            for (int tile = tile0; tile < P.ntiles; tile += tile_step, ++it) {
+                const Tile t = decode_tile(P, tile);
+                const int oyo = P.oyo[t.z], oxo = P.oxo[t.z];
+                const int set = nsets == 2 ? (it & 1) : 0;
+                const int use = nsets == 2 ? (it >> 1) : it;
+                const long long _te = DBG_ON ? clock64() : 0;
                 // ---- epilogue through shared memory + TMA: per 32-channel slab of an accumulator
                 //   TMEM -> registers -> y = act(acc*scale + shift + residual slab) -> bf16 slab in shared memory -> one
                 //   cp.async.bulk.tensor store of the 8 x 16 pixel box (the TMA unit clips pixels / channels outside the tensor).
@@ -1037,8 +843,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 __syncwarp();
                 if (lane == 0) mbar_arrive(BAR(ACC_EMPTY + set));
                 if (DBG_ON) t_epi += clock64() - _te;
-                continue;
             }
+            if (leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // my stores have been written
+        } else
+        for (int tile = tile0; tile < P.ntiles; tile += tile_step, ++it) {
+            const Tile t = decode_tile(P, tile);
+            const int oyo = P.oyo[t.z], oxo = P.oxo[t.z];
+            const int set = nsets == 2 ? (it & 1) : 0;
+            const int use = nsets == 2 ? (it >> 1) : it;
+            const long long _te = DBG_ON ? clock64() : 0;
             { DBG_T0(); mbar_wait<true>(BAR(ACC_FULL + set), use & 1); DBG_ACC(t_accfull); }
             tc_fence_after();
             if (kMode == MODE_HEADS) {
@@ -1060,7 +873,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 }
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) { if (kPair && rank != 0) mbar_arrive_remote(BAR(ACC_EMPTY + set), 0); else mbar_arrive(BAR(ACC_EMPTY + set)); }
+                if (lane == 0) mbar_arrive(BAR(ACC_EMPTY + set));
                 asm volatile("bar.sync 2, %0;" ::"n"(NEPI_WARPS * 32) : "memory");
                 for (int item = threadIdx.x - EPI_WARP0 * 32; item < 196 * ncols; item += NEPI_WARPS * 32) {
                     const int q = item / 196, pi = item - q * 196, iy = pi / 14, ix = pi - iy * 14;
@@ -1141,7 +954,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 }
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) { if (kPair && rank != 0) mbar_arrive_remote(BAR(ACC_EMPTY + set), 0); else mbar_arrive(BAR(ACC_EMPTY + set)); }
+                if (lane == 0) mbar_arrive(BAR(ACC_EMPTY + set));
                 continue;
             }
             const int n0 = t.n0;
@@ -1156,9 +969,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 const long long opix = ok ? ((long long)t.b * Ho + oy) * Wo + ox : 0;
                 const uint32_t trow = tmem_base + ((uint32_t)(32 * wq) << 16) + (uint32_t)(set * set_cols + j * bn);
                 const __nv_bfloat16 *rrow = res ? res + opix * res_stride + n0 : nullptr;
-                __nv_bfloat16 *orow = planar ? nullptr : outp + opix * out_stride + n0;
+                __nv_bfloat16 *orow = outp + opix * out_stride + n0;
                 __nv_bfloat16 *orow2 = P.out2 ? P.out2 + opix * P.out2_stride + n0 - P.split : nullptr;
-                const long long pp = (long long)oy * Wo + ox;
 
                 auto load_res = [&](int g, uint4 &r0, uint4 &r1) {
                     if (rrow && ok && (kMode == MODE_STD || n0 + 16 * g + 16 <= Cout)) {
@@ -1213,20 +1025,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                                         float y = f[4 * q4 + e] + (rp ? __ldg(rp + 4 * q4 + e) : 0.f);
                                         op[4 * q4 + e] = act <= RDFC_ACT_LEAKY02 ? fmaxf(y, slope * y) : apply_act(y, act);
                                     }
-                            }
-                        }
-                        return;
-                    }
-                    if (planar) {
-                        // fused decode heads: column q -> its own fp32 plane with its own activation
-#pragma unroll
-                        for (int q = 0; q < 16; ++q) {
-                            if (q < P.ncols) {
-                                const int a = P.act_col[q];
-                                float y = f[q];
-                                if (a == RDFC_ACT_TANH) y = tanhf(y);
-                                else if (a == RDFC_ACT_SIGMOID) y = 1.f / (1.f + expf(-y));
-                                P.plane[q][(long long)t.b * P.plane_bstride[q] + pp] = y;
                             }
                         }
                         return;
@@ -1300,18 +1098,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
             // this warp is done reading the accumulator set: hand it back to the MMA warp
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) { if (kPair && rank != 0) mbar_arrive_remote(BAR(ACC_EMPTY + set), 0); else mbar_arrive(BAR(ACC_EMPTY + set)); }
+            if (lane == 0) mbar_arrive(BAR(ACC_EMPTY + set));
             if (DBG_ON) t_epi += clock64() - _te;
         }
-        if (tma_epi && leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // my stores have been written
         if (DBG_ON && warp == EPI_WARP0 && lane == 0) { P.dbg[blockIdx.x * 16 + 9] = t_accfull; P.dbg[blockIdx.x * 16 + 10] = t_epi; }
-#undef planar
 #undef vec32
 #undef skip
     }
     tc_fence_before();
-    if constexpr (kPair) cluster_sync_all();          // the peer's shared memory / barriers stay valid until both CTAs are done
-    else __syncthreads();
+    __syncthreads();
     if (DBG_ON && threadIdx.x == 0) {
         P.dbg[blockIdx.x * 16 + 13] = clock64() - t_kernel0;
         unsigned long long gt; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
@@ -1319,10 +1114,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
     }
     if (warp == MMA_WARP) {
         tc_fence_after();
-        if constexpr (kPair)
-            asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)P.tmem_cols) : "memory");
-        else
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)P.tmem_cols) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)P.tmem_cols) : "memory");
     }
 }
 
@@ -1337,24 +1129,6 @@ int next_pow2_cols(int c) {
 }  // namespace
 
 // Host-side planning: planes, taps, tile shape, stage counts.
-typedef CUresult (*TmapEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                 const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-// cuTensorMapEncodeTiled through the runtime's driver entry point query: the library keeps linking only cudart
-static TmapEncodeFn tmap_encoder() {
-    static TmapEncodeFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        cudaDriverEntryPointQueryResult q;
-        void *p = nullptr;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = (TmapEncodeFn)p;
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
-
 int wadain_tile(int C) { return (2 * C) % 256 == 0 ? 256 : 128; }
 
 // split_c != 0: `d->in` is a split bf16 tensor [hi(split_c) | lo(split_c)] (see Params::split_c) and the filter bank holds
@@ -1407,7 +1181,7 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
         }
     }
     if (heads) {
-        P.planar = 2; P.ncols = heads->ncols;
+        P.ncols = heads->ncols;
         for (int q = 0; q < 16; ++q) {
             P.plane[q] = heads->out[q]; P.plane_bstride[q] = heads->out_bstride[q]; P.act_col[q] = heads->act[q];
         }
@@ -1476,26 +1250,18 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     }
     P.tiles_y = cdiv(P.Ht, P.tstep_y); P.tiles_x = cdiv(P.Wt, P.tstep_x);
 
-    // A operand through TMA tensor-map loads unless the producers have to build it (stem mode) or the driver entry
-    // point is missing; RDFC_UMMA_TMA=0 forces the cp.async producers (development knob)
-    P.a_tma = !stem && tmap_encoder() != nullptr;
-    if (const long long e = knob("RDFC_UMMA_TMA", KNOB_UNSET); e != KNOB_UNSET) P.a_tma = P.a_tma && (int)e != 0;
+    // A operand through TMA tensor-map loads unless the producers have to build it (stem mode)
+    P.a_tma = !stem;
+    RDFC_REQUIRE(!P.a_tma || tmap_encoder() != nullptr, "UMMA conv: the CUDA driver does not provide cuTensorMapEncodeTiled");
     P.px16 = P.a_tma ? 4 : 1;
-    // CTA pairs (tcgen05 cta_group::2, RDFC_UMMA_PAIR=1): each CTA stages half of every filter block and one stream of M = 256
-    // MMAs issued by the leader covers both CTAs' pixel tiles.  Correct (tests/test_gpu_conv.py runs it) but OFF by default:
-    // measured on B200 it is slower than two independent CTAs at the N <= 128 it was meant for (128 -> 128 @114x152: 108 cycles
-    // per M=256 N=128 MMA and 221 us, against 88 cycles per M=128 MMA and 166 us), and 1x1 / transposed convs lose 2x to the
-    // extra barrier hops (a peer's TMA cannot complete on the leader's mbarrier, so its "full" signals are forwarded).
-    P.pair = 0;
-    if (const long long e = knob("RDFC_UMMA_PAIR", KNOB_UNSET); e != KNOB_UNSET) P.pair = P.a_tma && P.bn % 32 == 0 && (int)e != 0;
-    P.dual = P.a_tma && !P.pair && P.nacc >= 2;
+    P.dual = P.a_tma && P.nacc >= 2;
     if (const long long e = knob("RDFC_UMMA_DUAL", KNOB_UNSET); e != KNOB_UNSET) P.dual = P.dual && (int)e != 0;      // development knob
-    P.ntiles = (P.pair ? (P.tiles_x * P.tiles_y + 1) / 2 : P.tiles_x * P.tiles_y) * P.B * P.nphases * P.n_tiles_n;   // pair mode: pairs of tiles
+    P.ntiles = P.tiles_x * P.tiles_y * P.B * P.nphases * P.n_tiles_n;
     // 1x1 convs: one tap per A stage means 2 * nacc MMAs per stage against ~500 cycles of barrier / commit / ring overhead in the issuing
     // warp (role timers, DESIGN 8.10).  Stage `kbs` consecutive 32-channel k-blocks at once: k-block j of a stage is "plane" j (the same
     // pixels, channel coordinate + 32 j) and "tap" j (its block of the packed filters), so the kernel's tap loop walks them inside one stage.
     P.kbs = 1;
-    if (k1 && P.a_tma && !heads && !stem && !split_c && !P.pair) {
+    if (k1 && P.a_tma && !heads && !split_c) {
         const int nkb_total = P.nkb;
         for (int cand = 3; cand >= 2; --cand)
             if (nkb_total % cand == 0) { P.kbs = cand; break; }
@@ -1542,7 +1308,7 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
         int pl[2][2];
         for (int py = 0; py < 2; ++py)
             for (int px = 0; px < 2; ++px)
-                pl[py][px] = add_plane(2, py ? -1 : 0, 2, px ? -1 : 0, TH + (P.a_tma ? 1 : py), TW + (P.a_tma ? 1 : px));   // one TMA box shape
+                pl[py][px] = add_plane(2, py ? -1 : 0, 2, px ? -1 : 0, TH + 1, TW + 1);   // one TMA box shape
         Phase &ph = phases[0];
         for (int ky = 0; ky < 3; ++ky)
             for (int kx = 0; kx < 3; ++kx)
@@ -1567,15 +1333,10 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
                                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         RDFC_REQUIRE(r == CUDA_SUCCESS, "UMMA conv: cuTensorMapEncodeTiled failed (%d)", (int)r);
     } else {
-        for (int pl = 0; pl < P.nplanes; ++pl)
-            RDFC_REQUIRE(P.planes[pl].ystep * (P.planes[pl].rows - 1) + 1 < 255 && P.planes[pl].xstep * (P.planes[pl].cols - 1) + 1 < 255,
-                         "UMMA conv: staged plane too large for the packed producer slot table");
-        RDFC_REQUIRE(P.npix <= JMAX * PIXPASS, "UMMA conv: staged halo (%d pixels) exceeds the producer slot table", P.npix);
-        RDFC_REQUIRE((long long)P.Hi * P.Wi * P.in_stride * 2 < (1ll << 32), "UMMA conv: image too large for 32-bit producer offsets");
         RDFC_REQUIRE(P.npix_pad < (1 << 14), "UMMA conv: staged halo too large for the descriptor LBO field");
     }
     P.w_kb_stride = (long long)KCH * P.CoutP * 8 * P.kbs;
-    P.b_contig = P.n_tiles_n == 1 && !P.pair;
+    P.b_contig = P.n_tiles_n == 1;
     for (int z = 0; z < P.nphases; ++z) {
         const Phase &ph = phases[z];
         P.ntaps[z] = ph.ntaps; P.oyo[z] = ph.oyo; P.oxo[z] = ph.oxo;
@@ -1610,7 +1371,6 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
               (!P.out2 || (((uintptr_t)P.out2 % 32) == 0 && P.out2_stride % 16 == 0 && P.split % 16 == 0)) &&
               (!d->residual.ptr || (((uintptr_t)d->residual.ptr % 32) == 0 && d->residual.pix_stride % 16 == 0));
     if (P.out_f32) P.vec32 = 0;                    // fp32 output: the general epilogue variant
-    RDFC_REQUIRE(!split_c || P.a_tma, "UMMA conv (split input) needs the TMA producer");
     const int a_stage = P.a_tma ? P.nplanes * P.a_plane_bytes : (KCH * P.npix_pad * 16 + 1023) / 1024 * 1024;
     const int stem_patch = stem ? 2 * ((P.stem_k / 9) * (TH + 2) * (TW + 2) + 4) * 4 : 0;  // two fp32 input patches of a tile (stem mode)
     const int heads_y = heads ? 256 * (P.bn + 1) * 4 : 0;                                   // shift-add heads: Y of a region
@@ -1621,10 +1381,10 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     // from the operand stages: stride-2 convs 121 -> 138 us, 256-wide + residual 144 -> 168 us, 128 -> 160 719 -> 769 us), so it
     // is selected per layer.  RDFC_UMMA_TMAOUT: 0 = never, 1 = where it pays (default), 2 = every eligible layer, transposed convs
     // (element-strided store boxes) included -- the tests run all three.
-    const int mode_std = !heads && !wad && !(P.planar || P.act > RDFC_ACT_LEAKY02 || !P.vec32 || P.Cout % 16 != 0);
+    const int mode_std = !heads && !wad && !(P.act > RDFC_ACT_LEAKY02 || !P.vec32 || P.Cout % 16 != 0);
     const long long tmaout_knob = knob("RDFC_UMMA_TMAOUT", 1);
     const bool tmaout_pays = d->residual.ptr && P.bn <= 128 && !d->transposed && d->stride == 1;
-    P.tma_out = mode_std && P.a_tma && !P.pair && !P.out2 && !stem && P.bn % 32 == 0 &&
+    P.tma_out = mode_std && P.a_tma && !P.out2 && P.bn % 32 == 0 &&
                 (tmaout_knob >= 2 || (tmaout_knob == 1 && tmaout_pays));
     if (P.tma_out) {
         const int es = d->transposed ? 2 : 1;
@@ -1646,11 +1406,11 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     // The issuing warp pays ~1000 cycles per filter stage (barrier wait, commits, ring bookkeeping) that the tensor pipe does
     // not overlap (role timers: issue is blocking at the pipe's rate), so a 3x3 conv stages all nine taps of a k-block at once
     // when two such stages and two A stages fit.
-    if (k3 && !d->transposed && !stem && 2 * a_stage + 2 * 9 * KCH * (P.pair ? P.bn / 2 : P.bn) * 16 + fixed <= budget) P.gtaps = 9;
+    if (k3 && !d->transposed && !stem && 2 * a_stage + 2 * 9 * KCH * P.bn * 16 + fixed <= budget) P.gtaps = 9;
     if (const long long e = knob("RDFC_UMMA_GTAPS", KNOB_UNSET); e != KNOB_UNSET) P.gtaps = (int)e;    // development knob (1, 3 or 9)
     // joff of accumulator 0 is 0 (jb = 0): the fast path needs nothing but the tap table
-    P.fast9 = P.gtaps == 9 && P.nacc == 1 && P.a_tma && !P.pair && P.nphases == 1 && !P.dual && knob("RDFC_UMMA_FAST9", 1) != 0;
-    const int b_stage = P.gtaps * KCH * (P.pair ? P.bn / 2 : P.bn) * 16;
+    P.fast9 = P.gtaps == 9 && P.nacc == 1 && P.a_tma && P.nphases == 1 && !P.dual && knob("RDFC_UMMA_FAST9", 1) != 0;
+    const int b_stage = P.gtaps * KCH * P.bn * 16;
     // A ring first (>= 2 stages: the producers publish k-block i while k-block i+1 is in flight), then B stages (2..6)
     // the filter stream is latency-bound: bytes in flight per SM = bandwidth x L2 latency (~2000 cycles), so keep
     // >= 64 KB of filter stages in flight when the tile allows it
@@ -1670,15 +1430,13 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     if (const long long e = knob("RDFC_UMMA_SA", KNOB_UNSET); e != KNOB_UNSET) P.sa = (int)e < P.sa ? (int)e : P.sa;
     RDFC_REQUIRE(P.sa >= 1 && P.sa <= 8 && P.sb >= 1 && P.sb <= 16, "UMMA conv: tile does not fit shared memory");
     const size_t smem = (size_t)P.sa * a_stage + (size_t)P.sb * b_stage + fixed + 1024;
+    void (*const kernels[4])(Params) = {conv_umma_kernel<MODE_STD>, conv_umma_kernel<MODE_GENERAL>, conv_umma_kernel<MODE_WADAIN>,
+                                        conv_umma_kernel<MODE_HEADS>};   // indexed by mode
     static bool attr_set[64] = {};                 // per device: the attribute belongs to the function ON a device
     int dev_id = 0;
     RDFC_CUDA(cudaGetDevice(&dev_id));
     if (!attr_set[dev_id & 63]) {
-#define RDFC_SMEM_ATTR(M)                                                                                                      \
-    RDFC_CUDA(cudaFuncSetAttribute(conv_umma_kernel<M, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));       \
-    RDFC_CUDA(cudaFuncSetAttribute(conv_umma_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024))
-        RDFC_SMEM_ATTR(MODE_STD); RDFC_SMEM_ATTR(MODE_GENERAL); RDFC_SMEM_ATTR(MODE_WADAIN); RDFC_SMEM_ATTR(MODE_HEADS);
-#undef RDFC_SMEM_ATTR
+        for (auto k : kernels) RDFC_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         attr_set[dev_id & 63] = true;
     }
     if (const long long e = knob("RDFC_UMMA_SKIP", KNOB_UNSET); e != KNOB_UNSET) P.dbg_flags = (int)e;
@@ -1692,38 +1450,18 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     int grid = P.ntiles < sm_count() ? P.ntiles : sm_count();
     if (const long long e = knob("RDFC_UMMA_GRID", KNOB_UNSET); e != KNOB_UNSET) grid = (int)e < P.ntiles ? (int)e : P.ntiles;   // development knob
     const int mode = heads ? MODE_HEADS : wad ? MODE_WADAIN
-                     : (P.planar || P.act > RDFC_ACT_LEAKY02 || !P.vec32 || P.Cout % 16 != 0) ? MODE_GENERAL : MODE_STD;
-    void (*kern)(Params) = nullptr;
-    switch (mode) {
-        case MODE_HEADS: kern = P.pair ? conv_umma_kernel<MODE_HEADS, true> : conv_umma_kernel<MODE_HEADS, false>; break;
-        case MODE_WADAIN: kern = P.pair ? conv_umma_kernel<MODE_WADAIN, true> : conv_umma_kernel<MODE_WADAIN, false>; break;
-        case MODE_GENERAL: kern = P.pair ? conv_umma_kernel<MODE_GENERAL, true> : conv_umma_kernel<MODE_GENERAL, false>; break;
-        default: kern = P.pair ? conv_umma_kernel<MODE_STD, true> : conv_umma_kernel<MODE_STD, false>; break;
-    }
-    if (P.pair) {
-        // one cluster of two CTAs per tile pair (P.ntiles counts pairs; grid = 2 x min(pairs, #SMs / 2))
-        int pairs = P.ntiles < sm_count() / 2 ? P.ntiles : sm_count() / 2;
-        if (const long long e = knob("RDFC_UMMA_GRID", KNOB_UNSET); e != KNOB_UNSET) pairs = (int)e / 2 < pairs ? ((int)e / 2 > 0 ? (int)e / 2 : 1) : pairs;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(2 * pairs); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        RDFC_CUDA(cudaLaunchKernelEx(&cfg, kern, P));
-    } else {
-        // measured with the two-lane graph: early launch of the next conv takes SMs the other lane's CTAs would have used, and the
-        // step does not get faster (10.61 / 10.63 ms with, 10.58 / 10.47 ms without), so it is off by default
-        static int pdl = -1;
-        if (pdl < 0) pdl = knob("RDFC_UMMA_PDL", 0) != 0;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = pdl;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        RDFC_CUDA(cudaLaunchKernelEx(&cfg, kern, P));
-    }
+                     : (P.act > RDFC_ACT_LEAKY02 || !P.vec32 || P.Cout % 16 != 0) ? MODE_GENERAL : MODE_STD;
+    // measured with the two-lane graph: early launch of the next conv takes SMs the other lane's CTAs would have used, and the
+    // step does not get faster (10.61 / 10.63 ms with, 10.58 / 10.47 ms without), so it is off by default
+    static int pdl = -1;
+    if (pdl < 0) pdl = knob("RDFC_UMMA_PDL", 0) != 0;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = pdl;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    RDFC_CUDA(cudaLaunchKernelEx(&cfg, kernels[mode], P));
     RDFC_CHECK_LAUNCH("conv_umma_kernel");
     return 0;
 }

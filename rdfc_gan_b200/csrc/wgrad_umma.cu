@@ -215,21 +215,6 @@ __global__ void __launch_bounds__(256) wgrad_umma_reduce_kernel(const float *__r
     }
 }
 
-typedef CUresult (*TmapEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
-                                 const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-TmapEncodeFn tmap_encoder() {
-    static TmapEncodeFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        cudaDriverEntryPointQueryResult q;
-        void *p = nullptr;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess) fn = (TmapEncodeFn)p;
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
-
 }  // namespace
 
 struct WuGeom { WuParams P; int nchunk; size_t smem; long long ws_floats; };

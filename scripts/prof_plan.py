@@ -62,8 +62,7 @@ def main():
         import numpy as np
         pats = sys.argv[sys.argv.index("--timers") + 1].split(",")
         names = {0: "MMA warp lifetime", 1: "MMA wait ACC_EMPTY", 2: "MMA wait A_FULL", 3: "MMA wait B_FULL", 5: "Bload wait B_EMPTY",
-                 6: "prod wait A_EMPTY", 7: "prod issue", 8: "prod wait_group", 9: "epi wait ACC_FULL", 10: "epi work",
-                 11: "MMA issue (elected)", 12: "MMA commits", 13: "CTA lifetime"}
+                 9: "epi wait ACC_FULL", 10: "epi work", 11: "MMA issue (elected)", 12: "MMA commits", 13: "CTA lifetime"}
         for f, n in zip(plan.steps, plan.names):
             if any(pat in n for pat in pats):
                 f(s)
@@ -71,8 +70,6 @@ def main():
                 buf = (ctypes.c_longlong * (148 * 16))()
                 C.lib.rdfc_dev_umma_timers(buf, 148 * 16)
                 a = np.frombuffer(buf, dtype=np.int64).reshape(148, 16).astype(np.float64)
-                if os.environ.get("RDFC_UMMA_PAIR") == "1":
-                    a = a[::2]                      # pair mode: the leader CTAs (even cluster ranks) issue the MMAs
                 a = a[a[:, 0] > 0]
                 print(f"role timers for step '{n}' (cycles, median over {len(a)} CTAs; CTA lifetime max {a[:, 13].max():.0f}, "
                       f"last CTA end - first CTA end {(a[:, 14].max() - a[:, 14].min()) / 1e3:.1f} us, "
