@@ -176,9 +176,12 @@ int rdfc_fuse_depth_forward(const float *d1, const float *c1, const float *d2, c
 /* ------------------------------------------------------------------ dense part (NHWC) ------------------------- */
 typedef enum { RDFC_ACT_NONE = 0, RDFC_ACT_RELU = 1, RDFC_ACT_LEAKY02 = 2, RDFC_ACT_TANH = 3, RDFC_ACT_SIGMOID = 4 }
     rdfc_act;
-/* RDFC_PATH_UMMA_F32X3: fp32 NHWC in / out on the bf16 tensor cores with split operands (x = x_hi + x_lo, W = W_hi + W_lo;
+/* RDFC_PATH_UMMA_F32X3: fp32 NHWC in / out on the 16-bit tensor cores with split fp16 operands (x = x_hi + x_lo, W = W_hi + W_lo;
  * x_hi W_hi + x_hi W_lo + x_lo W_hi accumulated in fp32): the <= 1e-4 parity mode at tensor-core speed.  `weight` is the UMMA
- * packing of [W_hi ; W_lo ; W_hi] along Cin (3 * Cin input channels); needs `workspace`. */
+ * packing of [W_hi ; W_lo ; W_hi] along Cin (3 * Cin input channels); needs `workspace`.  The input is scaled by the power of two
+ * s with max|x| * s in [1024, 2048) before it is split (as rdfc_split_scaled does; the factor stays on the device) and the kernel
+ * multiplies 1 / s into `scale`, so the split keeps 22 bits at any input magnitude.  A caller that scales the filter the same way
+ * folds its inverse into `scale` (rdfc_gan_b200.engine.pack_weight_x3 does, per output channel). */
 typedef enum { RDFC_PATH_SIMT_F32 = 0, RDFC_PATH_UMMA_BF16 = 1, RDFC_PATH_UMMA_F32X3 = 2 } rdfc_conv_path;
 
 /* A view of an NHWC tensor: element (b,y,x,c) lives at ptr[((b*H + y)*W + x)*pix_stride + c].
@@ -205,7 +208,8 @@ typedef struct {
     const void *weight;     /* packed by rdfc_gan_b200.engine: SIMT: fp32 [kh*kw][Cin][Cout]; UMMA: bf16 [kh*kw][Cin/8][Cout padded to 16][8] */
     const float *scale;     /* per-Cout multiplier (folded BN gamma/sqrt(var+eps)) or NULL (= 1) */
     const float *shift;     /* per-Cout addend (folded BN beta - mean*scale, or the conv bias) or NULL (= 0) */
-    void *workspace;        /* RDFC_PATH_UMMA_F32X3 only: B*Hi*Wi*Cin*4 bytes, 128-byte aligned (the split input) */
+    void *workspace;        /* RDFC_PATH_UMMA_F32X3 only: B*Hi*Wi*Cin*4 + 16 bytes, 128-byte aligned (the split input, then its
+                             * scale factor in a 16-byte tail) */
     size_t workspace_bytes;
 } rdfc_conv_desc;
 
@@ -226,8 +230,9 @@ typedef struct {
     int act[16];                 /* rdfc_act per column */
     float *out[16];              /* device plane base pointers */
     long long out_bstride[16];   /* elements between consecutive images of a plane */
-    void *workspace;             /* only when `in` is an fp32 view (tensor-core fp32 mode: weight packs [W_hi ; W_lo ; W_hi], fp16): */
-    size_t workspace_bytes;      /*   B*H*W*C*4 bytes, 128-byte aligned, receives the split input */
+    void *workspace;             /* only when `in` is an fp32 view (tensor-core fp32 mode: weight packs [W_hi ; W_lo ; W_hi], fp16, */
+    size_t workspace_bytes;      /*   unscaled): B*H*W*C*4 + 16 bytes, 128-byte aligned, receives the split input scaled as in
+                                  *   RDFC_PATH_UMMA_F32X3 and its factor (16-byte tail) */
 } rdfc_heads_desc;
 
 int rdfc_heads_forward(const rdfc_heads_desc *d, void *stream);

@@ -4,13 +4,33 @@
 namespace rdfc {
 int conv_simt_forward(const rdfc_conv_desc *d, cudaStream_t st);
 int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads_desc *heads, const rdfc_stem_desc *stem,
-                      const rdfc_wadain_conv_desc *wad, int split_c);
-int split_f32_forward(const rdfc_view *x, void *out_bf16, long long npix, cudaStream_t st);
+                      const rdfc_wadain_conv_desc *wad, int split_c, const float *split_factor = nullptr);
+int split_scaled_forward(const rdfc_view *x, void *out, int out_stride, long long npix, float *factor, cudaStream_t st);
 int wadain_tile(int C);
 int conv_umma_read_dbg(long long *host, int n);
 }  // namespace rdfc
 
 using namespace rdfc;
+
+// The fp32 input of RDFC_PATH_UMMA_F32X3 and of the fp32 heads: a 16-byte aligned NHWC view, and the caller's workspace of
+// npix*C*4 + 16 bytes, 128-byte aligned, that receives [hi | lo] of s * x (npix*C*4 bytes) followed by the factor s in a 16-byte tail.
+static int check_split_input(const rdfc_view *x, const void *workspace, size_t workspace_bytes, long long npix, const char *what) {
+    RDFC_REQUIRE(x->pix_stride % 4 == 0 && ((uintptr_t)x->ptr % 16) == 0,
+                 "%s: the fp32 input must be 16-byte aligned with a pixel stride that is a multiple of 4", what);
+    const size_t need = (size_t)npix * x->C * 4 + 16;
+    RDFC_REQUIRE(workspace && workspace_bytes >= need && ((uintptr_t)workspace % 128) == 0,
+                 "%s: workspace of %zu bytes (B*H*W*C*4 for the split input + 16 for its scale factor), 128-byte aligned, required", what,
+                 need);
+    return 0;
+}
+
+// split x into the workspace (see check_split_input) -> the bf16-typed [hi | lo] view the tcgen05 kernel reads, and the factor's address
+static int split_input(const rdfc_view *x, void *workspace, long long npix, cudaStream_t st, rdfc_view *split, float **factor) {
+    *factor = (float *)((char *)workspace + (size_t)npix * x->C * 4);
+    if (int rc = split_scaled_forward(x, workspace, 2 * x->C, npix, *factor, st)) return rc;
+    split->ptr = workspace; split->dtype = RDFC_BF16; split->C = 2 * x->C; split->pix_stride = 2 * x->C; split->nchw = 0;
+    return 0;
+}
 
 static int check_conv_geometry(const rdfc_conv_desc *d) {
     RDFC_REQUIRE(d != nullptr, "descriptor is NULL");
@@ -35,19 +55,19 @@ extern "C" int rdfc_conv_forward(const rdfc_conv_desc *d, void *stream) {
     if (d->path == RDFC_PATH_UMMA_BF16) return conv_umma_forward(d, st, nullptr, nullptr, nullptr, 0);
     if (d->path == RDFC_PATH_SIMT_F32) return conv_simt_forward(d, st);
     if (d->path == RDFC_PATH_UMMA_F32X3) {
-        // fp32-faithful contraction on the bf16 tensor cores: split the fp32 input into [hi | lo] bf16 halves (one HBM pass into the
-        // caller's workspace), then the tcgen05 kernel walks x_hi W_hi + x_hi W_lo + x_lo W_hi and writes fp32
+        // fp32-faithful contraction on the 16-bit tensor cores: scale the fp32 input by a power of two of its own and split it into
+        // [hi | lo] fp16 halves (an amax pass and one split pass into the caller's workspace), then the tcgen05 kernel walks
+        // x_hi W_hi + x_hi W_lo + x_lo W_hi, multiplies the exact inverse of the factor into the per-Cout scale and writes fp32
         RDFC_REQUIRE(d->in.dtype == RDFC_F32 && d->out.dtype == RDFC_F32 && !d->in.nchw && !d->out.nchw && !d->in2.ptr,
                      "conv (fp32 on tensor cores): single fp32 NHWC source and fp32 NHWC output");
         RDFC_REQUIRE(d->in.C % 32 == 0, "conv (fp32 on tensor cores): Cin (%d) must be a multiple of 32", d->in.C);
         const long long npix = (long long)d->B * d->Hi * d->Wi;
-        RDFC_REQUIRE(d->workspace && d->workspace_bytes >= (size_t)npix * d->in.C * 4 && ((uintptr_t)d->workspace % 128) == 0,
-                     "conv (fp32 on tensor cores): workspace of B*Hi*Wi*Cin*4 bytes (128-byte aligned) required");
-        if (int rc = split_f32_forward(&d->in, d->workspace, npix, st)) return rc;
+        if (int rc = check_split_input(&d->in, d->workspace, d->workspace_bytes, npix, "conv (fp32 on tensor cores)")) return rc;
         rdfc_conv_desc e = *d;
-        e.in.ptr = d->workspace; e.in.dtype = RDFC_BF16; e.in.C = 2 * d->in.C; e.in.pix_stride = 2 * d->in.C;
+        float *factor;
+        if (int rc = split_input(&d->in, d->workspace, npix, st, &e.in, &factor)) return rc;
         e.path = RDFC_PATH_UMMA_BF16;
-        return conv_umma_forward(&e, st, nullptr, nullptr, nullptr, d->in.C);
+        return conv_umma_forward(&e, st, nullptr, nullptr, nullptr, d->in.C, factor);
     }
     return fail(RDFC_ERR_INVALID, "conv: unknown path %d", d->path);
 }
@@ -80,17 +100,17 @@ extern "C" int rdfc_heads_forward(const rdfc_heads_desc *h, void *stream) {
     d.out.ptr = h->out[0]; d.out.dtype = RDFC_F32; d.out.C = (9 * h->ncols + 15) / 16 * 16; d.out.pix_stride = d.out.C;
     d.weight = h->weight; d.scale = nullptr; d.shift = h->shift;
     int split_c = 0;
+    float *factor = nullptr;
     if (h->in.dtype == RDFC_F32) {
-        // fp32 input (the tensor-core fp32 mode): split it into [hi | lo] fp16 halves first; the filter bank then holds 3 x C channels
+        // fp32 input (the tensor-core fp32 mode): scale and split it into [hi | lo] fp16 halves first (the filter bank then holds
+        // 3 x C channels); the shift-add multiplies each output's tap sum by the factor's exact inverse
         const long long npix = (long long)h->B * h->H * h->W;
         RDFC_REQUIRE(!h->in.nchw && h->in.C % 32 == 0, "heads (fp32 input): NHWC view with C %% 32 == 0");
-        RDFC_REQUIRE(h->workspace && h->workspace_bytes >= (size_t)npix * h->in.C * 4 && ((uintptr_t)h->workspace % 128) == 0,
-                     "heads (fp32 input): workspace of B*H*W*C*4 bytes (128-byte aligned) required");
-        if (int rc = split_f32_forward(&h->in, h->workspace, npix, (cudaStream_t)stream)) return rc;
+        if (int rc = check_split_input(&h->in, h->workspace, h->workspace_bytes, npix, "heads (fp32 input)")) return rc;
         split_c = h->in.C;
-        d.in.ptr = h->workspace; d.in.dtype = RDFC_BF16; d.in.C = 2 * split_c; d.in.pix_stride = 2 * split_c;
+        if (int rc = split_input(&h->in, h->workspace, npix, (cudaStream_t)stream, &d.in, &factor)) return rc;
     }
-    return conv_umma_forward(&d, (cudaStream_t)stream, h, nullptr, nullptr, split_c);
+    return conv_umma_forward(&d, (cudaStream_t)stream, h, nullptr, nullptr, split_c, factor);
 }
 
 extern "C" int rdfc_stem_forward(const rdfc_stem_desc *m, void *stream) {

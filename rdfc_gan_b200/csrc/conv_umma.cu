@@ -135,6 +135,10 @@ struct Params {
     int gtaps;                     // filter taps per B stage (3 for 3x3 convs: one wait / commit per filter row)
     int vec32;                     // output (and residual) slices are 32-byte aligned: 256-bit stores / loads
     int b_contig;                  // the 4 cin chunks of a stage are contiguous in the packed weights (one Cout tile)
+    // split_factor (with split_c): the device factor s of an input scaled by a power of two before its split (rdfc_conv_forward /
+    // rdfc_heads_forward on fp32 data), else NULL.  Its exact inverse is folded into s_scale when staged (convs) or applied to each
+    // tap sum (heads).
+    const float *split_factor;
 };
 
 struct Tile {
@@ -399,7 +403,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
         s_tap[threadIdx.x] = make_uint2(P.tap_alo[threadIdx.x / MAX_TAPS][threadIdx.x % MAX_TAPS],
                                         P.tap_ahi[threadIdx.x / MAX_TAPS][threadIdx.x % MAX_TAPS]);
     for (int i = threadIdx.x; i < P.CoutP; i += NTHREADS) {
-        s_scale[i] = (P.scale && i < P.Cout) ? P.scale[i] : 1.f;
+        // times the exact inverse of a scaled split's factor (a power of two)
+        s_scale[i] = ((P.scale && i < P.Cout) ? P.scale[i] : 1.f) * (P.split_factor ? __frcp_rn(__ldg(P.split_factor)) : 1.f);
         s_shift[i] = (P.shift && i < P.Cout) ? P.shift[i] : 0.f;
     }
 
@@ -875,14 +880,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_umma_kernel(const __grid_con
                 __syncwarp();
                 if (lane == 0) mbar_arrive(BAR(ACC_EMPTY + set));
                 asm volatile("bar.sync 2, %0;" ::"n"(NEPI_WARPS * 32) : "memory");
+                // a scaled split input (factor s): the taps are s times the output's, so the bias enters as bias * s and the sum
+                // is multiplied by 1 / s.  Both are exact: this is bias + taps / s rounded step by step.  Without a split both are 1.
+                const float fac = P.split_factor ? __ldg(P.split_factor) : 1.f, inv = __frcp_rn(fac);
                 for (int item = threadIdx.x - EPI_WARP0 * 32; item < 196 * ncols; item += NEPI_WARPS * 32) {
                     const int q = item / 196, pi = item - q * 196, iy = pi / 14, ix = pi - iy * 14;
                     const int oy = t.ty0 + 1 + iy, ox = t.tx0 + 1 + ix;
                     if (oy >= Ho || ox >= Wo) continue;
                     const float *yq = Ys + (iy * 16 + ix) * pitch + q;
-                    float acc = s_shift[q];
+                    float acc = s_shift[q] * fac;
 #pragma unroll
                     for (int t9 = 0; t9 < 9; ++t9) acc += yq[((t9 / 3) * 16 + (t9 % 3)) * pitch + t9 * ncols];
+                    acc *= inv;
                     const int a = P.act_col[q];
                     if (a == RDFC_ACT_TANH) acc = tanhf(acc);
                     else if (a == RDFC_ACT_SIGMOID) acc = 1.f / (1.f + expf(-acc));
@@ -1132,9 +1141,9 @@ int next_pow2_cols(int c) {
 int wadain_tile(int C) { return (2 * C) % 256 == 0 ? 256 : 128; }
 
 // split_c != 0: `d->in` is a split bf16 tensor [hi(split_c) | lo(split_c)] (see Params::split_c) and the filter bank holds
-// 3 * split_c input channels; the output (and residual) may then be fp32 NHWC.
+// 3 * split_c input channels; the output (and residual) may then be fp32 NHWC.  split_factor: see Params::split_factor.
 int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads_desc *heads, const rdfc_stem_desc *stem,
-                      const rdfc_wadain_conv_desc *wad, int split_c) {
+                      const rdfc_wadain_conv_desc *wad, int split_c, const float *split_factor) {
     RDFC_REQUIRE((stem || d->in.dtype == RDFC_BF16) && (heads || d->out.dtype == RDFC_BF16 || (split_c && d->out.dtype == RDFC_F32)),
                  "UMMA conv: bf16 in/out only");
     RDFC_REQUIRE(!d->in.nchw && !d->out.nchw && !d->in2.ptr, "UMMA conv: single NHWC source / NHWC output only");
@@ -1162,6 +1171,7 @@ int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads
     P.Cout = d->out.C; P.CoutP = (P.Cout + 15) / 16 * 16;
     P.cin_chunks = d->in.C / 8; P.nkb = d->in.C / BK;
     if (split_c) { P.split_c = split_c; P.cin_chunks = 3 * split_c / 8; P.nkb = 3 * split_c / BK; P.out_f32 = d->out.dtype == RDFC_F32; }
+    P.split_factor = split_factor;
     P.out = (__nv_bfloat16 *)d->out.ptr; P.out_stride = d->out.pix_stride; P.Ho = d->Ho; P.Wo = d->Wo;
     P.res = (const __nv_bfloat16 *)d->residual.ptr; P.res_stride = d->residual.pix_stride;
     P.scale = d->scale; P.shift = d->shift; P.act = d->act;

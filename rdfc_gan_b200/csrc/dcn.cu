@@ -12,7 +12,7 @@
 
 namespace rdfc {
 int conv_umma_forward(const rdfc_conv_desc *d, cudaStream_t st, const rdfc_heads_desc *heads, const rdfc_stem_desc *stem,
-                      const rdfc_wadain_conv_desc *wad, int split_c);
+                      const rdfc_wadain_conv_desc *wad, int split_c, const float *split_factor = nullptr);
 long long wgrad_umma_workspace_floats(const rdfc_wgrad_desc *d);
 int wgrad_umma_partials(const rdfc_wgrad_desc *d, float *workspace, int fp16, cudaStream_t st, int *nchunk);
 namespace {

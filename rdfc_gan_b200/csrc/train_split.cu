@@ -5,8 +5,8 @@
 //   rdfc_conv_wgrad_split   the filter gradient of wgrad_umma.cu on fp16 halves, run for the three products g_hi.x_hi, g_hi.x_lo,
 //                           g_lo.x_hi into consecutive chunk ranges of one workspace, then ONE reduction in a fixed order that also
 //                           applies 1 / (s_g s_x)  (bit-reproducible)
-// (the conv forward / data gradient on an already split input is rdfc_conv_forward_split, conv.cu.)  The split kernel also serves,
-// unscaled, the fp32 inputs of the inference path's RDFC_PATH_UMMA_F32X3 convs and fp32 heads (split_f32_forward).
+// (the conv forward / data gradient on an already split input is rdfc_conv_forward_split, conv.cu.)  The same scaled split serves
+// the fp32 inputs of the inference path's RDFC_PATH_UMMA_F32X3 convs and fp32 heads (split_scaled_forward, conv.cu).
 //
 // Why the scaling: fp16 keeps 11 significant bits down to 6.1e-5 only, and the training step's gradients start near 1e-5 (the
 // reference's image_loss_weight = mask / mask.sum()).  Scaled so that the largest magnitude lies in [1024, 2048), the low half keeps
@@ -37,13 +37,11 @@ __global__ void __launch_bounds__(256) split_amax_kernel(const float *__restrict
     if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(am, __float_as_uint(m));
 }
 
-// fp32 NHWC view -> fp16 [pixel][hi(C) | lo(C)] of s * x, hi = fp16(s x), lo = fp16(s x - hi).  8 channels per thread.
-// kScaled: s = pow2_scale(max |x|), read from `am`; otherwise s = 1 -- no load of `am`, no multiply (the inference path's split).
-template <bool kScaled>
+// fp32 NHWC view -> fp16 [pixel][hi(C) | lo(C)] of s * x, hi = fp16(s x), lo = fp16(s x - hi), s = pow2_scale(max |x|) read from
+// `am`.  8 channels per thread.
 __global__ void __launch_bounds__(256) split_kernel(const float *__restrict__ x, int C, int stride, __half *__restrict__ out, int out_stride,
                                                     long long npix, const unsigned *__restrict__ am) {
-    float s = 1.f;
-    if (kScaled) s = pow2_scale(__uint_as_float(__ldg(am)));
+    const float s = pow2_scale(__uint_as_float(__ldg(am)));
     const int cgs = C >> 3;
     const long long total = npix * cgs;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -51,9 +49,8 @@ __global__ void __launch_bounds__(256) split_kernel(const float *__restrict__ x,
         const int c0 = (int)(i - p * cgs) * 8;
         const float4 a = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0)), b = __ldg(reinterpret_cast<const float4 *>(x + p * stride + c0) + 1);
         float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-        if (kScaled)
 #pragma unroll
-            for (int q = 0; q < 8; ++q) v[q] *= s;
+        for (int q = 0; q < 8; ++q) v[q] *= s;
         uint32_t hi[4], lo[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
@@ -100,21 +97,21 @@ static int check_split_view(const rdfc_view *v, const char *what) {
     return 0;
 }
 
-template <bool kScaled>
-static int split_launch(const rdfc_view *x, __half *out, int out_stride, long long npix, const unsigned *am, cudaStream_t st) {
-    const int nblk = (int)min((long long)cdiv(npix * (x->C / 8), 256), (long long)sm_count() * 16);
-    split_kernel<kScaled><<<nblk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, out, out_stride, npix, am);
-    RDFC_CHECK_LAUNCH("split_kernel");
-    return 0;
-}
-
 namespace rdfc {
-// the unscaled split into a dense [hi | lo] workspace: the fp32 input of the RDFC_PATH_UMMA_F32X3 conv and of the fp32 heads (conv.cu)
-int split_f32_forward(const rdfc_view *x, void *out, long long npix, cudaStream_t st) {
-    RDFC_REQUIRE(x && x->ptr && out && x->dtype == RDFC_F32 && !x->nchw && x->C % 8 == 0 && x->pix_stride % 4 == 0 &&
-                     ((uintptr_t)x->ptr % 16) == 0,
-                 "split: 16-byte aligned fp32 NHWC view with C % 8 == 0 expected");
-    return split_launch<false>(x, (__half *)out, 2 * x->C, npix, nullptr, st);
+// amax -> scaled split -> factor, stream-ordered on the device (graph-capturable, no host synchronisation): out[p] = [hi | lo] of s * x
+// (out_stride halves per pixel), *factor = s.  The caller has validated x (fp32 NHWC, C % 8 == 0, 16-byte aligned, pixel stride % 4
+// == 0), out and factor.
+int split_scaled_forward(const rdfc_view *x, void *out, int out_stride, long long npix, float *factor, cudaStream_t st) {
+    RDFC_CUDA(cudaMemsetAsync(factor, 0, sizeof(float), st));
+    const int ablk = (int)min((long long)cdiv(npix * (x->C / 4), 256 * 8), (long long)sm_count() * 4);
+    split_amax_kernel<<<ablk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, npix, (unsigned *)factor);
+    RDFC_CHECK_LAUNCH("split_amax_kernel");
+    const int nblk = (int)min((long long)cdiv(npix * (x->C / 8), 256), (long long)sm_count() * 16);
+    split_kernel<<<nblk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, (__half *)out, out_stride, npix, (const unsigned *)factor);
+    RDFC_CHECK_LAUNCH("split_kernel");
+    split_factor_kernel<<<1, 1, 0, st>>>(factor);
+    RDFC_CHECK_LAUNCH("split_factor_kernel");
+    return 0;
 }
 }  // namespace rdfc
 
@@ -126,15 +123,7 @@ extern "C" int rdfc_split_scaled(const rdfc_view *x, long long npix, const rdfc_
     if (int rc = check_split_view(out, "split destination")) return rc;
     RDFC_REQUIRE(out->C == 2 * x->C, "split: destination has %d channels, 2 x %d expected", out->C, x->C);
     RDFC_REQUIRE(((uintptr_t)factor % 4) == 0, "split: factor must be 4-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    RDFC_CUDA(cudaMemsetAsync(factor, 0, sizeof(float), st));
-    const int ablk = (int)min((long long)cdiv(npix * (x->C / 4), 256 * 8), (long long)sm_count() * 4);
-    split_amax_kernel<<<ablk, 256, 0, st>>>((const float *)x->ptr, x->C, x->pix_stride, npix, (unsigned *)factor);
-    RDFC_CHECK_LAUNCH("split_amax_kernel");
-    if (int rc = split_launch<true>(x, (__half *)out->ptr, out->pix_stride, npix, (const unsigned *)factor, st)) return rc;
-    split_factor_kernel<<<1, 1, 0, st>>>(factor);
-    RDFC_CHECK_LAUNCH("split_factor_kernel");
-    return 0;
+    return split_scaled_forward(x, out->ptr, out->pix_stride, npix, factor, (cudaStream_t)stream);
 }
 
 // the per-product descriptor: `part` 0 = (g_hi, x_hi), 1 = (g_hi, x_lo), 2 = (g_lo, x_hi); 16-bit views of C channels

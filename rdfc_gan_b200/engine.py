@@ -45,6 +45,17 @@ def pack_weight(w, umma, x3=False):
     return g.reshape(CoutP, kh * kw, Cin // 8, 8).permute(1, 2, 0, 3).contiguous().to(torch.float16 if x3 else torch.bfloat16)
 
 
+def pack_weight_x3(w, scale):
+    """The RDFC_PATH_UMMA_F32X3 filters of the inference engines: (Cout, Cin, kh, kw) fp32 filters and their per-Cout epilogue
+    multiplier `scale` (Cout,) -> (pack_weight(w * s, x3), scale / s), s per output channel the power of two with
+    max|w_c| * s_c in [1024, 2048) (1 for an all-zero filter), the rule rdfc_split_scaled applies to activations.  Unscaled, the low
+    half of a filter of N(0, 1/K) is already in fp16's subnormal range; scaled, it keeps 11 bits.  Dividing by s is exact."""
+    amax = w.abs().amax(dim=(1, 2, 3))
+    _, e = torch.frexp(amax)
+    s = torch.where((amax > 0) & torch.isfinite(amax), torch.exp2((11 - e).clamp(-100, 100).float()), torch.ones_like(amax))
+    return pack_weight(w * s[:, None, None, None], True, True), (scale / s).contiguous()
+
+
 class _Packed:
     """Persistent device storage for one (possibly fused) conv layer's packed filters and epilogue vectors."""
 
@@ -133,7 +144,9 @@ class GeneratorEngine:
         # 'fp32_tc' fp32 tensors, GEMM-shaped convs (Cin % 32 == 0, Cout >= 16) and the decode heads on the 16-bit tensor cores with
         #           split operands (RDFC_PATH_UMMA_F32X3: x_hi W_hi + x_hi W_lo + x_lo W_hi, fp16 halves, fp32 accumulation):
         #           <= 1e-5 on the bench recipe, <= 2e-4 on the O(1)-activation stress goldens (the tensor cores' fp32 accumulation
-        #           is not IEEE round-to-nearest), ~6-10x faster than 'fp32'
+        #           is not IEEE round-to-nearest), ~6-10x faster than 'fp32'.  Every split input is scaled by a power of two of its own
+        #           (on the device) and every conv filter per output channel (pack_weight_x3), so fp16's range [6.1e-5, 65504] limits
+        #           no activation magnitude; the heads' filters stay unscaled (their low half resolves 2^-25 absolute)
         # 'bf16'    the throughput mode
         self.precision = 'fp32'
         self.use_cuda_graph = True
@@ -141,7 +154,7 @@ class GeneratorEngine:
         self._plans = {}         # (B, H, W, Cs, device, precision) -> Plan, in LRU order
         self._packed = {}        # (precision, layer name) -> _Packed
         self._wver = {}          # precision -> parameter version stamp
-        self._recipes = {}       # (precision, layer name) -> (sources, umma, transposed) for in-place re-packing
+        self._recipes = {}       # (precision, layer name) -> (sources, umma, transposed, x3, heads) for in-place re-packing
         self._device = None      # packed weights and plans live on ONE device; moving the module drops them
 
     def clear_plans(self, precision=None):
@@ -162,10 +175,11 @@ class GeneratorEngine:
         scale = bn.weight.detach().float() / torch.sqrt(bn.running_var.detach().float() + bn.eps)
         return scale, bn.bias.detach().float() - bn.running_mean.detach().float() * scale
 
-    def _pack(self, name, sources, precision, umma, transposed=False, x3=False):
+    def _pack(self, name, sources, precision, umma, transposed=False, x3=False, heads=False):
         """sources: list of (weight (Cout,Cin,kh,kw) or ConvT (Cin,Cout,kh,kw), bn module or None, bias or None),
-        fused along Cout."""
-        self._recipes[(precision, name)] = (sources, umma, transposed, x3)
+        fused along Cout.  x3: the RDFC_PATH_UMMA_F32X3 packing, per-Cout scaled (pack_weight_x3) for a conv, unscaled for the
+        fused heads (heads=True: rdfc_heads_forward has no per-column multiplier)."""
+        self._recipes[(precision, name)] = (sources, umma, transposed, x3, heads)
         ws, scs, shs = [], [], []
         for w, bn, bias in sources:
             w = (w() if callable(w) else w).detach().float()
@@ -180,9 +194,13 @@ class GeneratorEngine:
                 sh = bias.detach().float() if bias is not None else torch.zeros(w.shape[0], device=w.device)
             scs.append(sc)
             shs.append(sh)
-        packed = pack_weight(torch.cat(ws, 0), umma, x3)
+        w, scale = torch.cat(ws, 0), torch.cat(scs).contiguous()
+        if x3 and not heads:
+            packed, scale = pack_weight_x3(w, scale)
+        else:
+            packed = pack_weight(w, umma, x3)
         p = self._packed.setdefault((precision, name), _Packed())
-        p.store(packed, torch.cat(scs).contiguous(), torch.cat(shs).contiguous())
+        p.store(packed, scale, torch.cat(shs).contiguous())
         return p
 
     def _pack_nlspn(self, precision):
@@ -194,9 +212,9 @@ class GeneratorEngine:
 
     def _repack(self, precision):
         """Refresh every packed tensor of this precision in place (pointers, plans and CUDA graphs stay valid)."""
-        for (prec, name), (sources, umma, transposed, x3) in list(self._recipes.items()):
+        for (prec, name), (sources, umma, transposed, x3, heads) in list(self._recipes.items()):
             if prec == precision:
-                self._pack(name, sources, precision, umma, transposed, x3)
+                self._pack(name, sources, precision, umma, transposed, x3, heads)
         if (precision, 'nlspn') in self._packed:
             self._pack_nlspn(precision)
 
@@ -255,22 +273,23 @@ class GeneratorEngine:
             d.stride, d.pad, d.transposed, d.act = stride, pad, int(transposed), act
             d.path = C.PATH_UMMA_BF16 if umma else (C.PATH_UMMA_F32X3 if x3 else C.PATH_SIMT_F32)
             d.inp, d.in2, d.out, d.residual = vin, vin2, vout, vres
-            if x3:       # the split [hi | lo] copy of the input: one scratch buffer per lane (the two lanes run concurrently)
+            if x3:       # the split [hi | lo] copy of the input and its factor: one scratch buffer per lane (the two lanes run concurrently)
                 ws = x3_scratch[plan.cur_lane]
-                assert ws.numel() >= B * hin[0] * hin[1] * cin * 4, (name, cin, hin)
+                assert ws.numel() >= B * hin[0] * hin[1] * cin * 4 + 16, (name, cin, hin)
                 d.workspace, d.workspace_bytes = ws.data_ptr(), ws.numel()
             d.weight, d.scale, d.shift = pk.weight.data_ptr(), pk.scale.data_ptr(), pk.shift.data_ptr()
             plan.keep.append((d, pk))
             plan.names.append(f"conv {name} k{k} s{stride} T{int(transposed)} {vin.C}->{vout.C} {hin}->{hout} {'umma' if umma else ('umma_x3' if x3 else 'simt')}")
-            if x3:
-                plan.n_launch += 1
+            if x3:       # the split: amax, split and factor kernels
+                plan.n_launch += 3
             plan.steps.append(lambda s, d=d: C.check(C.lib.rdfc_conv_forward(ctypes.byref(d), s)))
             plan.n_launch += 1
 
         x3_scratch = None
         if tc32:
-            # largest split input: the 224-channel full-resolution head buffer (4 bytes per element, like the fp32 tensor itself)
-            x3_scratch = [new(B * H * W * 224 * 4, dtype=torch.uint8) for _ in range(2)]
+            # largest split input: the 224-channel full-resolution head buffer (4 bytes per element, like the fp32 tensor itself),
+            # + 16 bytes for the split's scale factor
+            x3_scratch = [new(B * H * W * 224 * 4 + 16, dtype=torch.uint8) for _ in range(2)]
 
         def seq_src(mod):           # conv_bn_relu / convt_bn_relu Sequential -> (weight, bn, bias)
             bn = mod[1] if len(mod) > 1 and isinstance(mod[1], torch.nn.BatchNorm2d) else None
@@ -512,15 +531,15 @@ class GeneratorEngine:
             return torch.cat([c['mod'].bias.detach().float() for c in cols] + [torch.zeros(NP - nc, device=buf.device)])
 
         tc32 = precision == 'fp32_tc'
-        pk = self._pack(name, [(fused_weight, None, fused_bias)], precision, True, x3=tc32)
+        pk = self._pack(name, [(fused_weight, None, fused_bias)], precision, True, x3=tc32, heads=True)
         d = C.HeadsDesc()
         d.B, d.H, d.W = B, H, W
         d.inp = C.view(buf)
-        if tc32:         # fp32 head buffer: split into fp16 halves inside the call (this lane's scratch)
+        if tc32:         # fp32 head buffer: scaled and split into fp16 halves inside the call (this lane's scratch; amax, split, factor)
             ws = x3_scratch[plan.cur_lane]
-            assert ws.numel() >= B * H * W * Ctot * 4
+            assert ws.numel() >= B * H * W * Ctot * 4 + 16
             d.workspace, d.workspace_bytes = ws.data_ptr(), ws.numel()
-            plan.n_launch += 1
+            plan.n_launch += 3
         d.weight, d.shift = pk.weight.data_ptr(), pk.shift.data_ptr()
         q = 0
         for c in cols:

@@ -16,7 +16,9 @@ C-ABI calls, captured in a CUDA graph), NHWC activations:
 ``set_precision`` selects the arithmetic, with the meanings of the generator's modes (engine.GeneratorEngine):
   'bf16'    (default) bf16 activations, the convs on the tcgen05 tensor cores (RDFC_PATH_UMMA_BF16): the throughput mode;
   'fp32'    fp32 activations, every conv on the CUDA cores in fp32 (RDFC_PATH_SIMT_F32): the parity mode;
-  'fp32_tc' fp32 activations, the convs on the tensor cores with split fp16 operands (RDFC_PATH_UMMA_F32X3).
+  'fp32_tc' fp32 activations, the convs on the tensor cores with split fp16 operands (RDFC_PATH_UMMA_F32X3): each conv's input
+            scaled by a power of two of its own before the split (on the device), each filter per output channel
+            (engine.pack_weight_x3), so the split keeps fp32's magnitude range.
 
 Covered configuration = the one the reference's scripts use (F/bash/test_nyuv2_Ts2T.sh:7-16): ResNet-18 / 34 BasicBlock encoder,
 ``weighting_in_encoder='SE-add'``, ``context_module='ppm'``, ``encoder_decoder_fusion='add'``,
@@ -29,7 +31,7 @@ import torch
 import torch.nn as nn
 
 from . import _cabi as C
-from .engine import pack_weight
+from .engine import pack_weight, pack_weight_x3
 
 _BLOCKS = {'resnet18': (2, 2, 2, 2), 'resnet34': (3, 4, 6, 3)}
 _PRECISIONS = ('bf16', 'fp32', 'fp32_tc')
@@ -261,7 +263,6 @@ def _build_plan(net, B, H, W, dev, precision='bf16'):
         # fp32_tc: the split-operand tensor-core path where its shape rules allow (all ESANet convs), else CUDA-core fp32
         x3 = precision == 'fp32_tc' and cin % 32 == 0 and out[2] >= 16
         umma = precision == 'bf16' or x3
-        packed = pack_weight(w, umma, x3)
         if bn is not None:
             scale, shift = _fold(bn)
             if conv_mod.bias is not None:            # conv bias in front of a BatchNorm (NonBottleneck1D): bn(conv + b) = scale conv + (scale b + shift)
@@ -269,6 +270,10 @@ def _build_plan(net, B, H, W, dev, precision='bf16'):
         else:
             scale = torch.ones(w.shape[0], device=dev)
             shift = conv_mod.bias.detach().float() if conv_mod.bias is not None else torch.zeros(w.shape[0], device=dev)
+        if x3:       # filters scaled per output channel by a power of two, its inverse folded into `scale`
+            packed, scale = pack_weight_x3(w, scale)
+        else:
+            packed = pack_weight(w, umma)
         scale, shift = scale.contiguous(), shift.contiguous()
         Hi, Wi = hin
         Ho, Wo = (Hi - 1) // stride + 1, (Wi - 1) // stride + 1
@@ -278,7 +283,7 @@ def _build_plan(net, B, H, W, dev, precision='bf16'):
         d.stride, d.pad, d.transposed, d.act = stride, (k - 1) // 2, 0, act
         d.path = C.PATH_UMMA_F32X3 if x3 else (C.PATH_UMMA_BF16 if umma else C.PATH_SIMT_F32)
         if x3:
-            x3_descs.append((d, B * Hi * Wi * cin * 4))
+            x3_descs.append((d, B * Hi * Wi * cin * 4 + 16))         # the split input and its scale factor
         d.inp, d.in2 = C.view(x[0], x[2], x[1]), C.view(None)
         d.out = C.view(out[0], out[2], out[1])
         d.residual = C.view(None) if residual is None else C.view(residual[0], residual[2], residual[1])

@@ -21,6 +21,10 @@ ESANET_BOUND = {"fp32": (5e-6, 5e-5), "fp32_tc": (3.5e-4, 3e-3)}
 # decoder carries activations up to 8e6, and the fp32 CPU oracle itself lands 0.076 from an fp64 run of it on depth_map_1, so no fp32
 # implementation meets 1e-4 there.  The guidance network's own share is within ESANET_BOUND (DESIGN.md section 7, rank 2).
 RDFGAN_FP32_BOUND = {"depth_map_1": 0.7, "confidence_map_1": 0.19, "depth_map_2": 0.046, "confidence_map_2": 6e-5, "pred_depth": 0.35}
+# RDF-GAN in fp32_tc (guidance network and generator) against the same pipeline in strict fp32 on that input, RMSE per map: twice
+# the distance measured on a B200.  RMSE, not max-abs: on this ill-conditioned input single pixels of the tanh / clamped maps differ
+# by up to 1.96 (fp32_tc's contractions are ~1e-5 relative where fp32's are ~1e-7), so a max-abs bound would not constrain them.
+RDFGAN_FP32_TC_BOUND = {"depth_map_1": 0.034, "confidence_map_1": 0.006, "depth_map_2": 0.091, "confidence_map_2": 1.6e-4, "pred_depth": 0.057}
 KEYS = ("depth_map_1", "confidence_map_1", "depth_map_2", "confidence_map_2", "pred_depth")
 NL = dict(prop_kernel=3, prop_time=18, affinity="TGASS", affinity_gamma=0.5, conf_prop=True, preserve_input=False)
 
@@ -302,12 +306,21 @@ def test_rdfgan_fp32_end_to_end():
     assert all(torch.equal(outs[k], b) for k, b in zip(KEYS, ref2))
 
 
-@pytest.mark.xfail(strict=True, reason="the generator's fp32_tc path splits activations into fp16 halves; this input drives the RGB "
-                                       "decoder to 8e6, beyond fp16's 65504, and the maps come out NaN (DESIGN.md section 7, rank 2)")
 def test_rdfgan_fp32_tc_end_to_end():
-    _, _, _, _, errs, (g_rmse, g_max), _ = _rdfgan_errors("fp32_tc")
+    """RDF-GAN in fp32_tc end to end on the input that drives the RGB decoder to activations of 8e6, beyond fp16's 65504 (every split
+    input is scaled by a power of two of its own first): finite maps, the guidance within ESANET_BOUND of the oracle, and every map
+    within RDFGAN_FP32_TC_BOUND (RMSE) of the same pipeline in strict fp32"""
+    G, _, _, (rgb_d, depth_d), errs, (g_rmse, g_max), outs = _rdfgan_errors("fp32_tc")
     assert g_rmse <= ESANET_BOUND["fp32_tc"][0] and g_max <= ESANET_BOUND["fp32_tc"][1], (g_rmse, g_max)
-    assert all(np.isfinite(e) for e in errs.values()), errs
+    outs = {k: v.clone() for k, v in outs.items()}
+    assert all(bool(torch.isfinite(outs[k]).all()) for k in KEYS), errs
+    G.set_precision("fp32")
+    G.global_guidance_module.set_precision("fp32")
+    with torch.no_grad():
+        ref = dict(zip(KEYS, G(rgb_d, depth_d)))
+    dist = {k: float((outs[k] - ref[k]).double().square().mean().sqrt()) for k in KEYS}
+    _dump("rdfgan_fp32_tc:c2_228x304_vs_fp32", {"rmse": dist, "max_abs": {k: float((outs[k] - ref[k]).abs().max()) for k in KEYS}})
+    assert all(dist[k] <= RDFGAN_FP32_TC_BOUND[k] for k in KEYS), dist
 
 
 def test_stream_with_fp32_guidance():
